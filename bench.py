@@ -2,6 +2,7 @@
 """bench.py -- GLL hot-path benchmark (BASELINE.json metric: GLL fwd+bwd calls/s, CG iterations/s vs HBM roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5|c5s] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one call of the hot path on one synthetic graph:
     pred = LaplaceLearningSparseHard.apply(X, Y, tau, eps); loss = custom_ce_loss(pred, y); loss.backward()
@@ -25,6 +26,8 @@ cpu_baseline : the fp64 numpy/scipy oracle (a port of the reference's GLL.py, se
          box's host cores, rank 0 at N=1 only, bounded sample; plus the reference's own stable_conjgrad semantics
          (GLL.py:247-276, alias included) timed on the C4 system: cpu_baseline.cg_iters_per_sec.
 --impl reference : only the oracle port, all host threads, same JSON line with "impl": "reference".
+--dump-outputs DIR : pred, loss and dX of the last step of the pass `value` is timed on, as DIR/<name>.npy (rank 0;
+         a tensor over 30 MB as a seeded sample of its rows).
 """
 import argparse
 import json
@@ -248,6 +251,28 @@ def algorithmic_work(name, shp, info):
     return "hbm", None, "B"
 
 
+DUMP_BYTES_PER_ARRAY = 30_000_000  # pred and dX: a dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes each tensor as out_dir/<name>.npy (float32 / float64, as computed), so that two builds can be
+    compared output for output.  A tensor above DUMP_BYTES_PER_ARRAY is cut to a sample of its rows drawn with a fixed
+    seed (sorted; the same rows in every run of the same workload)."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dtype not in (torch.float32, torch.float64):
+            raise TypeError(f"bench.py: output {name} is {t.dtype}, not float32/float64")
+        if t.numel() * t.element_size() > DUMP_BYTES_PER_ARRAY:
+            keep = DUMP_BYTES_PER_ARRAY // (t[0].numel() * t.element_size())
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], size=keep, replace=False))
+            print(f"bench.py: {name} dumped as a seeded sample of {keep} of its {t.shape[0]} rows", file=sys.stderr)
+            t = t[torch.as_tensor(rows, device=t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_b200(args, rank, world, local_rank):
     import torch
 
@@ -294,7 +319,9 @@ def run_b200(args, rank, world, local_rank):
         Xe = torch.empty_like(Xd).requires_grad_(True)
         Ye = torch.empty_like(Yd)
 
-        split = {"ev": None}  # set to a list to have resident() record (start, after forward+loss, end) events
+        # "ev": set to a list to have resident() record (start, after forward+loss, end) events;
+        # "out": (pred, loss, dX) of the latest resident() call, what a caller of the layer receives
+        split = {"ev": None, "out": None}
 
         def resident():
             Xd.grad = None
@@ -310,6 +337,7 @@ def run_b200(args, rank, world, local_rank):
             if ev is not None:
                 ev[2].record()
                 split["ev"].append(ev)
+            split["out"] = (pred.detach(), loss.detach(), Xd.grad)  # detached: the layer's state is freed with its graph
             return loss
 
         def e2e():
@@ -401,6 +429,7 @@ def run_b200(args, rank, world, local_rank):
     # the same step replayed from CUDA graphs (graphlearninglayer_b200.graphed: forward + loss and backward captured once,
     # two graph launches per step, the same kernels): this is `value`; the eager figure is kept beside it
     tot_ms, execution = eager_ms, "eager launches through LaplaceLearningSparseHard.apply"
+    outputs = split["out"]  # (pred, loss, dX) of the last step of the path `value` is timed on
     extra_cfg = {}
     if not sharded and not args.no_cuda_graph and args.loss == "fused":
         try:
@@ -409,8 +438,15 @@ def run_b200(args, rank, world, local_rank):
             tn = split["tensors"]
             gs = GraphedStep(shp["n"], shp["d"], shp["k_lab"], shp["l"], dev, tau=tn["tau"], epsilon=tn["eps"],
                              warmup_inputs=(tn["Xd"].detach(), tn["Yd"], tn["yq"]))
-            tot_ms = timed(lambda: gs(tn["Xd"], tn["Yd"], tn["yq"]), args.steps, args.warmup)
+            replayed = {}
+
+            def replay():
+                loss = gs(tn["Xd"], tn["Yd"], tn["yq"])
+                replayed["out"] = (gs.pred, loss, gs.dX)  # static tensors of gs, untouched by the other passes
+
+            tot_ms = timed(replay, args.steps, args.warmup)
             execution = "CUDA graph replay (GraphedStep: 2 graph launches per step, same kernels)"
+            outputs = replayed["out"]
         except Exception as e:  # capture not available: say so, keep the eager number
             execution += f" (graph capture failed: {type(e).__name__}: {e})"[:300]
         try:  # extra, NOT the headline: the same step with the loss fused behind the layer in one autograd node (8f-3)
@@ -421,6 +457,8 @@ def run_b200(args, rank, world, local_rank):
         except Exception as e:
             print(f"bench.py: loss-head variant not measured: {type(e).__name__}: {e}", file=sys.stderr)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("pred", "loss", "dX"), outputs)))
     e2e_ms = timed(e2e, args.steps, args.warmup)
     pipe_ms = None
     if not sharded:
@@ -705,7 +743,12 @@ def main():
     ap.add_argument("--no-sharded", action="store_true", help="skip the sharded c5 / c5s lines")
     ap.add_argument("--no-c5", action="store_true", help="skip the 1M-node graph (keeps the c5s parity lines at N > 1)")
     ap.add_argument("--cpu-cg", action="store_true", help="reference arm: also time the reference's CG on the C4 system")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path's last step returned (pred, loss, dX) as "
+                         "DIR/<name>.npy; inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the B200 arm's outputs; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     os.environ["GLL_B200_SHARD_CG"] = args.cg_partition
     rank = int(os.environ.get("RANK", "0"))

@@ -1,5 +1,5 @@
-import sys, time, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from graphlearninglayer_b200 import LaplaceLearningSparseHard, sharded as sh, last_info, _lib
 from graphlearninglayer_b200.losses import custom_ce_loss
 from graphlearninglayer_b200.synth import synth_inputs
