@@ -1,14 +1,16 @@
 """graphlearninglayer_b200 -- B200 (sm_100a) implementation of the GraphLearningLayer hot path.
 
     from graphlearninglayer_b200 import LaplaceLearningSparseHard, knn_sym_dist, stable_conjgrad
+    from graphlearninglayer_b200 import laplace_learning        # utils.laplace on GPU features, no host round trip
 
 The names resolve lazily so that ``python -m graphlearninglayer_b200.build`` can run before the shared library
 exists; the first access loads libgll_b200.so through ctypes and fails loudly if it is missing or stale.  There is no
 CPU or PyTorch fallback.
 """
 __all__ = ["LaplaceLearningSparseHard", "LaplaceLearningSparseHardNormalized", "knn_sym_dist", "stable_conjgrad", "last_info", "GLL",
-           "GraphedStep", "BaseSetEvaluator"]
-_ELSEWHERE = {"GraphedStep": ".graphed", "BaseSetEvaluator": ".evalcache"}
+           "GraphedStep", "BaseSetEvaluator", "laplace_learning", "LaplaceResult"]
+_ELSEWHERE = {"GraphedStep": ".graphed", "BaseSetEvaluator": ".evalcache", "laplace_learning": ".laplace_eval",
+              "LaplaceResult": ".laplace_eval"}
 
 
 def __getattr__(name):

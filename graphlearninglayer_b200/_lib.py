@@ -19,6 +19,7 @@ STATUS_KNN_FALLBACK = 8
 
 INFO_STATUS, INFO_NNZ, INFO_NNZ_UU, INFO_CG_ITERS_FWD, INFO_CG_ITERS_BWD = 0, 1, 2, 3, 4
 INFO_KNN_FALLBACK_ROWS, INFO_CG_RESID_FWD, INFO_CG_RESID_BWD = 5, 6, 7
+INFO_LAPLACE_ROUNDS, INFO_LAPLACE_CG_ITERS, INFO_LAPLACE_RESID, INFO_LAPLACE_RESID0, INFO_LAPLACE_ROUND_ITERS = 8, 9, 10, 11, 14
 INFO_WORDS = 16
 
 
@@ -108,6 +109,8 @@ def _load():
     sig("gll_forward", i32, [vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, f32, i32, vp, vp, i32, vp, sz, vp])
     sig("gll_backward", i32, [vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, i32, vp, vp, vp, sz, vp])
     sig("gll_backward_scaled", i32, [vp, vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, f32, i32, vp, vp, vp, sz, vp])
+    sig("gll_laplace_eval_workspace_bytes", sz, [i32, i32, i32, i32, i32])
+    sig("gll_laplace_eval", i32, [vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp, vp, vp, vp, sz, vp])
     return lib
 
 
@@ -124,7 +127,8 @@ EXPORTS = ["gll_last_error", "gll_version", "gll_device_sm_count", "gll_kernel_c
            "gll_cg_rows_peer_mail_bytes", "gll_cg_rows_peer_flag_bytes", "gll_cg_rows_init_p2p", "gll_cg_rows_spmv_p2p",
            "gll_cg_rows_update_p2p", "gll_csr_residual_f64", "gll_normalize_rows",
            "gll_normalize_rows_backward", "gll_debug_gram_tile", "gll_base_cache_bytes", "gll_base_cache_workspace_bytes",
-           "gll_base_cache_build", "gll_knn_cached_workspace_bytes", "gll_knn_cached"]
+           "gll_base_cache_build", "gll_knn_cached_workspace_bytes", "gll_knn_cached", "gll_laplace_eval_workspace_bytes",
+           "gll_laplace_eval"]
 
 
 def check(rc: int, what: str) -> None:

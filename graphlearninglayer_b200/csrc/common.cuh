@@ -94,7 +94,7 @@ __device__ __forceinline__ float ordered_to_float(uint32_t u) {
 // ---- per-kernel launch counter and optional CUDA-event timing (gll_profile_* in the C ABI) ----
 enum KernelId {
   KID_SQNORM = 0, KID_GRAM_TOPK, KID_GRAM_TOPK_TC, KID_RERANK, KID_KNN_FALLBACK, KID_GRAPH, KID_WEIGHTS, KID_CG, KID_PACK,
-  KID_EDGE_GRAD, KID_ROW_GATHER, KID_CONVERT, KID_CG_ROWS, KID_COUNT
+  KID_EDGE_GRAD, KID_ROW_GATHER, KID_CONVERT, KID_CG_ROWS, KID_LAPLACE_REFINE, KID_LAPLACE_FINISH, KID_COUNT
 };
 // RAII: counts the launch; when profiling is on, brackets it with two events on the launch stream.
 struct ProfScope {

@@ -1,0 +1,313 @@
+// Laplace-learning evaluation on the device (utils.py:570-593 `laplace`, used by test_GL_NP at utils.py:637-660):
+// features -> graph -> harmonic extension refined in fp64 to the reference's stop rule -> argmax labels and a hit count.
+//
+//   gll_laplace_eval:  K1 + K2/K3 (gll_forward's stages with the caller's k)
+//                      fp32 Jacobi-CG  (L_uu + tau I) x0 = -L_ul Y,  relative tolerance GLL_LAPLACE_CG_RTOL0
+//                      GLL_LAPLACE_ROUNDS x { laplace_refine ; fp32 correction CG at GLL_LAPLACE_CG_RTOL }
+//                      laplace_finish
+//
+// laplace_refine (round r) reads x_{r-1} (fp64) and the previous fp32 correction e_{r-1}, and writes x_r = x_{r-1} + e_{r-1}
+// to the OTHER fp64 buffer (neighbour rows are read while rows are written, so the rounds ping-pong between `pred` and a
+// workspace buffer).  In the same pass it forms the fp64 residual over the full-graph CSR,
+//     r_i = sum_j w_ij (u_j - x_i) - tau x_i,   u = [Y; x_r],
+// i.e. b - A x with A = D - W_uu + tau I, D = ROW sums of the stored fp32 weights accumulated in fp64, and the reference's
+// stop quantity per class column ||M r_c||_2 = sqrt(sum_i r_ic^2 / (D_i + tau + 1e-10)) (make_golden_eval.py:41-45).
+// Per-CTA column partials are added in CTA order by the last CTA (integer ticket): no floating-point atomics.  That CTA
+// writes the correction solve's right-hand-side scale: 1 while some column is above tol, else 0 -- a zero right-hand side
+// stops every CG kernel at iteration 0 and the correction is exactly zero, so the round count is fixed and no host decision
+// is needed.  laplace_finish adds the last correction, writes pred, the argmax labels and the hit count.
+#include "cg_common.cuh"
+#include "common.cuh"
+
+namespace gll {
+namespace {
+
+constexpr int LR_THREADS = 256;
+
+struct RefineParams {
+  const int* row_ptr;  // full graph, n rows
+  const int* col;
+  const float* w;
+  const float* Y;        // k_lab x l
+  const double* x_prev;  // m x l, or NULL (round 0)
+  const float* e;        // m x lp fp32 correction (round 0: the initial solution)
+  double* x_out;         // m x l
+  double* r_out;         // m x l: right-hand side of the correction solve
+  double* partial;       // [gridDim.x][l]
+  double* colnorm;       // [l]
+  double* scale;         // 1 scalar
+  unsigned* ticket;
+  int* info;
+  int n, k_lab, m, l, lp, cw, round;
+  double tau, tol;
+};
+
+// Block = RL row lanes x CW class columns (CW = min(l, 32)); blockIdx.y picks a chunk of CW columns.  A thread walks the rows
+// of its lane in a fixed order and keeps its own partial sum of r^2 / diag: the reduction order depends on nothing but the
+// launch shape.
+__global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(RefineParams P) {
+  __shared__ double red[LR_THREADS];
+  __shared__ bool last;
+  const int cw = P.cw, rl_count = LR_THREADS / cw;
+  const int tid = threadIdx.x, rl = tid / cw, cc = tid - rl * cw;
+  const int c = blockIdx.y * cw + cc;
+  const bool active = rl < rl_count && c < P.l;
+  double acc = 0.0;
+  if (active) {
+    const int l = P.l, lp = P.lp, k_lab = P.k_lab;
+    for (int i = blockIdx.x * rl_count + rl; i < P.m; i += gridDim.x * rl_count) {
+      const size_t o = (size_t)i * l + c;
+      const double xi = (P.x_prev ? __ldg(P.x_prev + o) : 0.0) + (double)__ldg(P.e + (size_t)i * lp + c);
+      P.x_out[o] = xi;
+      const int g = k_lab + i, e1 = __ldg(P.row_ptr + g + 1);
+      double s = 0.0, deg = 0.0;
+      for (int e = __ldg(P.row_ptr + g); e < e1; ++e) {
+        const int j = __ldg(P.col + e);
+        const double wv = (double)__ldg(P.w + e);
+        double uj;
+        if (j < k_lab) {
+          uj = (double)__ldg(P.Y + (size_t)j * l + c);
+        } else {
+          const int jj = j - k_lab;
+          uj = (P.x_prev ? __ldg(P.x_prev + (size_t)jj * l + c) : 0.0) + (double)__ldg(P.e + (size_t)jj * lp + c);
+        }
+        s = fma(wv, uj - xi, s);
+        deg += wv;
+      }
+      const double r = s - P.tau * xi;
+      P.r_out[o] = r;
+      acc = fma(r, r / (deg + P.tau + 1e-10), acc);
+    }
+  }
+  red[tid] = acc;
+  __syncthreads();
+  if (tid < cw && c < P.l) {
+    double t = 0.0;
+    for (int q = 0; q < rl_count; ++q) t += red[q * cw + tid];
+    P.partial[(size_t)blockIdx.x * P.l + c] = t;
+  }
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last = atomicAdd(P.ticket, 1u) == gridDim.x * gridDim.y - 1u;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  const int lane = tid & 31, warp = tid >> 5;
+  for (int cc2 = warp; cc2 < P.l; cc2 += LR_THREADS / 32) {
+    double t = 0.0;
+    for (int b = lane; b < (int)gridDim.x; b += 32) t += __ldcg(P.partial + (size_t)b * P.l + cc2);
+    t = warp_sum(t);
+    if (lane == 0) P.colnorm[cc2] = sqrt(t);
+  }
+  __syncthreads();
+  if (tid == 0) {
+    double mx = 0.0;
+    bool bad = false;
+    for (int cc2 = 0; cc2 < P.l; ++cc2) {
+      const double v = P.colnorm[cc2];
+      if (!(v == v) || isinf(v)) bad = true;
+      mx = fmax(mx, v);
+    }
+    const bool more = bad || !(mx <= P.tol);
+    *P.scale = more ? 1.0 : 0.0;
+    if (more) P.info[GLL_INFO_LAPLACE_ROUNDS] = P.round + 1;
+    if (bad) atomicOr(P.info + GLL_INFO_STATUS, GLL_STATUS_NONFINITE);
+    const float fr = bad ? __int_as_float(0x7fc00000) : (float)mx;
+    P.info[GLL_INFO_LAPLACE_RESID] = __float_as_int(fr);
+    if (P.round == 0) P.info[GLL_INFO_LAPLACE_RESID0] = __float_as_int(fr);
+    *P.ticket = 0u;  // rewound for the next round
+  }
+}
+
+// Thread per unlabeled row: pred = x + e (in place), labels = first maximal column, hits counted with one integer atomic per CTA.
+// CTA 0 also writes the correction-CG iteration counts and the convergence status.
+__global__ void __launch_bounds__(LR_THREADS)
+laplace_finish_kernel(double* __restrict__ pred, const float* __restrict__ e, int m, int l, int lp, long long* __restrict__ labels,
+                      const long long* __restrict__ targets, unsigned long long* __restrict__ correct, const double* __restrict__ scale,
+                      const int* __restrict__ round_iters, int rounds, int* __restrict__ info) {
+  __shared__ int part[LR_THREADS / 32];
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  int hit = 0;
+  if (i < m) {
+    double best = 0.0;
+    int arg = 0;
+    for (int c = 0; c < l; ++c) {
+      const size_t o = (size_t)i * l + c;
+      const double v = pred[o] + (double)__ldg(e + (size_t)i * lp + c);
+      pred[o] = v;
+      if (c == 0 || v > best) {
+        best = v;
+        arg = c;
+      }
+    }
+    labels[i] = arg;
+    if (targets != nullptr) {
+      const long long t = __ldg(targets + i);
+      hit = (t >= 0 && t == (long long)arg) ? 1 : 0;
+    }
+  }
+  if (correct != nullptr) {
+    hit = warp_sum(hit);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = hit;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      int s = 0;
+      for (int w = 0; w < LR_THREADS / 32; ++w) s += part[w];
+      if (s) atomicAdd(correct, (unsigned long long)s);
+    }
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    int tot = 0;
+    unsigned packed[2] = {0u, 0u};
+    for (int r = 0; r < rounds; ++r) {
+      const int it = round_iters[r];
+      tot += it;
+      if (r < 4) packed[r >> 1] |= (unsigned)min(it, 65535) << (16 * (r & 1));
+    }
+    info[GLL_INFO_LAPLACE_CG_ITERS] = tot;
+    info[GLL_INFO_LAPLACE_ROUND_ITERS] = (int)packed[0];
+    info[GLL_INFO_LAPLACE_ROUND_ITERS + 1] = (int)packed[1];
+    if (*scale != 0.0) atomicOr(info + GLL_INFO_STATUS, GLL_STATUS_CG_NOT_CONVERGED);  // tol unmet after the last round
+  }
+}
+
+int refine_grid_x(int m, int l) {
+  const int cw = min(l, 32), rl = LR_THREADS / cw;
+  return max(1, min(ceil_div(m, rl), 4 * device_info().sms));
+}
+
+// the evaluation's own buffers, behind the layer state and in front of the stage workspace
+struct EvalBufs {
+  double* xtmp;    // m x l
+  double* r;       // m x l
+  double* partial; // [refine grid][l]
+  double* colnorm; // [l]
+  double* scale;
+  unsigned* ticket;
+  int* round_iters;  // [GLL_LAPLACE_ROUNDS]
+};
+
+// base == NULL: size query only
+size_t eval_bufs(char* base, int m, int l, EvalBufs* B) {
+  Carver cv(base, ~(size_t)0);
+  EvalBufs b;
+  b.xtmp = cv.take<double>((size_t)m * l);
+  b.r = cv.take<double>((size_t)m * l);
+  b.partial = cv.take<double>((size_t)refine_grid_x(m, l) * l);
+  b.colnorm = cv.take<double>(l);
+  b.scale = cv.take<double>(1);
+  b.ticket = cv.take<unsigned>(1);
+  b.round_iters = cv.take<int>(GLL_LAPLACE_ROUNDS);
+  if (B) *B = b;
+  return align_up(cv.off, 256);
+}
+
+}  // namespace
+}  // namespace gll
+
+using namespace gll;
+
+extern "C" {
+
+size_t gll_laplace_eval_workspace_bytes(int n, int d, int k, int l, int k_lab) {
+  gll_layout L;
+  if (n < 2 || l < 1 || k_lab < 1 || k_lab >= n || gll_state_layout(n, k, l, k_lab, &L)) return 0;
+  return L.total + eval_bufs(nullptr, n - k_lab, l, nullptr) + gll_workspace_bytes(n, d, k, l, k_lab);
+}
+
+int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
+                     float tau, double tol, int cg_max_iter, double* pred, long long* labels, const long long* targets,
+                     long long* correct_out, int* info, void* workspace, size_t workspace_bytes, void* stream) {
+  GLL_REQUIRE(X && Y && pred && labels && info && workspace, "null pointer");
+  GLL_REQUIRE(k >= 2 && k <= 64 && (k <= 33 || n >= 256) && k <= n, "k must be in [2, 64] (n >= 256 when k > 33) and <= n");
+  GLL_REQUIRE(d >= 1 && l >= 1 && k_lab >= 1 && k_lab < n, "bad sizes");
+  GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
+  const size_t need = gll_laplace_eval_workspace_bytes(n, d, k, l, k_lab);
+  if (workspace_bytes < need) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, need);
+    return GLL_ERR_WORKSPACE;
+  }
+  gll_layout L;
+  if (gll_state_layout(n, k, l, k_lab, &L)) return GLL_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int m = n - k_lab, lp = padded_classes(l);
+  // workspace = [layer state | the evaluation's buffers | stage workspace]
+  char* S = (char*)workspace;
+  EvalBufs B;
+  const size_t eb = eval_bufs(S + L.total, m, l, &B);
+  void* ws = S + L.total + eb;
+  const size_t ws_bytes = workspace_bytes - L.total - eb;
+  int* sinfo = info;  // slots 12-13 are the on-chip CG's barrier words (zeroed here, rewound by the kernels)
+
+  GLL_CUDA_CHECK(cudaMemsetAsync(sinfo, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  GLL_CUDA_CHECK(cudaMemsetAsync(B.ticket, 0, sizeof(unsigned), st));
+  if (correct_out) GLL_CUDA_CHECK(cudaMemsetAsync(correct_out, 0, sizeof(long long), st));
+  int rc = knn_run(X, n, d, k, 0, n, (int*)(S + L.knn_idx), (float*)(S + L.knn_dist), sinfo, ws, ws_bytes, st);
+  if (rc) return rc;
+  rc = graph_weights_run((int*)(S + L.knn_idx), (float*)(S + L.knn_dist), Y, n, k, l, k_lab, eps_auto, eps_fixed, tau,
+                         (int*)(S + L.row_ptr), (int*)(S + L.col), (float*)(S + L.dist), (float*)(S + L.eps), (int*)(S + L.kappa),
+                         (float*)(S + L.w), (float*)(S + L.deg), (int*)(S + L.uu_ptr), (int*)(S + L.uu_col), (float*)(S + L.uu_val),
+                         (float*)(S + L.diag), (float*)(S + L.rhs), (float*)(S + L.ut), sinfo, ws, ws_bytes, st);
+  if (rc) return rc;
+  const int* uu_ptr = (int*)(S + L.uu_ptr);
+  const int* uu_col = (int*)(S + L.uu_col);
+  const float* uu_val = (float*)(S + L.uu_val);
+  const float* diag = (float*)(S + L.diag);
+  float* rhs = (float*)(S + L.rhs);
+  float* x0 = (float*)(S + L.ut) + (size_t)k_lab * lp;
+  float* corr = (float*)(S + L.wt);  // the adjoint's region, free in an evaluation
+  unsigned* barrier = (unsigned*)(sinfo + 12);
+  // No sparsity hint (0): the evaluation system is never routed to the cluster kernel.  No status pointer either: an inner solve
+  // that stops at the fp32 floor is not a failure -- the fp64 rounds decide convergence.
+  rc = cg_run(uu_ptr, uu_col, uu_val, diag, rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, x0, sinfo + GLL_INFO_CG_ITERS_FWD,
+              (float*)(sinfo + GLL_INFO_CG_RESID_FWD), nullptr, ws, ws_bytes, st, barrier, nullptr);
+  if (rc) return rc;
+
+  RefineParams P;
+  P.row_ptr = (int*)(S + L.row_ptr);
+  P.col = (int*)(S + L.col);
+  P.w = (float*)(S + L.w);
+  P.Y = Y;
+  P.r_out = B.r;
+  P.partial = B.partial;
+  P.colnorm = B.colnorm;
+  P.scale = B.scale;
+  P.ticket = B.ticket;
+  P.info = sinfo;
+  P.n = n;
+  P.k_lab = k_lab;
+  P.m = m;
+  P.l = l;
+  P.lp = lp;
+  P.cw = min(l, 32);
+  P.tau = (double)tau;
+  P.tol = tol;
+  const dim3 grid(refine_grid_x(m, l), ceil_div(l, P.cw));
+  const CgIo io = {B.r, 2, nullptr, 0, B.scale, 1, 0.f};
+  for (int r = 0; r < GLL_LAPLACE_ROUNDS; ++r) {
+    // the last round writes pred; rounds alternate between pred and the workspace buffer
+    double* out = ((GLL_LAPLACE_ROUNDS - 1 - r) % 2 == 0) ? pred : B.xtmp;
+    P.x_prev = (r == 0) ? nullptr : (out == pred ? B.xtmp : pred);
+    P.e = (r == 0) ? x0 : corr;
+    P.x_out = out;
+    P.round = r;
+    {
+      GLL_PROF(KID_LAPLACE_REFINE, st);
+      laplace_refine_kernel<<<grid, LR_THREADS, 0, st>>>(P);
+      GLL_LAUNCH_CHECK();
+    }
+    rc = cg_run(uu_ptr, uu_col, uu_val, diag, rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, corr, B.round_iters + r, nullptr,
+                nullptr, ws, ws_bytes, st, barrier, &io);
+    if (rc) return rc;
+  }
+  {
+    GLL_PROF(KID_LAPLACE_FINISH, st);
+    laplace_finish_kernel<<<ceil_div(m, LR_THREADS), LR_THREADS, 0, st>>>(pred, corr, m, l, lp, labels, targets,
+                                                                           (unsigned long long*)correct_out, B.scale, B.round_iters,
+                                                                           GLL_LAPLACE_ROUNDS, sinfo);
+    GLL_LAUNCH_CHECK();
+  }
+  return GLL_OK;
+}
+
+}  // extern "C"

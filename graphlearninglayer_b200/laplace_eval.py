@@ -1,0 +1,107 @@
+"""Laplace-learning evaluation on the device: the reference's ``utils.laplace`` (utils.py:570-593), as ``test_GL_NP``
+(utils.py:637-660) runs it on base + train + test features, in one call on features that are already on the GPU.
+
+    res = laplace_learning(features, label_matrix, k=50, epsilon='auto', tau=0.0, tol=1e-10, targets=None)
+    res.pred      (m, l) float64   harmonic extension on the unlabeled rows (m = n - k_lab)
+    res.labels    (m,) int64       argmax, first maximal column on ties
+    res.correct   0-dim int64      rows with targets >= 0 and labels == targets (None without targets)
+
+Same graph as the layer (kNN -> union graph -> weights, with this k); the system L_uu + tau I is solved in fp32 and refined
+in fp64 until every class column meets the reference's stop rule ||M (b - A x)||_2 <= tol with M = diag(A + 1e-10)^(-1/2)
+(see gll_laplace_eval in include/gll_b200.h, including the row-sum degree).  Everything is enqueued on the current stream:
+no host sync, no host round trip, so the call can be captured into a CUDA graph.  Status ('max iter reached' when tol is
+unmet, epsilon ~ 0) goes through the same deferred check as the layer.  Knob: GLL_B200_CG_MAXIT (iterations per CG solve).
+"""
+from __future__ import annotations
+
+from typing import NamedTuple, Optional
+
+import numpy as np
+import torch
+
+from . import _lib
+from .GLL import _bytes, _cg_maxit, _check_status, _require_cuda, _stream_ptr
+from ._lib import lib
+
+__all__ = ["laplace_learning", "LaplaceResult", "last_eval_info"]
+
+
+class LaplaceResult(NamedTuple):
+    pred: torch.Tensor
+    labels: torch.Tensor
+    correct: Optional[torch.Tensor]
+
+
+_last_info: Optional[torch.Tensor] = None
+
+
+def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto", tau: float = 0.0,
+                     tol: float = 1e-10, targets: Optional[torch.Tensor] = None) -> LaplaceResult:
+    """features (n, d) CUDA tensor with the k_lab labeled rows FIRST (GLL.py:11); label_matrix (k_lab, l) one-hot float32 or
+    int64; targets (m,) int64 or None, a negative target is not counted."""
+    if features.dim() != 2:
+        raise ValueError("features must be (n, d)")
+    if label_matrix.dim() != 2:
+        raise ValueError("label_matrix must be (k_lab, l)")
+    n, d = features.shape
+    k_lab, l = label_matrix.shape
+    k = int(k)
+    if not (0 < k_lab < n):
+        raise ValueError(f"need 0 < k_lab < n (k_lab={k_lab}, n={n}); labeled rows come first (GLL.py:11)")
+    if l < 1 or d < 1:
+        raise ValueError("need at least one class column and one feature")
+    if not (2 <= k <= 64) or k > n or (k > 33 and n < 256):
+        raise ValueError(f"k must be in [2, 64] and <= n, with n >= 256 when k > 33 (k={k}, n={n})")
+    if isinstance(epsilon, str):
+        if epsilon != "auto":
+            raise ValueError("epsilon must be a float or 'auto'")
+        eps_auto, eps_fixed = 1, 0.0
+    else:
+        eps_auto, eps_fixed = 0, float(epsilon)
+    if not tol > 0:
+        raise ValueError("tol must be > 0")
+    m = n - k_lab
+    if targets is not None and tuple(targets.shape) != (m,):
+        raise ValueError(f"targets must be ({m},), got {tuple(targets.shape)}")
+    _require_cuda(features, "features")
+    dev = features.device
+    Xc = features.detach()
+    if Xc.dtype != torch.float32:
+        Xc = Xc.float()
+    Xc = Xc.contiguous()
+    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
+    tg = None
+    if targets is not None:
+        tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
+    with torch.cuda.device(dev):
+        ws_bytes = lib.gll_laplace_eval_workspace_bytes(n, d, k, l, k_lab)
+        ws = _bytes(ws_bytes, dev)
+        pred = torch.empty((m, l), dtype=torch.float64, device=dev)
+        labels = torch.empty(m, dtype=torch.int64, device=dev)
+        correct = torch.empty((), dtype=torch.int64, device=dev) if tg is not None else None
+        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
+        rc = lib.gll_laplace_eval(Xc.data_ptr(), Y.data_ptr(), n, d, k, l, k_lab, eps_auto, eps_fixed, float(tau), float(tol),
+                                  _cg_maxit(), pred.data_ptr(), labels.data_ptr(), tg.data_ptr() if tg is not None else None,
+                                  correct.data_ptr() if correct is not None else None, info.data_ptr(), ws.data_ptr(), ws_bytes,
+                                  _stream_ptr(dev))
+    _lib.check(rc, "gll_laplace_eval")
+    global _last_info
+    _last_info = info
+    _check_status(info, "Laplace-learning")
+    return LaplaceResult(pred, labels, correct)
+
+
+def last_eval_info() -> dict:
+    """Device status block of the most recent laplace_learning call (synchronises).  Keys follow GLL_INFO_* in
+    include/gll_b200.h."""
+    if _last_info is None:
+        return {}
+    v = _last_info.cpu().numpy()
+    f = v.view(np.float32)
+    u = v.view(np.uint32)
+    round_iters = [int((u[_lib.INFO_LAPLACE_ROUND_ITERS + r // 2] >> (16 * (r % 2))) & 0xFFFF) for r in range(4)]
+    return dict(status=int(v[_lib.INFO_STATUS]), nnz=int(v[_lib.INFO_NNZ]), nnz_uu=int(v[_lib.INFO_NNZ_UU]),
+                cg_iters_first=int(v[_lib.INFO_CG_ITERS_FWD]), knn_fallback_rows=int(v[_lib.INFO_KNN_FALLBACK_ROWS]),
+                rounds=int(v[_lib.INFO_LAPLACE_ROUNDS]), cg_iters_correction=int(v[_lib.INFO_LAPLACE_CG_ITERS]),
+                round_iters=round_iters, resid_first=float(f[_lib.INFO_LAPLACE_RESID0]),
+                resid=float(f[_lib.INFO_LAPLACE_RESID]))

@@ -42,7 +42,20 @@ extern "C" {
 #define GLL_INFO_KNN_FALLBACK_ROWS 5
 #define GLL_INFO_CG_RESID_FWD 6 /* float bits: max_c ||r_c||_2 at exit */
 #define GLL_INFO_CG_RESID_BWD 7
+/* gll_laplace_eval only (slots 12-13 are the on-chip CG's barrier words in every call) */
+#define GLL_INFO_LAPLACE_ROUNDS 8       /* refinement rounds that ran a correction solve */
+#define GLL_INFO_LAPLACE_CG_ITERS 9     /* correction-CG iterations, all rounds */
+#define GLL_INFO_LAPLACE_RESID 10       /* float bits: max_c ||M r_c||_2 at the last refinement round */
+#define GLL_INFO_LAPLACE_RESID0 11      /* float bits: the same after the initial solve */
+#define GLL_INFO_LAPLACE_ROUND_ITERS 14 /* two words: correction-CG iterations of round r in bits [16 (r % 2), +16) of word 14 + r / 2 */
 #define GLL_INFO_WORDS 16
+
+/* gll_laplace_eval's refinement schedule (chosen from the CPU model in tests/test_laplace_eval_cpu.py): the initial fp32 solve
+ * stops at GLL_LAPLACE_CG_RTOL0 times its right-hand side's largest column norm, each correction solve at GLL_LAPLACE_CG_RTOL,
+ * and GLL_LAPLACE_ROUNDS fp64 residual rounds run. */
+#define GLL_LAPLACE_ROUNDS 4
+#define GLL_LAPLACE_CG_RTOL0 1e-5
+#define GLL_LAPLACE_CG_RTOL 1e-4
 
 const char* gll_last_error(void);
 int gll_version(void);
@@ -285,6 +298,24 @@ int gll_backward(const float* X, const void* grad_out, int grad_is_f64, int n, i
 int gll_backward_scaled(const float* X, const void* grad_out, int grad_is_f64, const void* scale, int scale_is_f64, int n, int d,
                         int k, int l, int k_lab, int eps_auto, float cg_tol, int cg_max_iter, void* state, float* dX,
                         void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Laplace-learning evaluation, the reference's utils.laplace (utils.py:570-593) as test_GL_NP calls it (utils.py:637-660):
+ * one graph over all n rows (labeled rows first), the unlabeled block solved to the reference's stop rule, argmax labels.
+ *   Graph: gll_forward's stages with this k (2 <= k <= 64; n >= 256 when k > 33), eps_auto / eps_fixed as there.
+ *   System: L = D - W from the stored fp32 W, evaluated in fp64, with D = ROW sums of W (the reference's csgraph.laplacian
+ *   takes column sums; W_ij and W_ji may differ in the last fp32 bit, so the two agree to ~1e-7 relative).
+ *   Solve (L_uu + tau I) x = -L_ul Y: fp32 Jacobi-CG, then GLL_LAPLACE_ROUNDS rounds of fp64 residual + fp32 correction solve,
+ *   stopping when every class column has ||M (b - A x)||_2 <= tol, M = diag(A + 1e-10)^(-1/2) -- the residual of the
+ *   reference's stable_conjgrad on the Jacobi-scaled system.  Rounds after convergence cost two launches and no iterations.
+ *   Outputs: pred m x l fp64 (m = n - k_lab), labels[m] int64 = first maximal column; with targets (m int64, may be NULL)
+ *   correct_out (one int64, may be NULL) = #{i : targets[i] >= 0 and labels[i] == targets[i]}.
+ *   info: GLL_INFO_WORDS int32 (device); GLL_STATUS_CG_NOT_CONVERGED when tol is unmet after the last round.
+ *   workspace: gll_laplace_eval_workspace_bytes(...) bytes (it also holds the graph state).  Nothing syncs with the host. */
+size_t gll_laplace_eval_workspace_bytes(int n, int d, int k, int l, int k_lab);
+int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
+                     float tau, double tol, int cg_max_iter, double* pred, long long* labels, const long long* targets,
+                     long long* correct_out, int* info, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
