@@ -23,7 +23,7 @@ from __future__ import annotations
 
 import os
 import warnings
-from typing import Optional, Union
+from typing import Optional, Tuple, Union
 
 import numpy as np
 import torch
@@ -64,6 +64,34 @@ def _require_cuda(t: torch.Tensor, what: str) -> None:
                            "the reference /root/reference/GLL.py is the CPU implementation)")
 
 
+def parse_epsilon(epsilon) -> Tuple[int, float]:
+    """(eps_auto, eps_fixed) of the C ABI: 'auto' (GLL.py:205) or a fixed bandwidth (GLL.py:226)."""
+    if isinstance(epsilon, str):
+        if epsilon != "auto":
+            raise ValueError("epsilon must be a float or 'auto'")
+        return 1, 0.0
+    return 0, float(epsilon)
+
+
+def pred_dtype() -> torch.dtype:
+    """dtype of the predictions (GLL_B200_PRED_DTYPE; float64 like the reference, GLL.py:66)."""
+    return torch.float32 if os.environ.get("GLL_B200_PRED_DTYPE", "float64") == "float32" else torch.float64
+
+
+def as_features(X: torch.Tensor) -> torch.Tensor:
+    """X detached as the float32, contiguous matrix the kernels read (no copy when it already is one)."""
+    X = X.detach()
+    if X.dtype != torch.float32:
+        X = X.float()
+    return X.contiguous()
+
+
+def decode_info(v: np.ndarray) -> dict:
+    """The keys every status block reports, from its host copy (int32 words, GLL_INFO_* in include/gll_b200.h)."""
+    return dict(status=int(v[_lib.INFO_STATUS]), nnz=int(v[_lib.INFO_NNZ]), nnz_uu=int(v[_lib.INFO_NNZ_UU]),
+                knn_fallback_rows=int(v[_lib.INFO_KNN_FALLBACK_ROWS]))
+
+
 _last_info: Optional[torch.Tensor] = None
 
 
@@ -74,10 +102,8 @@ def last_info() -> dict:
         return {}
     v = _last_info.cpu().numpy()
     f = v.view(np.float32)
-    return dict(status=int(v[_lib.INFO_STATUS]), nnz=int(v[_lib.INFO_NNZ]), nnz_uu=int(v[_lib.INFO_NNZ_UU]),
-                cg_iters_fwd=int(v[_lib.INFO_CG_ITERS_FWD]), cg_iters_bwd=int(v[_lib.INFO_CG_ITERS_BWD]),
-                knn_fallback_rows=int(v[_lib.INFO_KNN_FALLBACK_ROWS]), cg_resid_fwd=float(f[_lib.INFO_CG_RESID_FWD]),
-                cg_resid_bwd=float(f[_lib.INFO_CG_RESID_BWD]))
+    return dict(decode_info(v), cg_iters_fwd=int(v[_lib.INFO_CG_ITERS_FWD]), cg_iters_bwd=int(v[_lib.INFO_CG_ITERS_BWD]),
+                cg_resid_fwd=float(f[_lib.INFO_CG_RESID_FWD]), cg_resid_bwd=float(f[_lib.INFO_CG_RESID_BWD]))
 
 
 def _warn_from_status(info: torch.Tensor, where: str) -> None:
@@ -136,10 +162,7 @@ def _forward_impl(X: torch.Tensor, label_matrix: torch.Tensor, tau, epsilon, k: 
     if X.dim() != 2:
         raise ValueError("features must be (n, d)")
     dev = X.device
-    Xc = X.detach()
-    if Xc.dtype != torch.float32:
-        Xc = Xc.float()
-    Xc = Xc.contiguous()
+    Xc = as_features(X)
     Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()  # int64 one-hot allowed (t_a_a.py:545)
     if Y.dim() != 2:
         raise ValueError("label_matrix must be (k_lab, l)")
@@ -149,25 +172,19 @@ def _forward_impl(X: torch.Tensor, label_matrix: torch.Tensor, tau, epsilon, k: 
         raise ValueError(f"need 0 < k_lab < n (k_lab={k_lab}, n={n}); labeled rows come first (GLL.py:11)")
     if n < k:
         raise ValueError(f"need at least k={k} nodes, got {n}")
-    if isinstance(epsilon, str):
-        if epsilon != "auto":
-            raise ValueError("epsilon must be a float or 'auto'")
-        eps_auto, eps_fixed = 1, 0.0
-    else:
-        eps_auto, eps_fixed = 0, float(epsilon)
+    eps_auto, eps_fixed = parse_epsilon(epsilon)
     m = n - k_lab
     st = _State()
     st.layout = _lib.state_layout(n, k, l, k_lab)
     st.n, st.d, st.k, st.l, st.k_lab, st.eps_auto = n, d, k, l, k_lab, eps_auto
-    pred64 = os.environ.get("GLL_B200_PRED_DTYPE", "float64") != "float32"
     with torch.cuda.device(dev):
         st.buf = _bytes(st.layout.total, dev)
         ws_bytes = lib.gll_workspace_bytes(n, d, k, l, k_lab)
         ws = _bytes(ws_bytes, dev)
-        pred = torch.empty((m, l), dtype=torch.float64 if pred64 else torch.float32, device=dev)
+        pred = torch.empty((m, l), dtype=pred_dtype(), device=dev)
         rc = lib.gll_forward(Xc.data_ptr(), Y.data_ptr(), n, d, k, l, k_lab, eps_auto, eps_fixed, float(tau), _cg_tol(),
-                             _cg_maxit(), st.buf.data_ptr(), pred.data_ptr(), int(pred64), ws.data_ptr(), ws_bytes,
-                             _stream_ptr(dev))
+                             _cg_maxit(), st.buf.data_ptr(), pred.data_ptr(), int(pred.dtype == torch.float64), ws.data_ptr(),
+                             ws_bytes, _stream_ptr(dev))
     _lib.check(rc, "gll_forward")
     global _last_info
     _last_info = st.view("info", torch.int32, _lib.INFO_WORDS)
@@ -242,10 +259,7 @@ class LaplaceLearningSparseHardNormalized(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feat, label_matrix, tau=0, epsilon="auto"):
         _require_cuda(feat, "features")
-        f = feat.detach()
-        if f.dtype != torch.float32:
-            f = f.float()
-        f = f.contiguous()
+        f = as_features(feat)
         n, d = f.shape
         xn = torch.empty_like(f)
         inv = torch.empty(n, dtype=torch.float32, device=f.device)
@@ -283,46 +297,46 @@ def _device() -> torch.device:
     return torch.device("cuda", torch.cuda.current_device())
 
 
-def _graph_stages(Xc: torch.Tensor, k: int, epsilon):
-    """kNN -> CSR -> weights through the stage entry points; returns device tensors."""
-    dev = Xc.device
-    n, d = Xc.shape
-    emax = lib.gll_max_edges(n, k)
-    i32, f32 = torch.int32, torch.float32
-    knn_idx = torch.empty((n, k), dtype=i32, device=dev)
-    knn_dist = torch.empty((n, k), dtype=f32, device=dev)
-    row_ptr = torch.empty(n + 1, dtype=i32, device=dev)
-    col = torch.empty(emax, dtype=i32, device=dev)
-    dist = torch.empty(emax, dtype=f32, device=dev)
-    info = torch.zeros(_lib.INFO_WORDS, dtype=i32, device=dev)
-    s = _stream_ptr(dev)
-    wsb = max(lib.gll_knn_workspace_bytes(n, d, k), lib.gll_graph_workspace_bytes(n, k), lib.gll_weights_workspace_bytes(n, k))
-    ws = _bytes(wsb, dev)
-    _lib.check(lib.gll_knn(Xc.data_ptr(), n, d, k, knn_idx.data_ptr(), knn_dist.data_ptr(), info.data_ptr(), ws.data_ptr(),
-                           wsb, s), "gll_knn")
-    _lib.check(lib.gll_graph_build(knn_idx.data_ptr(), knn_dist.data_ptr(), n, k, row_ptr.data_ptr(), col.data_ptr(),
-                                   dist.data_ptr(), info.data_ptr(), ws.data_ptr(), wsb, s), "gll_graph_build")
-    eps_auto = isinstance(epsilon, str)
-    if eps_auto and epsilon != "auto":
-        raise ValueError("epsilon must be a float or 'auto'")
-    # the weights stage also emits the unlabeled-block system; with a 1-row dummy label block it is just ignored
-    k_lab, l = 1, 1
-    lp = lib.gll_padded_classes(l)
-    m = n - k_lab
-    Y = torch.zeros((k_lab, l), dtype=f32, device=dev)
-    out = dict(eps=torch.empty(n, dtype=f32, device=dev), kappa=torch.empty(n, dtype=i32, device=dev),
-               w=torch.empty(emax, dtype=f32, device=dev), deg=torch.empty(n, dtype=f32, device=dev))
-    scratch = dict(uu_ptr=torch.empty(m + 1, dtype=i32, device=dev), uu_col=torch.empty(emax, dtype=i32, device=dev),
-                   uu_val=torch.empty(emax, dtype=f32, device=dev), diag=torch.empty(m, dtype=f32, device=dev),
-                   rhs=torch.empty(m * lp, dtype=f32, device=dev), ut=torch.empty(n * lp, dtype=f32, device=dev))
-    _lib.check(lib.gll_edge_weights(knn_idx.data_ptr(), knn_dist.data_ptr(), row_ptr.data_ptr(), col.data_ptr(),
-                                    dist.data_ptr(), Y.data_ptr(), n, k, l, k_lab, int(eps_auto),
-                                    0.0 if eps_auto else float(epsilon), 0.0, out["eps"].data_ptr(),
-                                    out["kappa"].data_ptr(), out["w"].data_ptr(), out["deg"].data_ptr(),
-                                    scratch["uu_ptr"].data_ptr(), scratch["uu_col"].data_ptr(),
-                                    scratch["uu_val"].data_ptr(), scratch["diag"].data_ptr(), scratch["rhs"].data_ptr(),
-                                    scratch["ut"].data_ptr(), info.data_ptr(), ws.data_ptr(), wsb, s), "gll_edge_weights")
-    return dict(knn_idx=knn_idx, knn_dist=knn_dist, row_ptr=row_ptr, col=col, dist=dist, info=info, **out)
+class GraphStages:
+    """K2 + K3 (gll_graph_build, gll_edge_weights) on kNN lists the caller searched: the graph (row_ptr, col, dist), its
+    weights (eps, kappa, w, deg) and the unlabeled block's system (uu_ptr, uu_col, uu_val, diag, rhs) as device tensors, and
+    ut whose first k_lab rows hold Y.  knn_idx / knn_dist may have more than n rows (never read); ws is a byte tensor of at
+    least the graph and weights workspaces (None: one is allocated); ut is zero-filled when zero_ut."""
+
+    def __init__(self, knn_idx: torch.Tensor, knn_dist: torch.Tensor, Y: torch.Tensor, n: int, tau: float, epsilon,
+                 info: torch.Tensor, ws: Optional[torch.Tensor] = None, zero_ut: bool = False):
+        dev = knn_idx.device
+        k = knn_idx.shape[1]
+        k_lab, l = Y.shape
+        m, lp, emax = n - k_lab, lib.gll_padded_classes(l), lib.gll_max_edges(n, k)
+        self.n, self.k, self.l, self.k_lab, self.m, self.lp = n, k, l, k_lab, m, lp
+        self.eps_auto, eps_fixed = parse_epsilon(epsilon)
+        self.knn_idx, self.knn_dist, self.info = knn_idx, knn_dist, info
+        i32, f32 = torch.int32, torch.float32
+        self.row_ptr = torch.empty(n + 1, dtype=i32, device=dev)
+        self.col = torch.empty(emax, dtype=i32, device=dev)
+        self.dist = torch.empty(emax, dtype=f32, device=dev)
+        self.eps = torch.empty(n, dtype=f32, device=dev)
+        self.kappa = torch.empty(n, dtype=i32, device=dev)
+        self.w = torch.empty(emax, dtype=f32, device=dev)
+        self.deg = torch.empty(n, dtype=f32, device=dev)
+        self.uu_ptr = torch.empty(m + 1, dtype=i32, device=dev)
+        self.uu_col = torch.empty(emax, dtype=i32, device=dev)
+        self.uu_val = torch.empty(emax, dtype=f32, device=dev)
+        self.diag = torch.empty(m, dtype=f32, device=dev)
+        self.rhs = torch.empty((m, lp), dtype=f32, device=dev)
+        self.ut = (torch.zeros if zero_ut else torch.empty)((n, lp), dtype=f32, device=dev)
+        if ws is None:
+            ws = _bytes(max(lib.gll_graph_workspace_bytes(n, k), lib.gll_weights_workspace_bytes(n, k)), dev)
+        s = _stream_ptr(dev)
+        _lib.check(lib.gll_graph_build(knn_idx.data_ptr(), knn_dist.data_ptr(), n, k, self.row_ptr.data_ptr(), self.col.data_ptr(),
+                                       self.dist.data_ptr(), info.data_ptr(), ws.data_ptr(), ws.numel(), s), "gll_graph_build")
+        _lib.check(lib.gll_edge_weights(knn_idx.data_ptr(), knn_dist.data_ptr(), self.row_ptr.data_ptr(), self.col.data_ptr(),
+                                        self.dist.data_ptr(), Y.data_ptr(), n, k, l, k_lab, self.eps_auto, eps_fixed, float(tau),
+                                        self.eps.data_ptr(), self.kappa.data_ptr(), self.w.data_ptr(), self.deg.data_ptr(),
+                                        self.uu_ptr.data_ptr(), self.uu_col.data_ptr(), self.uu_val.data_ptr(),
+                                        self.diag.data_ptr(), self.rhs.data_ptr(), self.ut.data_ptr(), info.data_ptr(),
+                                        ws.data_ptr(), ws.numel(), s), "gll_edge_weights")
 
 
 def knn_sym_dist(data, k=K_NEIGHBOURS, epsilon="auto"):
@@ -338,27 +352,36 @@ def knn_sym_dist(data, k=K_NEIGHBOURS, epsilon="auto"):
 
     dev = _device()
     Xc = torch.as_tensor(np.ascontiguousarray(data, dtype=np.float32)).to(dev)
-    g = _graph_stages(Xc, int(k), epsilon)
-    n = Xc.shape[0]
-    indptr = g["row_ptr"].cpu().numpy()
+    n, d = Xc.shape
+    k = int(k)
+    knn_idx = torch.empty((n, k), dtype=torch.int32, device=dev)
+    knn_dist = torch.empty((n, k), dtype=torch.float32, device=dev)
+    info = torch.zeros(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
+    wsb = max(lib.gll_knn_workspace_bytes(n, d, k), lib.gll_graph_workspace_bytes(n, k), lib.gll_weights_workspace_bytes(n, k))
+    ws = _bytes(wsb, dev)
+    _lib.check(lib.gll_knn(Xc.data_ptr(), n, d, k, knn_idx.data_ptr(), knn_dist.data_ptr(), info.data_ptr(), ws.data_ptr(), wsb,
+                           _stream_ptr(dev)), "gll_knn")
+    # the weights stage also emits the unlabeled-block system; with a 1-row dummy label block it is just ignored
+    g = GraphStages(knn_idx, knn_dist, torch.zeros((1, 1), dtype=torch.float32, device=dev), n, 0.0, epsilon, info, ws)
+    indptr = g.row_ptr.cpu().numpy()
     E = int(indptr[-1])
-    cols = g["col"][:E].cpu().numpy()
-    dist = g["dist"][:E].cpu().numpy().astype(np.float64)
-    w = g["w"][:E].cpu().numpy().astype(np.float64)
-    eps = g["eps"].cpu().numpy().astype(np.float64)
-    if int(g["info"][_lib.INFO_STATUS].item()) & _lib.STATUS_EPS_TINY:
+    cols = g.col[:E].cpu().numpy()
+    dist = g.dist[:E].cpu().numpy().astype(np.float64)
+    w = g.w[:E].cpu().numpy().astype(np.float64)
+    eps = g.eps.cpu().numpy().astype(np.float64)
+    if int(info[_lib.INFO_STATUS].item()) & _lib.STATUS_EPS_TINY:
         warnings.warn("Epsilon in KNN is very close to zero.")  # GLL.py:240-241
     rows = np.repeat(np.arange(n), np.diff(indptr))
     with np.errstate(divide="ignore", invalid="ignore"):
         v = -8.0 * w / eps[rows] / eps[cols]
     W = sp.csr_matrix((w, cols, indptr), shape=(n, n))
     V = sp.csr_matrix((v, cols.copy(), indptr.copy()), shape=(n, n))
-    knn_ind = g["knn_idx"].cpu().numpy().astype(np.int64)
+    knn_ind = knn_idx.cpu().numpy().astype(np.int64)
     if isinstance(epsilon, str):
         with np.errstate(divide="ignore", invalid="ignore"):
             mv = dist * dist * v / (eps[rows] ** 2) / 2.0
         mod_V = sp.csr_matrix((mv, cols.copy(), indptr.copy()), shape=(n, n))
-        kappa = g["kappa"].cpu().numpy().astype(np.int64)
+        kappa = g.kappa.cpu().numpy().astype(np.int64)
         Cm = sp.csr_matrix((np.ones(n), (kappa, np.arange(n))), shape=(n, n))
         return W, V, mod_V, Cm, knn_ind
     return W, V, 0, 0, knn_ind  # placeholders of GLL.py:229-230

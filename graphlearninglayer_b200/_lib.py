@@ -20,6 +20,7 @@ STATUS_KNN_FALLBACK = 8
 INFO_STATUS, INFO_NNZ, INFO_NNZ_UU, INFO_CG_ITERS_FWD, INFO_CG_ITERS_BWD = 0, 1, 2, 3, 4
 INFO_KNN_FALLBACK_ROWS, INFO_CG_RESID_FWD, INFO_CG_RESID_BWD = 5, 6, 7
 INFO_LAPLACE_ROUNDS, INFO_LAPLACE_CG_ITERS, INFO_LAPLACE_RESID, INFO_LAPLACE_RESID0, INFO_LAPLACE_ROUND_ITERS = 8, 9, 10, 11, 14
+INFO_CG_BARRIER = 12  # two words: the on-chip CG's grid barrier
 INFO_WORDS = 16
 
 

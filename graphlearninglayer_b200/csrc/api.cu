@@ -294,6 +294,35 @@ static int make_layout(int n, int k, int l, int k_lab, gll_layout* L) {
   return GLL_OK;
 }
 
+// expected off-diagonal entries per row of L_uu: the solver's sparsity hint in gll_forward / gll_backward.  evalcache._uu_hint
+// repeats this float32 arithmetic bit for bit so that BaseSetEvaluator runs the same solver kernel.
+static float uu_degree_hint(int n, int k, int m) { return 1.2f * (float)(k - 1) * (float)m / (float)n; }
+
+GraphBufs graph_bufs(const gll_layout& L, void* state) {
+  char* S = (char*)state;
+  GraphBufs B;
+  B.knn_idx = (int*)(S + L.knn_idx);
+  B.knn_dist = (float*)(S + L.knn_dist);
+  B.row_ptr = (int*)(S + L.row_ptr);
+  B.col = (int*)(S + L.col);
+  B.dist = (float*)(S + L.dist);
+  B.w = (float*)(S + L.w);
+  B.gv = (float*)(S + L.gv);
+  B.eps = (float*)(S + L.eps);
+  B.kappa = (int*)(S + L.kappa);
+  B.deg = (float*)(S + L.deg);
+  B.bvec = (float*)(S + L.bvec);
+  B.uu_ptr = (int*)(S + L.uu_ptr);
+  B.uu_col = (int*)(S + L.uu_col);
+  B.uu_val = (float*)(S + L.uu_val);
+  B.diag = (float*)(S + L.diag);
+  B.rhs = (float*)(S + L.rhs);
+  B.ut = (float*)(S + L.ut);
+  B.wt = (float*)(S + L.wt);
+  B.info = (int*)(S + L.info);
+  return B;
+}
+
 }  // namespace gll
 
 using namespace gll;
@@ -395,15 +424,38 @@ int gll_knn_rows(const float* X, int n, int d, int k, int row_begin, int row_end
 
 int gll_graph_build(const int* knn_idx, const float* knn_dist, int n, int k, int* row_ptr, int* col, float* dist, int* info,
                     void* workspace, size_t workspace_bytes, void* stream) {
-  return graph_run(knn_idx, knn_dist, n, k, row_ptr, col, dist, info, workspace, workspace_bytes, (cudaStream_t)stream);
+  GraphBufs B = {};
+  B.knn_idx = const_cast<int*>(knn_idx);  // inputs: only read
+  B.knn_dist = const_cast<float*>(knn_dist);
+  B.row_ptr = row_ptr;
+  B.col = col;
+  B.dist = dist;
+  B.info = info;
+  return graph_stages_run(B, nullptr, n, k, 0, 0, 0, 0.f, 0.f, /*phases*/ 0, 4, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int gll_edge_weights(const int* knn_idx, const float* knn_dist, const int* row_ptr, const int* col, const float* dist,
                      const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau, float* eps,
                      int* kappa, float* w, float* deg, int* uu_ptr, int* uu_col, float* uu_val, float* diag, float* rhs,
                      float* ut, int* info, void* workspace, size_t workspace_bytes, void* stream) {
-  return weights_run(knn_idx, knn_dist, row_ptr, col, dist, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, eps, kappa, w, deg,
-                     uu_ptr, uu_col, uu_val, diag, rhs, ut, info, workspace, workspace_bytes, (cudaStream_t)stream);
+  GraphBufs B = {};
+  B.knn_idx = const_cast<int*>(knn_idx);  // inputs: only read
+  B.knn_dist = const_cast<float*>(knn_dist);
+  B.row_ptr = const_cast<int*>(row_ptr);
+  B.col = const_cast<int*>(col);
+  B.dist = const_cast<float*>(dist);
+  B.eps = eps;
+  B.kappa = kappa;
+  B.w = w;
+  B.deg = deg;
+  B.uu_ptr = uu_ptr;
+  B.uu_col = uu_col;
+  B.uu_val = uu_val;
+  B.diag = diag;
+  B.rhs = rhs;
+  B.ut = ut;
+  B.info = info;
+  return graph_stages_run(B, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, /*phases*/ 3, 6, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int gll_cg_solve(const int* uu_ptr, const int* uu_col, const float* uu_val, const float* diag, const float* rhs, int m, int l,
@@ -424,16 +476,26 @@ int gll_cg_solve_hint(const int* uu_ptr, const int* uu_col, const float* uu_val,
 int gll_backward_edges(const float* X, int n, int d, int l, int k_lab, int eps_auto, const int* row_ptr, const int* col,
                        const float* dist, const float* w, const float* eps, const int* kappa, const float* ut,
                        const float* wt, float* gv, float* bvec, float* dX, void* stream) {
-  return backward_edges_run(X, n, d, l, k_lab, eps_auto, row_ptr, col, dist, w, eps, kappa, ut, wt, gv, bvec, dX, 0, n, 3,
-                            (cudaStream_t)stream);
+  return gll_backward_edges_rows(X, n, d, l, k_lab, eps_auto, row_ptr, col, dist, w, eps, kappa, ut, wt, gv, bvec, dX, 0, n, 3,
+                                 stream);
 }
 
 int gll_backward_edges_rows(const float* X, int n, int d, int l, int k_lab, int eps_auto, const int* row_ptr, const int* col,
                             const float* dist, const float* w, const float* eps, const int* kappa, const float* ut,
                             const float* wt, float* gv, float* bvec, float* dX, int row_begin, int row_end, int phases,
                             void* stream) {
-  return backward_edges_run(X, n, d, l, k_lab, eps_auto, row_ptr, col, dist, w, eps, kappa, ut, wt, gv, bvec, dX, row_begin,
-                            row_end, phases, (cudaStream_t)stream);
+  GraphBufs B = {};
+  B.row_ptr = const_cast<int*>(row_ptr);  // inputs: only read
+  B.col = const_cast<int*>(col);
+  B.dist = const_cast<float*>(dist);
+  B.w = const_cast<float*>(w);
+  B.eps = const_cast<float*>(eps);
+  B.kappa = const_cast<int*>(kappa);
+  B.ut = const_cast<float*>(ut);
+  B.wt = const_cast<float*>(wt);
+  B.gv = gv;
+  B.bvec = bvec;
+  return backward_edges_run(X, n, d, l, k_lab, eps_auto, B, dX, row_begin, row_end, phases, (cudaStream_t)stream);
 }
 
 size_t gll_cg_rows_workspace_bytes(int rows_local, int l) { return cg_rows_ws_bytes(rows_local, l); }
@@ -561,35 +623,37 @@ int gll_pack_grad(const void* grad_out, int grad_is_f64, int m, int l, float* rh
   return pack_grad(grad_out, grad_is_f64, m, l, padded_classes(l), rhs, (cudaStream_t)stream);
 }
 
+// the state's arrays and the workspace check of gll_forward and gll_backward_scaled
+static int driver_bufs(int n, int d, int k, int l, int k_lab, void* state, size_t workspace_bytes, GraphBufs* B) {
+  gll_layout L;
+  if (gll_state_layout(n, k, l, k_lab, &L)) return GLL_ERR_ARG;
+  const size_t need = gll_workspace_bytes(n, d, k, l, k_lab);
+  if (workspace_bytes < need) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, need);
+    return GLL_ERR_WORKSPACE;
+  }
+  *B = graph_bufs(L, state);
+  return GLL_OK;
+}
+
 int gll_forward(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
                 float tau, float cg_tol, int cg_max_iter, void* state, void* pred_out, int pred_is_f64, void* workspace,
                 size_t workspace_bytes, void* stream) {
   GLL_REQUIRE(X && state && pred_out && workspace, "null pointer");
-  gll_layout L;
-  if (gll_state_layout(n, k, l, k_lab, &L)) return GLL_ERR_ARG;
-  if (workspace_bytes < gll_workspace_bytes(n, d, k, l, k_lab)) {
-    set_error("workspace too small: %zu < %zu", workspace_bytes, gll_workspace_bytes(n, d, k, l, k_lab));
-    return GLL_ERR_WORKSPACE;
-  }
+  GraphBufs B;
+  int rc = driver_bufs(n, d, k, l, k_lab, state, workspace_bytes, &B);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  char* S = (char*)state;
-  int* info = (int*)(S + L.info);
   const int m = n - k_lab, lp = padded_classes(l);
-  GLL_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int) * GLL_INFO_WORDS, st));
-  int rc = knn_run(X, n, d, k, 0, n, (int*)(S + L.knn_idx), (float*)(S + L.knn_dist), info, workspace, workspace_bytes, st);
+  GLL_CUDA_CHECK(cudaMemsetAsync(B.info, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  rc = knn_run(X, n, d, k, 0, n, B.knn_idx, B.knn_dist, B.info, workspace, workspace_bytes, st);
   if (rc) return rc;
-  rc = graph_weights_run((int*)(S + L.knn_idx), (float*)(S + L.knn_dist), Y, n, k, l, k_lab, eps_auto, eps_fixed, tau,
-                         (int*)(S + L.row_ptr), (int*)(S + L.col), (float*)(S + L.dist), (float*)(S + L.eps), (int*)(S + L.kappa),
-                         (float*)(S + L.w), (float*)(S + L.deg), (int*)(S + L.uu_ptr), (int*)(S + L.uu_col), (float*)(S + L.uu_val),
-                         (float*)(S + L.diag), (float*)(S + L.rhs), (float*)(S + L.ut), info, workspace, workspace_bytes, st);
+  rc = graph_stages_run(B, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, 0, 6, workspace, workspace_bytes, st);
   if (rc) return rc;
-  float* u_out = (float*)(S + L.ut) + (size_t)k_lab * lp;
-  const float uu_hint = 1.2f * (float)(k - 1) * (float)m / (float)n;  // expected off-diagonal entries per row of L_uu
-  const CgIo io = {nullptr, 0, pred_out, pred_is_f64, nullptr, 0, uu_hint};  // Pred (GLL.py:66) is written by the solver itself
-  return cg_run((int*)(S + L.uu_ptr), (int*)(S + L.uu_col), (float*)(S + L.uu_val), (float*)(S + L.diag),
-                (float*)(S + L.rhs), m, l, cg_tol, cg_max_iter, u_out, info + GLL_INFO_CG_ITERS_FWD,
-                (float*)(info + GLL_INFO_CG_RESID_FWD), info + GLL_INFO_STATUS, workspace, workspace_bytes, st,
-                (unsigned*)(info + 12), &io);  // info[12..13]: the on-chip CG's barrier words (zeroed with info, rewound by the kernel)
+  const CgIo io = {nullptr, 0, pred_out, pred_is_f64, nullptr, 0, uu_degree_hint(n, k, m)};  // Pred (GLL.py:66) is written by the solver itself
+  return cg_run(B.uu_ptr, B.uu_col, B.uu_val, B.diag, B.rhs, m, l, cg_tol, cg_max_iter, B.ut + (size_t)k_lab * lp,
+                B.info + GLL_INFO_CG_ITERS_FWD, (float*)(B.info + GLL_INFO_CG_RESID_FWD), B.info + GLL_INFO_STATUS, workspace,
+                workspace_bytes, st, (unsigned*)(B.info + GLL_INFO_CG_BARRIER), &io);
 }
 
 int gll_backward(const float* X, const void* grad_out, int grad_is_f64, int n, int d, int k, int l, int k_lab, int eps_auto,
@@ -603,28 +667,19 @@ int gll_backward_scaled(const float* X, const void* grad_out, int grad_is_f64, c
                         int l, int k_lab, int eps_auto, float cg_tol, int cg_max_iter, void* state, float* dX, void* workspace,
                         size_t workspace_bytes, void* stream) {
   GLL_REQUIRE(X && grad_out && state && dX && workspace, "null pointer");
-  gll_layout L;
-  if (gll_state_layout(n, k, l, k_lab, &L)) return GLL_ERR_ARG;
-  if (workspace_bytes < gll_workspace_bytes(n, d, k, l, k_lab)) {
-    set_error("workspace too small: %zu < %zu", workspace_bytes, gll_workspace_bytes(n, d, k, l, k_lab));
-    return GLL_ERR_WORKSPACE;
-  }
+  GraphBufs B;
+  int rc = driver_bufs(n, d, k, l, k_lab, state, workspace_bytes, &B);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  char* S = (char*)state;
-  int* info = (int*)(S + L.info);
   const int m = n - k_lab, lp = padded_classes(l);
-  float* wt = (float*)(S + L.wt);
   // GLL.py:104: the solver reads the incoming gradient itself; the labeled rows of the padded adjoint solution (zeros) are
   // never read -- edge_grad substitutes them
-  const CgIo io = {grad_out, grad_is_f64 ? 2 : 1, nullptr, 0, scale, scale_is_f64, 1.2f * (float)(k - 1) * (float)m / (float)n};
-  int rc = cg_run((int*)(S + L.uu_ptr), (int*)(S + L.uu_col), (float*)(S + L.uu_val), (float*)(S + L.diag),
-                  (float*)(S + L.rhs), m, l, cg_tol, cg_max_iter, wt + (size_t)k_lab * lp, info + GLL_INFO_CG_ITERS_BWD,
-                  (float*)(info + GLL_INFO_CG_RESID_BWD), info + GLL_INFO_STATUS, workspace, workspace_bytes, st,
-                  (unsigned*)(info + 12), &io);
+  const CgIo io = {grad_out, grad_is_f64 ? 2 : 1, nullptr, 0, scale, scale_is_f64, uu_degree_hint(n, k, m)};
+  rc = cg_run(B.uu_ptr, B.uu_col, B.uu_val, B.diag, B.rhs, m, l, cg_tol, cg_max_iter, B.wt + (size_t)k_lab * lp,
+              B.info + GLL_INFO_CG_ITERS_BWD, (float*)(B.info + GLL_INFO_CG_RESID_BWD), B.info + GLL_INFO_STATUS, workspace,
+              workspace_bytes, st, (unsigned*)(B.info + GLL_INFO_CG_BARRIER), &io);
   if (rc) return rc;
-  return backward_edges_run(X, n, d, l, k_lab, eps_auto, (int*)(S + L.row_ptr), (int*)(S + L.col), (float*)(S + L.dist),
-                            (float*)(S + L.w), (float*)(S + L.eps), (int*)(S + L.kappa), (float*)(S + L.ut), wt,
-                            (float*)(S + L.gv), (float*)(S + L.bvec), dX, 0, n, 3, st);
+  return backward_edges_run(X, n, d, l, k_lab, eps_auto, B, dX, 0, n, 3, st);
 }
 
 }  // extern "C"

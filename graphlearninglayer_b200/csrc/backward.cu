@@ -234,20 +234,18 @@ row_gather_warp_kernel(const float* __restrict__ X, int row_begin, int row_end, 
 
 }  // namespace
 
-int backward_edges_run(const float* X, int n, int d, int l, int k_lab, int eps_auto, const int* row_ptr, const int* col,
-                       const float* dist, const float* w, const float* eps, const int* kappa, const float* ut,
-                       const float* wt, float* gv, float* bvec, float* dX, int row_begin, int row_end, int phases,
-                       cudaStream_t st) {
-  GLL_REQUIRE(X && row_ptr && col && dist && w && eps && ut && wt && gv && bvec && dX, "null pointer");
-  GLL_REQUIRE(!eps_auto || kappa, "kappa missing");
+int backward_edges_run(const float* X, int n, int d, int l, int k_lab, int eps_auto, const GraphBufs& B, float* dX, int row_begin,
+                       int row_end, int phases, cudaStream_t st) {
+  GLL_REQUIRE(X && B.row_ptr && B.col && B.dist && B.w && B.eps && B.ut && B.wt && B.gv && B.bvec && dX, "null pointer");
+  GLL_REQUIRE(!eps_auto || B.kappa, "kappa missing");
   GLL_REQUIRE(0 <= row_begin && row_begin <= row_end && row_end <= n, "bad row range");
   const int rows = row_end - row_begin;
   if (rows == 0) return GLL_OK;
   const int lp = padded_classes(l);
   if (phases & 1) {  // K5: gv for the rows' edges, b for the rows
     GLL_PROF(KID_EDGE_GRAD, st);
-    edge_grad_kernel<<<ceil_div((long long)rows * 32, 256), 256, 0, st>>>(row_begin, row_end, lp, k_lab, eps_auto, row_ptr, col,
-                                                                          dist, w, eps, ut, wt, gv, bvec);
+    edge_grad_kernel<<<ceil_div((long long)rows * 32, 256), 256, 0, st>>>(row_begin, row_end, lp, k_lab, eps_auto, B.row_ptr, B.col,
+                                                                          B.dist, B.w, B.eps, B.ut, B.wt, B.gv, B.bvec);
   }
   GLL_LAUNCH_CHECK();
   if (phases & 2) {  // K6: needs b of ALL rows (neighbours j with kappa(j) = i)
@@ -258,13 +256,13 @@ int backward_edges_run(const float* X, int n, int d, int l, int k_lab, int eps_a
     if (vec4) {
       const int grid = ceil_div(rows, 4);
       if (cols <= 32)
-        row_gather_warp_kernel<1><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, row_ptr, col, kappa, gv, bvec, dX);
+        row_gather_warp_kernel<1><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
       else if (cols <= 64)
-        row_gather_warp_kernel<2><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, row_ptr, col, kappa, gv, bvec, dX);
+        row_gather_warp_kernel<2><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
       else
-        row_gather_warp_kernel<4><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, row_ptr, col, kappa, gv, bvec, dX);
+        row_gather_warp_kernel<4><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
     } else
-      row_gather_kernel<1><<<rows, threads, 0, st>>>(X, row_begin, d, eps_auto, row_ptr, col, kappa, gv, bvec, dX);
+      row_gather_kernel<1><<<rows, threads, 0, st>>>(X, row_begin, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
   }
   GLL_LAUNCH_CHECK();
   return GLL_OK;

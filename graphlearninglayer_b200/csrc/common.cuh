@@ -120,20 +120,38 @@ void knn_tc_set_trace(void* device_buf);  // debug timeline of the Gram kernel's
 int knn_debug_gram_tile(const float* X, int n, int d, int row_tile, int col_tile, float* acc_out, float* rscale_out, void* ws,
                         size_t ws_bytes, cudaStream_t st);
 
-int graph_run(const int* knn_idx, const float* knn_dist, int n, int k, int* row_ptr, int* col, float* dist,
-              int* info, void* ws, size_t ws_bytes, cudaStream_t st);
-size_t graph_ws_bytes(int n, int k);
+// One typed pointer per array of gll_layout: the graph, its system and the backward scratch, as the stages pass them on.
+// The stage entry points fill only what they use and leave the rest NULL.
+struct GraphBufs {
+  int* knn_idx;
+  float* knn_dist;
+  int* row_ptr;
+  int* col;
+  float* dist;
+  float* w;
+  float* gv;
+  float* eps;
+  int* kappa;
+  float* deg;
+  float* bvec;
+  int* uu_ptr;
+  int* uu_col;
+  float* uu_val;
+  float* diag;
+  float* rhs;
+  float* ut;
+  float* wt;
+  int* info;
+};
+// the arrays of a state buffer laid out by gll_state_layout
+GraphBufs graph_bufs(const gll_layout& L, void* state);
 
-int weights_run(const int* knn_idx, const float* knn_dist, const int* row_ptr, const int* col, const float* dist,
-                const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau,
-                float* eps, int* kappa, float* w, float* deg, int* uu_ptr, int* uu_col, float* uu_val,
-                float* diag, float* rhs, float* ut, int* info, void* ws, size_t ws_bytes, cudaStream_t st);
+// K2 (phases 0-3: CSR with sorted rows) and K3 (phases 3-5: weights and the unlabeled system) as one cooperative launch over
+// the phases [phase_begin, phase_end): 0-4 is K2, 3-6 K3 on sorted rows, 0-6 both (graph.cu)
+int graph_stages_run(const GraphBufs& B, const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau,
+                     int phase_begin, int phase_end, void* ws, size_t ws_bytes, cudaStream_t st);
+size_t graph_ws_bytes(int n, int k);
 size_t weights_ws_bytes(int n, int k);
-// K2 + K3 in one cooperative launch (graph.cu)
-int graph_weights_run(const int* knn_idx, const float* knn_dist, const float* Y, int n, int k, int l, int k_lab, int eps_auto,
-                      float eps_fixed, float tau, int* row_ptr, int* col, float* dist, float* eps, int* kappa, float* w, float* deg,
-                      int* uu_ptr, int* uu_col, float* uu_val, float* diag, float* rhs, float* ut, int* info, void* ws, size_t ws_bytes,
-                      cudaStream_t st);
 size_t graph_weights_ws_bytes(int n, int k);
 
 // optional fused conversions of the layer: rhs_src = the caller's [m][l] right-hand side (rhs_kind 1 fp32 / 2 fp64; `rhs` is then
@@ -166,10 +184,9 @@ int cg_rows_update(const float* diag, int m, int l, int row_lo, int row_hi, cons
                    float* x, float* u_full, int* ctrl, float* resid_out, void* ws, size_t ws_bytes, const gll_peers* peers,
                    unsigned epoch, cudaStream_t st);
 
-int backward_edges_run(const float* X, int n, int d, int l, int k_lab, int eps_auto, const int* row_ptr,
-                       const int* col, const float* dist, const float* w, const float* eps, const int* kappa,
-                       const float* ut, const float* wt, float* gv, float* bvec, float* dX, int row_begin, int row_end,
-                       int phases, cudaStream_t st);
+// reads row_ptr, col, dist, w, eps, kappa, ut, wt of B; writes gv, bvec
+int backward_edges_run(const float* X, int n, int d, int l, int k_lab, int eps_auto, const GraphBufs& B, float* dX, int row_begin,
+                       int row_end, int phases, cudaStream_t st);
 
 // column slices of m x lp class matrices (sharded solves): dst[r][c] = src[r][c0 + c] for c < cnt (zero padding), and back
 int pack_columns(const float* src, int rows, int lp_src, int c0, int cnt, float* dst, int lp_dst, cudaStream_t st);

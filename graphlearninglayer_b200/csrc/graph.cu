@@ -357,17 +357,6 @@ __global__ void __launch_bounds__(GF_THREADS, 1) graph_weights_kernel(GfParams P
 int gf_grid() { return device_info().sms; }
 size_t gf_common_bytes() { return 256 + align_up(sizeof(int) * (size_t)(gf_grid() + 1), 256); }
 
-// common = [barrier counter (256 B) | tile sums]; counter_cleared: the caller's memset covered the counter already
-int gf_launch(GfParams& P, void* common, cudaStream_t st, int kid, bool counter_cleared) {
-  P.counter = (unsigned*)common;
-  P.tile_sums = (int*)((char*)common + 256);
-  if (!counter_cleared) GLL_CUDA_CHECK(cudaMemsetAsync(P.counter, 0, 64, st));
-  void* args[] = {&P};
-  ProfScope prof(kid, st);
-  GLL_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)graph_weights_kernel, dim3(gf_grid()), dim3(GF_THREADS), args, 0, st));
-  return GLL_OK;
-}
-
 }  // namespace
 
 size_t graph_ws_bytes(int n, int k) {
@@ -381,135 +370,76 @@ size_t weights_ws_bytes(int n, int k) {
 }
 size_t graph_weights_ws_bytes(int n, int k) { return graph_ws_bytes(n, k) + weights_ws_bytes(n, k); }
 
-// carve the K2 scratch; the barrier counter, len and cursor are adjacent 256-aligned blocks: ONE memset clears all three
-static int carve_graph(GfParams& P, Carver& cv, int n, int k, void** common, cudaStream_t st) {
-  const size_t emax = gll_max_edges(n, k);
-  *common = cv.take<char>(gf_common_bytes());
-  P.len = cv.take<int>(n + 1);
-  P.cursor = cv.take<int>(n + 1);
-  P.col_tmp = cv.take<int>(emax);
-  P.dist_tmp = cv.take<float>(emax);
-  P.flag = cv.take<unsigned char>((size_t)n * k);
-  GLL_CUDA_CHECK(cudaMemsetAsync(*common, 0, (size_t)((char*)P.cursor - (char*)*common) + sizeof(int) * (size_t)(n + 1), st));
-  return GLL_OK;
-}
-
-int graph_run(const int* knn_idx, const float* knn_dist, int n, int k, int* row_ptr, int* col, float* dist, int* info,
-              void* ws, size_t ws_bytes, cudaStream_t st) {
-  GLL_REQUIRE(knn_idx && knn_dist && row_ptr && col && dist && ws, "null pointer");
+int graph_stages_run(const GraphBufs& B, const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau,
+                     int phase_begin, int phase_end, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const bool build = phase_begin == 0;  // K2 from the kNN lists; otherwise the rows are sorted already (col_tmp stays NULL)
+  const bool weights = phase_end > 4;   // K3; otherwise phase 3 only sorts the rows (w stays NULL)
+  GLL_REQUIRE(B.knn_idx && B.knn_dist && B.row_ptr && B.col && B.dist && ws, "null pointer");
   GLL_REQUIRE(n >= 1 && k >= 2, "bad sizes");
-  if (ws_bytes < graph_ws_bytes(n, k)) {
-    set_error("graph workspace too small: %zu < %zu", ws_bytes, graph_ws_bytes(n, k));
+  if (weights) {
+    GLL_REQUIRE(B.eps && B.kappa && B.w && B.deg && B.uu_ptr && B.uu_col && B.uu_val && B.diag && B.rhs && B.ut, "null pointer");
+    GLL_REQUIRE(k_lab >= 0 && k_lab < n && l >= 1, "need 0 <= k_lab < n and l >= 1");
+    GLL_REQUIRE(k_lab == 0 || Y != nullptr, "label matrix missing");
+  }
+  const size_t need = (build ? graph_ws_bytes(n, k) : 0) + (weights ? weights_ws_bytes(n, k) : 0);
+  if (ws_bytes < need) {
+    set_error("%s workspace too small: %zu < %zu", build ? "graph" : "weights", ws_bytes, need);
     return GLL_ERR_WORKSPACE;
   }
   GfParams P;
   memset(&P, 0, sizeof(P));
   P.trace = (unsigned long long*)cg_get_trace();
-  Carver cv(ws, ws_bytes);
-  void* common;
-  int rc = carve_graph(P, cv, n, k, &common, st);
-  if (rc) return rc;
-  P.knn_idx = knn_idx;
-  P.knn_dist = knn_dist;
+  P.knn_idx = B.knn_idx;
+  P.knn_dist = B.knn_dist;
   P.n = n;
   P.k = k;
-  P.row_ptr = row_ptr;
-  P.col = col;
-  P.dist = dist;
-  P.info = info;
-  P.phase_begin = 0;
-  P.phase_end = 4;  // phase 3 sorts the rows and, with no weight outputs given, stops there
-  return gf_launch(P, common, st, KID_GRAPH, true);
-}
-
-static void set_weights(GfParams& P, const float* Y, int l, int k_lab, int eps_auto, float eps_fixed, float tau, float* eps, int* kappa,
-                        float* w, float* deg, int* uu_ptr, int* uu_col, float* uu_val, float* diag, float* rhs, float* ut) {
-  P.Y = Y;
-  P.l = l;
-  P.lp = padded_classes(l);
-  P.k_lab = k_lab;
-  P.eps_auto = eps_auto;
-  P.eps_fixed = eps_fixed;
-  P.tau = tau;
-  P.eps = eps;
-  P.kappa = kappa;
-  P.w = w;
-  P.deg = deg;
-  P.uu_ptr = uu_ptr;
-  P.uu_col = uu_col;
-  P.uu_val = uu_val;
-  P.diag = diag;
-  P.rhs = rhs;
-  P.ut = ut;
-}
-
-int weights_run(const int* knn_idx, const float* knn_dist, const int* row_ptr, const int* col, const float* dist,
-                const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau, float* eps,
-                int* kappa, float* w, float* deg, int* uu_ptr, int* uu_col, float* uu_val, float* diag, float* rhs,
-                float* ut, int* info, void* ws, size_t ws_bytes, cudaStream_t st) {
-  GLL_REQUIRE(knn_idx && knn_dist && row_ptr && col && dist && eps && kappa && w && deg && uu_ptr && uu_col && uu_val &&
-                  diag && rhs && ut && ws,
-              "null pointer");
-  GLL_REQUIRE(k_lab >= 0 && k_lab < n && l >= 1, "need 0 <= k_lab < n and l >= 1");
-  GLL_REQUIRE(k_lab == 0 || Y != nullptr, "label matrix missing");
-  if (ws_bytes < weights_ws_bytes(n, k)) {
-    set_error("weights workspace too small: %zu < %zu", ws_bytes, weights_ws_bytes(n, k));
-    return GLL_ERR_WORKSPACE;
+  P.row_ptr = B.row_ptr;
+  P.col = B.col;
+  P.dist = B.dist;
+  P.info = B.info;
+  P.phase_begin = phase_begin;
+  P.phase_end = phase_end;
+  // common = [barrier counter (256 B) | tile sums], then the K2 scratch, then uu_cnt
+  Carver cv(ws, ws_bytes);
+  char* common = cv.take<char>(gf_common_bytes());
+  P.counter = (unsigned*)common;
+  P.tile_sums = (int*)(common + 256);
+  size_t zero_bytes = 64;  // the barrier counter
+  if (build) {
+    const size_t emax = gll_max_edges(n, k);
+    P.len = cv.take<int>(n + 1);
+    P.cursor = cv.take<int>(n + 1);
+    P.col_tmp = cv.take<int>(emax);
+    P.dist_tmp = cv.take<float>(emax);
+    P.flag = cv.take<unsigned char>((size_t)n * k);
+    // the counter, len and cursor are adjacent 256-aligned blocks: ONE memset clears all three
+    zero_bytes = (size_t)((char*)P.cursor - common) + sizeof(int) * (size_t)(n + 1);
   }
-  GfParams P;
-  memset(&P, 0, sizeof(P));
-  P.trace = (unsigned long long*)cg_get_trace();
-  Carver cv(ws, ws_bytes);
-  P.uu_cnt = cv.take<int>(n + 1);
-  void* common = cv.take<char>(gf_common_bytes());
-  P.knn_idx = knn_idx;
-  P.knn_dist = knn_dist;
-  P.n = n;
-  P.k = k;
-  P.row_ptr = const_cast<int*>(row_ptr);  // read only from phase 3 on
-  P.col = const_cast<int*>(col);
-  P.dist = const_cast<float*>(dist);
-  P.info = info;
-  set_weights(P, Y, l, k_lab, eps_auto, eps_fixed, tau, eps, kappa, w, deg, uu_ptr, uu_col, uu_val, diag, rhs, ut);
-  P.phase_begin = 3;  // col_tmp == NULL: the rows are sorted already
-  P.phase_end = 6;
-  return gf_launch(P, common, st, KID_WEIGHTS, false);
-}
-
-// K2 + K3 in one launch (gll_forward)
-int graph_weights_run(const int* knn_idx, const float* knn_dist, const float* Y, int n, int k, int l, int k_lab, int eps_auto,
-                      float eps_fixed, float tau, int* row_ptr, int* col, float* dist, float* eps, int* kappa, float* w, float* deg,
-                      int* uu_ptr, int* uu_col, float* uu_val, float* diag, float* rhs, float* ut, int* info, void* ws, size_t ws_bytes,
-                      cudaStream_t st) {
-  GLL_REQUIRE(knn_idx && knn_dist && row_ptr && col && dist && eps && kappa && w && deg && uu_ptr && uu_col && uu_val && diag &&
-                  rhs && ut && ws,
-              "null pointer");
-  GLL_REQUIRE(n >= 1 && k >= 2 && k_lab >= 0 && k_lab < n && l >= 1, "bad sizes");
-  GLL_REQUIRE(k_lab == 0 || Y != nullptr, "label matrix missing");
-  if (ws_bytes < graph_weights_ws_bytes(n, k)) {
-    set_error("graph workspace too small: %zu < %zu", ws_bytes, graph_weights_ws_bytes(n, k));
-    return GLL_ERR_WORKSPACE;
+  if (weights) {
+    P.uu_cnt = cv.take<int>(n + 1);
+    P.Y = Y;
+    P.l = l;
+    P.lp = padded_classes(l);
+    P.k_lab = k_lab;
+    P.eps_auto = eps_auto;
+    P.eps_fixed = eps_fixed;
+    P.tau = tau;
+    P.eps = B.eps;
+    P.kappa = B.kappa;
+    P.w = B.w;
+    P.deg = B.deg;
+    P.uu_ptr = B.uu_ptr;
+    P.uu_col = B.uu_col;
+    P.uu_val = B.uu_val;
+    P.diag = B.diag;
+    P.rhs = B.rhs;
+    P.ut = B.ut;
   }
-  GfParams P;
-  memset(&P, 0, sizeof(P));
-  P.trace = (unsigned long long*)cg_get_trace();
-  Carver cv(ws, ws_bytes);
-  void* common;
-  int rc = carve_graph(P, cv, n, k, &common, st);
-  if (rc) return rc;
-  P.uu_cnt = cv.take<int>(n + 1);
-  P.knn_idx = knn_idx;
-  P.knn_dist = knn_dist;
-  P.n = n;
-  P.k = k;
-  P.row_ptr = row_ptr;
-  P.col = col;
-  P.dist = dist;
-  P.info = info;
-  set_weights(P, Y, l, k_lab, eps_auto, eps_fixed, tau, eps, kappa, w, deg, uu_ptr, uu_col, uu_val, diag, rhs, ut);
-  P.phase_begin = 0;
-  P.phase_end = 6;
-  return gf_launch(P, common, st, KID_GRAPH, true);
+  GLL_CUDA_CHECK(cudaMemsetAsync(common, 0, zero_bytes, st));
+  void* args[] = {&P};
+  ProfScope prof(phase_begin == 3 ? KID_WEIGHTS : KID_GRAPH, st);
+  GLL_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)graph_weights_kernel, dim3(gf_grid()), dim3(GF_THREADS), args, 0, st));
+  return GLL_OK;
 }
 
 }  // namespace gll

@@ -233,47 +233,40 @@ int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l,
   const int m = n - k_lab, lp = padded_classes(l);
   // workspace = [layer state | the evaluation's buffers | stage workspace]
   char* S = (char*)workspace;
+  GraphBufs G = graph_bufs(L, S);
+  G.info = info;  // the caller's info block in place of the state's
   EvalBufs B;
   const size_t eb = eval_bufs(S + L.total, m, l, &B);
   void* ws = S + L.total + eb;
   const size_t ws_bytes = workspace_bytes - L.total - eb;
-  int* sinfo = info;  // slots 12-13 are the on-chip CG's barrier words (zeroed here, rewound by the kernels)
 
-  GLL_CUDA_CHECK(cudaMemsetAsync(sinfo, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  GLL_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int) * GLL_INFO_WORDS, st));
   GLL_CUDA_CHECK(cudaMemsetAsync(B.ticket, 0, sizeof(unsigned), st));
   if (correct_out) GLL_CUDA_CHECK(cudaMemsetAsync(correct_out, 0, sizeof(long long), st));
-  int rc = knn_run(X, n, d, k, 0, n, (int*)(S + L.knn_idx), (float*)(S + L.knn_dist), sinfo, ws, ws_bytes, st);
+  int rc = knn_run(X, n, d, k, 0, n, G.knn_idx, G.knn_dist, info, ws, ws_bytes, st);
   if (rc) return rc;
-  rc = graph_weights_run((int*)(S + L.knn_idx), (float*)(S + L.knn_dist), Y, n, k, l, k_lab, eps_auto, eps_fixed, tau,
-                         (int*)(S + L.row_ptr), (int*)(S + L.col), (float*)(S + L.dist), (float*)(S + L.eps), (int*)(S + L.kappa),
-                         (float*)(S + L.w), (float*)(S + L.deg), (int*)(S + L.uu_ptr), (int*)(S + L.uu_col), (float*)(S + L.uu_val),
-                         (float*)(S + L.diag), (float*)(S + L.rhs), (float*)(S + L.ut), sinfo, ws, ws_bytes, st);
+  rc = graph_stages_run(G, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, 0, 6, ws, ws_bytes, st);
   if (rc) return rc;
-  const int* uu_ptr = (int*)(S + L.uu_ptr);
-  const int* uu_col = (int*)(S + L.uu_col);
-  const float* uu_val = (float*)(S + L.uu_val);
-  const float* diag = (float*)(S + L.diag);
-  float* rhs = (float*)(S + L.rhs);
-  float* x0 = (float*)(S + L.ut) + (size_t)k_lab * lp;
-  float* corr = (float*)(S + L.wt);  // the adjoint's region, free in an evaluation
-  unsigned* barrier = (unsigned*)(sinfo + 12);
+  float* x0 = G.ut + (size_t)k_lab * lp;
+  float* corr = G.wt;  // the adjoint's region, free in an evaluation
+  unsigned* barrier = (unsigned*)(info + GLL_INFO_CG_BARRIER);  // zeroed with info, rewound by the kernels
   // No sparsity hint (0): the evaluation system is never routed to the cluster kernel.  No status pointer either: an inner solve
   // that stops at the fp32 floor is not a failure -- the fp64 rounds decide convergence.
-  rc = cg_run(uu_ptr, uu_col, uu_val, diag, rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, x0, sinfo + GLL_INFO_CG_ITERS_FWD,
-              (float*)(sinfo + GLL_INFO_CG_RESID_FWD), nullptr, ws, ws_bytes, st, barrier, nullptr);
+  rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, x0,
+              info + GLL_INFO_CG_ITERS_FWD, (float*)(info + GLL_INFO_CG_RESID_FWD), nullptr, ws, ws_bytes, st, barrier, nullptr);
   if (rc) return rc;
 
   RefineParams P;
-  P.row_ptr = (int*)(S + L.row_ptr);
-  P.col = (int*)(S + L.col);
-  P.w = (float*)(S + L.w);
+  P.row_ptr = G.row_ptr;
+  P.col = G.col;
+  P.w = G.w;
   P.Y = Y;
   P.r_out = B.r;
   P.partial = B.partial;
   P.colnorm = B.colnorm;
   P.scale = B.scale;
   P.ticket = B.ticket;
-  P.info = sinfo;
+  P.info = info;
   P.n = n;
   P.k_lab = k_lab;
   P.m = m;
@@ -296,15 +289,15 @@ int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l,
       laplace_refine_kernel<<<grid, LR_THREADS, 0, st>>>(P);
       GLL_LAUNCH_CHECK();
     }
-    rc = cg_run(uu_ptr, uu_col, uu_val, diag, rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, corr, B.round_iters + r, nullptr,
-                nullptr, ws, ws_bytes, st, barrier, &io);
+    rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, corr, B.round_iters + r,
+                nullptr, nullptr, ws, ws_bytes, st, barrier, &io);
     if (rc) return rc;
   }
   {
     GLL_PROF(KID_LAPLACE_FINISH, st);
     laplace_finish_kernel<<<ceil_div(m, LR_THREADS), LR_THREADS, 0, st>>>(pred, corr, m, l, lp, labels, targets,
                                                                            (unsigned long long*)correct_out, B.scale, B.round_iters,
-                                                                           GLL_LAPLACE_ROUNDS, sinfo);
+                                                                           GLL_LAPLACE_ROUNDS, info);
     GLL_LAUNCH_CHECK();
   }
   return GLL_OK;

@@ -17,17 +17,15 @@ Forward only (evaluation); CUDA tensors only; needs at least 256 base rows.
 """
 from __future__ import annotations
 
-import os
-
 import torch
 
 from . import _lib
 from ._lib import lib
-from .GLL import K_NEIGHBOURS, _bytes, _cg_maxit, _cg_tol, _require_cuda, _stream_ptr
+from .GLL import K_NEIGHBOURS, GraphStages, _bytes, _cg_maxit, _cg_tol, _require_cuda, _stream_ptr, as_features, parse_epsilon, pred_dtype
 
 
 def _uu_hint(k: int, m: int, n: int) -> float:
-    """gll_forward's own number, in its own float32 arithmetic (api.cu): 1.2f * (k - 1) * m / n."""
+    """gll_forward's sparsity hint, uu_degree_hint in csrc/api.cu, in the same float32 arithmetic: 1.2f * (k - 1) * m / n."""
     import numpy as np
 
     return float(np.float32(1.2) * np.float32(k - 1) * np.float32(m) / np.float32(n))
@@ -37,9 +35,8 @@ class BaseSetEvaluator:
     def __init__(self, base_features: torch.Tensor, label_matrix: torch.Tensor, tau: float = 0.0, epsilon="auto",
                  k: int = K_NEIGHBOURS):
         _require_cuda(base_features, "base features")
-        if isinstance(epsilon, str) and epsilon != "auto":
-            raise ValueError("epsilon must be a float or 'auto'")
-        self.base = base_features.detach().to(torch.float32).contiguous()
+        parse_epsilon(epsilon)
+        self.base = as_features(base_features)
         self.Y = label_matrix.detach().to(device=self.base.device, dtype=torch.float32).contiguous()
         self.n_base, self.d = self.base.shape
         if self.Y.shape[0] != self.n_base:
@@ -72,49 +69,25 @@ class BaseSetEvaluator:
         dev = X.device
         n, d, k, l, k_lab = X.shape[0], self.d, self.k, self.l, self.n_base
         m = n - k_lab
-        lp = lib.gll_padded_classes(l)
-        emax = lib.gll_max_edges(n, k)
-        i32, f32 = torch.int32, torch.float32
         s = _stream_ptr(dev)
-        eps_auto = isinstance(self.epsilon, str)
         with torch.cuda.device(dev):
-            info = torch.zeros(_lib.INFO_WORDS, dtype=i32, device=dev)
-            knn_idx = torch.empty((n, k), dtype=i32, device=dev)
-            knn_dist = torch.empty((n, k), dtype=f32, device=dev)
+            info = torch.zeros(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
+            knn_idx = torch.empty((n, k), dtype=torch.int32, device=dev)
+            knn_dist = torch.empty((n, k), dtype=torch.float32, device=dev)
             wsb = max(lib.gll_knn_cached_workspace_bytes(n, d, k, k_lab), lib.gll_graph_workspace_bytes(n, k),
                       lib.gll_weights_workspace_bytes(n, k), lib.gll_cg_workspace_bytes(m, l))
             ws = _bytes(wsb, dev)
             _lib.check(lib.gll_knn_cached(X.data_ptr(), n, d, k, k_lab, self.cache.data_ptr(), knn_idx.data_ptr(), knn_dist.data_ptr(),
                                           info.data_ptr(), ws.data_ptr(), wsb, s), "gll_knn_cached")
-            row_ptr = torch.empty(n + 1, dtype=i32, device=dev)
-            col = torch.empty(emax, dtype=i32, device=dev)
-            dist = torch.empty(emax, dtype=f32, device=dev)
-            _lib.check(lib.gll_graph_build(knn_idx.data_ptr(), knn_dist.data_ptr(), n, k, row_ptr.data_ptr(), col.data_ptr(),
-                                           dist.data_ptr(), info.data_ptr(), ws.data_ptr(), wsb, s), "gll_graph_build")
-            eps = torch.empty(n, dtype=f32, device=dev)
-            kappa = torch.empty(n, dtype=i32, device=dev)
-            w = torch.empty(emax, dtype=f32, device=dev)
-            deg = torch.empty(n, dtype=f32, device=dev)
-            uu_ptr = torch.empty(m + 1, dtype=i32, device=dev)
-            uu_col = torch.empty(emax, dtype=i32, device=dev)
-            uu_val = torch.empty(emax, dtype=f32, device=dev)
-            diag = torch.empty(m, dtype=f32, device=dev)
-            rhs = torch.empty((m, lp), dtype=f32, device=dev)
-            ut = torch.empty((n, lp), dtype=f32, device=dev)
-            _lib.check(lib.gll_edge_weights(knn_idx.data_ptr(), knn_dist.data_ptr(), row_ptr.data_ptr(), col.data_ptr(),
-                                            dist.data_ptr(), self.Y.data_ptr(), n, k, l, k_lab, int(eps_auto),
-                                            0.0 if eps_auto else float(self.epsilon), self.tau, eps.data_ptr(), kappa.data_ptr(),
-                                            w.data_ptr(), deg.data_ptr(), uu_ptr.data_ptr(), uu_col.data_ptr(), uu_val.data_ptr(),
-                                            diag.data_ptr(), rhs.data_ptr(), ut.data_ptr(), info.data_ptr(), ws.data_ptr(), wsb, s),
-                       "gll_edge_weights")
-            u = ut[k_lab:]
+            g = GraphStages(knn_idx, knn_dist, self.Y, n, self.tau, self.epsilon, info, ws)
+            u = g.ut[k_lab:]
             # the same sparsity hint as gll_forward passes, so that the same solver kernel runs: bit-identical predictions
-            _lib.check(lib.gll_cg_solve_hint(uu_ptr.data_ptr(), uu_col.data_ptr(), uu_val.data_ptr(), diag.data_ptr(), rhs.data_ptr(), m,
-                                             l, _cg_tol(), _cg_maxit(), u.data_ptr(), info[_lib.INFO_CG_ITERS_FWD:].data_ptr(),
-                                             info[_lib.INFO_CG_RESID_FWD:].data_ptr(), info[_lib.INFO_STATUS:].data_ptr(),
-                                             ws.data_ptr(), wsb, s, _uu_hint(k, m, n)), "gll_cg_solve")
-            pred64 = os.environ.get("GLL_B200_PRED_DTYPE", "float64") != "float32"
-            pred = torch.empty((m, l), dtype=torch.float64 if pred64 else f32, device=dev)
-            _lib.check(lib.gll_unpack_pred(u.data_ptr(), m, l, pred.data_ptr(), int(pred64), s), "gll_unpack_pred")
+            _lib.check(lib.gll_cg_solve_hint(g.uu_ptr.data_ptr(), g.uu_col.data_ptr(), g.uu_val.data_ptr(), g.diag.data_ptr(),
+                                             g.rhs.data_ptr(), m, l, _cg_tol(), _cg_maxit(), u.data_ptr(),
+                                             info[_lib.INFO_CG_ITERS_FWD:].data_ptr(), info[_lib.INFO_CG_RESID_FWD:].data_ptr(),
+                                             info[_lib.INFO_STATUS:].data_ptr(), ws.data_ptr(), wsb, s, _uu_hint(k, m, n)),
+                       "gll_cg_solve")
+            pred = torch.empty((m, l), dtype=pred_dtype(), device=dev)
+            _lib.check(lib.gll_unpack_pred(u.data_ptr(), m, l, pred.data_ptr(), int(pred.dtype == torch.float64), s), "gll_unpack_pred")
         self.info, self.knn_idx, self.knn_dist = info, knn_idx, knn_dist
         return pred

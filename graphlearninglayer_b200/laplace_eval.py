@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .GLL import _bytes, _cg_maxit, _check_status, _require_cuda, _stream_ptr
+from .GLL import _bytes, _cg_maxit, _check_status, _require_cuda, _stream_ptr, as_features, decode_info, parse_epsilon
 from ._lib import lib
 
 __all__ = ["laplace_learning", "LaplaceResult", "last_eval_info"]
@@ -52,12 +52,7 @@ def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int 
         raise ValueError("need at least one class column and one feature")
     if not (2 <= k <= 64) or k > n or (k > 33 and n < 256):
         raise ValueError(f"k must be in [2, 64] and <= n, with n >= 256 when k > 33 (k={k}, n={n})")
-    if isinstance(epsilon, str):
-        if epsilon != "auto":
-            raise ValueError("epsilon must be a float or 'auto'")
-        eps_auto, eps_fixed = 1, 0.0
-    else:
-        eps_auto, eps_fixed = 0, float(epsilon)
+    eps_auto, eps_fixed = parse_epsilon(epsilon)
     if not tol > 0:
         raise ValueError("tol must be > 0")
     m = n - k_lab
@@ -65,10 +60,7 @@ def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int 
         raise ValueError(f"targets must be ({m},), got {tuple(targets.shape)}")
     _require_cuda(features, "features")
     dev = features.device
-    Xc = features.detach()
-    if Xc.dtype != torch.float32:
-        Xc = Xc.float()
-    Xc = Xc.contiguous()
+    Xc = as_features(features)
     Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
     tg = None
     if targets is not None:
@@ -100,8 +92,6 @@ def last_eval_info() -> dict:
     f = v.view(np.float32)
     u = v.view(np.uint32)
     round_iters = [int((u[_lib.INFO_LAPLACE_ROUND_ITERS + r // 2] >> (16 * (r % 2))) & 0xFFFF) for r in range(4)]
-    return dict(status=int(v[_lib.INFO_STATUS]), nnz=int(v[_lib.INFO_NNZ]), nnz_uu=int(v[_lib.INFO_NNZ_UU]),
-                cg_iters_first=int(v[_lib.INFO_CG_ITERS_FWD]), knn_fallback_rows=int(v[_lib.INFO_KNN_FALLBACK_ROWS]),
-                rounds=int(v[_lib.INFO_LAPLACE_ROUNDS]), cg_iters_correction=int(v[_lib.INFO_LAPLACE_CG_ITERS]),
-                round_iters=round_iters, resid_first=float(f[_lib.INFO_LAPLACE_RESID0]),
+    return dict(decode_info(v), cg_iters_first=int(v[_lib.INFO_CG_ITERS_FWD]), rounds=int(v[_lib.INFO_LAPLACE_ROUNDS]),
+                cg_iters_correction=int(v[_lib.INFO_LAPLACE_CG_ITERS]), round_iters=round_iters, resid_first=float(f[_lib.INFO_LAPLACE_RESID0]),
                 resid=float(f[_lib.INFO_LAPLACE_RESID]))

@@ -30,7 +30,7 @@ import torch.distributed as dist
 
 from . import _lib
 from ._lib import lib
-from .GLL import K_NEIGHBOURS, _bytes, _cg_maxit, _cg_tol, _require_cuda, _stream_ptr
+from .GLL import K_NEIGHBOURS, GraphStages, _bytes, _cg_maxit, _cg_tol, _require_cuda, _stream_ptr, as_features, decode_info, pred_dtype
 
 ROW_ALIGN = 128  # row blocks start on a tensor-core row tile
 
@@ -93,35 +93,18 @@ class _Comm:
                 parts[r].copy_(total)
 
 
-class _Graph:
-    pass
-
-
 def _forward(X: torch.Tensor, Y: torch.Tensor, tau: float, epsilon, comm: _Comm, k: int = K_NEIGHBOURS,
              cg_partition: str = "columns"):
     dev = X.device
     n, d = X.shape
-    k_lab, l = Y.shape
-    m = n - k_lab
-    i32, f32 = torch.int32, torch.float32
     s = _stream_ptr(dev)
-    g = _Graph()
-    g.n, g.d, g.k, g.l, g.k_lab, g.m = n, d, k, l, k_lab, m
-    g.cg_partition = cg_partition
-    g.lp = lib.gll_padded_classes(l)
-    emax = lib.gll_max_edges(n, k)
-    eps_auto = isinstance(epsilon, str)
-    if eps_auto and epsilon != "auto":
-        raise ValueError("epsilon must be a float or 'auto'")
-    g.eps_auto = int(eps_auto)
-    info = torch.zeros(_lib.INFO_WORDS, dtype=i32, device=dev)
-    g.info = info
+    info = torch.zeros(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
 
     # ---- K1, rows: every rank searches its block of nodes against all n columns ----
     _, _, per = row_block(n, 0, comm.world)
     idx_parts, dist_parts = {}, {}
-    knn_idx = torch.empty((comm.world * per, k), dtype=i32, device=dev)
-    knn_dist = torch.empty((comm.world * per, k), dtype=f32, device=dev)
+    knn_idx = torch.empty((comm.world * per, k), dtype=torch.int32, device=dev)
+    knn_dist = torch.empty((comm.world * per, k), dtype=torch.float32, device=dev)
     for r in comm.ranks:
         lo, hi, _ = row_block(n, r, comm.world)
         if hi > lo:
@@ -134,39 +117,18 @@ def _forward(X: torch.Tensor, Y: torch.Tensor, tau: float, epsilon, comm: _Comm,
     if comm.real:  # (emulation wrote every block into the shared arrays already)
         knn_idx = torch.cat(comm.all_gather(idx_parts, knn_idx), 0)
         knn_dist = torch.cat(comm.all_gather(dist_parts, knn_dist), 0)
-    g.knn_idx, g.knn_dist = knn_idx, knn_dist  # rows >= n are padding and never read
 
-    # ---- K2, K3 replicated ----
-    g.row_ptr = torch.empty(n + 1, dtype=i32, device=dev)
-    g.col = torch.empty(emax, dtype=i32, device=dev)
-    g.dist = torch.empty(emax, dtype=f32, device=dev)
-    wsb = max(lib.gll_graph_workspace_bytes(n, k), lib.gll_weights_workspace_bytes(n, k))
-    ws = _bytes(wsb, dev)
-    _lib.check(lib.gll_graph_build(knn_idx.data_ptr(), knn_dist.data_ptr(), n, k, g.row_ptr.data_ptr(), g.col.data_ptr(),
-                                   g.dist.data_ptr(), info.data_ptr(), ws.data_ptr(), wsb, s), "gll_graph_build")
-    g.eps = torch.empty(n, dtype=f32, device=dev)
-    g.kappa = torch.empty(n, dtype=i32, device=dev)
-    g.w = torch.empty(emax, dtype=f32, device=dev)
-    g.deg = torch.empty(n, dtype=f32, device=dev)
-    g.uu_ptr = torch.empty(m + 1, dtype=i32, device=dev)
-    g.uu_col = torch.empty(emax, dtype=i32, device=dev)
-    g.uu_val = torch.empty(emax, dtype=f32, device=dev)
-    g.diag = torch.empty(m, dtype=f32, device=dev)
-    rhs = torch.empty((m, g.lp), dtype=f32, device=dev)
-    g.ut = torch.zeros((n, g.lp), dtype=f32, device=dev)
-    _lib.check(lib.gll_edge_weights(knn_idx.data_ptr(), knn_dist.data_ptr(), g.row_ptr.data_ptr(), g.col.data_ptr(),
-                                    g.dist.data_ptr(), Y.data_ptr(), n, k, l, k_lab, g.eps_auto,
-                                    0.0 if eps_auto else float(epsilon), float(tau), g.eps.data_ptr(), g.kappa.data_ptr(),
-                                    g.w.data_ptr(), g.deg.data_ptr(), g.uu_ptr.data_ptr(), g.uu_col.data_ptr(),
-                                    g.uu_val.data_ptr(), g.diag.data_ptr(), rhs.data_ptr(), g.ut.data_ptr(), info.data_ptr(),
-                                    ws.data_ptr(), wsb, s), "gll_edge_weights")
+    # ---- K2, K3 replicated (kNN rows >= n are padding and never read) ----
+    g = GraphStages(knn_idx, knn_dist, Y, n, tau, epsilon, info, zero_ut=True)
+    g.d, g.cg_partition = d, cg_partition
+    rhs, g.rhs = g.rhs, None  # the backward packs its own right-hand side
 
     # ---- K4, columns: each rank solves its block of class columns ----
-    g.iters_fwd = torch.zeros(comm.world, dtype=i32, device=dev)
-    _solve(g, rhs, g.ut[k_lab:], _cg_tol(), comm, g.iters_fwd)
-    pred64 = os.environ.get("GLL_B200_PRED_DTYPE", "float64") != "float32"
-    pred = torch.empty((m, l), dtype=torch.float64 if pred64 else f32, device=dev)
-    _lib.check(lib.gll_unpack_pred(g.ut[k_lab:].data_ptr(), m, l, pred.data_ptr(), int(pred64), s), "gll_unpack_pred")
+    g.iters_fwd = torch.zeros(comm.world, dtype=torch.int32, device=dev)
+    _solve(g, rhs, g.ut[g.k_lab:], _cg_tol(), comm, g.iters_fwd)
+    pred = torch.empty((g.m, g.l), dtype=pred_dtype(), device=dev)
+    _lib.check(lib.gll_unpack_pred(g.ut[g.k_lab:].data_ptr(), g.m, g.l, pred.data_ptr(), int(pred.dtype == torch.float64), s),
+               "gll_unpack_pred")
     return pred, g
 
 
@@ -425,7 +387,7 @@ class ShardedLaplaceLearning(torch.autograd.Function):
     @staticmethod
     def forward(ctx, X, label_matrix, tau=0, epsilon="auto", group=None, emulate=0, cg_partition=None):
         _require_cuda(X, "features")
-        Xc = X.detach().float().contiguous()
+        Xc = as_features(X)
         Y = label_matrix.detach().to(device=X.device, dtype=torch.float32).contiguous()
         if not (0 < Y.shape[0] < Xc.shape[0]):
             raise ValueError("need 0 < k_lab < n; labeled rows come first (GLL.py:11)")
@@ -458,10 +420,8 @@ def last_info() -> dict:
     g = _last_graph
     if g is None:
         return {}
-    v = g.info.cpu().numpy()
     solve_ms = [a.elapsed_time(b) for a, b in getattr(g, "solve_events", [])]
-    return dict(cg_partition=g.cg_partition, cg_solve_ms=solve_ms,
-                status=int(v[_lib.INFO_STATUS]), nnz=int(v[_lib.INFO_NNZ]), nnz_uu=int(v[_lib.INFO_NNZ_UU]),
+    return dict(decode_info(g.info.cpu().numpy()), cg_partition=g.cg_partition, cg_solve_ms=solve_ms,
                 cg_iters_fwd=int(g.iters_fwd.max().item()),
                 cg_iters_bwd=int(g.iters_bwd.max().item()) if hasattr(g, "iters_bwd") else 0,
-                knn_fallback_rows=int(v[_lib.INFO_KNN_FALLBACK_ROWS]), cg_resid_fwd=float("nan"), cg_resid_bwd=float("nan"))
+                cg_resid_fwd=float("nan"), cg_resid_bwd=float("nan"))

@@ -42,11 +42,12 @@ extern "C" {
 #define GLL_INFO_KNN_FALLBACK_ROWS 5
 #define GLL_INFO_CG_RESID_FWD 6 /* float bits: max_c ||r_c||_2 at exit */
 #define GLL_INFO_CG_RESID_BWD 7
-/* gll_laplace_eval only (slots 12-13 are the on-chip CG's barrier words in every call) */
+/* gll_laplace_eval only */
 #define GLL_INFO_LAPLACE_ROUNDS 8       /* refinement rounds that ran a correction solve */
 #define GLL_INFO_LAPLACE_CG_ITERS 9     /* correction-CG iterations, all rounds */
 #define GLL_INFO_LAPLACE_RESID 10       /* float bits: max_c ||M r_c||_2 at the last refinement round */
 #define GLL_INFO_LAPLACE_RESID0 11      /* float bits: the same after the initial solve */
+#define GLL_INFO_CG_BARRIER 12          /* two words, every fused call: the on-chip CG's grid barrier (zeroed with info, rewound by the kernel) */
 #define GLL_INFO_LAPLACE_ROUND_ITERS 14 /* two words: correction-CG iterations of round r in bits [16 (r % 2), +16) of word 14 + r / 2 */
 #define GLL_INFO_WORDS 16
 
