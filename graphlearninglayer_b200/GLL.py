@@ -2,6 +2,7 @@
 (``/root/reference/GLL.py``; ``utils.py:25`` imports all three), backed by libgll_b200.so.
 
     LaplaceLearningSparseHard.apply(X, label_matrix, tau=0, epsilon='auto')   GLL.py:10-177
+    LaplaceLearningSparseHardBatched.apply(X, label_matrix, tau, epsilon)    B independent graphs, X (B, n, d)
     knn_sym_dist(data, k=25, epsilon='auto')                                  GLL.py:180-244
     stable_conjgrad(A, b, x0=None, max_iter=1e5, tol=1e-10)                   GLL.py:247-276
 
@@ -33,7 +34,7 @@ from ._lib import lib
 
 K_NEIGHBOURS = 25  # hard-coded in the reference at GLL.py:27
 
-__all__ = ["LaplaceLearningSparseHard", "LaplaceLearningSparseHardNormalized", "knn_sym_dist", "stable_conjgrad", "last_info"]
+__all__ = ["LaplaceLearningSparseHard", "LaplaceLearningSparseHardNormalized", "LaplaceLearningSparseHardBatched", "knn_sym_dist", "stable_conjgrad", "last_info"]
 
 
 def _env_float(name: str, default: float) -> float:
@@ -286,6 +287,92 @@ class LaplaceLearningSparseHardNormalized(torch.autograd.Function):
         if dx.dtype != ctx.x_dtype:
             dx = dx.to(ctx.x_dtype)
         return dx, None, None, None
+
+
+def labeled_first(X: torch.Tensor, k_lab: int) -> torch.Tensor:
+    """(B, n, d) -> (B n, d) in the batched layer's row order: all graphs' labeled rows, then all graphs' unlabeled rows."""
+    d = X.shape[2]
+    return torch.cat((X[:, :k_lab].reshape(-1, d), X[:, k_lab:].reshape(-1, d)))
+
+
+def natural_order(Xg: torch.Tensor, B: int, k_lab: int) -> torch.Tensor:
+    """Inverse of labeled_first: (B n, d) -> (B, n, d)."""
+    d = Xg.shape[1]
+    m = Xg.shape[0] // B - k_lab
+    return torch.cat((Xg[:B * k_lab].reshape(B, k_lab, d), Xg[B * k_lab:].reshape(B, m, d)), dim=1)
+
+
+def _batched_forward_impl(X: torch.Tensor, label_matrix: torch.Tensor, tau, epsilon, k: int = K_NEIGHBOURS):
+    if X.dim() != 3:
+        raise ValueError("features must be (B, n, d)")
+    B, n, d = X.shape
+    if label_matrix.dim() != 3 or label_matrix.shape[0] != B:
+        raise ValueError(f"label_matrix must be (B, k_lab, l) with B = {B}, got {tuple(label_matrix.shape)}")
+    _, k_lab, l = label_matrix.shape
+    if k_lab < 1 or n - k_lab < 1 or l < 1 or d < 1:
+        raise ValueError(f"need 1 <= k_lab < n, l >= 1 and d >= 1 (k_lab={k_lab}, n={n}, l={l}, d={d}); labeled rows come first")
+    if n < k:
+        raise ValueError(f"every graph needs at least k={k} nodes, got n={n}")
+    eps_auto, eps_fixed = parse_epsilon(epsilon)
+    _require_cuda(X, "features")
+    dev = X.device
+    Xc = as_features(X)
+    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()  # int64 one-hot allowed
+    st = _State()
+    st.layout = _lib.state_layout(B * n, k, l, B * k_lab)
+    st.n, st.d, st.k, st.l, st.k_lab, st.eps_auto = B * n, d, k, l, B * k_lab, eps_auto
+    with torch.cuda.device(dev):
+        st.buf = _bytes(st.layout.total, dev)
+        ws_bytes = lib.gll_batched_workspace_bytes(B, n, d, k, l, k_lab)
+        ws = _bytes(ws_bytes, dev)
+        pred = torch.empty((B, n - k_lab, l), dtype=pred_dtype(), device=dev)
+        rc = lib.gll_forward_batched(Xc.data_ptr(), Y.data_ptr(), B, n, d, k, l, k_lab, eps_auto, eps_fixed, float(tau), _cg_tol(),
+                                     _cg_maxit(), st.buf.data_ptr(), pred.data_ptr(), int(pred.dtype == torch.float64), ws.data_ptr(),
+                                     ws_bytes, _stream_ptr(dev))
+        _lib.check(rc, "gll_forward_batched")
+        Xg = labeled_first(Xc, k_lab)  # the backward's rows, in the order of the block-diagonal graph
+    global _last_info
+    _last_info = st.view("info", torch.int32, _lib.INFO_WORDS)
+    _check_status(_last_info, "forward")
+    return pred, st, Xg
+
+
+class LaplaceLearningSparseHardBatched(torch.autograd.Function):
+    """B independent graphs of the same shape in one call: ``LaplaceLearningSparseHard`` applied to each ``X[b]`` with
+    ``label_matrix[b]``.
+
+    forward(X, label_matrix, tau=0, epsilon='auto'): X is (B, n, d) with each graph's k_lab labeled rows first,
+    label_matrix (B, k_lab, l) one-hot (float32 or int64); returns (B, n - k_lab, l) in the layer's prediction dtype.
+    backward gives dX (B, n, d) in X's dtype.
+
+    The B graphs are solved as one block-diagonal graph: the kNN search never crosses graphs, and the kNN lists, the graph,
+    epsilon, the weights and the degrees are bit-identical to per-graph calls.  One multi-right-hand-side CG solves all B
+    systems, so its step lengths are shared across graphs and each class column stops when its residual over all graphs
+    meets the tolerance (which bounds every graph's residual): predictions and gradients agree with per-graph calls to the
+    solver tolerance, not bit for bit when B > 1, and iteration counts in last_info() are the batch's.  B = 1 is
+    bit-identical to LaplaceLearningSparseHard.
+    """
+
+    @staticmethod
+    def forward(ctx, X, label_matrix, tau=0, epsilon="auto"):
+        pred, st, Xg = _batched_forward_impl(X, label_matrix, tau, epsilon)
+        ctx.gll_state = st
+        ctx.x_dtype = X.dtype
+        ctx.batch = (X.shape[0], label_matrix.shape[1])
+        ctx.save_for_backward(Xg)
+        ctx.set_materialize_grads(True)
+        return pred
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_output):
+        (Xg,) = ctx.saved_tensors
+        B, k_lab = ctx.batch
+        dXg = _backward_impl(ctx.gll_state, Xg, grad_output.reshape(-1, grad_output.shape[-1]))
+        dX = natural_order(dXg, B, k_lab)
+        if dX.dtype != ctx.x_dtype:
+            dX = dX.to(ctx.x_dtype)
+        return dX, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------------------

@@ -2,12 +2,13 @@
 
     from graphlearninglayer_b200 import LaplaceLearningSparseHard, knn_sym_dist, stable_conjgrad
     from graphlearninglayer_b200 import laplace_learning        # utils.laplace on GPU features, no host round trip
+    from graphlearninglayer_b200 import LaplaceLearningSparseHardBatched  # B independent graphs (B, n, d) in one call
 
 The names resolve lazily so that ``python -m graphlearninglayer_b200.build`` can run before the shared library
 exists; the first access loads libgll_b200.so through ctypes and fails loudly if it is missing or stale.  There is no
 CPU or PyTorch fallback.
 """
-__all__ = ["LaplaceLearningSparseHard", "LaplaceLearningSparseHardNormalized", "knn_sym_dist", "stable_conjgrad", "last_info", "GLL",
+__all__ = ["LaplaceLearningSparseHard", "LaplaceLearningSparseHardNormalized", "LaplaceLearningSparseHardBatched", "knn_sym_dist", "stable_conjgrad", "last_info", "GLL",
            "GraphedStep", "BaseSetEvaluator", "laplace_learning", "LaplaceResult"]
 _ELSEWHERE = {"GraphedStep": ".graphed", "BaseSetEvaluator": ".evalcache", "laplace_learning": ".laplace_eval",
               "LaplaceResult": ".laplace_eval"}

@@ -110,6 +110,12 @@ def _load():
     sig("gll_forward", i32, [vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, f32, i32, vp, vp, i32, vp, sz, vp])
     sig("gll_backward", i32, [vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, i32, vp, vp, vp, sz, vp])
     sig("gll_backward_scaled", i32, [vp, vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, f32, i32, vp, vp, vp, sz, vp])
+    ip, llp = C.POINTER(C.c_int), C.POINTER(C.c_longlong)
+    sig("gll_knn_segments_workspace_bytes", sz, [i32, i32, i32, ip, i32])
+    sig("gll_knn_segments", i32, [vp, i32, i32, i32, ip, i32, vp, vp, vp, vp, sz, vp])
+    sig("gll_knn_segments_units", None, [i32, i32, ip, i32, llp, llp])
+    sig("gll_batched_workspace_bytes", sz, [i32, i32, i32, i32, i32, i32])
+    sig("gll_forward_batched", i32, [vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, f32, f32, i32, vp, vp, i32, vp, sz, vp])
     sig("gll_laplace_eval_workspace_bytes", sz, [i32, i32, i32, i32, i32])
     sig("gll_laplace_eval", i32, [vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp, vp, vp, vp, sz, vp])
     return lib
@@ -129,7 +135,8 @@ EXPORTS = ["gll_last_error", "gll_version", "gll_device_sm_count", "gll_kernel_c
            "gll_cg_rows_update_p2p", "gll_csr_residual_f64", "gll_normalize_rows",
            "gll_normalize_rows_backward", "gll_debug_gram_tile", "gll_base_cache_bytes", "gll_base_cache_workspace_bytes",
            "gll_base_cache_build", "gll_knn_cached_workspace_bytes", "gll_knn_cached", "gll_laplace_eval_workspace_bytes",
-           "gll_laplace_eval"]
+           "gll_laplace_eval", "gll_knn_segments_workspace_bytes", "gll_knn_segments", "gll_knn_segments_units",
+           "gll_batched_workspace_bytes", "gll_forward_batched"]
 
 
 def check(rc: int, what: str) -> None:
@@ -142,6 +149,12 @@ def state_layout(n: int, k: int, l: int, k_lab: int) -> Layout:
     L = Layout()
     check(lib.gll_state_layout(n, k, l, k_lab, C.byref(L)), "gll_state_layout")
     return L
+
+
+def seg_ptr_array(seg_ptr) -> "C.Array":
+    """Host int32 array of segment offsets for gll_knn_segments* (seg_ptr_host)."""
+    v = [int(x) for x in seg_ptr]
+    return (C.c_int * len(v))(*v)
 
 
 def launch_count(kernel_id: int = -1) -> int:

@@ -2,6 +2,7 @@
 #include <stdarg.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <vector>
@@ -70,7 +71,8 @@ std::atomic<int> g_prof_on{0};
 std::atomic<long long> g_launches[KID_COUNT];
 const char* const g_kernel_names[KID_COUNT] = {
     "sqnorm", "knn_gram_topk_simt", "knn_gram_topk_tcgen05", "knn_rerank", "knn_fallback", "graph_build", "edge_weights",
-    "cg_persistent", "pack_unpack", "edge_grad", "row_gather", "convert", "cg_rows", "laplace_refine", "laplace_finish"};
+    "cg_persistent", "pack_unpack", "edge_grad", "row_gather", "convert", "cg_rows", "laplace_refine", "laplace_finish",
+    "knn_segment_setup", "batch_reorder"};
 }  // namespace
 
 ProfScope::ProfScope(int id_, cudaStream_t st_) : id(id_), st(st_), slot(nullptr) {
@@ -212,6 +214,24 @@ __global__ void unpack_pred_kernel(const float* __restrict__ u, int m, int l, in
     ((double*)pred)[t] = (double)v;
   else
     ((float*)pred)[t] = v;
+}
+
+// Batched layer: natural order (graph b, row t) -> the block-diagonal graph's order, all graphs' labeled rows first, then all
+// graphs' unlabeled rows, each graph's rows in their own order
+__device__ __forceinline__ int labeled_first_row(int r, int n, int k_lab, int B) {
+  const int b = r / n, t = r - b * n;
+  return (t < k_lab) ? b * k_lab + t : B * k_lab + b * (n - k_lab) + (t - k_lab);
+}
+
+// kNN lists of the stacked graphs in natural order -> rows and indices in labeled-first order
+__global__ void knn_to_labeled_first_kernel(const int* __restrict__ idx_in, const float* __restrict__ dist_in, int B, int n, int k,
+                                            int k_lab, int* __restrict__ idx_out, float* __restrict__ dist_out) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (long long)B * n * k) return;
+  const int r = (int)(t / k), s = (int)(t - (long long)r * k);
+  const size_t o = (size_t)labeled_first_row(r, n, k_lab, B) * k + s;
+  idx_out[o] = labeled_first_row(idx_in[t], n, k_lab, B);
+  dist_out[o] = dist_in[t];
 }
 
 __global__ void pack_columns_kernel(const float* __restrict__ src, int rows, int lp_src, int c0, int cnt, float* __restrict__ dst,
@@ -623,11 +643,10 @@ int gll_pack_grad(const void* grad_out, int grad_is_f64, int m, int l, float* rh
   return pack_grad(grad_out, grad_is_f64, m, l, padded_classes(l), rhs, (cudaStream_t)stream);
 }
 
-// the state's arrays and the workspace check of gll_forward and gll_backward_scaled
-static int driver_bufs(int n, int d, int k, int l, int k_lab, void* state, size_t workspace_bytes, GraphBufs* B) {
+// the state's arrays and the workspace check of the fused drivers (need: the driver's workspace size)
+static int driver_bufs(int n, int k, int l, int k_lab, void* state, size_t need, size_t workspace_bytes, GraphBufs* B) {
   gll_layout L;
   if (gll_state_layout(n, k, l, k_lab, &L)) return GLL_ERR_ARG;
-  const size_t need = gll_workspace_bytes(n, d, k, l, k_lab);
   if (workspace_bytes < need) {
     set_error("workspace too small: %zu < %zu", workspace_bytes, need);
     return GLL_ERR_WORKSPACE;
@@ -636,24 +655,96 @@ static int driver_bufs(int n, int d, int k, int l, int k_lab, void* state, size_
   return GLL_OK;
 }
 
-int gll_forward(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
-                float tau, float cg_tol, int cg_max_iter, void* state, void* pred_out, int pred_is_f64, void* workspace,
-                size_t workspace_bytes, void* stream) {
-  GLL_REQUIRE(X && state && pred_out && workspace, "null pointer");
-  GraphBufs B;
-  int rc = driver_bufs(n, d, k, l, k_lab, state, workspace_bytes, &B);
-  if (rc) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
+// gll_forward after the kNN search: graph, weights and the unlabeled system from B.knn_idx / B.knn_dist, then the CG solve
+static int forward_solve(const GraphBufs& B, const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau,
+                         float cg_tol, int cg_max_iter, void* pred_out, int pred_is_f64, void* workspace, size_t workspace_bytes,
+                         cudaStream_t st) {
   const int m = n - k_lab, lp = padded_classes(l);
-  GLL_CUDA_CHECK(cudaMemsetAsync(B.info, 0, sizeof(int) * GLL_INFO_WORDS, st));
-  rc = knn_run(X, n, d, k, 0, n, B.knn_idx, B.knn_dist, B.info, workspace, workspace_bytes, st);
-  if (rc) return rc;
-  rc = graph_stages_run(B, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, 0, 6, workspace, workspace_bytes, st);
+  int rc = graph_stages_run(B, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, 0, 6, workspace, workspace_bytes, st);
   if (rc) return rc;
   const CgIo io = {nullptr, 0, pred_out, pred_is_f64, nullptr, 0, uu_degree_hint(n, k, m)};  // Pred (GLL.py:66) is written by the solver itself
   return cg_run(B.uu_ptr, B.uu_col, B.uu_val, B.diag, B.rhs, m, l, cg_tol, cg_max_iter, B.ut + (size_t)k_lab * lp,
                 B.info + GLL_INFO_CG_ITERS_FWD, (float*)(B.info + GLL_INFO_CG_RESID_FWD), B.info + GLL_INFO_STATUS, workspace,
                 workspace_bytes, st, (unsigned*)(B.info + GLL_INFO_CG_BARRIER), &io);
+}
+
+int gll_forward(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
+                float tau, float cg_tol, int cg_max_iter, void* state, void* pred_out, int pred_is_f64, void* workspace,
+                size_t workspace_bytes, void* stream) {
+  GLL_REQUIRE(X && state && pred_out && workspace, "null pointer");
+  GraphBufs B;
+  int rc = driver_bufs(n, k, l, k_lab, state, gll_workspace_bytes(n, d, k, l, k_lab), workspace_bytes, &B);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  GLL_CUDA_CHECK(cudaMemsetAsync(B.info, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  rc = knn_run(X, n, d, k, 0, n, B.knn_idx, B.knn_dist, B.info, workspace, workspace_bytes, st);
+  if (rc) return rc;
+  return forward_solve(B, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, cg_tol, cg_max_iter, pred_out, pred_is_f64, workspace,
+                       workspace_bytes, st);
+}
+
+size_t gll_knn_segments_workspace_bytes(int n, int d, int k, const int* seg_ptr_host, int nseg) {
+  return knn_seg_ws_bytes(n, d, k, seg_ptr_host, nseg);
+}
+
+int gll_knn_segments(const float* X, int n, int d, int k, const int* seg_ptr_host, int nseg, int* knn_idx, float* knn_dist, int* info,
+                     void* workspace, size_t workspace_bytes, void* stream) {
+  return knn_run_segments(X, n, d, k, seg_ptr_host, nseg, knn_idx, knn_dist, info, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+void gll_knn_segments_units(int n, int d, const int* seg_ptr_host, int nseg, long long* seg_units, long long* uniform_units) {
+  long long a = 0, b = 0;
+  knn_seg_units(n, d, seg_ptr_host, nseg, &a, &b);
+  if (seg_units) *seg_units = a;
+  if (uniform_units) *uniform_units = b;
+}
+
+// k <= 33: the segmented search serves one candidate round (gll_knn_segments)
+static bool batched_sizes_ok(int B, int n, int d, int k, int l, int k_lab) {
+  return B >= 1 && n >= k && k >= 2 && k <= 33 && d >= 1 && l >= 1 && k_lab >= 1 && k_lab < n && (long long)B * n <= 0x7fffffffLL;
+}
+
+static std::vector<int> uniform_segments(int B, int n) {
+  std::vector<int> seg(B + 1);
+  for (int b = 0; b <= B; ++b) seg[b] = b * n;
+  return seg;
+}
+
+size_t gll_batched_workspace_bytes(int B, int n, int d, int k, int l, int k_lab) {
+  if (!batched_sizes_ok(B, n, d, k, l, k_lab)) return 0;
+  const int N = B * n;
+  const std::vector<int> seg = uniform_segments(B, n);
+  const size_t lists = 2 * align_up(sizeof(int) * (size_t)N * k, 256);  // the search's lists in natural order
+  size_t b = lists + knn_seg_ws_bytes(N, d, k, seg.data(), B) + 256;
+  b = std::max(b, graph_weights_ws_bytes(N, k));
+  return std::max(b, cg_ws_bytes(N - B * k_lab, l));
+}
+
+int gll_forward_batched(const float* X, const float* Y, int B, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
+                        float tau, float cg_tol, int cg_max_iter, void* state, void* pred_out, int pred_is_f64, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  GLL_REQUIRE(X && Y && state && pred_out && workspace, "null pointer");
+  GLL_REQUIRE(batched_sizes_ok(B, n, d, k, l, k_lab), "need B >= 1, 2 <= k <= 33, n >= k, 1 <= k_lab < n, B n < 2^31");
+  const int N = B * n, K = B * k_lab;
+  GraphBufs G;
+  int rc = driver_bufs(N, k, l, K, state, gll_batched_workspace_bytes(B, n, d, k, l, k_lab), workspace_bytes, &G);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  GLL_CUDA_CHECK(cudaMemsetAsync(G.info, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  Carver cv(workspace, workspace_bytes);
+  int* idx = cv.take<int>((size_t)N * k);
+  float* dist = cv.take<float>((size_t)N * k);
+  char* kws = cv.take<char>(0);
+  const std::vector<int> seg = uniform_segments(B, n);
+  rc = knn_run_segments(X, N, d, k, seg.data(), B, idx, dist, G.info, kws, workspace_bytes - (size_t)(kws - (char*)workspace), st);
+  if (rc) return rc;
+  {
+    GLL_PROF(KID_BATCH_REORDER, st);
+    knn_to_labeled_first_kernel<<<ceil_div((long long)N * k, 256), 256, 0, st>>>(idx, dist, B, n, k, k_lab, G.knn_idx, G.knn_dist);
+  }
+  GLL_LAUNCH_CHECK();
+  return forward_solve(G, Y, N, k, l, K, eps_auto, eps_fixed, tau, cg_tol, cg_max_iter, pred_out, pred_is_f64, workspace, workspace_bytes,
+                       st);
 }
 
 int gll_backward(const float* X, const void* grad_out, int grad_is_f64, int n, int d, int k, int l, int k_lab, int eps_auto,
@@ -668,7 +759,7 @@ int gll_backward_scaled(const float* X, const void* grad_out, int grad_is_f64, c
                         size_t workspace_bytes, void* stream) {
   GLL_REQUIRE(X && grad_out && state && dX && workspace, "null pointer");
   GraphBufs B;
-  int rc = driver_bufs(n, d, k, l, k_lab, state, workspace_bytes, &B);
+  int rc = driver_bufs(n, k, l, k_lab, state, gll_workspace_bytes(n, d, k, l, k_lab), workspace_bytes, &B);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int m = n - k_lab, lp = padded_classes(l);

@@ -94,7 +94,10 @@ __device__ __forceinline__ float ordered_to_float(uint32_t u) {
 // ---- per-kernel launch counter and optional CUDA-event timing (gll_profile_* in the C ABI) ----
 enum KernelId {
   KID_SQNORM = 0, KID_GRAM_TOPK, KID_GRAM_TOPK_TC, KID_RERANK, KID_KNN_FALLBACK, KID_GRAPH, KID_WEIGHTS, KID_CG, KID_PACK,
-  KID_EDGE_GRAD, KID_ROW_GATHER, KID_CONVERT, KID_CG_ROWS, KID_LAPLACE_REFINE, KID_LAPLACE_FINISH, KID_COUNT
+  KID_EDGE_GRAD, KID_ROW_GATHER, KID_CONVERT, KID_CG_ROWS, KID_LAPLACE_REFINE, KID_LAPLACE_FINISH,
+  KID_KNN_SEGMENTS,   // segmented search: upload of seg_ptr and the unit table, per-row column windows
+  KID_BATCH_REORDER,  // batched layer: kNN lists to the labeled-first order of the block-diagonal graph
+  KID_COUNT
 };
 // RAII: counts the launch; when profiling is on, brackets it with two events on the launch stream.
 struct ProfScope {
@@ -116,6 +119,12 @@ int knn_base_cache_build(const float* Xbase, int n_base, int d, void* cache, voi
 size_t knn_cached_ws_bytes(int n, int d, int k, int n_base);
 int knn_run_cached(const float* X, int n, int d, int k, int n_base, const void* cache, int* knn_idx, float* knn_dist, int* info,
                    void* ws, size_t ws_bytes, cudaStream_t st);
+// segmented search: independent graphs as row segments, seg_ptr on the host (knn.cu)
+int knn_seg_check(int n, int d, int k, const int* seg_ptr, int nseg);
+size_t knn_seg_ws_bytes(int n, int d, int k, const int* seg_ptr, int nseg);
+int knn_run_segments(const float* X, int n, int d, int k, const int* seg_ptr, int nseg, int* knn_idx, float* knn_dist, int* info,
+                     void* ws, size_t ws_bytes, cudaStream_t st);
+void knn_seg_units(int n, int d, const int* seg_ptr, int nseg, long long* seg_units, long long* uniform_units);
 void knn_tc_set_trace(void* device_buf);  // debug timeline of the Gram kernel's CTA 0 (knn_tc.cu)
 int knn_debug_gram_tile(const float* X, int n, int d, int row_tile, int col_tile, float* acc_out, float* rscale_out, void* ws,
                         size_t ws_bytes, cudaStream_t st);

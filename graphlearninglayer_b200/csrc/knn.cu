@@ -17,6 +17,10 @@
 // reuses the rerank / fallback kernels through knn_finish().
 #include <math.h>
 #include <stdlib.h>
+#include <string.h>
+
+#include <algorithm>
+#include <vector>
 
 #include <cuda_fp16.h>
 #include <cuda_fp16.h>
@@ -241,10 +245,11 @@ __device__ __forceinline__ void store_tile_smem(float* __restrict__ S, int lds, 
 }
 
 // grid: (row tiles, column splits).  cand: [n][splits][KC] sorted keys.
-template <bool VEC4>
+// SEG: segmented search, row i only sees the columns win[i]; the splits divide the union of the row tile's windows.
+template <bool VEC4, bool SEG>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 knn_gemm_topk_kernel(const float* __restrict__ X, const float* __restrict__ sq, int n, int d, int cols_per_split,
-                     int splits, u64* __restrict__ cand, int row_begin, int row_end) {
+                     int splits, u64* __restrict__ cand, int row_begin, int row_end, const int2* __restrict__ win) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* As = reinterpret_cast<float*>(smem_raw);
   float* Bs = As + 2 * BK * LDS_A;
@@ -257,8 +262,13 @@ knn_gemm_topk_kernel(const float* __restrict__ X, const float* __restrict__ sq, 
   const int tx = tid & 15, ty = tid >> 4;
   const int row0 = row_begin + blockIdx.x * BM;
   const int split = blockIdx.y;
-  const int c_begin = split * cols_per_split;
-  const int c_end = min(n, c_begin + cols_per_split);
+  int t_lo = 0, t_hi = n;  // columns any row of the tile may see
+  if (SEG) {
+    t_lo = __ldg(&win[row0].x);
+    t_hi = __ldg(&win[min(row_end, row0 + BM) - 1].y);
+  }
+  const int c_begin = t_lo + split * cols_per_split;  // a split past the windows runs no tile and writes empty lists
+  const int c_end = min(t_hi, c_begin + cols_per_split);
 
   for (int t = tid; t < BM * KC; t += GEMM_THREADS) topk[t] = KEY_INF;
   for (int t = tid; t < BM; t += GEMM_THREADS) {
@@ -325,9 +335,15 @@ knn_gemm_topk_kernel(const float* __restrict__ X, const float* __restrict__ sq, 
       if (gi >= row_end) continue;
       float t = thr[rr];
       float sqi = __ldg(sq + gi);
+      int w_lo = 0, w_hi = n;
+      if (SEG) {
+        const int2 w = __ldg(win + gi);
+        w_lo = w.x;
+        w_hi = w.y;
+      }
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        if (gjv[j] < c_end && gjv[j] != gi) {
+        if (gjv[j] < c_end && gjv[j] != gi && (!SEG || (gjv[j] >= w_lo && gjv[j] < w_hi))) {
           float dist = fmaf(-2.f, acc[i][j], sqi + sqj[j]);
           if (dist < t) {
             int p = atomicAdd(&pcnt[rr], 1);
@@ -457,10 +473,9 @@ knn_rerank_kernel(const float* __restrict__ X, const float* __restrict__ sq, con
 
   u64 mine = KEY_INF;
   int splits = lay.stride;
-  if (lay.tc == 1) {  // lists written for this row's tile: one per CTA that touched it (knn_tc.cu)
-    const long long rt = (i - lay.row_begin) / lay.row_tile;
-    const int b0 = (int)(((rt * lay.col_tiles + 1) * lay.grid - 1) / lay.units);
-    const int b1 = (int)((((rt + 1) * lay.col_tiles) * lay.grid - 1) / lay.units);
+  if (lay.tc == 1 || lay.tc == 3) {  // lists written for this row's tile: one per CTA that touched it (knn_tc.cu)
+    int b0, b1;
+    cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
     splits = 2 * (b1 - b0 + 1);  // every CTA writes two lists per row (the column halves of its epilogue)
   }
   if (splits == 1 && lay.tc == 0) {
@@ -632,7 +647,7 @@ __global__ void __launch_bounds__(FB_WARPS * 32)
 knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const int* __restrict__ flag_count,
                          const int* __restrict__ flag_rows, int* __restrict__ knn_idx, float* __restrict__ knn_dist,
                          int* __restrict__ info, double* __restrict__ part_d, int* __restrict__ part_j,
-                         unsigned* __restrict__ ticket) {
+                         unsigned* __restrict__ ticket, const int2* __restrict__ win) {
   extern __shared__ __align__(16) float xs[];
   __shared__ double sd[FB_WARPS][32];
   __shared__ int sj[FB_WARPS][32];
@@ -649,7 +664,8 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
   for (long long t = blockIdx.x; t < T; t += G) {
     const int f = (int)(t / C), c = (int)(t - (long long)f * C);
     const int i = flag_rows[f];
-    const int j0 = (int)((long long)n * c / C), j1 = (int)((long long)n * (c + 1) / C);
+    const int2 w = (win != nullptr) ? win[i] : make_int2(0, n);  // a segmented search scans the row's own segment
+    const int j0 = w.x + (int)((long long)(w.y - w.x) * c / C), j1 = w.x + (int)((long long)(w.y - w.x) * (c + 1) / C);
     __syncthreads();  // the previous task's readers of xs / sd / sj are done
     for (int q = threadIdx.x; q < d; q += blockDim.x) xs[q] = X[(size_t)i * d + q];
     __syncthreads();
@@ -780,9 +796,8 @@ knn_merge_kernel(int row_end, CandLayout lay, const u64* __restrict__ cand, u64*
   if (i >= row_end) return;
   int splits = lay.stride;
   if (lay.tc == 1) {
-    const long long rt = (i - lay.row_begin) / lay.row_tile;
-    const int b0 = (int)(((rt * lay.col_tiles + 1) * lay.grid - 1) / lay.units);
-    const int b1 = (int)((((rt + 1) * lay.col_tiles) * lay.grid - 1) / lay.units);
+    int b0, b1;
+    cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
     splits = 2 * (b1 - b0 + 1);  // every CTA writes two lists per row (the column halves of its epilogue)
   }
   u64 mine = KEY_INF;
@@ -877,7 +892,7 @@ size_t knn_fallback_scratch_bytes() { return align_up((size_t)knn_fallback_grid(
 
 int knn_finish(const float* X, const float* sq, const unsigned* sqmax_bits, int n, int d, int k, int row_begin, int row_end,
                CandLayout lay, const u64* cand, float err_coef, int* knn_idx, float* knn_dist, int* flag_count, int* flag_rows,
-               int* info, void* fb_scratch, cudaStream_t st) {
+               int* info, void* fb_scratch, cudaStream_t st, const int2* win) {
   const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
   size_t smem = sizeof(float) * (size_t)RERANK_WARPS * d;
   lay.row_begin = row_begin;
@@ -913,10 +928,10 @@ int knn_finish(const float* X, const float* sq, const unsigned* sqmax_bits, int 
     GLL_PROF(KID_KNN_FALLBACK, st);
     if (vec4)
       knn_fallback_scan_kernel<true><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info,
-                                                                           part_d, part_j, ticket);
+                                                                           part_d, part_j, ticket, win);
     else
       knn_fallback_scan_kernel<false><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info,
-                                                                            part_d, part_j, ticket);
+                                                                            part_d, part_j, ticket, win);
   }
   GLL_LAUNCH_CHECK();
   return GLL_OK;
@@ -974,21 +989,110 @@ static int cand_stride(int n, int d, int row_begin, int row_end) {
   return simt_splits(n, row_end - row_begin, &cps);
 }
 
-size_t knn_ws_bytes(int n, int d, int k, int row_begin, int row_end) {
-  (void)k;
-  const size_t rows = (size_t)(row_end - row_begin);
+// The buffers every search carves from its workspace (KnnBufs, knn_carve) and their size for `rows` searched rows with `stride`
+// candidate lists per row.  knn_run and knn_run_segments append their own buffers behind them.
+static size_t knn_common_bytes(int n, int d, size_t rows, int stride) {
   size_t b = 0;
-  b += align_up(sizeof(float) * (size_t)n, 256);                                                   // sq
-  b += 256;                                                                                        // sqmax + flag_count
-  b += align_up(sizeof(u64) * rows * (size_t)cand_stride(n, d, row_begin, row_end) * KC, 256);     // cand
-  b += align_up(sizeof(int) * rows, 256);                                                          // flag_rows
+  b += align_up(sizeof(float) * (size_t)n, 256);                        // sq
+  b += 256;                                                             // sqmax + flag_count
+  b += align_up(sizeof(u64) * rows * (size_t)stride * KC, 256);         // cand
+  b += align_up(sizeof(int) * rows, 256);                               // flag_rows
   b += knn_tc_ws_upper(n, d);                                           // 16-bit hi / lo copies for the tensor-core path
   b += align_up(sizeof(unsigned) * (size_t)n, 256);                     // per-row shared thresholds
   b += align_up(sizeof(float) * (size_t)n, 256);                        // per-row operand scale (f16x2 split)
-  if (k > KC + 1) b += 2 * align_up(sizeof(u64) * rows * KC, 256) + align_up(sizeof(u64) * (size_t)n, 256);  // merged lists, excl
   b += knn_fallback_scratch_bytes() + 256;                              // chunk lists of the brute-force fallback
+  return b;
+}
+
+size_t knn_ws_bytes(int n, int d, int k, int row_begin, int row_end) {
+  const size_t rows = (size_t)(row_end - row_begin);
+  size_t b = knn_common_bytes(n, d, rows, cand_stride(n, d, row_begin, row_end));
+  if (k > KC + 1) b += 2 * align_up(sizeof(u64) * rows * KC, 256) + align_up(sizeof(u64) * (size_t)n, 256);  // merged lists, excl
   return b + 1024;
 }
+
+namespace {
+
+struct KnnBufs {
+  float* sq;
+  unsigned* small;   // small[0]: bits of max |x|^2, small[1]: flag_count, small[7]: fallback ticket (zeroed per search)
+  int* flag_count;
+  u64* cand;         // indexed by GLOBAL row: where row 0 would live
+  int* flag_rows;
+  char* tc_ws;
+  unsigned* thr_g;   // NULL when GLL_B200_KNN_SHARE=0
+  float* rscale;     // per-row power-of-two scale of the fp16 operands
+  void* fb_scratch;
+};
+
+KnnBufs knn_carve(Carver& cv, int n, int d, int row_begin, int row_end, int stride) {
+  const int rows = row_end - row_begin;
+  KnnBufs b;
+  b.sq = cv.take<float>(n);
+  b.small = cv.take<unsigned>(64);
+  b.flag_count = reinterpret_cast<int*>(b.small + 1);
+  b.cand = cv.take<u64>((size_t)rows * stride * KC) - (size_t)row_begin * stride * KC;
+  b.flag_rows = cv.take<int>(rows);
+  b.tc_ws = cv.take<char>(knn_tc_ws_upper(n, d));
+  b.thr_g = cv.take<unsigned>(n);
+  b.rscale = cv.take<float>(n);
+  b.fb_scratch = cv.take<char>(knn_fallback_scratch_bytes());
+  const char* sh = getenv("GLL_B200_KNN_SHARE");  // "0": every candidate set keeps its own threshold (experiments)
+  if (sh && sh[0] == '0') b.thr_g = nullptr;
+  return b;
+}
+
+// candidate-list layout of a tensor-core search; gfirst != NULL: the segmented unit grid
+CandLayout layout_of(const TcPlan& plan, int row_begin, const int* gfirst = nullptr) {
+  CandLayout lay;
+  lay.stride = plan.max_splits;
+  lay.tc = plan.aligned ? 2 : (gfirst != nullptr ? 3 : 1);
+  lay.row_tile = 128 * plan.rstep;  // rows per row group
+  lay.col_tiles = plan.col_tiles;
+  lay.grid = plan.grid;
+  lay.units = plan.units;
+  lay.row_begin = row_begin;
+  lay.gfirst = gfirst;
+  return lay;
+}
+
+// ... and of the SIMT search (or of lists merged into one sorted list per row)
+CandLayout simt_layout(int splits) {
+  CandLayout lay;
+  lay.stride = splits;
+  lay.tc = 0;
+  lay.row_tile = lay.col_tiles = lay.grid = 0;
+  lay.units = 0;
+  lay.row_begin = 0;
+  lay.gfirst = nullptr;
+  return lay;
+}
+
+// |fl(d~^2) - d^2| <= (gamma_d + 4u)(|x_i|^2 + |x_j|^2), gamma_d = d u/(1 - d u), u = 2^-24 (sequential fp32 FMA chain)
+float simt_err_coef(int d) {
+  const double u = 5.9604644775390625e-8;
+  return (float)(((double)d * u / (1.0 - (double)d * u) + 4.0 * u) * 1.0001);
+}
+
+// fp32 SIMT Gram with the fused top-k epilogue; win != NULL: segmented search (column windows per row)
+int launch_simt(const float* X, const float* sq, int n, int d, int cps, int splits, u64* cand, int row_begin, int row_end,
+                const int2* win, cudaStream_t st) {
+  const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
+  const bool seg = win != nullptr;
+  auto kern = vec4 ? (seg ? knn_gemm_topk_kernel<true, true> : knn_gemm_topk_kernel<true, false>)
+                   : (seg ? knn_gemm_topk_kernel<false, true> : knn_gemm_topk_kernel<false, false>);
+  const dim3 grid(ceil_div(row_end - row_begin, BM), splits);
+  const size_t smem = gemm_smem_bytes();
+  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)smem));
+  {
+    GLL_PROF(KID_GRAM_TOPK, st);
+    kern<<<grid, GEMM_THREADS, smem, st>>>(X, sq, n, d, cps, splits, cand, row_begin, row_end, win);
+  }
+  GLL_LAUNCH_CHECK();
+  return GLL_OK;
+}
+
+}  // namespace
 
 // fp16 operand split + norms: rows of up to 1024 padded columns stay in registers (one sweep over X)
 static int launch_split_f16(const float* X, int n, int d, const TcPlan& plan, float* sq, unsigned* small, char* tc_ws, float* rscale,
@@ -1004,6 +1108,15 @@ static int launch_split_f16(const float* X, int n, int d, const TcPlan& plan, fl
     sqnorm_split_f16_kernel<16><<<grid, 256, 0, st>>>(X, n, d, plan.d_pad, sq, small, H, L, rscale, thr_g);
   else
     sqnorm_split_f16_kernel<0><<<grid, 256, 0, st>>>(X, n, d, plan.d_pad, sq, small, H, L, rscale, thr_g);
+  GLL_LAUNCH_CHECK();
+  return GLL_OK;
+}
+
+// |x_i|^2 and the global max for the search, plus the fp16 operand split when the tensor-core plan runs
+static int launch_norms(const float* X, int n, int d, const TcPlan& plan, const KnnBufs& b, cudaStream_t st) {
+  GLL_PROF(KID_SQNORM, st);
+  if (plan.ok) return launch_split_f16(X, n, d, plan, b.sq, b.small, b.tc_ws, b.rscale, b.thr_g, st);
+  sqnorm_kernel<<<ceil_div((long long)n * 32, 256), 256, 0, st>>>(X, n, d, b.sq, b.small);
   GLL_LAUNCH_CHECK();
   return GLL_OK;
 }
@@ -1044,38 +1157,25 @@ int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int
     return GLL_ERR_WORKSPACE;
   }
   const int rows = row_end - row_begin;
-  const int stride = cand_stride(n, d, row_begin, row_end);
   Carver cv(ws, ws_bytes);
-  float* sq = cv.take<float>(n);
-  unsigned* small = cv.take<unsigned>(64);
+  const KnnBufs kb = knn_carve(cv, n, d, row_begin, row_end, cand_stride(n, d, row_begin, row_end));
+  float* sq = kb.sq;
+  unsigned* small = kb.small;
   unsigned* sqmax_bits = small;
-  int* flag_count = reinterpret_cast<int*>(small + 1);
-  u64* cand_store = cv.take<u64>((size_t)rows * stride * KC);
-  // kernels index candidate sets by GLOBAL row: hand them the pointer where row 0 would live
-  u64* cand = cand_store - (size_t)row_begin * stride * KC;
-  int* flag_rows = cv.take<int>(rows);
-  char* tc_ws = cv.take<char>(knn_tc_ws_upper(n, d));
-  unsigned* thr_g = cv.take<unsigned>(n);
-  float* rscale = cv.take<float>(n);  // per-row power-of-two scale of the fp16 operands
-  void* fb_scratch = cv.take<char>(knn_fallback_scratch_bytes());
-  {
-    const char* sh = getenv("GLL_B200_KNN_SHARE");  // "0": every candidate set keeps its own threshold (experiments)
-    if (sh && sh[0] == '0') thr_g = nullptr;
-  }
+  int* flag_count = kb.flag_count;
+  u64* cand = kb.cand;
+  int* flag_rows = kb.flag_rows;
+  char* tc_ws = kb.tc_ws;
+  unsigned* thr_g = kb.thr_g;
+  float* rscale = kb.rscale;
 
   CandLayout lay;
   float err_coef;
   const TcPlan plan = knn_tc_plan(n, d, row_begin, row_end);
   GLL_CUDA_CHECK(cudaMemsetAsync(small, 0, 256, st));
   {
-    GLL_PROF(KID_SQNORM, st);
-    if (plan.ok) {
-      const int rcs = launch_split_f16(X, n, d, plan, sq, small, tc_ws, rscale, thr_g, st);
-      if (rcs) return rcs;
-    } else {
-      sqnorm_kernel<<<ceil_div((long long)n * 32, 256), 256, 0, st>>>(X, n, d, sq, sqmax_bits);
-      GLL_LAUNCH_CHECK();
-    }
+    const int rcs = launch_norms(X, n, d, plan, kb, st);
+    if (rcs) return rcs;
   }
 
   if (k > KC + 1) {
@@ -1084,13 +1184,7 @@ int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int
     u64* merged1 = cv.take<u64>((size_t)rows * KC);
     u64* merged2 = cv.take<u64>((size_t)rows * KC);
     u64* excl = cv.take<u64>(n);
-    lay.stride = plan.max_splits;
-    lay.tc = plan.aligned ? 2 : 1;
-    lay.row_tile = 128 * plan.rstep;
-    lay.col_tiles = plan.col_tiles;
-    lay.grid = plan.grid;
-    lay.units = plan.units;
-    lay.row_begin = row_begin;
+    lay = layout_of(plan, row_begin);
     const int mblocks = ceil_div(rows, RERANK_WARPS);
     int rc = knn_tc_candidates(X, sq, rscale, small, n, d, row_end, plan, tc_ws, cand, nullptr, thr_g, st);
     if (rc) return rc;
@@ -1112,45 +1206,174 @@ int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int
   if (plan.ok) {  // tcgen05 / TMA Gram GEMM with the fused top-k epilogue
     int rc = knn_tc_candidates(X, sq, rscale, small, n, d, row_end, plan, tc_ws, cand, nullptr, thr_g, st);
     if (rc) return rc;
-    lay.stride = plan.max_splits;
-    lay.tc = plan.aligned ? 2 : 1;
-    lay.row_tile = 128 * plan.rstep;  // rows per row group
-    lay.col_tiles = plan.col_tiles;
-    lay.grid = plan.grid;
-    lay.units = plan.units;
+    lay = layout_of(plan, row_begin);
     err_coef = knn_tc_err_coef(d, plan.passes);
   } else {  // fp32 SIMT Gram (tiny graphs, or forced by GLL_B200_KNN_PATH=simt)
     int cps;
     const int splits = simt_splits(n, rows, &cps);
-    const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
-    dim3 grid(ceil_div(rows, BM), splits);
-    size_t smem = gemm_smem_bytes();
-    if (vec4) {
-      GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_gemm_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      {
-        GLL_PROF(KID_GRAM_TOPK, st);
-        knn_gemm_topk_kernel<true><<<grid, GEMM_THREADS, smem, st>>>(X, sq, n, d, cps, splits, cand, row_begin, row_end);
-      }
-    } else {
-      GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_gemm_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      {
-        GLL_PROF(KID_GRAM_TOPK, st);
-        knn_gemm_topk_kernel<false><<<grid, GEMM_THREADS, smem, st>>>(X, sq, n, d, cps, splits, cand, row_begin, row_end);
-      }
-    }
-    GLL_LAUNCH_CHECK();
-    lay.stride = splits;
-    lay.tc = 0;
-    lay.row_tile = lay.col_tiles = lay.grid = 0;
-    lay.units = 0;
-    // |fl(d~^2) - d^2| <= (gamma_d + 4u)(|x_i|^2 + |x_j|^2), gamma_d = d u/(1 - d u), u = 2^-24 (sequential fp32 FMA chain)
-    const double u = 5.9604644775390625e-8;
-    err_coef = (float)(((double)d * u / (1.0 - (double)d * u) + 4.0 * u) * 1.0001);
+    const int rc = launch_simt(X, sq, n, d, cps, splits, cand, row_begin, row_end, nullptr, st);
+    if (rc) return rc;
+    lay = simt_layout(splits);
+    err_coef = simt_err_coef(d);
   }
   return knn_finish(X, sq, sqmax_bits, n, d, k, row_begin, row_end, lay, cand, err_coef, knn_idx, knn_dist, flag_count, flag_rows,
-                    info, fb_scratch, st);
+                    info, kb.fb_scratch, st);
 }
 
+
+// ------------------------------------------------------------------------------------------------------------------------
+// Segmented search (gll_knn_segments): independent graphs stacked as row segments; row i of segment s gets its k nearest
+// neighbours among the rows of s only.  Every kernel sees the rows' column windows win[i] = [lo, hi): the Gram kernels only
+// visit the column tiles that meet a row tile's windows and mask the rest per row, the fallback scans the window, and the
+// re-rank is unchanged (columns outside the window never enter a set, so its completeness proof covers the window).
+// ------------------------------------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int UPLOAD_INTS = 1000;
+struct IntChunk {
+  int v[UPLOAD_INTS];
+};
+// host ints -> device through the kernel parameters: no host memory is read when the work runs, so the call can be captured
+// in a CUDA graph (a copy from pageable host memory cannot)
+__global__ void upload_ints_kernel(IntChunk c, int count, int* __restrict__ dst) {
+  for (int t = threadIdx.x; t < count; t += blockDim.x) dst[t] = c.v[t];
+}
+
+// win[i] = [seg_ptr[s], seg_ptr[s + 1]) for the rows i of segment s = blockIdx.x
+__global__ void seg_windows_kernel(const int* __restrict__ seg_ptr, int2* __restrict__ win) {
+  const int lo = seg_ptr[blockIdx.x], hi = seg_ptr[blockIdx.x + 1];
+  for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) win[i] = make_int2(lo, hi);
+}
+
+// SIMT column splits of a segmented search: the widest union of windows over a 128-row tile takes the place of n
+int simt_seg_splits(int n, const int* seg_ptr, int* cols_per_split) {
+  int wmax = 1;
+  for (int r0 = 0, s = 0; r0 < n; r0 += BM) {
+    while (seg_ptr[s + 1] <= r0) ++s;
+    int t = s;
+    const int r1 = min(n, r0 + BM) - 1;
+    while (seg_ptr[t + 1] <= r1) ++t;
+    wmax = max(wmax, seg_ptr[t + 1] - seg_ptr[s]);
+  }
+  return simt_splits(wmax, n, cols_per_split);
+}
+
+struct SegPlan {
+  TcPlan tc;
+  std::vector<int> tab;  // gfirst, gct, bstart of the tensor-core plan
+  int stride, cps;       // candidate lists per row; SIMT: columns per split
+};
+
+SegPlan seg_plan(int n, int d, const int* seg_ptr, int nseg) {
+  SegPlan p;
+  p.tc = knn_tc_plan_segments(n, d, seg_ptr, nseg, &p.tab);
+  p.cps = 0;
+  if (p.tc.ok) {
+    p.stride = p.tc.max_splits;
+  } else {
+    p.tab.clear();
+    p.stride = simt_seg_splits(n, seg_ptr, &p.cps);
+  }
+  return p;
+}
+
+}  // namespace
+
+int knn_seg_check(int n, int d, int k, const int* seg_ptr, int nseg) {
+  GLL_REQUIRE(seg_ptr != nullptr, "null seg_ptr");
+  GLL_REQUIRE(nseg >= 1 && n >= 1 && d >= 1, "bad sizes");
+  GLL_REQUIRE(k >= 2 && k <= KC + 1, "the segmented search serves 2 <= k <= 33");
+  GLL_REQUIRE(seg_ptr[0] == 0 && seg_ptr[nseg] == n, "seg_ptr must run from 0 to n");
+  for (int s = 0; s < nseg; ++s)
+    if (seg_ptr[s + 1] - seg_ptr[s] < k) {
+      set_error("segment %d has %d rows, fewer than k = %d (or seg_ptr is not increasing)", s, seg_ptr[s + 1] - seg_ptr[s], k);
+      return GLL_ERR_ARG;
+    }
+  return GLL_OK;
+}
+
+size_t knn_seg_ws_bytes(int n, int d, int k, const int* seg_ptr, int nseg) {
+  if (knn_seg_check(n, d, k, seg_ptr, nseg) != GLL_OK) return 0;
+  if (nseg == 1) return knn_ws_bytes(n, d, k, 0, n);
+  const SegPlan p = seg_plan(n, d, seg_ptr, nseg);
+  size_t b = knn_common_bytes(n, d, (size_t)n, p.stride);
+  b += align_up(sizeof(int2) * (size_t)n, 256);                                      // windows
+  b += align_up(sizeof(int) * ((size_t)nseg + 1 + p.tab.size()), 256);               // seg_ptr + unit table
+  return b + 2048;
+}
+
+int knn_run_segments(const float* X, int n, int d, int k, const int* seg_ptr, int nseg, int* knn_idx, float* knn_dist, int* info,
+                     void* ws, size_t ws_bytes, cudaStream_t st) {
+  GLL_REQUIRE(X && knn_idx && knn_dist && ws, "null pointer");
+  const int rc0 = knn_seg_check(n, d, k, seg_ptr, nseg);
+  if (rc0) return rc0;
+  if (nseg == 1) return knn_run(X, n, d, k, 0, n, knn_idx, knn_dist, info, ws, ws_bytes, st);  // the unsegmented search as is
+  const size_t need = knn_seg_ws_bytes(n, d, k, seg_ptr, nseg);
+  if (ws_bytes < need) {
+    set_error("kNN workspace too small: %zu < %zu", ws_bytes, need);
+    return GLL_ERR_WORKSPACE;
+  }
+  const SegPlan sp = seg_plan(n, d, seg_ptr, nseg);
+  const TcPlan& plan = sp.tc;
+  Carver cv(ws, ws_bytes);
+  const KnnBufs kb = knn_carve(cv, n, d, 0, n, sp.stride);
+  int2* win = cv.take<int2>(n);
+  int* ints = cv.take<int>((size_t)nseg + 1 + sp.tab.size());  // seg_ptr, then gfirst, gct, bstart
+  GLL_CUDA_CHECK(cudaMemsetAsync(kb.small, 0, 256, st));
+  {
+    GLL_PROF(KID_KNN_SEGMENTS, st);
+    std::vector<int> host(seg_ptr, seg_ptr + nseg + 1);
+    host.insert(host.end(), sp.tab.begin(), sp.tab.end());
+    for (size_t o = 0; o < host.size(); o += UPLOAD_INTS) {
+      IntChunk c;
+      const int cnt = (int)std::min<size_t>(UPLOAD_INTS, host.size() - o);
+      memcpy(c.v, host.data() + o, sizeof(int) * (size_t)cnt);
+      upload_ints_kernel<<<1, 256, 0, st>>>(c, cnt, ints + o);
+    }
+    seg_windows_kernel<<<nseg, 256, 0, st>>>(ints, win);
+    GLL_LAUNCH_CHECK();
+  }
+  {
+    const int rcs = launch_norms(X, n, d, plan, kb, st);
+    if (rcs) return rcs;
+  }
+  CandLayout lay;
+  float err_coef;
+  if (plan.ok) {
+    const int RG = plan.row_tiles;
+    SegDev sd;
+    sd.win = win;
+    sd.gfirst = ints + nseg + 1;
+    sd.gct = sd.gfirst + RG + 1;
+    sd.bstart = sd.gct + RG;
+    const int rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, n, plan, kb.tc_ws, kb.cand, nullptr, kb.thr_g, st, &sd);
+    if (rc) return rc;
+    lay = layout_of(plan, 0, sd.gfirst);
+    err_coef = knn_tc_err_coef(d, plan.passes);
+  } else {
+    const int rc = launch_simt(X, kb.sq, n, d, sp.cps, sp.stride, kb.cand, 0, n, win, st);
+    if (rc) return rc;
+    lay = simt_layout(sp.stride);
+    err_coef = simt_err_coef(d);
+  }
+  return knn_finish(X, kb.sq, kb.small, n, d, k, 0, n, lay, kb.cand, err_coef, knn_idx, knn_dist, kb.flag_count, kb.flag_rows, info,
+                    kb.fb_scratch, st, win);
+}
+
+// units the tensor-core search of a segmented call issues, and those of the uniform grid over the same rows (0, 0: SIMT path)
+void knn_seg_units(int n, int d, const int* seg_ptr, int nseg, long long* seg_units, long long* uniform_units) {
+  *seg_units = *uniform_units = 0;
+  if (knn_seg_check(n, d, 2, seg_ptr, nseg) != GLL_OK) return;
+  const TcPlan u = knn_tc_plan(n, d, 0, n);
+  if (!u.ok) return;
+  *uniform_units = u.units;
+  if (nseg == 1) {
+    *seg_units = u.units;
+    return;
+  }
+  std::vector<int> tab;
+  *seg_units = knn_tc_plan_segments(n, d, seg_ptr, nseg, &tab).units;
+}
 
 // ------------------------------------------------------------------------------------------------------------------------
 // Base-set reuse across evaluation batches (SURVEY 8f-4; utils.py:596-621: test_network calls the layer on
@@ -1192,25 +1415,12 @@ knn_merge_cached_kernel(int r0, int n, CandLayout layA, const u64* __restrict__ 
   u64 mine = base ? cache[(size_t)i * KC + lane] : KEY_INF;
   int splits = lay.stride;
   if (lay.tc == 1) {
-    const long long rt = (i - lay.row_begin) / lay.row_tile;
-    const int b0 = (int)(((rt * lay.col_tiles + 1) * lay.grid - 1) / lay.units);
-    const int b1 = (int)((((rt + 1) * lay.col_tiles) * lay.grid - 1) / lay.units);
+    int b0, b1;
+    cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
     splits = 2 * (b1 - b0 + 1);
   }
   for (int s = 0; s < splits; ++s) list_merge_set(mine, cand[((size_t)i * lay.stride + s) * KC + lane], lane);
   merged[(size_t)i * KC + lane] = mine;
-}
-
-CandLayout layout_of(const TcPlan& plan, int row_begin) {
-  CandLayout lay;
-  lay.stride = plan.max_splits;
-  lay.tc = plan.aligned ? 2 : 1;
-  lay.row_tile = 128 * plan.rstep;
-  lay.col_tiles = plan.col_tiles;
-  lay.grid = plan.grid;
-  lay.units = plan.units;
-  lay.row_begin = row_begin;
-  return lay;
 }
 
 }  // namespace
@@ -1319,12 +1529,7 @@ int knn_run_cached(const float* X, int n, int d, int k, int nb, const void* cach
                                                                                    cache, merged);
   }
   GLL_LAUNCH_CHECK();
-  CandLayout lay;
-  lay.stride = 1;
-  lay.tc = 0;
-  lay.row_tile = lay.col_tiles = lay.grid = 0;
-  lay.units = 0;
-  return knn_finish(X, sq, small, n, d, k, 0, n, lay, merged, knn_tc_err_coef(d, pa.passes), knn_idx, knn_dist, flag_count, flag_rows, info,
+  return knn_finish(X, sq, small, n, d, k, 0, n, simt_layout(1), merged, knn_tc_err_coef(d, pa.passes), knn_idx, knn_dist, flag_count, flag_rows, info,
                     fb_scratch, st);
 }
 

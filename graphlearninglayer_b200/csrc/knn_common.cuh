@@ -1,5 +1,7 @@
 // Pieces shared by the SIMT (knn.cu) and tensor-core (knn_tc.cu) kNN candidate kernels.
 #pragma once
+#include <vector>
+
 #include "common.cuh"
 
 namespace gll {
@@ -76,10 +78,23 @@ struct TcPlan {
   size_t ws_bytes;  // fp16 hi / lo copies of X
 };
 
+// Segmented search (gll_knn_segments): row i only sees the columns of its own segment, win[i] = [lo, hi).  The tensor-core
+// unit grid then has, per row group g, only the column tiles [gct[g], gct[g] + gfirst[g + 1] - gfirst[g]) that meet the
+// windows of its rows; units are numbered row group by row group (gfirst[g] = first unit of g), and bstart[b] is the row
+// group of owner b's first unit.  Device arrays in the workspace; all NULL for an unsegmented search.
+struct SegDev {
+  const int2* win;
+  const int* gfirst;
+  const int* gct;
+  const int* bstart;
+};
+
 TcPlan knn_tc_plan(int n, int d, int row_begin, int row_end, int col_begin = 0);
+// the plan of a segmented search over all n rows; *tab receives gfirst, gct and bstart (in that order, see SegDev)
+TcPlan knn_tc_plan_segments(int n, int d, const int* seg_ptr, int nseg, std::vector<int>* tab);
 size_t knn_tc_ws_upper(int n, int d);
 int knn_tc_candidates(const float* X, const float* sq, const float* rscale, const unsigned* small, int n, int d, int row_end, const TcPlan& plan,
-                      void* tc_ws, u64* cand, const u64* excl, unsigned* thr_g, cudaStream_t st);
+                      void* tc_ws, u64* cand, const u64* excl, unsigned* thr_g, cudaStream_t st, const SegDev* seg = nullptr);
 float knn_tc_err_coef(int d, int passes);
 // verification: raw accumulator of one (row tile, column tile) unit, acc_out[128][256] (knn_gram_tile_debug_kernel)
 int knn_tc_debug_tile(const TcPlan& plan, int n, void* tc_ws, int rt, int ct, float* acc_out, cudaStream_t st);
@@ -88,15 +103,26 @@ int knn_tc_debug_tile(const TcPlan& plan, int n, void* tc_ws, int rt, int ct, fl
 // or the tensor-core work split (row tile rt was touched by CTAs b0(rt)..b1(rt); slot = b - b0).
 struct CandLayout {
   int stride;      // lists allocated per row
-  int tc;          // 0: every row has `stride` sorted lists; 1: tensor-core work split; 2: one unsorted set per row
+  int tc;          // 0: every row has `stride` sorted lists; 1: tensor-core work split; 2: one unsorted set per row;
+                   // 3: tensor-core work split over a segmented unit grid (row group g owns units [gfirst[g], gfirst[g + 1]))
   int row_begin;   // first row of this call's row range (row tiles are counted from it)
   int row_tile, col_tiles, grid;
   long long units;
+  const int* gfirst;  // tc == 3 only (SegDev::gfirst)
 };
 
+// CTAs of a G-CTA tensor-core launch over `units` units that wrote candidate sets for row group rt: b0 .. b1
+__device__ __forceinline__ void cand_owner_range(const CandLayout& lay, long long rt, int& b0, int& b1) {
+  const long long f0 = (lay.tc == 3) ? (long long)__ldg(lay.gfirst + rt) : rt * lay.col_tiles;
+  const long long f1 = (lay.tc == 3) ? (long long)__ldg(lay.gfirst + rt + 1) : (rt + 1) * lay.col_tiles;
+  b0 = (int)(((f0 + 1) * lay.grid - 1) / lay.units);
+  b1 = (int)((f1 * lay.grid - 1) / lay.units);
+}
+
+// win: NULL, or the rows' column windows of a segmented search (the brute-force fallback scans only the window)
 int knn_finish(const float* X, const float* sq, const unsigned* sqmax_bits, int n, int d, int k, int row_begin, int row_end,
                CandLayout lay,
                const u64* cand, float err_coef, int* knn_idx, float* knn_dist, int* flag_count, int* flag_rows,
-               int* info, void* fb_scratch, cudaStream_t st);
+               int* info, void* fb_scratch, cudaStream_t st, const int2* win = nullptr);
 
 }  // namespace gll

@@ -44,6 +44,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
+
 #include "knn_common.cuh"
 
 namespace gll {
@@ -244,16 +246,26 @@ __host__ __device__ inline uint32_t a_bytes_of(int passes) { return passes == 2 
 // CTA that owns unit u when `units` units are dealt contiguously to G CTAs (CTA b owns [b*units/G, (b+1)*units/G))
 __host__ __device__ inline int tc_cta_of_unit(long long u, int G, long long units) { return (int)(((u + 1) * G - 1) / units); }
 
+// Segmented unit grid: row group r's column-tile count and first column tile (r == row_tiles: past the end, left alone)
+__device__ __forceinline__ void seg_group(const SegDev& S, int row_tiles, int r, int& cnt, int& ctl) {
+  if (r < row_tiles) {
+    cnt = __ldg(S.gfirst + r + 1) - __ldg(S.gfirst + r);
+    ctl = __ldg(S.gct + r);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------- the GEMM + top-k kernel
 // PAIR: launched as clusters of two CTAs (one TPC) that process the SAME column tile for two adjacent row tiles with ONE
 // tcgen05.mma.cta_group::2 of M = 256: each CTA stages its own 128 rows of A and HALF of the B tile (128 of the 256
 // columns), so the operand bytes a CTA pulls from L2 drop by a third -- which is what bounds the one-pass kernel
 // (measured: ~70 GB/s per SM whatever the stage count, profiles/r02k_knn_experiments_c2.txt).  The leader CTA issues the
 // MMAs; both CTAs run their own TMA producer and their own epilogue on their own 128 accumulator rows.
-template <bool PAIR>
+// SEG: segmented search.  Row group r_idx has cnt column tiles from ctl on (S); the uniform grid has cnt = C, ctl = ct0.  S is
+// a parameter of its own: inside TcParams it would push the struct past the size up to which the compiler keeps it in registers.
+template <bool PAIR, bool SEG>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_constant__ CUtensorMap mapAL,
-                        const __grid_constant__ CUtensorMap mapBH, TcParams P) {
+                        const __grid_constant__ CUtensorMap mapBH, TcParams P, SegDev S) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;  // 128B-swizzled operand tiles need 1024 B alignment
@@ -270,12 +282,30 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
     if (tracing && ui < TC_TRACE_UNITS) P.trace[((size_t)w * TC_TRACE_UNITS + ui) * TC_TRACE_PHASES + ph] = (unsigned long long)val;
   };
   long long u_begin, u_end;
-  if (P.aligned) {
-    u_begin = ((long long)b * P.row_tiles / G) * C;
-    u_end = ((long long)(b + 1) * P.row_tiles / G) * C;
+  // SEG: coordinates of unit u_begin (row-group ordinal, column-tile ordinal inside it, the group's tile count and first tile).
+  // The uniform grid keeps its own arithmetic below, in each warp role, exactly as without segments.
+  int r_begin = 0, c_begin0 = 0, cnt0 = C, ctl0 = P.ct0;
+  if constexpr (SEG) {
+    if (P.aligned) {
+      const int g0 = (int)((long long)b * P.row_tiles / G), g1 = (int)((long long)(b + 1) * P.row_tiles / G);
+      u_begin = (long long)__ldg(S.gfirst + g0);
+      u_end = (long long)__ldg(S.gfirst + g1);
+      r_begin = g0;
+    } else {
+      u_begin = (long long)b * P.units / G;
+      u_end = (long long)(b + 1) * P.units / G;
+      r_begin = __ldg(S.bstart + b);
+    }
+    seg_group(S, P.row_tiles, r_begin, cnt0, ctl0);
+    c_begin0 = (r_begin < P.row_tiles) ? (int)(u_begin - __ldg(S.gfirst + r_begin)) : 0;
   } else {
-    u_begin = (long long)b * P.units / G;
-    u_end = (long long)(b + 1) * P.units / G;
+    if (P.aligned) {
+      u_begin = ((long long)b * P.row_tiles / G) * C;
+      u_end = ((long long)(b + 1) * P.row_tiles / G) * C;
+    } else {
+      u_begin = (long long)b * P.units / G;
+      u_end = (long long)(b + 1) * P.units / G;
+    }
   }
 
   const bool two = P.passes == 2;
@@ -339,7 +369,9 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
     // counts.  (The split dates from the lane-0 issue form, where one cp.async.bulk.tensor cost its thread ~280 cycles.)
     if (ares && warp == 0) {
       // resident A: one load of all K blocks per row tile, after the MMAs of the previous row tile have retired
-      int r_idx = (int)(u_begin / C), c_idx = (int)(u_begin % C);
+      int r_idx = SEG ? r_begin : (int)(u_begin / C), c_idx = SEG ? c_begin0 : (int)(u_begin % C);
+      int cnt = cnt0, ctl = ctl0;  // SEG only
+      (void)ctl;
       uint32_t ph_free = 0;
       for (long long u = u_begin; u < u_end;) {
         const int rt = P.rt0 + RSTEP * r_idx + crank;
@@ -363,9 +395,10 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
           }
         }
         __syncwarp();
-        u += C - c_idx;  // on to the CTA's next row tile
+        u += (SEG ? cnt : C) - c_idx;  // on to the CTA's next row tile
         c_idx = 0;
         ++r_idx;
+        if constexpr (SEG) seg_group(S, P.row_tiles, r_idx, cnt, ctl);
       }
     } else {
       const bool is_a = warp == 0;
@@ -373,12 +406,15 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
       uint32_t phase = 0;
       const uint32_t my_bytes = is_a ? a_bytes : b_bytes;
       const uint32_t b_off = ares ? 0u : a_bytes;  // where the B block sits inside a stage
-      int r_idx = (int)(u_begin / C), c_idx = (int)(u_begin % C);  // the unit's row-tile ordinal and column tile, kept incrementally
+      // the unit's row-tile ordinal and column tile, kept incrementally
+      int r_idx = SEG ? r_begin : (int)(u_begin / C), c_idx = SEG ? c_begin0 : (int)(u_begin % C);
+      int cnt = cnt0, ctl = ctl0;  // SEG only
       for (long long u = u_begin; u < u_end; ++u) {
-        const int rt = P.rt0 + RSTEP * r_idx + crank, ct = P.ct0 + c_idx;
-        if (++c_idx == C) {
+        const int rt = P.rt0 + RSTEP * r_idx + crank, ct = (SEG ? ctl : P.ct0) + c_idx;
+        if (++c_idx == (SEG ? cnt : C)) {
           c_idx = 0;
           ++r_idx;
+          if constexpr (SEG) seg_group(S, P.row_tiles, r_idx, cnt, ctl);
         }
         if (is_a && tracing) stamp(3, u - u_begin, 0, clock64());
         for (int kk = 0; kk < KB; ++kk) {
@@ -420,7 +456,9 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
     uint32_t phase = 0, acc_phase = 0;
     const int nprod = P.passes;
     const uint32_t idesc = PAIR ? TC_IDESC_F16_PAIR : TC_IDESC_F16;
-    int c_idx = (int)(u_begin % C);
+    int c_idx = SEG ? c_begin0 : (int)(u_begin % C);
+    int r_idx = r_begin, cnt = cnt0, ctl = ctl0;  // SEG only
+    (void)ctl;
     uint32_t ph_afull = 0;
     bool need_a = ares;
     for (long long u = (PAIR && crank != 0) ? u_end : u_begin; u < u_end; ++u) {
@@ -431,8 +469,11 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
         ph_afull ^= 1u;
         need_a = false;
       }
-      const bool row_done = (++c_idx == C);  // last unit of the row tile
+      const bool row_done = (++c_idx == (SEG ? cnt : C));  // last unit of the row tile
       if (row_done) c_idx = 0;
+      if constexpr (SEG) {
+        if (row_done) seg_group(S, P.row_tiles, ++r_idx, cnt, ctl);
+      }
       tc_fence_after();
       if (tracing) stamp(0, u - u_begin, 1, clock64());
       const uint32_t d_tmem = tmem_base + (uint32_t)acc * TC_ACC_STRIDE;
@@ -534,7 +575,11 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
 
     auto flush = [&](int rt) {
       __syncwarp();
-      const int slot = 2 * (P.aligned ? 0 : b - tc_cta_of_unit((long long)((rt - P.rt0) / RSTEP) * C, G, P.units)) + half;
+      int slot;
+      if constexpr (SEG)
+        slot = 2 * (P.aligned ? 0 : b - tc_cta_of_unit(__ldg(S.gfirst + (rt - P.rt0) / RSTEP), G, P.units)) + half;
+      else
+        slot = 2 * (P.aligned ? 0 : b - tc_cta_of_unit((long long)((rt - P.rt0) / RSTEP) * C, G, P.units)) + half;
       const uint32_t* wk = Lk - lane;
       const int* wi = Li - lane;
       for (int r = 0; r < 32; ++r) {  // lane = slot index e here; 256 B coalesced store per row
@@ -569,17 +614,22 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
       r.w = (j + 3 < P.n) ? __ldg(P.rscale + j + 3) : 1.f;
       return r;
     };
-    int r_idx = (int)(u_begin / C), c_idx = (int)(u_begin % C);  // kept incrementally: no 64-bit divisions per unit
+    // kept incrementally: no 64-bit divisions per unit
+    int r_idx = SEG ? r_begin : (int)(u_begin / C), c_idx = SEG ? c_begin0 : (int)(u_begin % C);
+    int cnt = cnt0, ctl = ctl0;  // SEG only
+    // SEG: my row's column window [my_lo, my_hi), and the part [w_lo, w_hi) that every row of the warp shares
+    int my_lo = 0, my_hi = 0, w_lo = 0, w_hi = 0;
     float4 nsq = make_float4(0.f, 0.f, 0.f, 0.f), ncj = nsq;
     if (u_begin < u_end) {
-      nsq = col_sq(P.ct0 + c_idx);
-      if (!uniform) ncj = col_cj(P.ct0 + c_idx);
+      nsq = col_sq((SEG ? ctl : P.ct0) + c_idx);
+      if (!uniform) ncj = col_cj((SEG ? ctl : P.ct0) + c_idx);
     }
     for (long long u = u_begin; u < u_end; ++u) {
-      const int rt = P.rt0 + RSTEP * r_idx + crank, ct = P.ct0 + c_idx;
-      if (++c_idx == C) {
+      const int rt = P.rt0 + RSTEP * r_idx + crank, ct = (SEG ? ctl : P.ct0) + c_idx;
+      if (++c_idx == (SEG ? cnt : C)) {
         c_idx = 0;
         ++r_idx;
+        if constexpr (SEG) seg_group(S, P.row_tiles, r_idx, cnt, ctl);
       }
       if (rt != cur_rt) {
         if (cur_rt >= 0) flush(cur_rt);
@@ -595,6 +645,13 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
         if (P.excl != nullptr) {
           excl_row = (gi < P.n) ? __ldg(P.excl + gi) : 0ull;
           sqi_row = (gi < P.n) ? __ldg(P.sq + gi) : 0.f;
+        }
+        if constexpr (SEG) {  // rows past n see every column; their sets are never flushed
+          const int2 w = (gi < P.n) ? __ldg(S.win + gi) : make_int2(0, 0x7fffffff);
+          my_lo = w.x;
+          my_hi = w.y;
+          w_lo = __reduce_max_sync(FULL, my_lo);
+          w_hi = __reduce_min_sync(FULL, my_hi);
         }
       }
       const int c_begin = ct * TC_BN;
@@ -613,8 +670,8 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
       if (!uniform) *reinterpret_cast<float4*>(cj_w + 4 * lane) = make_float4(-2.f * ncj.x, -2.f * ncj.y, -2.f * ncj.z, -2.f * ncj.w);
       __syncwarp();
       if (u + 1 < u_end) {
-        nsq = col_sq(P.ct0 + c_idx);
-        if (!uniform) ncj = col_cj(P.ct0 + c_idx);
+        nsq = col_sq((SEG ? ctl : P.ct0) + c_idx);
+        if (!uniform) ncj = col_cj((SEG ? ctl : P.ct0) + c_idx);
       }
       // ... and what the row's other sets have published (once per unit; folded in after the first 32 columns, when the
       // load has landed)
@@ -654,6 +711,15 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
             v[4 * c4 + 1] = fmaf(ri * __uint_as_float(raw[4 * c4 + 1]), c4v.y, s4.y);
             v[4 * c4 + 2] = fmaf(ri * __uint_as_float(raw[4 * c4 + 2]), c4v.z, s4.z);
             v[4 * c4 + 3] = fmaf(ri * __uint_as_float(raw[4 * c4 + 3]), c4v.w, s4.w);
+          }
+        }
+        // segmented search: a chunk inside every window of the warp's rows costs one warp-uniform test; one that crosses a
+        // window edge masks the columns outside each row's own window (they then never enter a set: +inf is the empty key)
+        if constexpr (SEG) {
+          if (!(j0 >= w_lo && j0 + TC_CHUNK <= w_hi)) {
+#pragma unroll
+            for (int c = 0; c < TC_CHUNK; ++c)
+              if (j0 + c < my_lo || j0 + c >= my_hi) v[c] = INFINITY;
           }
         }
         if (diag && j0 < wrow0 + 32 && j0 + TC_CHUNK > wrow0) {  // warp-uniform, true for at most 2 chunks of one unit
@@ -973,6 +1039,60 @@ TcPlan knn_tc_plan(int n, int d, int row_begin, int row_end, int col_begin) {
   return p;
 }
 
+// Segmented unit grid: row group g (rstep row tiles) gets the column tiles that meet [lo of its first row, hi of its last row)
+// -- segments are contiguous row ranges, so that is the union of its rows' windows.  Units are dealt to the owners exactly as
+// in the uniform grid (contiguously, tc_cta_of_unit); the kernel, the flush slots and the re-rank all read gfirst.
+TcPlan knn_tc_plan_segments(int n, int d, const int* seg_ptr, int nseg, std::vector<int>* tab) {
+  TcPlan p = knn_tc_plan(n, d, 0, n);
+  if (p.d_pad == 0) return p;  // SIMT path (tiny graph or forced)
+  const int RG = p.row_tiles, rows_g = TC_BM * p.rstep;
+  std::vector<int> gfirst(RG + 1), gct(RG);
+  int s = 0, max_cnt = 1;
+  long long units = 0;
+  for (int g = 0; g < RG; ++g) {
+    const int r0 = g * rows_g, r1 = std::min(n, r0 + rows_g) - 1;
+    while (seg_ptr[s + 1] <= r0) ++s;
+    const int lo = seg_ptr[s];
+    int t = s;
+    while (seg_ptr[t + 1] <= r1) ++t;
+    const int hi = seg_ptr[t + 1];
+    gct[g] = lo / TC_BN;
+    const int cnt = ceil_div(hi, TC_BN) - gct[g];
+    gfirst[g] = (int)units;
+    units += cnt;
+    max_cnt = std::max(max_cnt, cnt);
+  }
+  gfirst[RG] = (int)units;
+  (void)nseg;
+  p.units = units;
+  p.col_tiles = max_cnt;
+  const int owners = device_info().sms / p.rstep;
+  p.grid = (int)std::min<long long>(units, owners);
+  std::vector<int> bstart;
+  for (;;) {
+    if (!p.aligned) p.grid = std::max(1, std::min(p.grid, RG * (KNN_MAX_SPLITS / 2 - 1)));
+    int ms = 1;
+    if (!p.aligned)
+      for (int g = 0; g < RG; ++g)
+        ms = std::max(ms, tc_cta_of_unit(gfirst[g + 1] - 1, p.grid, units) - tc_cta_of_unit(gfirst[g], p.grid, units) + 1);
+    p.max_splits = 2 * ms;
+    if (p.max_splits <= KNN_MAX_SPLITS || p.grid == 1) break;
+    p.grid = std::max(1, p.grid * 3 / 4);  // a long row group shared by too many owners: fewer owners
+  }
+  p.ok = (p.max_splits <= KNN_MAX_SPLITS) ? 1 : 0;
+  bstart.resize(p.grid);
+  for (int b = 0, g = 0; b < p.grid; ++b) {
+    const long long u0 = (long long)b * units / p.grid;
+    while (g + 1 < RG && gfirst[g + 1] <= u0) ++g;
+    bstart[b] = g;
+  }
+  tab->clear();
+  tab->insert(tab->end(), gfirst.begin(), gfirst.end());
+  tab->insert(tab->end(), gct.begin(), gct.end());
+  tab->insert(tab->end(), bstart.begin(), bstart.end());
+  return p;
+}
+
 size_t knn_tc_ws_upper(int n, int d) { return 2 * align_up((size_t)n * (size_t)(ceil_div(d, TC_BK) * TC_BK) * 2, 256) + 512; }
 
 // |d~^2 - d^2| <= coef (|xi|^2 + max|x|^2) + [the rho term of knn_err_bound()].  coef budgets what rho does not measure:
@@ -1009,7 +1129,7 @@ static unsigned long long* g_knn_trace = nullptr;  // debug only: [TC_TRACE_WARP
 void knn_tc_set_trace(void* device_buf) { g_knn_trace = reinterpret_cast<unsigned long long*>(device_buf); }
 
 int knn_tc_candidates(const float* X, const float* sq, const float* rscale, const unsigned* small, int n, int d, int row_end, const TcPlan& plan,
-                      void* tc_ws, u64* cand, const u64* excl, unsigned* thr_g, cudaStream_t st) {
+                      void* tc_ws, u64* cand, const u64* excl, unsigned* thr_g, cudaStream_t st, const SegDev* seg) {
   __half* H = reinterpret_cast<__half*>(tc_ws);
   __half* L = reinterpret_cast<__half*>((char*)tc_ws + align_up((size_t)n * plan.d_pad * 2, 256));
   // H and L (fp16 hi / lo of the scaled rows, row stride d_pad) were written by sqnorm_split_f16_kernel (knn.cu); with one
@@ -1038,6 +1158,10 @@ int knn_tc_candidates(const float* X, const float* sq, const float* rscale, cons
   P.passes = plan.passes;
   P.rscale = rscale;
   P.small = small;
+  const bool segd = seg != nullptr;
+  SegDev S;
+  if (segd) S = *seg;
+  else memset(&S, 0, sizeof(S));
   {
     const char* dbg = getenv("GLL_B200_KNN_DEBUG");
     P.debug = dbg ? atoi(dbg) : 0;
@@ -1051,8 +1175,9 @@ int knn_tc_candidates(const float* X, const float* sq, const float* rscale, cons
     const char* e = getenv("GLL_B200_KNN_ARES");
     P.ares = (fits && (e ? atoi(e) != 0 : plan.aligned != 0)) ? 1 : 0;
   }
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)knn_gram_topk_tc_kernel<false>, (int)TC_SMEM_BYTES));
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)knn_gram_topk_tc_kernel<true>, (int)TC_SMEM_BYTES));
+  auto kern = segd ? (plan.rstep == 2 ? knn_gram_topk_tc_kernel<true, true> : knn_gram_topk_tc_kernel<false, true>)
+                   : (plan.rstep == 2 ? knn_gram_topk_tc_kernel<true, false> : knn_gram_topk_tc_kernel<false, false>);
+  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)TC_SMEM_BYTES));
   {
     GLL_PROF(KID_GRAM_TOPK_TC, st);
     if (plan.rstep == 2) {
@@ -1069,9 +1194,9 @@ int knn_tc_candidates(const float* X, const float* sq, const float* rscale, cons
       attr[0].val.clusterDim.z = 1;
       cfg.attrs = attr;
       cfg.numAttrs = 1;
-      GLL_CUDA_CHECK(cudaLaunchKernelEx(&cfg, knn_gram_topk_tc_kernel<true>, mAH, mAL, mBH, P));
+      GLL_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, mAH, mAL, mBH, P, S));
     } else {
-      knn_gram_topk_tc_kernel<false><<<plan.grid, TC_THREADS, TC_SMEM_BYTES, st>>>(mAH, mAL, mBH, P);
+      kern<<<plan.grid, TC_THREADS, TC_SMEM_BYTES, st>>>(mAH, mAL, mBH, P, S);
     }
   }
   GLL_LAUNCH_CHECK();

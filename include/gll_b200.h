@@ -129,6 +129,20 @@ size_t gll_knn_workspace_bytes(int n, int d, int k);
 int gll_knn(const float* X, int n, int d, int k, int* knn_idx, float* knn_dist, int* info,
             void* workspace, size_t workspace_bytes, void* stream);
 
+/* K1 over independent graphs stacked as row segments: segment s is rows [seg_ptr_host[s], seg_ptr_host[s+1]) of X (n x d),
+ * seg_ptr_host a HOST array of nseg + 1 offsets from 0 to n (the search is planned on the host: no sync).  Row i of segment s
+ * gets its k nearest neighbours among the rows of s only (global row numbers, self in slot 0, then by (distance, index)):
+ * bit-identical to gll_knn on each segment alone plus the segment's offset, because those lists are exact.  Every segment
+ * needs >= k rows; 2 <= k <= 33.  The tensor-core search only issues the (row tile, column tile) units whose columns meet
+ * the segments of the tile's rows, O(sum n_s^2 d) work instead of O(n^2 d).  nseg == 1 runs gll_knn.  Bad arguments
+ * return GLL_ERR_ARG before any CUDA call; the workspace query returns 0 for them.  gll_knn_segments_units (host query,
+ * for benchmarks): tensor-core units such a call issues, and those of the uniform grid over the same rows (0, 0 when
+ * the SIMT path runs). */
+size_t gll_knn_segments_workspace_bytes(int n, int d, int k, const int* seg_ptr_host, int nseg);
+int gll_knn_segments(const float* X, int n, int d, int k, const int* seg_ptr_host, int nseg, int* knn_idx, float* knn_dist,
+                     int* info, void* workspace, size_t workspace_bytes, void* stream);
+void gll_knn_segments_units(int n, int d, const int* seg_ptr_host, int nseg, long long* seg_units, long long* uniform_units);
+
 /* K2. Symmetrise (elementwise max == union graph) and build the CSR; zero distances and self loops are
  * not edges.  Replaces the scipy sequence at GLL.py:192-198. col/dist need gll_max_edges(n,k) entries. */
 size_t gll_graph_workspace_bytes(int n, int k);
@@ -299,6 +313,20 @@ int gll_backward(const float* X, const void* grad_out, int grad_is_f64, int n, i
 int gll_backward_scaled(const float* X, const void* grad_out, int grad_is_f64, const void* scale, int scale_is_f64, int n, int d,
                         int k, int l, int k_lab, int eps_auto, float cg_tol, int cg_max_iter, void* state, float* dX,
                         void* workspace, size_t workspace_bytes, void* stream);
+
+/* Batched forward of B independent graphs of the same shape (LaplaceLearningSparseHardBatched): X is B x n x d and Y is
+ * B x k_lab x l, each graph's labeled rows first.  The B graphs are ONE block-diagonal graph whose rows are ordered labeled
+ * first: all graphs' labeled rows (graph-major), then all graphs' unlabeled rows (graph-major), each graph's rows in their
+ * own order.  The kNN search runs per graph (gll_knn_segments); graph, weights and the CG are gll_forward's stages on the
+ * union, so state has the layout of gll_state_layout(B n, k, l, B k_lab), its kNN lists, CSR, eps, kappa, W and degrees are
+ * per graph bit-identical to gll_forward's, and pred_out (B*(n - k_lab)) x l is graph-major: a (B, m, l) tensor.  One
+ * multi-RHS CG solves all graphs (step lengths shared, each class column stops when its residual over all graphs is
+ * <= cg_tol, which bounds every graph's), so pred matches per-graph calls to the solver tolerance, not bit for bit, for B > 1.
+ * The backward is gll_backward_scaled(Xg, ..., B n, d, k, l, B k_lab, ...) on Xg = X in labeled-first order. */
+size_t gll_batched_workspace_bytes(int B, int n, int d, int k, int l, int k_lab);
+int gll_forward_batched(const float* X, const float* Y, int B, int n, int d, int k, int l, int k_lab, int eps_auto,
+                        float eps_fixed, float tau, float cg_tol, int cg_max_iter, void* state, void* pred_out,
+                        int pred_is_f64, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Laplace-learning evaluation, the reference's utils.laplace (utils.py:570-593) as test_GL_NP calls it (utils.py:637-660):
