@@ -118,6 +118,9 @@ def _load():
     sig("gll_forward_batched", i32, [vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, f32, f32, i32, vp, vp, i32, vp, sz, vp])
     sig("gll_laplace_eval_workspace_bytes", sz, [i32, i32, i32, i32, i32])
     sig("gll_laplace_eval", i32, [vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp, vp, vp, vp, sz, vp])
+    sig("gll_laplace_eval_batched_workspace_bytes", sz, [i32, i32, i32, i32, i32, i32])
+    sig("gll_laplace_eval_batched", i32, [vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp, vp, vp,
+                                          vp, vp, sz, vp])
     return lib
 
 
@@ -136,7 +139,7 @@ EXPORTS = ["gll_last_error", "gll_version", "gll_device_sm_count", "gll_kernel_c
            "gll_normalize_rows_backward", "gll_debug_gram_tile", "gll_base_cache_bytes", "gll_base_cache_workspace_bytes",
            "gll_base_cache_build", "gll_knn_cached_workspace_bytes", "gll_knn_cached", "gll_laplace_eval_workspace_bytes",
            "gll_laplace_eval", "gll_knn_segments_workspace_bytes", "gll_knn_segments", "gll_knn_segments_units",
-           "gll_batched_workspace_bytes", "gll_forward_batched"]
+           "gll_batched_workspace_bytes", "gll_forward_batched", "gll_laplace_eval_batched_workspace_bytes", "gll_laplace_eval_batched"]
 
 
 def check(rc: int, what: str) -> None:

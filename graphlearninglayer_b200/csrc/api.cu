@@ -710,14 +710,45 @@ static std::vector<int> uniform_segments(int B, int n) {
   return seg;
 }
 
-size_t gll_batched_workspace_bytes(int B, int n, int d, int k, int l, int k_lab) {
-  if (!batched_sizes_ok(B, n, d, k, l, k_lab)) return 0;
+}  // extern "C"
+
+namespace gll {
+
+size_t batched_ws_bytes(int B, int n, int d, int k, int l, int k_lab) {
   const int N = B * n;
   const std::vector<int> seg = uniform_segments(B, n);
   const size_t lists = 2 * align_up(sizeof(int) * (size_t)N * k, 256);  // the search's lists in natural order
-  size_t b = lists + knn_seg_ws_bytes(N, d, k, seg.data(), B) + 256;
+  const size_t s = knn_seg_ws_bytes(N, d, k, seg.data(), B);
+  if (s == 0) return 0;
+  size_t b = lists + s + 256;
   b = std::max(b, graph_weights_ws_bytes(N, k));
   return std::max(b, cg_ws_bytes(N - B * k_lab, l));
+}
+
+int batched_knn_run(const float* X, int B, int n, int d, int k, int k_lab, const GraphBufs& G, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const int N = B * n;
+  Carver cv(ws, ws_bytes);
+  int* idx = cv.take<int>((size_t)N * k);
+  float* dist = cv.take<float>((size_t)N * k);
+  char* kws = cv.take<char>(0);
+  const std::vector<int> seg = uniform_segments(B, n);
+  const int rc = knn_run_segments(X, N, d, k, seg.data(), B, idx, dist, G.info, kws, ws_bytes - (size_t)(kws - (char*)ws), st);
+  if (rc) return rc;
+  {
+    GLL_PROF(KID_BATCH_REORDER, st);
+    knn_to_labeled_first_kernel<<<ceil_div((long long)N * k, 256), 256, 0, st>>>(idx, dist, B, n, k, k_lab, G.knn_idx, G.knn_dist);
+  }
+  GLL_LAUNCH_CHECK();
+  return GLL_OK;
+}
+
+}  // namespace gll
+
+extern "C" {
+
+size_t gll_batched_workspace_bytes(int B, int n, int d, int k, int l, int k_lab) {
+  if (!batched_sizes_ok(B, n, d, k, l, k_lab)) return 0;
+  return batched_ws_bytes(B, n, d, k, l, k_lab);
 }
 
 int gll_forward_batched(const float* X, const float* Y, int B, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
@@ -731,18 +762,8 @@ int gll_forward_batched(const float* X, const float* Y, int B, int n, int d, int
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   GLL_CUDA_CHECK(cudaMemsetAsync(G.info, 0, sizeof(int) * GLL_INFO_WORDS, st));
-  Carver cv(workspace, workspace_bytes);
-  int* idx = cv.take<int>((size_t)N * k);
-  float* dist = cv.take<float>((size_t)N * k);
-  char* kws = cv.take<char>(0);
-  const std::vector<int> seg = uniform_segments(B, n);
-  rc = knn_run_segments(X, N, d, k, seg.data(), B, idx, dist, G.info, kws, workspace_bytes - (size_t)(kws - (char*)workspace), st);
+  rc = batched_knn_run(X, B, n, d, k, k_lab, G, workspace, workspace_bytes, st);
   if (rc) return rc;
-  {
-    GLL_PROF(KID_BATCH_REORDER, st);
-    knn_to_labeled_first_kernel<<<ceil_div((long long)N * k, 256), 256, 0, st>>>(idx, dist, B, n, k, k_lab, G.knn_idx, G.knn_dist);
-  }
-  GLL_LAUNCH_CHECK();
   return forward_solve(G, Y, N, k, l, K, eps_auto, eps_fixed, tau, cg_tol, cg_max_iter, pred_out, pred_is_f64, workspace, workspace_bytes,
                        st);
 }

@@ -160,6 +160,11 @@ GraphBufs graph_bufs(const gll_layout& L, void* state);
 int graph_stages_run(const GraphBufs& B, const float* Y, int n, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau,
                      int phase_begin, int phase_end, void* ws, size_t ws_bytes, cudaStream_t st);
 size_t graph_ws_bytes(int n, int k);
+// B stacked graphs of n rows (api.cu): the stage workspace of the batched drivers (the segmented search and its lists in natural
+// order, the graph stages and the CG on the union; 0 for sizes the search refuses), and the segmented search itself followed by
+// the reorder of its lists into B.knn_idx / B.knn_dist in labeled-first order
+size_t batched_ws_bytes(int B, int n, int d, int k, int l, int k_lab);
+int batched_knn_run(const float* X, int B, int n, int d, int k, int k_lab, const GraphBufs& G, void* ws, size_t ws_bytes, cudaStream_t st);
 size_t weights_ws_bytes(int n, int k);
 size_t graph_weights_ws_bytes(int n, int k);
 

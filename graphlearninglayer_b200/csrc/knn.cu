@@ -579,7 +579,7 @@ template <bool VEC4>
 __global__ void __launch_bounds__(FB_WARPS * 32)
 knn_fallback_kernel(const float* __restrict__ X, int n, int d, int k, const int* __restrict__ flag_count,
                     const int* __restrict__ flag_rows, int* __restrict__ knn_idx, float* __restrict__ knn_dist,
-                    int* __restrict__ info) {
+                    int* __restrict__ info, const int2* __restrict__ win) {
   extern __shared__ __align__(16) float xs[];
   __shared__ double sd[FB_WARPS][32];
   __shared__ int sj[FB_WARPS][32];
@@ -591,6 +591,7 @@ knn_fallback_kernel(const float* __restrict__ X, int n, int d, int k, const int*
   }
   for (int f = blockIdx.x; f < nflag; f += gridDim.x) {
     const int i = flag_rows[f];
+    const int2 w = (win != nullptr) ? win[i] : make_int2(0, n);  // a segmented search scans the row's own segment
     for (int t = threadIdx.x; t < d; t += blockDim.x) xs[t] = X[(size_t)i * d + t];
     __syncthreads();
     // k - 1 <= 32 neighbours fit one 32-wide list; larger k takes a second scan that only admits pairs beyond the 32nd
@@ -600,7 +601,7 @@ knn_fallback_kernel(const float* __restrict__ X, int n, int d, int k, const int*
     for (int pass = 0; pass * 32 < k - 1; ++pass) {
       double md = INFINITY;
       int mj = 0x7fffffff;
-      for (int j = warp; j < n; j += FB_WARPS) {
+      for (int j = w.x + warp; j < w.y; j += FB_WARPS) {
         if (j == i) continue;
         double v = exact_d2<VEC4>(xs, X + (size_t)j * d, d, lane);
         if (v > ex_d || (v == ex_d && j > ex_j)) list_insert_d(md, mj, v, j, lane);
@@ -795,7 +796,7 @@ knn_merge_kernel(int row_end, CandLayout lay, const u64* __restrict__ cand, u64*
   const int i = lay.row_begin + blockIdx.x * RERANK_WARPS + warp;
   if (i >= row_end) return;
   int splits = lay.stride;
-  if (lay.tc == 1) {
+  if (lay.tc == 1 || lay.tc == 3) {
     int b0, b1;
     cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
     splits = 2 * (b1 - b0 + 1);  // every CTA writes two lists per row (the column halves of its epilogue)
@@ -813,7 +814,7 @@ __global__ void __launch_bounds__(RERANK_WARPS * 32)
 knn_rerank64_kernel(const float* __restrict__ X, const float* __restrict__ sq, const unsigned* __restrict__ sqmax_bits, int n, int d,
                     int k, int row_begin, int row_end, const u64* __restrict__ m1, const u64* __restrict__ m2, float err_coef,
                     int* __restrict__ knn_idx, float* __restrict__ knn_dist, int* __restrict__ flag_count,
-                    int* __restrict__ flag_rows) {
+                    int* __restrict__ flag_rows, int force_rows) {
   extern __shared__ __align__(16) float xs[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int i = row_begin + blockIdx.x * RERANK_WARPS + warp;
@@ -879,6 +880,7 @@ knn_rerank64_kernel(const float* __restrict__ X, const float* __restrict__ sq, c
     const double errb = knn_err_bound(err_coef, sq[i], sqmax_bits);
     ok = ((double)lower - errb > dk) || (lower == INFINITY);
   }
+  if (i - row_begin < force_rows) ok = false;  // GLL_B200_KNN_FORCE_FALLBACK (tests): treat the first rows as unproven
   if (!ok && lane == 0) {
     int p = atomicAdd(flag_count, 1);
     flag_rows[p] = i;
@@ -939,22 +941,24 @@ int knn_finish(const float* X, const float* sq, const unsigned* sqmax_bits, int 
 
 static int knn_finish64(const float* X, const float* sq, const unsigned* sqmax_bits, int n, int d, int k, int row_begin, int row_end,
                        const u64* m1, const u64* m2, float err_coef, int* knn_idx, float* knn_dist, int* flag_count,
-                       int* flag_rows, int* info, cudaStream_t st) {
+                       int* flag_rows, int* info, cudaStream_t st, const int2* win) {
   const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
   const size_t smem = sizeof(float) * (size_t)RERANK_WARPS * d;
   const int blocks = ceil_div(row_end - row_begin, RERANK_WARPS);
+  int force_rows = 0;
+  if (const char* e = getenv("GLL_B200_KNN_FORCE_FALLBACK")) force_rows = atoi(e);
   {
     GLL_PROF(KID_RERANK, st);
     if (vec4) {
       if (smem > 48 * 1024)
         GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_rerank64_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       knn_rerank64_kernel<true><<<blocks, RERANK_WARPS * 32, smem, st>>>(X, sq, sqmax_bits, n, d, k, row_begin, row_end, m1, m2,
-                                                                          err_coef, knn_idx, knn_dist, flag_count, flag_rows);
+                                                                          err_coef, knn_idx, knn_dist, flag_count, flag_rows, force_rows);
     } else {
       if (smem > 48 * 1024)
         GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_rerank64_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       knn_rerank64_kernel<false><<<blocks, RERANK_WARPS * 32, smem, st>>>(X, sq, sqmax_bits, n, d, k, row_begin, row_end, m1, m2,
-                                                                           err_coef, knn_idx, knn_dist, flag_count, flag_rows);
+                                                                           err_coef, knn_idx, knn_dist, flag_count, flag_rows, force_rows);
     }
   }
   GLL_LAUNCH_CHECK();
@@ -964,9 +968,9 @@ static int knn_finish64(const float* X, const float* sq, const unsigned* sqmax_b
   {
     GLL_PROF(KID_KNN_FALLBACK, st);
     if (vec4)
-      knn_fallback_kernel<true><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info);
+      knn_fallback_kernel<true><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info, win);
     else
-      knn_fallback_kernel<false><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info);
+      knn_fallback_kernel<false><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info, win);
   }
   GLL_LAUNCH_CHECK();
   return GLL_OK;
@@ -1146,6 +1150,35 @@ int knn_debug_gram_tile(const float* X, int n, int d, int row_tile, int col_tile
   return knn_tc_debug_tile(plan, n, tc_ws, row_tile, col_tile, acc_out, st);
 }
 
+// ---- k in (33, 64]: two rounds of the tensor-core search, the second admits only keys beyond the first round's 32nd ----
+// The merged lists and excl are carved from cv behind the search's buffers; seg != NULL: the segmented unit grid (lay.tc == 3,
+// or 2 when aligned), whose masked columns never enter a set in either round.
+static int knn_run64(const float* X, const KnnBufs& kb, Carver& cv, int n, int d, int k, int row_begin, int row_end, const TcPlan& plan,
+                     const CandLayout& lay, int* knn_idx, float* knn_dist, int* info, cudaStream_t st, const SegDev* seg) {
+  const int rows = row_end - row_begin;
+  u64* merged1 = cv.take<u64>((size_t)rows * KC);
+  u64* merged2 = cv.take<u64>((size_t)rows * KC);
+  u64* excl = cv.take<u64>(n);
+  const int mblocks = ceil_div(rows, RERANK_WARPS);
+  int rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, row_end, plan, kb.tc_ws, kb.cand, nullptr, kb.thr_g, st, seg);
+  if (rc) return rc;
+  {
+    GLL_PROF(KID_RERANK, st);
+    knn_merge_kernel<<<mblocks, RERANK_WARPS * 32, 0, st>>>(row_end, lay, kb.cand, merged1, excl);
+  }
+  GLL_LAUNCH_CHECK();
+  // second round: own thresholds
+  rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, row_end, plan, kb.tc_ws, kb.cand, excl, nullptr, st, seg);
+  if (rc) return rc;
+  {
+    GLL_PROF(KID_RERANK, st);
+    knn_merge_kernel<<<mblocks, RERANK_WARPS * 32, 0, st>>>(row_end, lay, kb.cand, merged2, nullptr);
+  }
+  GLL_LAUNCH_CHECK();
+  return knn_finish64(X, kb.sq, kb.small, n, d, k, row_begin, row_end, merged1, merged2, knn_tc_err_coef(d, plan.passes), knn_idx, knn_dist,
+                      kb.flag_count, kb.flag_rows, info, st, seg ? seg->win : nullptr);
+}
+
 int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int* knn_idx, float* knn_dist, int* info,
             void* ws, size_t ws_bytes, cudaStream_t st) {
   GLL_REQUIRE(X && knn_idx && knn_dist && ws, "null pointer");
@@ -1179,29 +1212,8 @@ int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int
   }
 
   if (k > KC + 1) {
-    // ---- k in (33, 64]: two rounds of the tensor-core search, the second admits only keys beyond the first round's 32nd ----
     GLL_REQUIRE(plan.ok, "k > 33 needs the tensor-core path (n >= 256, row range starting on a multiple of 128)");
-    u64* merged1 = cv.take<u64>((size_t)rows * KC);
-    u64* merged2 = cv.take<u64>((size_t)rows * KC);
-    u64* excl = cv.take<u64>(n);
-    lay = layout_of(plan, row_begin);
-    const int mblocks = ceil_div(rows, RERANK_WARPS);
-    int rc = knn_tc_candidates(X, sq, rscale, small, n, d, row_end, plan, tc_ws, cand, nullptr, thr_g, st);
-    if (rc) return rc;
-    {
-      GLL_PROF(KID_RERANK, st);
-      knn_merge_kernel<<<mblocks, RERANK_WARPS * 32, 0, st>>>(row_end, lay, cand, merged1, excl);
-    }
-    GLL_LAUNCH_CHECK();
-    rc = knn_tc_candidates(X, sq, rscale, small, n, d, row_end, plan, tc_ws, cand, excl, nullptr, st);  // second round: own thresholds
-    if (rc) return rc;
-    {
-      GLL_PROF(KID_RERANK, st);
-      knn_merge_kernel<<<mblocks, RERANK_WARPS * 32, 0, st>>>(row_end, lay, cand, merged2, nullptr);
-    }
-    GLL_LAUNCH_CHECK();
-    return knn_finish64(X, sq, sqmax_bits, n, d, k, row_begin, row_end, merged1, merged2, knn_tc_err_coef(d, plan.passes), knn_idx, knn_dist,
-                        flag_count, flag_rows, info, st);
+    return knn_run64(X, kb, cv, n, d, k, row_begin, row_end, plan, layout_of(plan, row_begin), knn_idx, knn_dist, info, st, nullptr);
   }
   if (plan.ok) {  // tcgen05 / TMA Gram GEMM with the fused top-k epilogue
     int rc = knn_tc_candidates(X, sq, rscale, small, n, d, row_end, plan, tc_ws, cand, nullptr, thr_g, st);
@@ -1282,7 +1294,7 @@ SegPlan seg_plan(int n, int d, const int* seg_ptr, int nseg) {
 int knn_seg_check(int n, int d, int k, const int* seg_ptr, int nseg) {
   GLL_REQUIRE(seg_ptr != nullptr, "null seg_ptr");
   GLL_REQUIRE(nseg >= 1 && n >= 1 && d >= 1, "bad sizes");
-  GLL_REQUIRE(k >= 2 && k <= KC + 1, "the segmented search serves 2 <= k <= 33");
+  GLL_REQUIRE(k >= 2 && k <= 2 * KC && (k <= KC + 1 || n >= 2 * 128), "need 2 <= k <= 64, and n >= 256 when k > 33");
   GLL_REQUIRE(seg_ptr[0] == 0 && seg_ptr[nseg] == n, "seg_ptr must run from 0 to n");
   for (int s = 0; s < nseg; ++s)
     if (seg_ptr[s + 1] - seg_ptr[s] < k) {
@@ -1299,6 +1311,7 @@ size_t knn_seg_ws_bytes(int n, int d, int k, const int* seg_ptr, int nseg) {
   size_t b = knn_common_bytes(n, d, (size_t)n, p.stride);
   b += align_up(sizeof(int2) * (size_t)n, 256);                                      // windows
   b += align_up(sizeof(int) * ((size_t)nseg + 1 + p.tab.size()), 256);               // seg_ptr + unit table
+  if (k > KC + 1) b += 2 * align_up(sizeof(u64) * (size_t)n * KC, 256) + align_up(sizeof(u64) * (size_t)n, 256);  // merged lists, excl
   return b + 2048;
 }
 
@@ -1315,6 +1328,7 @@ int knn_run_segments(const float* X, int n, int d, int k, const int* seg_ptr, in
   }
   const SegPlan sp = seg_plan(n, d, seg_ptr, nseg);
   const TcPlan& plan = sp.tc;
+  GLL_REQUIRE(k <= KC + 1 || plan.ok, "k > 33 needs the tensor-core path");
   Carver cv(ws, ws_bytes);
   const KnnBufs kb = knn_carve(cv, n, d, 0, n, sp.stride);
   int2* win = cv.take<int2>(n);
@@ -1346,9 +1360,10 @@ int knn_run_segments(const float* X, int n, int d, int k, const int* seg_ptr, in
     sd.gfirst = ints + nseg + 1;
     sd.gct = sd.gfirst + RG + 1;
     sd.bstart = sd.gct + RG;
+    lay = layout_of(plan, 0, sd.gfirst);
+    if (k > KC + 1) return knn_run64(X, kb, cv, n, d, k, 0, n, plan, lay, knn_idx, knn_dist, info, st, &sd);
     const int rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, n, plan, kb.tc_ws, kb.cand, nullptr, kb.thr_g, st, &sd);
     if (rc) return rc;
-    lay = layout_of(plan, 0, sd.gfirst);
     err_coef = knn_tc_err_coef(d, plan.passes);
   } else {
     const int rc = launch_simt(X, kb.sq, n, d, sp.cps, sp.stride, kb.cand, 0, n, win, st);

@@ -33,29 +33,35 @@ struct RefineParams {
   const float* e;        // m x lp fp32 correction (round 0: the initial solution)
   double* x_out;         // m x l
   double* r_out;         // m x l: right-hand side of the correction solve
-  double* partial;       // [gridDim.x][l]
-  double* colnorm;       // [l]
+  double* partial;       // [B][gx][l]
+  double* colnorm;       // [B][l]
+  double* gmax;          // [B]: per graph, the largest column norm (NaN: a column is not finite)
+  double* resid;         // [B] or NULL: the caller's copy of gmax
   double* scale;         // 1 scalar
-  unsigned* ticket;
+  unsigned* ticket;      // [B + 1]: CTAs done per graph, then graphs done
   int* info;
-  int n, k_lab, m, l, lp, cw, round;
+  int n, k_lab, m, mb, B, gx, l, lp, cw, round;
   double tau, tol;
 };
 
-// Block = RL row lanes x CW class columns (CW = min(l, 32)); blockIdx.y picks a chunk of CW columns.  A thread walks the rows
-// of its lane in a fixed order and keeps its own partial sum of r^2 / diag: the reduction order depends on nothing but the
-// launch shape.
+// B graphs whose unlabeled rows are the consecutive ranges [b mb, (b + 1) mb) of the m = B mb unlabeled rows (B = 1: one graph).
+// Block = RL row lanes x CW class columns (CW = min(l, 32)); blockIdx.x = b gx + (CTA of graph b), blockIdx.y picks a chunk of CW
+// columns.  A thread walks the rows of its lane in graph b in a fixed order and keeps its own partial sum of r^2 / diag: the
+// reduction order depends on nothing but the launch shape.  The last CTA of graph b (integer ticket) adds that graph's per-CTA
+// column partials in CTA order and writes the graph's largest column norm; the last graph to finish takes the maximum over
+// graphs, which decides the correction scale and the info slots.  No floating-point atomics.
 __global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(RefineParams P) {
   __shared__ double red[LR_THREADS];
   __shared__ bool last;
   const int cw = P.cw, rl_count = LR_THREADS / cw;
   const int tid = threadIdx.x, rl = tid / cw, cc = tid - rl * cw;
   const int c = blockIdx.y * cw + cc;
+  const int b = blockIdx.x / P.gx, bx = blockIdx.x - b * P.gx;
   const bool active = rl < rl_count && c < P.l;
   double acc = 0.0;
   if (active) {
-    const int l = P.l, lp = P.lp, k_lab = P.k_lab;
-    for (int i = blockIdx.x * rl_count + rl; i < P.m; i += gridDim.x * rl_count) {
+    const int l = P.l, lp = P.lp, k_lab = P.k_lab, i_end = (b + 1) * P.mb;
+    for (int i = b * P.mb + bx * rl_count + rl; i < i_end; i += P.gx * rl_count) {
       const size_t o = (size_t)i * l + c;
       const double xi = (P.x_prev ? __ldg(P.x_prev + o) : 0.0) + (double)__ldg(P.e + (size_t)i * lp + c);
       P.x_out[o] = xi;
@@ -88,26 +94,53 @@ __global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(RefineParams
   }
   __threadfence();
   __syncthreads();
-  if (tid == 0) last = atomicAdd(P.ticket, 1u) == gridDim.x * gridDim.y - 1u;
+  if (tid == 0) last = atomicAdd(P.ticket + b, 1u) == P.gx * gridDim.y - 1u;
   __syncthreads();
   if (!last) return;
   __threadfence();
   const int lane = tid & 31, warp = tid >> 5;
+  const double* part = P.partial + (size_t)b * P.gx * P.l;
+  double* colnorm = P.colnorm + (size_t)b * P.l;
   for (int cc2 = warp; cc2 < P.l; cc2 += LR_THREADS / 32) {
     double t = 0.0;
-    for (int b = lane; b < (int)gridDim.x; b += 32) t += __ldcg(P.partial + (size_t)b * P.l + cc2);
+    for (int q = lane; q < P.gx; q += 32) t += __ldcg(part + (size_t)q * P.l + cc2);
     t = warp_sum(t);
-    if (lane == 0) P.colnorm[cc2] = sqrt(t);
+    if (lane == 0) colnorm[cc2] = sqrt(t);
   }
   __syncthreads();
   if (tid == 0) {
     double mx = 0.0;
     bool bad = false;
     for (int cc2 = 0; cc2 < P.l; ++cc2) {
-      const double v = P.colnorm[cc2];
+      const double v = colnorm[cc2];
       if (!(v == v) || isinf(v)) bad = true;
       mx = fmax(mx, v);
     }
+    const double gv = bad ? __longlong_as_double(0x7ff8000000000000LL) : mx;
+    P.gmax[b] = gv;
+    if (P.resid != nullptr) P.resid[b] = gv;
+    P.ticket[b] = 0u;  // rewound for the next round
+    __threadfence();
+    last = atomicAdd(P.ticket + P.B, 1u) == (unsigned)P.B - 1u;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  // maximum over graphs: exact, so the order of the reduction does not matter
+  double mx = 0.0;
+  bool bad = false;
+  for (int g = tid; g < P.B; g += LR_THREADS) {
+    const double v = __ldcg(P.gmax + g);
+    if (!(v == v)) bad = true;
+    mx = fmax(mx, v);
+  }
+  bad = __syncthreads_or(bad) != 0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(FULL, mx, o));
+  if (lane == 0) red[warp] = mx;
+  __syncthreads();
+  if (tid == 0) {
+    for (int w = 1; w < LR_THREADS / 32; ++w) mx = fmax(mx, red[w]);
     const bool more = bad || !(mx <= P.tol);
     *P.scale = more ? 1.0 : 0.0;
     if (more) P.info[GLL_INFO_LAPLACE_ROUNDS] = P.round + 1;
@@ -115,20 +148,21 @@ __global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(RefineParams
     const float fr = bad ? __int_as_float(0x7fc00000) : (float)mx;
     P.info[GLL_INFO_LAPLACE_RESID] = __float_as_int(fr);
     if (P.round == 0) P.info[GLL_INFO_LAPLACE_RESID0] = __float_as_int(fr);
-    *P.ticket = 0u;  // rewound for the next round
+    P.ticket[P.B] = 0u;
   }
 }
 
-// Thread per unlabeled row: pred = x + e (in place), labels = first maximal column, hits counted with one integer atomic per CTA.
-// CTA 0 also writes the correction-CG iteration counts and the convergence status.
+// Thread per unlabeled row: pred = x + e (in place), labels = first maximal column, hits counted with one integer atomic per CTA
+// into correct[b].  The fb CTAs of graph b cover its rows [b mb, (b + 1) mb).  CTA 0 also writes the correction-CG iteration
+// counts and the convergence status.
 __global__ void __launch_bounds__(LR_THREADS)
-laplace_finish_kernel(double* __restrict__ pred, const float* __restrict__ e, int m, int l, int lp, long long* __restrict__ labels,
+laplace_finish_kernel(double* __restrict__ pred, const float* __restrict__ e, int mb, int fb, int l, int lp, long long* __restrict__ labels,
                       const long long* __restrict__ targets, unsigned long long* __restrict__ correct, const double* __restrict__ scale,
                       const int* __restrict__ round_iters, int rounds, int* __restrict__ info) {
   __shared__ int part[LR_THREADS / 32];
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int b = blockIdx.x / fb, t = (blockIdx.x - b * fb) * blockDim.x + threadIdx.x, i = b * mb + t;
   int hit = 0;
-  if (i < m) {
+  if (t < mb) {
     double best = 0.0;
     int arg = 0;
     for (int c = 0; c < l; ++c) {
@@ -142,8 +176,8 @@ laplace_finish_kernel(double* __restrict__ pred, const float* __restrict__ e, in
     }
     labels[i] = arg;
     if (targets != nullptr) {
-      const long long t = __ldg(targets + i);
-      hit = (t >= 0 && t == (long long)arg) ? 1 : 0;
+      const long long tg = __ldg(targets + i);
+      hit = (tg >= 0 && tg == (long long)arg) ? 1 : 0;
     }
   }
   if (correct != nullptr) {
@@ -153,7 +187,7 @@ laplace_finish_kernel(double* __restrict__ pred, const float* __restrict__ e, in
     if (threadIdx.x == 0) {
       int s = 0;
       for (int w = 0; w < LR_THREADS / 32; ++w) s += part[w];
-      if (s) atomicAdd(correct, (unsigned long long)s);
+      if (s) atomicAdd(correct + b, (unsigned long long)s);
     }
   }
   if (blockIdx.x == 0 && threadIdx.x == 0) {
@@ -171,35 +205,146 @@ laplace_finish_kernel(double* __restrict__ pred, const float* __restrict__ e, in
   }
 }
 
-int refine_grid_x(int m, int l) {
+// CTAs per graph of laplace_refine (mb unlabeled rows per graph)
+int refine_grid_x(int mb, int l) {
   const int cw = min(l, 32), rl = LR_THREADS / cw;
-  return max(1, min(ceil_div(m, rl), 4 * device_info().sms));
+  return max(1, min(ceil_div(mb, rl), 4 * device_info().sms));
 }
 
 // the evaluation's own buffers, behind the layer state and in front of the stage workspace
 struct EvalBufs {
   double* xtmp;    // m x l
   double* r;       // m x l
-  double* partial; // [refine grid][l]
-  double* colnorm; // [l]
+  double* partial; // [B][refine grid][l]
+  double* colnorm; // [B][l]
+  double* gmax;    // [B]
   double* scale;
-  unsigned* ticket;
+  unsigned* ticket;  // [B + 1]
   int* round_iters;  // [GLL_LAPLACE_ROUNDS]
 };
 
 // base == NULL: size query only
-size_t eval_bufs(char* base, int m, int l, EvalBufs* B) {
+size_t eval_bufs(char* base, int B, int mb, int l, EvalBufs* E) {
   Carver cv(base, ~(size_t)0);
+  const size_t m = (size_t)B * mb;
   EvalBufs b;
-  b.xtmp = cv.take<double>((size_t)m * l);
-  b.r = cv.take<double>((size_t)m * l);
-  b.partial = cv.take<double>((size_t)refine_grid_x(m, l) * l);
-  b.colnorm = cv.take<double>(l);
+  b.xtmp = cv.take<double>(m * l);
+  b.r = cv.take<double>(m * l);
+  b.partial = cv.take<double>((size_t)B * refine_grid_x(mb, l) * l);
+  b.colnorm = cv.take<double>((size_t)B * l);
+  b.gmax = cv.take<double>(B);
   b.scale = cv.take<double>(1);
-  b.ticket = cv.take<unsigned>(1);
+  b.ticket = cv.take<unsigned>((size_t)B + 1);
   b.round_iters = cv.take<int>(GLL_LAPLACE_ROUNDS);
-  if (B) *B = b;
+  if (E) *E = b;
   return align_up(cv.off, 256);
+}
+
+// workspace of B graphs of n rows: [layer state of the union | the evaluation's buffers | stage workspace]; 0 for sizes the stages
+// refuse
+size_t eval_ws_bytes(int B, int n, int d, int k, int l, int k_lab) {
+  gll_layout L;
+  if (gll_state_layout(B * n, k, l, B * k_lab, &L)) return 0;
+  const size_t stage = (B == 1) ? gll_workspace_bytes(n, d, k, l, k_lab) : batched_ws_bytes(B, n, d, k, l, k_lab);
+  if (stage == 0) return 0;
+  return L.total + eval_bufs(nullptr, B, n - k_lab, l, nullptr) + stage;
+}
+
+// the sizes gll_laplace_eval_batched accepts
+bool eval_batched_sizes_ok(int B, int n, int d, int k, int l, int k_lab) {
+  if (B < 1 || n < 1 || (long long)B * n > 0x7fffffffLL) return false;
+  return k >= 2 && k <= 64 && k <= n && (k <= 33 || (long long)B * n >= 256) && d >= 1 && l >= 1 && k_lab >= 1 && k_lab < n;
+}
+
+// gll_laplace_eval (B = 1) and gll_laplace_eval_batched: sizes are checked by the callers
+int eval_run(const float* X, const float* Y, int B, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed, float tau,
+             double tol, int cg_max_iter, double* pred, long long* labels, const long long* targets, long long* correct_out,
+             double* resid_out, int* info, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const size_t need = eval_ws_bytes(B, n, d, k, l, k_lab);
+  if (workspace_bytes < need) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, need);
+    return GLL_ERR_WORKSPACE;
+  }
+  const int N = B * n, K = B * k_lab, mb = n - k_lab, m = N - K, lp = padded_classes(l);
+  gll_layout L;
+  if (gll_state_layout(N, k, l, K, &L)) return GLL_ERR_ARG;
+  // workspace = [layer state | the evaluation's buffers | stage workspace]
+  char* S = (char*)workspace;
+  GraphBufs G = graph_bufs(L, S);
+  G.info = info;  // the caller's info block in place of the state's
+  EvalBufs E;
+  const size_t eb = eval_bufs(S + L.total, B, mb, l, &E);
+  void* ws = S + L.total + eb;
+  const size_t ws_bytes = workspace_bytes - L.total - eb;
+
+  GLL_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  GLL_CUDA_CHECK(cudaMemsetAsync(E.ticket, 0, sizeof(unsigned) * ((size_t)B + 1), st));
+  if (correct_out) GLL_CUDA_CHECK(cudaMemsetAsync(correct_out, 0, sizeof(long long) * (size_t)B, st));
+  int rc = (B == 1) ? knn_run(X, n, d, k, 0, n, G.knn_idx, G.knn_dist, info, ws, ws_bytes, st)
+                    : batched_knn_run(X, B, n, d, k, k_lab, G, ws, ws_bytes, st);
+  if (rc) return rc;
+  rc = graph_stages_run(G, Y, N, k, l, K, eps_auto, eps_fixed, tau, 0, 6, ws, ws_bytes, st);
+  if (rc) return rc;
+  float* x0 = G.ut + (size_t)K * lp;
+  float* corr = G.wt;  // the adjoint's region, free in an evaluation
+  unsigned* barrier = (unsigned*)(info + GLL_INFO_CG_BARRIER);  // zeroed with info, rewound by the kernels
+  // No sparsity hint (0): the evaluation system is never routed to the cluster kernel.  No status pointer either: an inner solve
+  // that stops at the fp32 floor is not a failure -- the fp64 rounds decide convergence.  B graphs are one block-diagonal system:
+  // every CG solves them together, with step lengths shared by the graphs (per class column).
+  rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, x0,
+              info + GLL_INFO_CG_ITERS_FWD, (float*)(info + GLL_INFO_CG_RESID_FWD), nullptr, ws, ws_bytes, st, barrier, nullptr);
+  if (rc) return rc;
+
+  RefineParams P;
+  P.row_ptr = G.row_ptr;
+  P.col = G.col;
+  P.w = G.w;
+  P.Y = Y;
+  P.r_out = E.r;
+  P.partial = E.partial;
+  P.colnorm = E.colnorm;
+  P.gmax = E.gmax;
+  P.resid = resid_out;
+  P.scale = E.scale;
+  P.ticket = E.ticket;
+  P.info = info;
+  P.n = N;
+  P.k_lab = K;
+  P.m = m;
+  P.mb = mb;
+  P.B = B;
+  P.gx = refine_grid_x(mb, l);
+  P.l = l;
+  P.lp = lp;
+  P.cw = min(l, 32);
+  P.tau = (double)tau;
+  P.tol = tol;
+  const dim3 grid(B * P.gx, ceil_div(l, P.cw));
+  const CgIo io = {E.r, 2, nullptr, 0, E.scale, 1, 0.f};
+  for (int r = 0; r < GLL_LAPLACE_ROUNDS; ++r) {
+    // the last round writes pred; rounds alternate between pred and the workspace buffer
+    double* out = ((GLL_LAPLACE_ROUNDS - 1 - r) % 2 == 0) ? pred : E.xtmp;
+    P.x_prev = (r == 0) ? nullptr : (out == pred ? E.xtmp : pred);
+    P.e = (r == 0) ? x0 : corr;
+    P.x_out = out;
+    P.round = r;
+    {
+      GLL_PROF(KID_LAPLACE_REFINE, st);
+      laplace_refine_kernel<<<grid, LR_THREADS, 0, st>>>(P);
+      GLL_LAUNCH_CHECK();
+    }
+    rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, corr, E.round_iters + r,
+                nullptr, nullptr, ws, ws_bytes, st, barrier, &io);
+    if (rc) return rc;
+  }
+  {
+    GLL_PROF(KID_LAPLACE_FINISH, st);
+    const int fb = ceil_div(mb, LR_THREADS);
+    laplace_finish_kernel<<<B * fb, LR_THREADS, 0, st>>>(pred, corr, mb, fb, l, lp, labels, targets, (unsigned long long*)correct_out,
+                                                         E.scale, E.round_iters, GLL_LAPLACE_ROUNDS, info);
+    GLL_LAUNCH_CHECK();
+  }
+  return GLL_OK;
 }
 
 }  // namespace
@@ -210,9 +355,8 @@ using namespace gll;
 extern "C" {
 
 size_t gll_laplace_eval_workspace_bytes(int n, int d, int k, int l, int k_lab) {
-  gll_layout L;
-  if (n < 2 || l < 1 || k_lab < 1 || k_lab >= n || gll_state_layout(n, k, l, k_lab, &L)) return 0;
-  return L.total + eval_bufs(nullptr, n - k_lab, l, nullptr) + gll_workspace_bytes(n, d, k, l, k_lab);
+  if (n < 2 || l < 1 || k_lab < 1 || k_lab >= n) return 0;
+  return eval_ws_bytes(1, n, d, k, l, k_lab);
 }
 
 int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
@@ -222,85 +366,27 @@ int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l,
   GLL_REQUIRE(k >= 2 && k <= 64 && (k <= 33 || n >= 256) && k <= n, "k must be in [2, 64] (n >= 256 when k > 33) and <= n");
   GLL_REQUIRE(d >= 1 && l >= 1 && k_lab >= 1 && k_lab < n, "bad sizes");
   GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
-  const size_t need = gll_laplace_eval_workspace_bytes(n, d, k, l, k_lab);
-  if (workspace_bytes < need) {
-    set_error("workspace too small: %zu < %zu", workspace_bytes, need);
-    return GLL_ERR_WORKSPACE;
-  }
-  gll_layout L;
-  if (gll_state_layout(n, k, l, k_lab, &L)) return GLL_ERR_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int m = n - k_lab, lp = padded_classes(l);
-  // workspace = [layer state | the evaluation's buffers | stage workspace]
-  char* S = (char*)workspace;
-  GraphBufs G = graph_bufs(L, S);
-  G.info = info;  // the caller's info block in place of the state's
-  EvalBufs B;
-  const size_t eb = eval_bufs(S + L.total, m, l, &B);
-  void* ws = S + L.total + eb;
-  const size_t ws_bytes = workspace_bytes - L.total - eb;
+  return eval_run(X, Y, 1, n, d, k, l, k_lab, eps_auto, eps_fixed, tau, tol, cg_max_iter, pred, labels, targets, correct_out, nullptr, info,
+                  workspace, workspace_bytes, (cudaStream_t)stream);
+}
 
-  GLL_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int) * GLL_INFO_WORDS, st));
-  GLL_CUDA_CHECK(cudaMemsetAsync(B.ticket, 0, sizeof(unsigned), st));
-  if (correct_out) GLL_CUDA_CHECK(cudaMemsetAsync(correct_out, 0, sizeof(long long), st));
-  int rc = knn_run(X, n, d, k, 0, n, G.knn_idx, G.knn_dist, info, ws, ws_bytes, st);
-  if (rc) return rc;
-  rc = graph_stages_run(G, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, 0, 6, ws, ws_bytes, st);
-  if (rc) return rc;
-  float* x0 = G.ut + (size_t)k_lab * lp;
-  float* corr = G.wt;  // the adjoint's region, free in an evaluation
-  unsigned* barrier = (unsigned*)(info + GLL_INFO_CG_BARRIER);  // zeroed with info, rewound by the kernels
-  // No sparsity hint (0): the evaluation system is never routed to the cluster kernel.  No status pointer either: an inner solve
-  // that stops at the fp32 floor is not a failure -- the fp64 rounds decide convergence.
-  rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, x0,
-              info + GLL_INFO_CG_ITERS_FWD, (float*)(info + GLL_INFO_CG_RESID_FWD), nullptr, ws, ws_bytes, st, barrier, nullptr);
-  if (rc) return rc;
+size_t gll_laplace_eval_batched_workspace_bytes(int B, int n, int d, int k, int l, int k_lab) {
+  if (!eval_batched_sizes_ok(B, n, d, k, l, k_lab)) return 0;
+  return eval_ws_bytes(B, n, d, k, l, k_lab);
+}
 
-  RefineParams P;
-  P.row_ptr = G.row_ptr;
-  P.col = G.col;
-  P.w = G.w;
-  P.Y = Y;
-  P.r_out = B.r;
-  P.partial = B.partial;
-  P.colnorm = B.colnorm;
-  P.scale = B.scale;
-  P.ticket = B.ticket;
-  P.info = info;
-  P.n = n;
-  P.k_lab = k_lab;
-  P.m = m;
-  P.l = l;
-  P.lp = lp;
-  P.cw = min(l, 32);
-  P.tau = (double)tau;
-  P.tol = tol;
-  const dim3 grid(refine_grid_x(m, l), ceil_div(l, P.cw));
-  const CgIo io = {B.r, 2, nullptr, 0, B.scale, 1, 0.f};
-  for (int r = 0; r < GLL_LAPLACE_ROUNDS; ++r) {
-    // the last round writes pred; rounds alternate between pred and the workspace buffer
-    double* out = ((GLL_LAPLACE_ROUNDS - 1 - r) % 2 == 0) ? pred : B.xtmp;
-    P.x_prev = (r == 0) ? nullptr : (out == pred ? B.xtmp : pred);
-    P.e = (r == 0) ? x0 : corr;
-    P.x_out = out;
-    P.round = r;
-    {
-      GLL_PROF(KID_LAPLACE_REFINE, st);
-      laplace_refine_kernel<<<grid, LR_THREADS, 0, st>>>(P);
-      GLL_LAUNCH_CHECK();
-    }
-    rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, corr, B.round_iters + r,
-                nullptr, nullptr, ws, ws_bytes, st, barrier, &io);
-    if (rc) return rc;
-  }
-  {
-    GLL_PROF(KID_LAPLACE_FINISH, st);
-    laplace_finish_kernel<<<ceil_div(m, LR_THREADS), LR_THREADS, 0, st>>>(pred, corr, m, l, lp, labels, targets,
-                                                                           (unsigned long long*)correct_out, B.scale, B.round_iters,
-                                                                           GLL_LAPLACE_ROUNDS, info);
-    GLL_LAUNCH_CHECK();
-  }
-  return GLL_OK;
+int gll_laplace_eval_batched(const float* X, const float* Y, int B, int n, int d, int k, int l, int k_lab, int eps_auto,
+                             float eps_fixed, float tau, double tol, int cg_max_iter, double* pred, long long* labels,
+                             const long long* targets, long long* correct_out, double* resid_out, int* info, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+  GLL_REQUIRE(X && Y && pred && labels && info && workspace, "null pointer");
+  GLL_REQUIRE(B >= 1 && n >= 1 && (long long)B * n <= 0x7fffffffLL, "need B >= 1 and B n < 2^31");
+  GLL_REQUIRE(k >= 2 && k <= 64 && k <= n && (k <= 33 || (long long)B * n >= 256),
+              "k must be in [2, 64] and <= n, with B n >= 256 when k > 33");
+  GLL_REQUIRE(d >= 1 && l >= 1 && k_lab >= 1 && k_lab < n, "bad sizes");
+  GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
+  return eval_run(X, Y, B, n, d, k, l, k_lab, eps_auto, eps_fixed, tau, tol, cg_max_iter, pred, labels, targets, correct_out, resid_out,
+                  info, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -11,6 +11,13 @@ in fp64 until every class column meets the reference's stop rule ||M (b - A x)||
 (see gll_laplace_eval in include/gll_b200.h, including the row-sum degree).  Everything is enqueued on the current stream:
 no host sync, no host round trip, so the call can be captured into a CUDA graph.  Status ('max iter reached' when tol is
 unmet, epsilon ~ 0) goes through the same deferred check as the layer.  Knob: GLL_B200_CG_MAXIT (iterations per CG solve).
+
+    res = laplace_learning_batched(features, label_matrix, k=50, epsilon='auto', tau=0.0, tol=1e-10, targets=None)
+
+B independent graphs of the same shape in one call (features (B, n, d), label_matrix (B, k_lab, l), targets (B, m)); pred
+(B, m, l), labels (B, m), correct (B,).  Every graph meets the stop rule on its own; the solver's step lengths are shared by
+the graphs, so pred matches per-graph laplace_learning calls to solver accuracy (bit for bit at B = 1).  See
+gll_laplace_eval_batched in include/gll_b200.h.
 """
 from __future__ import annotations
 
@@ -23,7 +30,7 @@ from . import _lib
 from .GLL import _bytes, _cg_maxit, _check_status, _require_cuda, _stream_ptr, as_features, decode_info, parse_epsilon
 from ._lib import lib
 
-__all__ = ["laplace_learning", "LaplaceResult", "last_eval_info"]
+__all__ = ["laplace_learning", "laplace_learning_batched", "LaplaceResult", "last_eval_info"]
 
 
 class LaplaceResult(NamedTuple):
@@ -33,6 +40,21 @@ class LaplaceResult(NamedTuple):
 
 
 _last_info: Optional[torch.Tensor] = None
+_last_resid: Optional[torch.Tensor] = None  # per-graph residuals of the last call when it was batched
+
+
+def _check_args(n, d, k_lab, l, k, epsilon, tol, total_rows, rows_name):
+    """The size, epsilon and tol checks both entry points share; returns (eps_auto, eps_fixed)."""
+    if not (0 < k_lab < n):
+        raise ValueError(f"need 0 < k_lab < n (k_lab={k_lab}, n={n}); labeled rows come first (GLL.py:11)")
+    if l < 1 or d < 1:
+        raise ValueError("need at least one class column and one feature")
+    if not (2 <= k <= 64) or k > n or (k > 33 and total_rows < 256):
+        raise ValueError(f"k must be in [2, 64] and <= n, with {rows_name} >= 256 when k > 33 (k={k}, n={n})")
+    eps = parse_epsilon(epsilon)
+    if not tol > 0:
+        raise ValueError("tol must be > 0")
+    return eps
 
 
 def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto", tau: float = 0.0,
@@ -46,15 +68,7 @@ def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int 
     n, d = features.shape
     k_lab, l = label_matrix.shape
     k = int(k)
-    if not (0 < k_lab < n):
-        raise ValueError(f"need 0 < k_lab < n (k_lab={k_lab}, n={n}); labeled rows come first (GLL.py:11)")
-    if l < 1 or d < 1:
-        raise ValueError("need at least one class column and one feature")
-    if not (2 <= k <= 64) or k > n or (k > 33 and n < 256):
-        raise ValueError(f"k must be in [2, 64] and <= n, with n >= 256 when k > 33 (k={k}, n={n})")
-    eps_auto, eps_fixed = parse_epsilon(epsilon)
-    if not tol > 0:
-        raise ValueError("tol must be > 0")
+    eps_auto, eps_fixed = _check_args(n, d, k_lab, l, k, epsilon, tol, n, "n")
     m = n - k_lab
     if targets is not None and tuple(targets.shape) != (m,):
         raise ValueError(f"targets must be ({m},), got {tuple(targets.shape)}")
@@ -77,15 +91,63 @@ def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int 
                                   correct.data_ptr() if correct is not None else None, info.data_ptr(), ws.data_ptr(), ws_bytes,
                                   _stream_ptr(dev))
     _lib.check(rc, "gll_laplace_eval")
-    global _last_info
-    _last_info = info
+    global _last_info, _last_resid
+    _last_info, _last_resid = info, None
+    _check_status(info, "Laplace-learning")
+    return LaplaceResult(pred, labels, correct)
+
+
+def laplace_learning_batched(features: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto", tau: float = 0.0,
+                             tol: float = 1e-10, targets: Optional[torch.Tensor] = None) -> LaplaceResult:
+    """laplace_learning over B independent graphs of the same shape.  features (B, n, d) CUDA tensor, each graph's k_lab labeled
+    rows FIRST; label_matrix (B, k_lab, l) one-hot float32 or int64; targets (B, m) int64 or None, a negative target is not
+    counted.  Returns pred (B, m, l) float64, labels (B, m) int64 and correct (B,) int64 (None without targets)."""
+    if features.dim() != 3:
+        raise ValueError("features must be (B, n, d)")
+    if label_matrix.dim() != 3:
+        raise ValueError("label_matrix must be (B, k_lab, l)")
+    B, n, d = features.shape
+    if B < 1 or label_matrix.shape[0] != B:
+        raise ValueError(f"label_matrix must be (B, k_lab, l) with B = {B} >= 1, got {tuple(label_matrix.shape)}")
+    if B * n >= 2 ** 31:
+        raise ValueError(f"B n must be < 2^31 (B={B}, n={n})")
+    _, k_lab, l = label_matrix.shape
+    k = int(k)
+    eps_auto, eps_fixed = _check_args(n, d, k_lab, l, k, epsilon, tol, B * n, "B n")
+    m = n - k_lab
+    if targets is not None and tuple(targets.shape) != (B, m):
+        raise ValueError(f"targets must be ({B}, {m}), got {tuple(targets.shape)}")
+    _require_cuda(features, "features")
+    dev = features.device
+    Xc = as_features(features)
+    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
+    tg = None
+    if targets is not None:
+        tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
+    with torch.cuda.device(dev):
+        ws_bytes = lib.gll_laplace_eval_batched_workspace_bytes(B, n, d, k, l, k_lab)
+        ws = _bytes(ws_bytes, dev)
+        pred = torch.empty((B, m, l), dtype=torch.float64, device=dev)
+        labels = torch.empty((B, m), dtype=torch.int64, device=dev)
+        correct = torch.empty(B, dtype=torch.int64, device=dev) if tg is not None else None
+        resid = torch.empty(B, dtype=torch.float64, device=dev)
+        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
+        rc = lib.gll_laplace_eval_batched(Xc.data_ptr(), Y.data_ptr(), B, n, d, k, l, k_lab, eps_auto, eps_fixed, float(tau),
+                                          float(tol), _cg_maxit(), pred.data_ptr(), labels.data_ptr(),
+                                          tg.data_ptr() if tg is not None else None,
+                                          correct.data_ptr() if correct is not None else None, resid.data_ptr(), info.data_ptr(),
+                                          ws.data_ptr(), ws_bytes, _stream_ptr(dev))
+    _lib.check(rc, "gll_laplace_eval_batched")
+    global _last_info, _last_resid
+    _last_info, _last_resid = info, resid
     _check_status(info, "Laplace-learning")
     return LaplaceResult(pred, labels, correct)
 
 
 def last_eval_info() -> dict:
-    """Device status block of the most recent laplace_learning call (synchronises).  Keys follow GLL_INFO_* in
-    include/gll_b200.h."""
+    """Device status block of the most recent laplace_learning or laplace_learning_batched call (synchronises).  Keys follow
+    GLL_INFO_* in include/gll_b200.h; after a batched call the residuals are the maximum over graphs, the iteration counts those
+    of the whole batch, and resid_per_graph lists each graph's largest column norm of the last round."""
     if _last_info is None:
         return {}
     v = _last_info.cpu().numpy()
@@ -94,4 +156,5 @@ def last_eval_info() -> dict:
     round_iters = [int((u[_lib.INFO_LAPLACE_ROUND_ITERS + r // 2] >> (16 * (r % 2))) & 0xFFFF) for r in range(4)]
     return dict(decode_info(v), cg_iters_first=int(v[_lib.INFO_CG_ITERS_FWD]), rounds=int(v[_lib.INFO_LAPLACE_ROUNDS]),
                 cg_iters_correction=int(v[_lib.INFO_LAPLACE_CG_ITERS]), round_iters=round_iters, resid_first=float(f[_lib.INFO_LAPLACE_RESID0]),
-                resid=float(f[_lib.INFO_LAPLACE_RESID]))
+                resid=float(f[_lib.INFO_LAPLACE_RESID]),
+                **({} if _last_resid is None else dict(resid_per_graph=[float(x) for x in _last_resid.cpu().numpy()])))

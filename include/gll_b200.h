@@ -133,8 +133,9 @@ int gll_knn(const float* X, int n, int d, int k, int* knn_idx, float* knn_dist, 
  * seg_ptr_host a HOST array of nseg + 1 offsets from 0 to n (the search is planned on the host: no sync).  Row i of segment s
  * gets its k nearest neighbours among the rows of s only (global row numbers, self in slot 0, then by (distance, index)):
  * bit-identical to gll_knn on each segment alone plus the segment's offset, because those lists are exact.  Every segment
- * needs >= k rows; 2 <= k <= 33.  The tensor-core search only issues the (row tile, column tile) units whose columns meet
- * the segments of the tile's rows, O(sum n_s^2 d) work instead of O(n^2 d).  nseg == 1 runs gll_knn.  Bad arguments
+ * needs >= k rows; 2 <= k <= 64, with n >= 256 when k > 33 (as gll_knn: k > 33 runs two tensor-core candidate rounds,
+ * the second above the first round's 32nd key).  The tensor-core search only issues the (row tile, column tile) units whose
+ * columns meet the segments of the tile's rows, O(sum n_s^2 d) work instead of O(n^2 d).  nseg == 1 runs gll_knn.  Bad arguments
  * return GLL_ERR_ARG before any CUDA call; the workspace query returns 0 for them.  gll_knn_segments_units (host query,
  * for benchmarks): tensor-core units such a call issues, and those of the uniform grid over the same rows (0, 0 when
  * the SIMT path runs). */
@@ -345,6 +346,26 @@ size_t gll_laplace_eval_workspace_bytes(int n, int d, int k, int l, int k_lab);
 int gll_laplace_eval(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
                      float tau, double tol, int cg_max_iter, double* pred, long long* labels, const long long* targets,
                      long long* correct_out, int* info, void* workspace, size_t workspace_bytes, void* stream);
+
+/* gll_laplace_eval over B independent graphs of the same shape: X is B x n x d and Y is B x k_lab x l, each graph's labeled
+ * rows first.  As gll_forward_batched, the graphs are one block-diagonal graph in labeled-first order: the kNN search runs per
+ * graph (gll_knn_segments, so every graph's lists, CSR and W are bit-identical to a per-graph call), then the stages, the
+ * solves and the refinement of gll_laplace_eval run on the union.  The stop rule is per graph: the refinement stops when every
+ * class column of EVERY graph has ||M (b - A x)||_2 <= tol over that graph's rows; while one graph is above tol all graphs get
+ * corrections.  The CG step lengths are shared by the graphs, so pred matches per-graph gll_laplace_eval calls to solver
+ * accuracy, not bit for bit; B = 1 is bit-identical to gll_laplace_eval.
+ *   Sizes: B >= 1, B n < 2^31, 2 <= k <= 64, k <= n, B n >= 256 when k > 33, 1 <= k_lab < n, l >= 1, tol > 0, cg_max_iter >= 1.
+ *   Outputs: pred (B m) x l fp64 and labels[B m] int64 are graph-major ((B, m, l) and (B, m), m = n - k_lab); targets
+ *   (B m int64, may be NULL) line up with them; correct_out (B int64, may be NULL) counts hits per graph; resid_out (B fp64,
+ *   may be NULL) = per graph the largest column norm of the last round (GLL_INFO_LAPLACE_RESID's meaning, per graph).
+ *   info: as gll_laplace_eval, the residual slots holding the maximum over graphs and the iteration counts those of the whole
+ *   batch.  Bad arguments return GLL_ERR_ARG before any CUDA call; the workspace query returns 0 for them.  Nothing syncs with
+ *   the host, so the call can be captured in a CUDA graph. */
+size_t gll_laplace_eval_batched_workspace_bytes(int B, int n, int d, int k, int l, int k_lab);
+int gll_laplace_eval_batched(const float* X, const float* Y, int B, int n, int d, int k, int l, int k_lab, int eps_auto,
+                             float eps_fixed, float tau, double tol, int cg_max_iter, double* pred, long long* labels,
+                             const long long* targets, long long* correct_out, double* resid_out, int* info,
+                             void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
