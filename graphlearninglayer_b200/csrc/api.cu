@@ -714,25 +714,34 @@ static std::vector<int> uniform_segments(int B, int n) {
 
 namespace gll {
 
+// the segmented search's lists in natural order, in front of the search's own workspace; returns their bytes (ws == NULL: size
+// query only)
+static size_t batched_lists(void* ws, int N, int k, int** idx, float** dist) {
+  Carver cv(ws, ~(size_t)0);
+  int* i = cv.take<int>((size_t)N * k);
+  float* x = cv.take<float>((size_t)N * k);
+  if (idx) *idx = i;
+  if (dist) *dist = x;
+  return align_up(cv.off, 256);
+}
+
 size_t batched_ws_bytes(int B, int n, int d, int k, int l, int k_lab) {
   const int N = B * n;
   const std::vector<int> seg = uniform_segments(B, n);
-  const size_t lists = 2 * align_up(sizeof(int) * (size_t)N * k, 256);  // the search's lists in natural order
   const size_t s = knn_seg_ws_bytes(N, d, k, seg.data(), B);
   if (s == 0) return 0;
-  size_t b = lists + s + 256;
+  size_t b = batched_lists(nullptr, N, k, nullptr, nullptr) + s;
   b = std::max(b, graph_weights_ws_bytes(N, k));
   return std::max(b, cg_ws_bytes(N - B * k_lab, l));
 }
 
 int batched_knn_run(const float* X, int B, int n, int d, int k, int k_lab, const GraphBufs& G, void* ws, size_t ws_bytes, cudaStream_t st) {
   const int N = B * n;
-  Carver cv(ws, ws_bytes);
-  int* idx = cv.take<int>((size_t)N * k);
-  float* dist = cv.take<float>((size_t)N * k);
-  char* kws = cv.take<char>(0);
+  int* idx;
+  float* dist;
+  const size_t lists = batched_lists(ws, N, k, &idx, &dist);
   const std::vector<int> seg = uniform_segments(B, n);
-  const int rc = knn_run_segments(X, N, d, k, seg.data(), B, idx, dist, G.info, kws, ws_bytes - (size_t)(kws - (char*)ws), st);
+  const int rc = knn_run_segments(X, N, d, k, seg.data(), B, idx, dist, G.info, (char*)ws + lists, ws_bytes - lists, st);
   if (rc) return rc;
   {
     GLL_PROF(KID_BATCH_REORDER, st);

@@ -13,8 +13,8 @@
 //   fallback    : brute-force fp64 search for the queued rows only.
 //
 // This file holds the fp32 SIMT Gram path (tiny graphs; any d, any alignment), the operand-split kernels, re-rank and
-// fallback.  The tcgen05/TMA Gram path (n >= 256, any d: rows are zero-padded to a multiple of 32) lives in knn_tc.cu and
-// reuses the rerank / fallback kernels through knn_finish().
+// fallback, and the host code of every search.  The tcgen05/TMA Gram path (n >= 256, any d: rows are zero-padded to a multiple
+// of 32) lives in knn_tc.cu; both paths end in the same re-rank and fallback (knn_finish).
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -22,7 +22,6 @@
 #include <algorithm>
 #include <vector>
 
-#include <cuda_fp16.h>
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -472,12 +471,7 @@ knn_rerank_kernel(const float* __restrict__ X, const float* __restrict__ sq, con
   }
 
   u64 mine = KEY_INF;
-  int splits = lay.stride;
-  if (lay.tc == 1 || lay.tc == 3) {  // lists written for this row's tile: one per CTA that touched it (knn_tc.cu)
-    int b0, b1;
-    cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
-    splits = 2 * (b1 - b0 + 1);  // every CTA writes two lists per row (the column halves of its epilogue)
-  }
+  const int splits = cand_lists(lay, i);
   if (splits == 1 && lay.tc == 0) {
     mine = cand[(size_t)i * lay.stride * KC + lane];  // SIMT lists are sorted
   } else {
@@ -795,12 +789,7 @@ knn_merge_kernel(int row_end, CandLayout lay, const u64* __restrict__ cand, u64*
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int i = lay.row_begin + blockIdx.x * RERANK_WARPS + warp;
   if (i >= row_end) return;
-  int splits = lay.stride;
-  if (lay.tc == 1 || lay.tc == 3) {
-    int b0, b1;
-    cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
-    splits = 2 * (b1 - b0 + 1);  // every CTA writes two lists per row (the column halves of its epilogue)
-  }
+  const int splits = cand_lists(lay, i);
   u64 mine = KEY_INF;
   for (int s = 0; s < splits; ++s) {
     list_merge_set(mine, cand[((size_t)i * lay.stride + s) * KC + lane], lane);
@@ -892,92 +881,11 @@ knn_rerank64_kernel(const float* __restrict__ X, const float* __restrict__ sq, c
 int knn_fallback_grid() { return 2 * device_info().sms; }
 size_t knn_fallback_scratch_bytes() { return align_up((size_t)knn_fallback_grid() * 32 * (sizeof(double) + sizeof(int)), 256); }
 
-int knn_finish(const float* X, const float* sq, const unsigned* sqmax_bits, int n, int d, int k, int row_begin, int row_end,
-               CandLayout lay, const u64* cand, float err_coef, int* knn_idx, float* knn_dist, int* flag_count, int* flag_rows,
-               int* info, void* fb_scratch, cudaStream_t st, const int2* win) {
-  const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
-  size_t smem = sizeof(float) * (size_t)RERANK_WARPS * d;
-  lay.row_begin = row_begin;
-  int blocks = ceil_div(row_end - row_begin, RERANK_WARPS);
-  int force_rows = 0;
-  if (const char* e = getenv("GLL_B200_KNN_FORCE_FALLBACK")) force_rows = atoi(e);
-  if (vec4) {
-    if (smem > 48 * 1024)
-      GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_rerank_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    {
-      GLL_PROF(KID_RERANK, st);
-      knn_rerank_kernel<true><<<blocks, RERANK_WARPS * 32, smem, st>>>(X, sq, sqmax_bits, n, d, k, row_end, lay, cand,
-                                                                      err_coef, knn_idx, knn_dist, flag_count, flag_rows, force_rows);
-    }
-  } else {
-    if (smem > 48 * 1024)
-      GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_rerank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    {
-      GLL_PROF(KID_RERANK, st);
-      knn_rerank_kernel<false><<<blocks, RERANK_WARPS * 32, smem, st>>>(X, sq, sqmax_bits, n, d, k, row_end, lay, cand,
-                                                                       err_coef, knn_idx, knn_dist, flag_count, flag_rows, force_rows);
-    }
-  }
-  GLL_LAUNCH_CHECK();
-  size_t fsmem = sizeof(float) * (size_t)d;
-  if (getenv("GLL_B200_KNN_DEBUG") != nullptr) return GLL_OK;  // timing experiments: every row would be "unproven"
-  {
-    // rows whose completeness proof failed: exact brute force, the rows' column ranges dealt to all CTAs
-    const int fblocks = knn_fallback_grid();
-    double* part_d = reinterpret_cast<double*>(fb_scratch);
-    int* part_j = reinterpret_cast<int*>(part_d + (size_t)fblocks * 32);
-    unsigned* ticket = reinterpret_cast<unsigned*>(flag_count) + 7;  // small[8]: zeroed with flag_count at the start of the search
-    GLL_PROF(KID_KNN_FALLBACK, st);
-    if (vec4)
-      knn_fallback_scan_kernel<true><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info,
-                                                                           part_d, part_j, ticket, win);
-    else
-      knn_fallback_scan_kernel<false><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info,
-                                                                            part_d, part_j, ticket, win);
-  }
-  GLL_LAUNCH_CHECK();
-  return GLL_OK;
-}
+namespace {
 
-static int knn_finish64(const float* X, const float* sq, const unsigned* sqmax_bits, int n, int d, int k, int row_begin, int row_end,
-                       const u64* m1, const u64* m2, float err_coef, int* knn_idx, float* knn_dist, int* flag_count,
-                       int* flag_rows, int* info, cudaStream_t st, const int2* win) {
-  const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
-  const size_t smem = sizeof(float) * (size_t)RERANK_WARPS * d;
-  const int blocks = ceil_div(row_end - row_begin, RERANK_WARPS);
-  int force_rows = 0;
-  if (const char* e = getenv("GLL_B200_KNN_FORCE_FALLBACK")) force_rows = atoi(e);
-  {
-    GLL_PROF(KID_RERANK, st);
-    if (vec4) {
-      if (smem > 48 * 1024)
-        GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_rerank64_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      knn_rerank64_kernel<true><<<blocks, RERANK_WARPS * 32, smem, st>>>(X, sq, sqmax_bits, n, d, k, row_begin, row_end, m1, m2,
-                                                                          err_coef, knn_idx, knn_dist, flag_count, flag_rows, force_rows);
-    } else {
-      if (smem > 48 * 1024)
-        GLL_CUDA_CHECK(cudaFuncSetAttribute(knn_rerank64_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      knn_rerank64_kernel<false><<<blocks, RERANK_WARPS * 32, smem, st>>>(X, sq, sqmax_bits, n, d, k, row_begin, row_end, m1, m2,
-                                                                           err_coef, knn_idx, knn_dist, flag_count, flag_rows, force_rows);
-    }
-  }
-  GLL_LAUNCH_CHECK();
-  const size_t fsmem = sizeof(float) * (size_t)d;
-  const int fblocks = device_info().sms;
-  if (getenv("GLL_B200_KNN_DEBUG") != nullptr) return GLL_OK;  // timing experiments: every row would be "unproven"
-  {
-    GLL_PROF(KID_KNN_FALLBACK, st);
-    if (vec4)
-      knn_fallback_kernel<true><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info, win);
-    else
-      knn_fallback_kernel<false><<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, flag_count, flag_rows, knn_idx, knn_dist, info, win);
-  }
-  GLL_LAUNCH_CHECK();
-  return GLL_OK;
-}
-
-static int simt_splits(int n, int rows, int* cols_per_split) {
-  int row_tiles = ceil_div(rows, BM), col_tiles = ceil_div(n, BN);
+int simt_splits(int n, int rows, int* cols_per_split) {
+  // at least one row tile: size queries of shapes the search refuses (an empty row range) must not divide by zero
+  int row_tiles = max(1, ceil_div(rows, BM)), col_tiles = ceil_div(n, BN);
   int want = ceil_div(2 * device_info().sms, row_tiles);
   want = max(1, min(want, min(col_tiles, KNN_MAX_SPLITS)));
   int tiles_per = ceil_div(col_tiles, want);
@@ -985,97 +893,116 @@ static int simt_splits(int n, int rows, int* cols_per_split) {
   return ceil_div(col_tiles, tiles_per);
 }
 
-// candidate sets per row the chosen Gram path will write for this row range
-static int cand_stride(int n, int d, int row_begin, int row_end) {
-  const TcPlan plan = knn_tc_plan(n, d, row_begin, row_end);
-  if (plan.ok) return plan.max_splits;
-  int cps;
-  return simt_splits(n, row_end - row_begin, &cps);
-}
-
-// The buffers every search carves from its workspace (KnnBufs, knn_carve) and their size for `rows` searched rows with `stride`
-// candidate lists per row.  knn_run and knn_run_segments append their own buffers behind them.
-static size_t knn_common_bytes(int n, int d, size_t rows, int stride) {
-  size_t b = 0;
-  b += align_up(sizeof(float) * (size_t)n, 256);                        // sq
-  b += 256;                                                             // sqmax + flag_count
-  b += align_up(sizeof(u64) * rows * (size_t)stride * KC, 256);         // cand
-  b += align_up(sizeof(int) * rows, 256);                               // flag_rows
-  b += knn_tc_ws_upper(n, d);                                           // 16-bit hi / lo copies for the tensor-core path
-  b += align_up(sizeof(unsigned) * (size_t)n, 256);                     // per-row shared thresholds
-  b += align_up(sizeof(float) * (size_t)n, 256);                        // per-row operand scale (f16x2 split)
-  b += knn_fallback_scratch_bytes() + 256;                              // chunk lists of the brute-force fallback
-  return b;
-}
-
-size_t knn_ws_bytes(int n, int d, int k, int row_begin, int row_end) {
-  const size_t rows = (size_t)(row_end - row_begin);
-  size_t b = knn_common_bytes(n, d, rows, cand_stride(n, d, row_begin, row_end));
-  if (k > KC + 1) b += 2 * align_up(sizeof(u64) * rows * KC, 256) + align_up(sizeof(u64) * (size_t)n, 256);  // merged lists, excl
-  return b + 1024;
-}
-
-namespace {
-
-struct KnnBufs {
-  float* sq;
-  unsigned* small;   // small[0]: bits of max |x|^2, small[1]: flag_count, small[7]: fallback ticket (zeroed per search)
-  int* flag_count;
-  u64* cand;         // indexed by GLOBAL row: where row 0 would live
-  int* flag_rows;
-  char* tc_ws;
-  unsigned* thr_g;   // NULL when GLL_B200_KNN_SHARE=0
-  float* rscale;     // per-row power-of-two scale of the fp16 operands
-  void* fb_scratch;
-};
-
-KnnBufs knn_carve(Carver& cv, int n, int d, int row_begin, int row_end, int stride) {
-  const int rows = row_end - row_begin;
-  KnnBufs b;
-  b.sq = cv.take<float>(n);
-  b.small = cv.take<unsigned>(64);
-  b.flag_count = reinterpret_cast<int*>(b.small + 1);
-  b.cand = cv.take<u64>((size_t)rows * stride * KC) - (size_t)row_begin * stride * KC;
-  b.flag_rows = cv.take<int>(rows);
-  b.tc_ws = cv.take<char>(knn_tc_ws_upper(n, d));
-  b.thr_g = cv.take<unsigned>(n);
-  b.rscale = cv.take<float>(n);
-  b.fb_scratch = cv.take<char>(knn_fallback_scratch_bytes());
-  const char* sh = getenv("GLL_B200_KNN_SHARE");  // "0": every candidate set keeps its own threshold (experiments)
-  if (sh && sh[0] == '0') b.thr_g = nullptr;
-  return b;
-}
-
-// candidate-list layout of a tensor-core search; gfirst != NULL: the segmented unit grid
-CandLayout layout_of(const TcPlan& plan, int row_begin, const int* gfirst = nullptr) {
-  CandLayout lay;
-  lay.stride = plan.max_splits;
-  lay.tc = plan.aligned ? 2 : (gfirst != nullptr ? 3 : 1);
-  lay.row_tile = 128 * plan.rstep;  // rows per row group
-  lay.col_tiles = plan.col_tiles;
-  lay.grid = plan.grid;
-  lay.units = plan.units;
-  lay.row_begin = row_begin;
-  lay.gfirst = gfirst;
-  return lay;
-}
-
-// ... and of the SIMT search (or of lists merged into one sorted list per row)
-CandLayout simt_layout(int splits) {
-  CandLayout lay;
-  lay.stride = splits;
-  lay.tc = 0;
-  lay.row_tile = lay.col_tiles = lay.grid = 0;
-  lay.units = 0;
-  lay.row_begin = 0;
-  lay.gfirst = nullptr;
-  return lay;
+// the widest union of segment windows over a 128-row tile: the columns a SIMT row tile of a segmented search may see
+int widest_tile_window(int n, const int* seg_ptr) {
+  int wmax = 1;
+  for (int r0 = 0, s = 0; r0 < n; r0 += BM) {
+    while (seg_ptr[s + 1] <= r0) ++s;
+    int t = s;
+    const int r1 = min(n, r0 + BM) - 1;
+    while (seg_ptr[t + 1] <= r1) ++t;
+    wmax = max(wmax, seg_ptr[t + 1] - seg_ptr[s]);
+  }
+  return wmax;
 }
 
 // |fl(d~^2) - d^2| <= (gamma_d + 4u)(|x_i|^2 + |x_j|^2), gamma_d = d u/(1 - d u), u = 2^-24 (sequential fp32 FMA chain)
 float simt_err_coef(int d) {
   const double u = 5.9604644775390625e-8;
   return (float)(((double)d * u / (1.0 - (double)d * u) + 4.0 * u) * 1.0001);
+}
+
+// How a search over rows [row_begin, row_end) runs: the Gram path, the candidate lists it leaves and the error bound of their
+// approximate distances.
+struct KnnPlan {
+  int row_begin, row_end;
+  TcPlan tc;              // tc.ok: the tensor-core Gram path; otherwise the SIMT kernel with lay.stride column splits of cps columns
+  int cps;
+  CandLayout lay;         // lay.stride lists per row; lay.gfirst is set once the unit table is on the device
+  float err_coef;
+  std::vector<int> ints;  // segmented search: seg_ptr, then the tensor-core unit table (gfirst, gct, bstart; see SegDev)
+};
+
+// nseg > 1: the segmented search over all n rows (row_begin = 0, row_end = n); col_begin: columns before it are not searched
+KnnPlan knn_plan(int n, int d, int row_begin, int row_end, int col_begin = 0, const int* seg_ptr = nullptr, int nseg = 1) {
+  const bool seg = nseg > 1;
+  KnnPlan p;
+  p.row_begin = row_begin;
+  p.row_end = row_end;
+  std::vector<int> tab;
+  p.tc = seg ? knn_tc_plan_segments(n, d, seg_ptr, nseg, &tab) : knn_tc_plan(n, d, row_begin, row_end, col_begin);
+  memset(&p.lay, 0, sizeof(p.lay));
+  p.lay.row_begin = row_begin;
+  if (p.tc.ok) {
+    p.cps = 0;
+    p.lay.stride = p.tc.max_splits;
+    p.lay.tc = p.tc.aligned ? 2 : (seg ? 3 : 1);
+    p.lay.row_tile = 128 * p.tc.rstep;  // rows per row group
+    p.lay.col_tiles = p.tc.col_tiles;
+    p.lay.grid = p.tc.grid;
+    p.lay.units = p.tc.units;
+    p.err_coef = knn_tc_err_coef(d, p.tc.passes);
+  } else {
+    tab.clear();
+    p.lay.stride = simt_splits(seg ? widest_tile_window(n, seg_ptr) : n, row_end - row_begin, &p.cps);
+    p.err_coef = simt_err_coef(d);
+  }
+  if (seg) {
+    p.ints.assign(seg_ptr, seg_ptr + nseg + 1);
+    p.ints.insert(p.ints.end(), tab.begin(), tab.end());
+  }
+  return p;
+}
+
+// What a kNN entry takes from its workspace; the members it does not use stay NULL.
+struct KnnBufs {
+  float* sq;
+  unsigned* small;     // small[0]: bits of max |x|^2, small[1]: flag_count, small[8]: fallback ticket (zeroed per search)
+  int* flag_count;
+  u64* cand;           // the plan's rows x lay.stride lists, indexed by GLOBAL row: where row 0 would live
+  int* flag_rows;
+  char* tc_ws;         // fp16 hi / lo operands of the tensor-core path
+  unsigned* thr_g;     // per-row shared thresholds
+  float* rscale;       // per-row power-of-two scale of the fp16 operands
+  void* fb_scratch;    // chunk lists of the brute-force fallback
+  u64* merged;         // k > 33: the two rounds' merged lists [2][rows][KC]; cached search: [n][KC]
+  u64* excl;           // k > 33: the first round's 32nd key per row
+  int2* win;           // segmented search: the rows' column windows
+  int* ints;           // segmented search: KnnPlan::ints
+  u64* cand_base;      // cached search: the base x batch-columns lists of base rows [0, p.row_begin)
+};
+
+// Sizes and carves the workspace of every kNN entry; returns the bytes needed (ws == NULL: size query only).  pb != NULL: the
+// cached search, whose two candidate launches follow the tensor-core plans p and *pb (max_splits = 0 when one declines).
+size_t knn_bufs(void* ws, int n, int d, int k, const KnnPlan& p, const KnnPlan* pb, KnnBufs* out) {
+  Carver cv(ws, ~(size_t)0);
+  const size_t rows = (size_t)(p.row_end - p.row_begin);
+  const size_t stride = (size_t)(pb ? p.tc.max_splits : p.lay.stride);
+  KnnBufs b;
+  memset(&b, 0, sizeof(b));
+  b.sq = cv.take<float>(n);
+  b.small = cv.take<unsigned>(64);
+  b.flag_count = reinterpret_cast<int*>(b.small + 1);
+  b.cand = cv.take<u64>(rows * stride * KC) - (size_t)p.row_begin * stride * KC;
+  b.flag_rows = cv.take<int>(pb ? (size_t)n : rows);
+  b.tc_ws = cv.take<char>(knn_tc_ws_upper(n, d));
+  b.thr_g = cv.take<unsigned>(n);
+  b.rscale = cv.take<float>(n);
+  b.fb_scratch = cv.take<char>(knn_fallback_scratch_bytes());
+  if (k > KC + 1) {
+    b.merged = cv.take<u64>(2 * rows * KC);
+    b.excl = cv.take<u64>(n);
+  }
+  if (!p.ints.empty()) {
+    b.win = cv.take<int2>(n);
+    b.ints = cv.take<int>(p.ints.size());
+  }
+  if (pb) {
+    b.cand_base = cv.take<u64>((size_t)p.row_begin * pb->tc.max_splits * KC);
+    b.merged = cv.take<u64>((size_t)n * KC);
+  }
+  if (out) *out = b;
+  return cv.off;
 }
 
 // fp32 SIMT Gram with the fused top-k epilogue; win != NULL: segmented search (column windows per row)
@@ -1096,11 +1023,9 @@ int launch_simt(const float* X, const float* sq, int n, int d, int cps, int spli
   return GLL_OK;
 }
 
-}  // namespace
-
 // fp16 operand split + norms: rows of up to 1024 padded columns stay in registers (one sweep over X)
-static int launch_split_f16(const float* X, int n, int d, const TcPlan& plan, float* sq, unsigned* small, char* tc_ws, float* rscale,
-                            unsigned* thr_g, cudaStream_t st) {
+int launch_split_f16(const float* X, int n, int d, const TcPlan& plan, float* sq, unsigned* small, char* tc_ws, float* rscale,
+                     unsigned* thr_g, cudaStream_t st) {
   __half* H = reinterpret_cast<__half*>(tc_ws);
   __half* L = (plan.passes == 2) ? reinterpret_cast<__half*>(tc_ws + align_up((size_t)n * plan.d_pad * 2, 256)) : nullptr;
   const int grid = ceil_div((long long)ceil_div(n, plan.d_pad <= 1024 ? 2 : 1) * 32, 256);  // two rows per warp when the row fits registers
@@ -1117,7 +1042,7 @@ static int launch_split_f16(const float* X, int n, int d, const TcPlan& plan, fl
 }
 
 // |x_i|^2 and the global max for the search, plus the fp16 operand split when the tensor-core plan runs
-static int launch_norms(const float* X, int n, int d, const TcPlan& plan, const KnnBufs& b, cudaStream_t st) {
+int launch_norms(const float* X, int n, int d, const TcPlan& plan, const KnnBufs& b, cudaStream_t st) {
   GLL_PROF(KID_SQNORM, st);
   if (plan.ok) return launch_split_f16(X, n, d, plan, b.sq, b.small, b.tc_ws, b.rscale, b.thr_g, st);
   sqnorm_kernel<<<ceil_div((long long)n * 32, 256), 256, 0, st>>>(X, n, d, b.sq, b.small);
@@ -1125,113 +1050,54 @@ static int launch_norms(const float* X, int n, int d, const TcPlan& plan, const 
   return GLL_OK;
 }
 
-// Verification entry (gll_debug_gram_tile): operand split of the whole matrix as knn_run does it, then the raw tensor-core
-// accumulator of unit (row_tile, col_tile) and the rows' operand scale 2^E_i.
-int knn_debug_gram_tile(const float* X, int n, int d, int row_tile, int col_tile, float* acc_out, float* rscale_out, void* ws,
-                        size_t ws_bytes, cudaStream_t st) {
-  GLL_REQUIRE(X && acc_out && rscale_out && ws, "null pointer");
-  GLL_REQUIRE(n >= 256 && d >= 1, "the tensor-core path needs n >= 256");
-  if (ws_bytes < knn_ws_bytes(n, d, 25, 0, n)) {
-    set_error("workspace too small: %zu < %zu", ws_bytes, knn_ws_bytes(n, d, 25, 0, n));
-    return GLL_ERR_WORKSPACE;
-  }
-  const TcPlan plan = knn_tc_plan(n, d, 0, n);
-  GLL_REQUIRE(plan.ok, "tensor-core plan not available for this shape");
-  GLL_REQUIRE(row_tile >= 0 && row_tile * 128 < n && col_tile >= 0 && col_tile * 256 < n, "tile out of range");
-  Carver cv(ws, ws_bytes);
-  float* sq = cv.take<float>(n);
-  unsigned* small = cv.take<unsigned>(64);
-  char* tc_ws = cv.take<char>(knn_tc_ws_upper(n, d));
-  float* rscale = cv.take<float>(n);
-  GLL_CUDA_CHECK(cudaMemsetAsync(small, 0, 256, st));
-  const int rcs = launch_split_f16(X, n, d, plan, sq, small, tc_ws, rscale, nullptr, st);
-  if (rcs) return rcs;
-  GLL_CUDA_CHECK(cudaMemcpyAsync(rscale_out, rscale, sizeof(float) * (size_t)n, cudaMemcpyDeviceToDevice, st));
-  return knn_tc_debug_tile(plan, n, tc_ws, row_tile, col_tile, acc_out, st);
-}
-
-// ---- k in (33, 64]: two rounds of the tensor-core search, the second admits only keys beyond the first round's 32nd ----
-// The merged lists and excl are carved from cv behind the search's buffers; seg != NULL: the segmented unit grid (lay.tc == 3,
-// or 2 when aligned), whose masked columns never enter a set in either round.
-static int knn_run64(const float* X, const KnnBufs& kb, Carver& cv, int n, int d, int k, int row_begin, int row_end, const TcPlan& plan,
-                     const CandLayout& lay, int* knn_idx, float* knn_dist, int* info, cudaStream_t st, const SegDev* seg) {
-  const int rows = row_end - row_begin;
-  u64* merged1 = cv.take<u64>((size_t)rows * KC);
-  u64* merged2 = cv.take<u64>((size_t)rows * KC);
-  u64* excl = cv.take<u64>(n);
-  const int mblocks = ceil_div(rows, RERANK_WARPS);
-  int rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, row_end, plan, kb.tc_ws, kb.cand, nullptr, kb.thr_g, st, seg);
-  if (rc) return rc;
-  {
+// Exact re-rank of rows [lay.row_begin, row_end), their completeness proof, and the brute-force search of the rows it could not
+// prove.  k <= 33: the candidate lists `cand` under `lay`; k > 33: b.merged, the two rounds' merged lists.
+int knn_finish(const float* X, int n, int d, int k, int row_end, const CandLayout& lay, const u64* cand, float err_coef,
+               const KnnBufs& b, int* knn_idx, float* knn_dist, int* info, cudaStream_t st) {
+  const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
+  const bool two_rounds = k > KC + 1;
+  const int row_begin = lay.row_begin, blocks = ceil_div(row_end - row_begin, RERANK_WARPS);
+  const size_t smem = sizeof(float) * (size_t)RERANK_WARPS * d, fsmem = sizeof(float) * (size_t)d;
+  const char* force = getenv("GLL_B200_KNN_FORCE_FALLBACK");
+  const int force_rows = force ? atoi(force) : 0;
+  const bool no_fallback = getenv("GLL_B200_KNN_DEBUG") != nullptr;  // timing experiments: every row would be "unproven"
+  if (two_rounds) {
+    auto kern = vec4 ? knn_rerank64_kernel<true> : knn_rerank64_kernel<false>;
+    GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)smem));
     GLL_PROF(KID_RERANK, st);
-    knn_merge_kernel<<<mblocks, RERANK_WARPS * 32, 0, st>>>(row_end, lay, kb.cand, merged1, excl);
+    kern<<<blocks, RERANK_WARPS * 32, smem, st>>>(X, b.sq, b.small, n, d, k, row_begin, row_end, b.merged,
+                                                 b.merged + (size_t)(row_end - row_begin) * KC, err_coef, knn_idx, knn_dist,
+                                                 b.flag_count, b.flag_rows, force_rows);
+  } else {
+    auto kern = vec4 ? knn_rerank_kernel<true> : knn_rerank_kernel<false>;
+    GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)smem));
+    GLL_PROF(KID_RERANK, st);
+    kern<<<blocks, RERANK_WARPS * 32, smem, st>>>(X, b.sq, b.small, n, d, k, row_end, lay, cand, err_coef, knn_idx, knn_dist,
+                                                 b.flag_count, b.flag_rows, force_rows);
   }
   GLL_LAUNCH_CHECK();
-  // second round: own thresholds
-  rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, row_end, plan, kb.tc_ws, kb.cand, excl, nullptr, st, seg);
-  if (rc) return rc;
-  {
-    GLL_PROF(KID_RERANK, st);
-    knn_merge_kernel<<<mblocks, RERANK_WARPS * 32, 0, st>>>(row_end, lay, kb.cand, merged2, nullptr);
+  if (no_fallback) return GLL_OK;
+  if (two_rounds) {
+    auto kern = vec4 ? knn_fallback_kernel<true> : knn_fallback_kernel<false>;
+    GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)fsmem));
+    GLL_PROF(KID_KNN_FALLBACK, st);
+    kern<<<device_info().sms, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, b.flag_count, b.flag_rows, knn_idx, knn_dist, info, b.win);
+  } else {
+    // the rows' column ranges dealt to all CTAs
+    const int fblocks = knn_fallback_grid();
+    double* part_d = reinterpret_cast<double*>(b.fb_scratch);
+    int* part_j = reinterpret_cast<int*>(part_d + (size_t)fblocks * 32);
+    auto kern = vec4 ? knn_fallback_scan_kernel<true> : knn_fallback_scan_kernel<false>;
+    GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)fsmem));
+    GLL_PROF(KID_KNN_FALLBACK, st);
+    kern<<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, b.flag_count, b.flag_rows, knn_idx, knn_dist, info, part_d, part_j,
+                                                b.small + 8, b.win);
   }
   GLL_LAUNCH_CHECK();
-  return knn_finish64(X, kb.sq, kb.small, n, d, k, row_begin, row_end, merged1, merged2, knn_tc_err_coef(d, plan.passes), knn_idx, knn_dist,
-                      kb.flag_count, kb.flag_rows, info, st, seg ? seg->win : nullptr);
+  return GLL_OK;
 }
 
-int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int* knn_idx, float* knn_dist, int* info,
-            void* ws, size_t ws_bytes, cudaStream_t st) {
-  GLL_REQUIRE(X && knn_idx && knn_dist && ws, "null pointer");
-  GLL_REQUIRE(n >= k && k >= 2 && k <= 2 * KC, "need n >= k and 2 <= k <= 64");
-  GLL_REQUIRE(d >= 1, "d must be positive");
-  GLL_REQUIRE(0 <= row_begin && row_begin < row_end && row_end <= n, "bad row range");
-  if (ws_bytes < knn_ws_bytes(n, d, k, row_begin, row_end)) {
-    set_error("kNN workspace too small: %zu < %zu", ws_bytes, knn_ws_bytes(n, d, k, row_begin, row_end));
-    return GLL_ERR_WORKSPACE;
-  }
-  const int rows = row_end - row_begin;
-  Carver cv(ws, ws_bytes);
-  const KnnBufs kb = knn_carve(cv, n, d, row_begin, row_end, cand_stride(n, d, row_begin, row_end));
-  float* sq = kb.sq;
-  unsigned* small = kb.small;
-  unsigned* sqmax_bits = small;
-  int* flag_count = kb.flag_count;
-  u64* cand = kb.cand;
-  int* flag_rows = kb.flag_rows;
-  char* tc_ws = kb.tc_ws;
-  unsigned* thr_g = kb.thr_g;
-  float* rscale = kb.rscale;
-
-  CandLayout lay;
-  float err_coef;
-  const TcPlan plan = knn_tc_plan(n, d, row_begin, row_end);
-  GLL_CUDA_CHECK(cudaMemsetAsync(small, 0, 256, st));
-  {
-    const int rcs = launch_norms(X, n, d, plan, kb, st);
-    if (rcs) return rcs;
-  }
-
-  if (k > KC + 1) {
-    GLL_REQUIRE(plan.ok, "k > 33 needs the tensor-core path (n >= 256, row range starting on a multiple of 128)");
-    return knn_run64(X, kb, cv, n, d, k, row_begin, row_end, plan, layout_of(plan, row_begin), knn_idx, knn_dist, info, st, nullptr);
-  }
-  if (plan.ok) {  // tcgen05 / TMA Gram GEMM with the fused top-k epilogue
-    int rc = knn_tc_candidates(X, sq, rscale, small, n, d, row_end, plan, tc_ws, cand, nullptr, thr_g, st);
-    if (rc) return rc;
-    lay = layout_of(plan, row_begin);
-    err_coef = knn_tc_err_coef(d, plan.passes);
-  } else {  // fp32 SIMT Gram (tiny graphs, or forced by GLL_B200_KNN_PATH=simt)
-    int cps;
-    const int splits = simt_splits(n, rows, &cps);
-    const int rc = launch_simt(X, sq, n, d, cps, splits, cand, row_begin, row_end, nullptr, st);
-    if (rc) return rc;
-    lay = simt_layout(splits);
-    err_coef = simt_err_coef(d);
-  }
-  return knn_finish(X, sq, sqmax_bits, n, d, k, row_begin, row_end, lay, cand, err_coef, knn_idx, knn_dist, flag_count, flag_rows,
-                    info, kb.fb_scratch, st);
-}
-
+}  // namespace
 
 // ------------------------------------------------------------------------------------------------------------------------
 // Segmented search (gll_knn_segments): independent graphs stacked as row segments; row i of segment s gets its k nearest
@@ -1257,39 +1123,84 @@ __global__ void seg_windows_kernel(const int* __restrict__ seg_ptr, int2* __rest
   for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) win[i] = make_int2(lo, hi);
 }
 
-// SIMT column splits of a segmented search: the widest union of windows over a 128-row tile takes the place of n
-int simt_seg_splits(int n, const int* seg_ptr, int* cols_per_split) {
-  int wmax = 1;
-  for (int r0 = 0, s = 0; r0 < n; r0 += BM) {
-    while (seg_ptr[s + 1] <= r0) ++s;
-    int t = s;
-    const int r1 = min(n, r0 + BM) - 1;
-    while (seg_ptr[t + 1] <= r1) ++t;
-    wmax = max(wmax, seg_ptr[t + 1] - seg_ptr[s]);
+// The plain search of rows [row_begin, row_end) and (nseg > 1) the segmented search: checks, norms, one candidate round (two for
+// k > 33, the second admitting only keys beyond the first round's 32nd), finish.  The arguments are checked by the callers.
+int knn_search(const float* X, int n, int d, int k, int row_begin, int row_end, const int* seg_ptr, int nseg, int* knn_idx,
+               float* knn_dist, int* info, void* ws, size_t ws_bytes, cudaStream_t st) {
+  KnnPlan p = knn_plan(n, d, row_begin, row_end, 0, seg_ptr, nseg);
+  KnnBufs b;
+  const size_t need = knn_bufs(ws, n, d, k, p, nullptr, &b);
+  if (ws_bytes < need) {
+    set_error("kNN workspace too small: %zu < %zu", ws_bytes, need);
+    return GLL_ERR_WORKSPACE;
   }
-  return simt_splits(wmax, n, cols_per_split);
-}
-
-struct SegPlan {
-  TcPlan tc;
-  std::vector<int> tab;  // gfirst, gct, bstart of the tensor-core plan
-  int stride, cps;       // candidate lists per row; SIMT: columns per split
-};
-
-SegPlan seg_plan(int n, int d, const int* seg_ptr, int nseg) {
-  SegPlan p;
-  p.tc = knn_tc_plan_segments(n, d, seg_ptr, nseg, &p.tab);
-  p.cps = 0;
-  if (p.tc.ok) {
-    p.stride = p.tc.max_splits;
-  } else {
-    p.tab.clear();
-    p.stride = simt_seg_splits(n, seg_ptr, &p.cps);
+  GLL_REQUIRE(k <= KC + 1 || p.tc.ok, "k > 33 needs the tensor-core path (n >= 256, row range starting on a multiple of 128)");
+  const char* sh = getenv("GLL_B200_KNN_SHARE");  // "0": every candidate set keeps its own threshold (experiments)
+  if (sh && sh[0] == '0') b.thr_g = nullptr;
+  SegDev sd;
+  memset(&sd, 0, sizeof(sd));
+  const SegDev* seg = nullptr;
+  GLL_CUDA_CHECK(cudaMemsetAsync(b.small, 0, 256, st));
+  if (b.win) {
+    {
+      GLL_PROF(KID_KNN_SEGMENTS, st);
+      for (size_t o = 0; o < p.ints.size(); o += UPLOAD_INTS) {
+        IntChunk c;
+        const int cnt = (int)std::min<size_t>(UPLOAD_INTS, p.ints.size() - o);
+        memcpy(c.v, p.ints.data() + o, sizeof(int) * (size_t)cnt);
+        upload_ints_kernel<<<1, 256, 0, st>>>(c, cnt, b.ints + o);
+      }
+      seg_windows_kernel<<<nseg, 256, 0, st>>>(b.ints, b.win);
+      GLL_LAUNCH_CHECK();
+    }
+    if (p.tc.ok) {
+      sd.win = b.win;
+      sd.gfirst = b.ints + nseg + 1;
+      sd.gct = sd.gfirst + p.tc.row_tiles + 1;
+      sd.bstart = sd.gct + p.tc.row_tiles;
+      p.lay.gfirst = sd.gfirst;
+      seg = &sd;
+    }
   }
-  return p;
+  int rc = launch_norms(X, n, d, p.tc, b, st);
+  if (rc) return rc;
+  if (k > KC + 1) {
+    const int rows = row_end - row_begin;
+    for (int round = 0; round < 2; ++round) {
+      rc = knn_tc_candidates(X, b.sq, b.rscale, b.small, n, d, row_end, p.tc, b.tc_ws, b.cand, round ? b.excl : nullptr,
+                             round ? nullptr : b.thr_g, st, seg);  // the second round keeps its own thresholds
+      if (rc) return rc;
+      {
+        GLL_PROF(KID_RERANK, st);
+        knn_merge_kernel<<<ceil_div(rows, RERANK_WARPS), RERANK_WARPS * 32, 0, st>>>(row_end, p.lay, b.cand,
+                                                                                    b.merged + (size_t)round * rows * KC,
+                                                                                    round ? nullptr : b.excl);
+      }
+      GLL_LAUNCH_CHECK();
+    }
+  } else if (p.tc.ok) {  // tcgen05 / TMA Gram GEMM with the fused top-k epilogue
+    rc = knn_tc_candidates(X, b.sq, b.rscale, b.small, n, d, row_end, p.tc, b.tc_ws, b.cand, nullptr, b.thr_g, st, seg);
+  } else {  // fp32 SIMT Gram (tiny graphs, or forced by GLL_B200_KNN_PATH=simt)
+    rc = launch_simt(X, b.sq, n, d, p.cps, p.lay.stride, b.cand, row_begin, row_end, b.win, st);
+  }
+  if (rc) return rc;
+  return knn_finish(X, n, d, k, row_end, p.lay, b.cand, p.err_coef, b, knn_idx, knn_dist, info, st);
 }
 
 }  // namespace
+
+size_t knn_ws_bytes(int n, int d, int k, int row_begin, int row_end) {
+  return knn_bufs(nullptr, n, d, k, knn_plan(n, d, row_begin, row_end), nullptr, nullptr);
+}
+
+int knn_run(const float* X, int n, int d, int k, int row_begin, int row_end, int* knn_idx, float* knn_dist, int* info,
+            void* ws, size_t ws_bytes, cudaStream_t st) {
+  GLL_REQUIRE(X && knn_idx && knn_dist && ws, "null pointer");
+  GLL_REQUIRE(n >= k && k >= 2 && k <= 2 * KC, "need n >= k and 2 <= k <= 64");
+  GLL_REQUIRE(d >= 1, "d must be positive");
+  GLL_REQUIRE(0 <= row_begin && row_begin < row_end && row_end <= n, "bad row range");
+  return knn_search(X, n, d, k, row_begin, row_end, nullptr, 1, knn_idx, knn_dist, info, ws, ws_bytes, st);
+}
 
 int knn_seg_check(int n, int d, int k, const int* seg_ptr, int nseg) {
   GLL_REQUIRE(seg_ptr != nullptr, "null seg_ptr");
@@ -1306,73 +1217,16 @@ int knn_seg_check(int n, int d, int k, const int* seg_ptr, int nseg) {
 
 size_t knn_seg_ws_bytes(int n, int d, int k, const int* seg_ptr, int nseg) {
   if (knn_seg_check(n, d, k, seg_ptr, nseg) != GLL_OK) return 0;
-  if (nseg == 1) return knn_ws_bytes(n, d, k, 0, n);
-  const SegPlan p = seg_plan(n, d, seg_ptr, nseg);
-  size_t b = knn_common_bytes(n, d, (size_t)n, p.stride);
-  b += align_up(sizeof(int2) * (size_t)n, 256);                                      // windows
-  b += align_up(sizeof(int) * ((size_t)nseg + 1 + p.tab.size()), 256);               // seg_ptr + unit table
-  if (k > KC + 1) b += 2 * align_up(sizeof(u64) * (size_t)n * KC, 256) + align_up(sizeof(u64) * (size_t)n, 256);  // merged lists, excl
-  return b + 2048;
+  return knn_bufs(nullptr, n, d, k, knn_plan(n, d, 0, n, 0, seg_ptr, nseg), nullptr, nullptr);
 }
 
+// nseg == 1 is the plain search over all rows
 int knn_run_segments(const float* X, int n, int d, int k, const int* seg_ptr, int nseg, int* knn_idx, float* knn_dist, int* info,
                      void* ws, size_t ws_bytes, cudaStream_t st) {
   GLL_REQUIRE(X && knn_idx && knn_dist && ws, "null pointer");
-  const int rc0 = knn_seg_check(n, d, k, seg_ptr, nseg);
-  if (rc0) return rc0;
-  if (nseg == 1) return knn_run(X, n, d, k, 0, n, knn_idx, knn_dist, info, ws, ws_bytes, st);  // the unsegmented search as is
-  const size_t need = knn_seg_ws_bytes(n, d, k, seg_ptr, nseg);
-  if (ws_bytes < need) {
-    set_error("kNN workspace too small: %zu < %zu", ws_bytes, need);
-    return GLL_ERR_WORKSPACE;
-  }
-  const SegPlan sp = seg_plan(n, d, seg_ptr, nseg);
-  const TcPlan& plan = sp.tc;
-  GLL_REQUIRE(k <= KC + 1 || plan.ok, "k > 33 needs the tensor-core path");
-  Carver cv(ws, ws_bytes);
-  const KnnBufs kb = knn_carve(cv, n, d, 0, n, sp.stride);
-  int2* win = cv.take<int2>(n);
-  int* ints = cv.take<int>((size_t)nseg + 1 + sp.tab.size());  // seg_ptr, then gfirst, gct, bstart
-  GLL_CUDA_CHECK(cudaMemsetAsync(kb.small, 0, 256, st));
-  {
-    GLL_PROF(KID_KNN_SEGMENTS, st);
-    std::vector<int> host(seg_ptr, seg_ptr + nseg + 1);
-    host.insert(host.end(), sp.tab.begin(), sp.tab.end());
-    for (size_t o = 0; o < host.size(); o += UPLOAD_INTS) {
-      IntChunk c;
-      const int cnt = (int)std::min<size_t>(UPLOAD_INTS, host.size() - o);
-      memcpy(c.v, host.data() + o, sizeof(int) * (size_t)cnt);
-      upload_ints_kernel<<<1, 256, 0, st>>>(c, cnt, ints + o);
-    }
-    seg_windows_kernel<<<nseg, 256, 0, st>>>(ints, win);
-    GLL_LAUNCH_CHECK();
-  }
-  {
-    const int rcs = launch_norms(X, n, d, plan, kb, st);
-    if (rcs) return rcs;
-  }
-  CandLayout lay;
-  float err_coef;
-  if (plan.ok) {
-    const int RG = plan.row_tiles;
-    SegDev sd;
-    sd.win = win;
-    sd.gfirst = ints + nseg + 1;
-    sd.gct = sd.gfirst + RG + 1;
-    sd.bstart = sd.gct + RG;
-    lay = layout_of(plan, 0, sd.gfirst);
-    if (k > KC + 1) return knn_run64(X, kb, cv, n, d, k, 0, n, plan, lay, knn_idx, knn_dist, info, st, &sd);
-    const int rc = knn_tc_candidates(X, kb.sq, kb.rscale, kb.small, n, d, n, plan, kb.tc_ws, kb.cand, nullptr, kb.thr_g, st, &sd);
-    if (rc) return rc;
-    err_coef = knn_tc_err_coef(d, plan.passes);
-  } else {
-    const int rc = launch_simt(X, kb.sq, n, d, sp.cps, sp.stride, kb.cand, 0, n, win, st);
-    if (rc) return rc;
-    lay = simt_layout(sp.stride);
-    err_coef = simt_err_coef(d);
-  }
-  return knn_finish(X, kb.sq, kb.small, n, d, k, 0, n, lay, kb.cand, err_coef, knn_idx, knn_dist, kb.flag_count, kb.flag_rows, info,
-                    kb.fb_scratch, st, win);
+  const int rc = knn_seg_check(n, d, k, seg_ptr, nseg);
+  if (rc) return rc;
+  return knn_search(X, n, d, k, 0, n, seg_ptr, nseg, knn_idx, knn_dist, info, ws, ws_bytes, st);
 }
 
 // units the tensor-core search of a segmented call issues, and those of the uniform grid over the same rows (0, 0: SIMT path)
@@ -1388,6 +1242,28 @@ void knn_seg_units(int n, int d, const int* seg_ptr, int nseg, long long* seg_un
   }
   std::vector<int> tab;
   *seg_units = knn_tc_plan_segments(n, d, seg_ptr, nseg, &tab).units;
+}
+
+// Verification entry (gll_debug_gram_tile): operand split of the whole matrix as knn_run does it, then the raw tensor-core
+// accumulator of unit (row_tile, col_tile) and the rows' operand scale 2^E_i.
+int knn_debug_gram_tile(const float* X, int n, int d, int row_tile, int col_tile, float* acc_out, float* rscale_out, void* ws,
+                        size_t ws_bytes, cudaStream_t st) {
+  GLL_REQUIRE(X && acc_out && rscale_out && ws, "null pointer");
+  GLL_REQUIRE(n >= 256 && d >= 1, "the tensor-core path needs n >= 256");
+  const KnnPlan p = knn_plan(n, d, 0, n);
+  KnnBufs b;
+  const size_t need = knn_bufs(ws, n, d, 2, p, nullptr, &b);
+  if (ws_bytes < need) {
+    set_error("workspace too small: %zu < %zu", ws_bytes, need);
+    return GLL_ERR_WORKSPACE;
+  }
+  GLL_REQUIRE(p.tc.ok, "tensor-core plan not available for this shape");
+  GLL_REQUIRE(row_tile >= 0 && row_tile * 128 < n && col_tile >= 0 && col_tile * 256 < n, "tile out of range");
+  GLL_CUDA_CHECK(cudaMemsetAsync(b.small, 0, 256, st));
+  const int rcs = launch_norms(X, n, d, p.tc, b, st);
+  if (rcs) return rcs;
+  GLL_CUDA_CHECK(cudaMemcpyAsync(rscale_out, b.rscale, sizeof(float) * (size_t)n, cudaMemcpyDeviceToDevice, st));
+  return knn_tc_debug_tile(p.tc, n, b.tc_ws, row_tile, col_tile, acc_out, st);
 }
 
 // ------------------------------------------------------------------------------------------------------------------------
@@ -1428,48 +1304,44 @@ knn_merge_cached_kernel(int r0, int n, CandLayout layA, const u64* __restrict__ 
   const CandLayout& lay = base ? layB : layA;
   const u64* cand = base ? candB : candA;
   u64 mine = base ? cache[(size_t)i * KC + lane] : KEY_INF;
-  int splits = lay.stride;
-  if (lay.tc == 1) {
-    int b0, b1;
-    cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
-    splits = 2 * (b1 - b0 + 1);
-  }
+  const int splits = cand_lists(lay, i);
   for (int s = 0; s < splits; ++s) list_merge_set(mine, cand[((size_t)i * lay.stride + s) * KC + lane], lane);
   merged[(size_t)i * KC + lane] = mine;
+}
+
+// The plans and the workspace of a cached search: batch rows [r0, n) against all columns, base rows [0, r0) against the batch
+// columns.  One candidate round whatever k: the cached search serves k <= 33.
+size_t cached_bufs(void* ws, int n, int d, int nb, KnnPlan* pa, KnnPlan* pb, KnnBufs* b) {
+  const int r0 = nb / 128 * 128;  // base rows [r0, n_base) ride along with the batch rows (row ranges start on a tile)
+  *pa = knn_plan(n, d, r0, n);
+  *pb = knn_plan(n, d, 0, r0 > 0 ? r0 : 128, nb);
+  return knn_bufs(ws, n, d, KC + 1, *pa, pb, b);
 }
 
 }  // namespace
 
 size_t knn_base_cache_bytes(int n_base) { return align_up(sizeof(u64) * (size_t)n_base * KC, 256); }
 
+// sized like gll_knn on the base rows (gll_base_cache_workspace_bytes)
 int knn_base_cache_build(const float* Xb, int nb, int d, void* cache, void* ws, size_t ws_bytes, cudaStream_t st) {
   GLL_REQUIRE(Xb && cache && ws, "null pointer");
   GLL_REQUIRE(nb >= KC + 1 && d >= 1, "bad sizes");
-  if (ws_bytes < knn_ws_bytes(nb, d, 25, 0, nb)) {
-    set_error("kNN workspace too small: %zu < %zu", ws_bytes, knn_ws_bytes(nb, d, 25, 0, nb));
+  const KnnPlan p = knn_plan(nb, d, 0, nb);
+  KnnBufs b;
+  const size_t need = knn_bufs(ws, nb, d, 2, p, nullptr, &b);
+  if (ws_bytes < need) {
+    set_error("kNN workspace too small: %zu < %zu", ws_bytes, need);
     return GLL_ERR_WORKSPACE;
   }
-  const TcPlan plan = knn_tc_plan(nb, d, 0, nb);
-  GLL_REQUIRE(plan.ok, "the base-set cache needs the tensor-core search (n_base >= 256)");
-  Carver cv(ws, ws_bytes);
-  float* sq = cv.take<float>(nb);
-  unsigned* small = cv.take<unsigned>(64);
-  u64* cand = cv.take<u64>((size_t)nb * plan.max_splits * KC);
-  char* tc_ws = cv.take<char>(knn_tc_ws_upper(nb, d));
-  unsigned* thr_g = cv.take<unsigned>(nb);
-  float* rscale = cv.take<float>(nb);
-  GLL_CUDA_CHECK(cudaMemsetAsync(small, 0, 256, st));
-  int rc;
-  {
-    GLL_PROF(KID_SQNORM, st);
-    rc = launch_split_f16(Xb, nb, d, plan, sq, small, tc_ws, rscale, thr_g, st);
-  }
+  GLL_REQUIRE(p.tc.ok, "the base-set cache needs the tensor-core search (n_base >= 256)");
+  GLL_CUDA_CHECK(cudaMemsetAsync(b.small, 0, 256, st));
+  int rc = launch_norms(Xb, nb, d, p.tc, b, st);
   if (rc) return rc;
-  rc = knn_tc_candidates(Xb, sq, rscale, small, nb, d, nb, plan, tc_ws, cand, nullptr, thr_g, st);
+  rc = knn_tc_candidates(Xb, b.sq, b.rscale, b.small, nb, d, nb, p.tc, b.tc_ws, b.cand, nullptr, b.thr_g, st);
   if (rc) return rc;
   {
     GLL_PROF(KID_RERANK, st);
-    knn_merge_kernel<<<ceil_div(nb, RERANK_WARPS), RERANK_WARPS * 32, 0, st>>>(nb, layout_of(plan, 0), cand, (u64*)cache, nullptr);
+    knn_merge_kernel<<<ceil_div(nb, RERANK_WARPS), RERANK_WARPS * 32, 0, st>>>(nb, p.lay, b.cand, (u64*)cache, nullptr);
   }
   GLL_LAUNCH_CHECK();
   return GLL_OK;
@@ -1477,18 +1349,8 @@ int knn_base_cache_build(const float* Xb, int nb, int d, void* cache, void* ws, 
 
 size_t knn_cached_ws_bytes(int n, int d, int k, int nb) {
   (void)k;
-  const int r0 = nb / 128 * 128;
-  const TcPlan pa = knn_tc_plan(n, d, r0, n), pb = knn_tc_plan(n, d, 0, r0 > 0 ? r0 : 128, nb);
-  size_t b = 0;
-  b += align_up(sizeof(float) * (size_t)n, 256) + 256;
-  b += align_up(sizeof(u64) * (size_t)(n - r0) * (size_t)(pa.ok ? pa.max_splits : 1) * KC, 256);
-  b += align_up(sizeof(u64) * (size_t)r0 * (size_t)(pb.ok ? pb.max_splits : 1) * KC, 256);
-  b += align_up(sizeof(int) * (size_t)n, 256);
-  b += knn_tc_ws_upper(n, d);
-  b += 2 * align_up(sizeof(unsigned) * (size_t)n, 256);
-  b += align_up(sizeof(u64) * (size_t)n * KC, 256);
-  b += knn_fallback_scratch_bytes() + 256;
-  return b + 2048;
+  KnnPlan pa, pb;
+  return cached_bufs(nullptr, n, d, nb, &pa, &pb, nullptr);
 }
 
 int knn_run_cached(const float* X, int n, int d, int k, int nb, const void* cache_v, int* knn_idx, float* knn_dist, int* info, void* ws,
@@ -1496,56 +1358,41 @@ int knn_run_cached(const float* X, int n, int d, int k, int nb, const void* cach
   GLL_REQUIRE(X && cache_v && knn_idx && knn_dist && ws, "null pointer");
   GLL_REQUIRE(k >= 2 && k <= KC + 1, "the base-set cache serves k <= 33");
   GLL_REQUIRE(nb >= KC + 1 && nb < n && d >= 1, "need 32 < n_base < n");
-  if (ws_bytes < knn_cached_ws_bytes(n, d, k, nb)) {
-    set_error("kNN workspace too small: %zu < %zu", ws_bytes, knn_cached_ws_bytes(n, d, k, nb));
+  KnnPlan pa, pb;
+  KnnBufs b;
+  const size_t need = cached_bufs(ws, n, d, nb, &pa, &pb, &b);
+  if (ws_bytes < need) {
+    set_error("kNN workspace too small: %zu < %zu", ws_bytes, need);
     return GLL_ERR_WORKSPACE;
   }
   const u64* cache = (const u64*)cache_v;
-  const int r0 = nb / 128 * 128;  // base rows [r0, n_base) ride along with the batch rows (row ranges start on a tile)
-  const TcPlan pa = knn_tc_plan(n, d, r0, n);
-  GLL_REQUIRE(pa.ok, "tensor-core plan not available for this shape");
-  TcPlan pb;
-  memset(&pb, 0, sizeof(pb));
-  if (r0 > 0) {
-    pb = knn_tc_plan(n, d, 0, r0, nb);
-    GLL_REQUIRE(pb.ok, "tensor-core plan not available for this shape");
-  }
-  Carver cv(ws, ws_bytes);
-  float* sq = cv.take<float>(n);
-  unsigned* small = cv.take<unsigned>(64);
-  int* flag_count = reinterpret_cast<int*>(small + 1);
-  u64* candA_store = cv.take<u64>((size_t)(n - r0) * pa.max_splits * KC);
-  u64* candA = candA_store - (size_t)r0 * pa.max_splits * KC;  // indexed by GLOBAL row
-  u64* candB = cv.take<u64>((size_t)r0 * (pb.ok ? pb.max_splits : 1) * KC);
-  int* flag_rows = cv.take<int>(n);
-  char* tc_ws = cv.take<char>(knn_tc_ws_upper(n, d));
-  unsigned* thr_g = cv.take<unsigned>(n);
-  float* rscale = cv.take<float>(n);
-  u64* merged = cv.take<u64>((size_t)n * KC);
-  void* fb_scratch = cv.take<char>(knn_fallback_scratch_bytes());
-  GLL_CUDA_CHECK(cudaMemsetAsync(small, 0, 256, st));
+  const int r0 = pa.row_begin;
+  GLL_REQUIRE(pa.tc.ok, "tensor-core plan not available for this shape");
+  GLL_REQUIRE(r0 == 0 || pb.tc.ok, "tensor-core plan not available for this shape");
+  GLL_CUDA_CHECK(cudaMemsetAsync(b.small, 0, 256, st));
   int rc;
   {
     GLL_PROF(KID_SQNORM, st);
-    rc = launch_split_f16(X, n, d, pa, sq, small, tc_ws, rscale, thr_g, st);
+    rc = launch_split_f16(X, n, d, pa.tc, b.sq, b.small, b.tc_ws, b.rscale, b.thr_g, st);
     if (rc) return rc;
-    if (r0 > 0) base_thr_init_kernel<<<ceil_div(r0, 256), 256, 0, st>>>(cache, sq, small, r0, thr_g);
+    if (r0 > 0) base_thr_init_kernel<<<ceil_div(r0, 256), 256, 0, st>>>(cache, b.sq, b.small, r0, b.thr_g);
     GLL_LAUNCH_CHECK();
   }
-  rc = knn_tc_candidates(X, sq, rscale, small, n, d, n, pa, tc_ws, candA, nullptr, thr_g, st);
+  rc = knn_tc_candidates(X, b.sq, b.rscale, b.small, n, d, n, pa.tc, b.tc_ws, b.cand, nullptr, b.thr_g, st);
   if (rc) return rc;
   if (r0 > 0) {
-    rc = knn_tc_candidates(X, sq, rscale, small, n, d, r0, pb, tc_ws, candB, nullptr, thr_g, st);
+    rc = knn_tc_candidates(X, b.sq, b.rscale, b.small, n, d, r0, pb.tc, b.tc_ws, b.cand_base, nullptr, b.thr_g, st);
     if (rc) return rc;
   }
   {
     GLL_PROF(KID_RERANK, st);
-    knn_merge_cached_kernel<<<ceil_div(n, RERANK_WARPS), RERANK_WARPS * 32, 0, st>>>(r0, n, layout_of(pa, r0), candA, layout_of(pb, 0), candB,
-                                                                                   cache, merged);
+    knn_merge_cached_kernel<<<ceil_div(n, RERANK_WARPS), RERANK_WARPS * 32, 0, st>>>(r0, n, pa.lay, b.cand, pb.lay, b.cand_base,
+                                                                                   cache, b.merged);
   }
   GLL_LAUNCH_CHECK();
-  return knn_finish(X, sq, small, n, d, k, 0, n, simt_layout(1), merged, knn_tc_err_coef(d, pa.passes), knn_idx, knn_dist, flag_count, flag_rows, info,
-                    fb_scratch, st);
+  CandLayout one_list{};  // one sorted list per row
+  one_list.stride = 1;
+  return knn_finish(X, n, d, k, n, one_list, b.merged, pa.err_coef, b, knn_idx, knn_dist, info, st);
 }
 
 }  // namespace gll

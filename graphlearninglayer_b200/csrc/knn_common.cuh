@@ -119,10 +119,13 @@ __device__ __forceinline__ void cand_owner_range(const CandLayout& lay, long lon
   b1 = (int)((f1 * lay.grid - 1) / lay.units);
 }
 
-// win: NULL, or the rows' column windows of a segmented search (the brute-force fallback scans only the window)
-int knn_finish(const float* X, const float* sq, const unsigned* sqmax_bits, int n, int d, int k, int row_begin, int row_end,
-               CandLayout lay,
-               const u64* cand, float err_coef, int* knn_idx, float* knn_dist, int* flag_count, int* flag_rows,
-               int* info, void* fb_scratch, cudaStream_t st, const int2* win = nullptr);
+// candidate lists written for row i: `stride`, or under the tensor-core work split two per CTA that touched the row's group
+// (the column halves of its epilogue)
+__device__ __forceinline__ int cand_lists(const CandLayout& lay, int i) {
+  if (lay.tc != 1 && lay.tc != 3) return lay.stride;
+  int b0, b1;
+  cand_owner_range(lay, (i - lay.row_begin) / lay.row_tile, b0, b1);
+  return 2 * (b1 - b0 + 1);
+}
 
 }  // namespace gll

@@ -124,8 +124,9 @@ def run_cg(_lib, Luu: sp.csr_matrix, B: np.ndarray, tol=1e-7, max_iter=5000):
 # ----------------------------------------------------------------------------------------------------------------
 # K1: kNN
 # ----------------------------------------------------------------------------------------------------------------
+# d = 13000: the brute-force fallback's row copy (4 d bytes) is past the 48 KB that needs no dynamic shared memory opt-in
 KNN_SHAPES = [(0, 300, 500, 64, 10, 2.0), (3, 37, 91, 19, 3, 1.0), (1, 1000, 1000, 128, 10, 3.0),
-              (4, 2048, 1024, 512, 10, 4.5), (6, 10, 20, 7, 2, 0.5), (8, 500, 700, 130, 5, 2.0)]
+              (4, 2048, 1024, 512, 10, 4.5), (6, 10, 20, 7, 2, 0.5), (8, 500, 700, 130, 5, 2.0), (9, 30, 270, 13000, 5, 2.0)]
 
 
 def _set_knn_path(monkeypatch, path):
