@@ -115,6 +115,8 @@ def _warn_from_status(info: torch.Tensor, where: str) -> None:
         warnings.warn(f"max iter reached in the {where} CG solve")  # GLL.py:273-274 prints
     if st & _lib.STATUS_NONFINITE:
         warnings.warn(f"non-finite values in the {where} solve (singular L_uu or epsilon = 0)")
+    if st & _lib.STATUS_BAD_INDEX:
+        warnings.warn(f"{where}: a trial's labeled-row indices are out of range or repeated; that trial is invalid (NaN / -1)")
 
 
 class _DeferredStatus:

@@ -16,6 +16,7 @@ STATUS_CG_NOT_CONVERGED = 1
 STATUS_EPS_TINY = 2
 STATUS_NONFINITE = 4
 STATUS_KNN_FALLBACK = 8
+STATUS_BAD_INDEX = 16
 
 INFO_STATUS, INFO_NNZ, INFO_NNZ_UU, INFO_CG_ITERS_FWD, INFO_CG_ITERS_BWD = 0, 1, 2, 3, 4
 INFO_KNN_FALLBACK_ROWS, INFO_CG_RESID_FWD, INFO_CG_RESID_BWD = 5, 6, 7
@@ -121,6 +122,9 @@ def _load():
     sig("gll_laplace_eval_batched_workspace_bytes", sz, [i32, i32, i32, i32, i32, i32])
     sig("gll_laplace_eval_batched", i32, [vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp, vp, vp,
                                           vp, vp, sz, vp])
+    sig("gll_laplace_eval_trials_workspace_bytes", sz, [i32, i32, i32, i32, i32, i32])
+    sig("gll_laplace_eval_trials", i32, [vp, i32, i32, i32, vp, i32, vp, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp,
+                                         vp, vp, vp, vp, sz, vp])
     return lib
 
 
@@ -139,7 +143,8 @@ EXPORTS = ["gll_last_error", "gll_version", "gll_device_sm_count", "gll_kernel_c
            "gll_normalize_rows_backward", "gll_debug_gram_tile", "gll_base_cache_bytes", "gll_base_cache_workspace_bytes",
            "gll_base_cache_build", "gll_knn_cached_workspace_bytes", "gll_knn_cached", "gll_laplace_eval_workspace_bytes",
            "gll_laplace_eval", "gll_knn_segments_workspace_bytes", "gll_knn_segments", "gll_knn_segments_units",
-           "gll_batched_workspace_bytes", "gll_forward_batched", "gll_laplace_eval_batched_workspace_bytes", "gll_laplace_eval_batched"]
+           "gll_batched_workspace_bytes", "gll_forward_batched", "gll_laplace_eval_batched_workspace_bytes", "gll_laplace_eval_batched",
+           "gll_laplace_eval_trials_workspace_bytes", "gll_laplace_eval_trials"]
 
 
 def check(rc: int, what: str) -> None:

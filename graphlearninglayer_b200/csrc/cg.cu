@@ -107,7 +107,17 @@ __device__ __forceinline__ void grid_reduce(float4 (&acc)[NV], const CgParams& P
   __syncthreads();
 }
 
-__global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P) {
+// Masked operator of laplace_learning_trials: column c of this solve is column col0 + c of `trials` trials of `cols` columns each,
+// and A p is zeroed at (row i, trial t) when slot[i trials + t] >= 0.  A separate parameter, so that CgParams (shared with the
+// on-chip kernels) keeps its layout.
+struct CgMask {
+  const int* slot;
+  int trials, cols, col0;
+};
+
+// MASK = false is the unmasked solve and never reads M
+template <bool MASK>
+__global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P, CgMask M) {
   extern __shared__ __align__(16) double sm[];
   const int lp = P.lp, Q = lp >> 2, S = 32 / Q;
   double* wpart = sm;                            // [2][CG_WARPS][lp]
@@ -203,7 +213,11 @@ __global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P
         const size_t o = (size_t)i * lp + 4 * lane;
         const float4 pi = ldcg4(P.p + o);
         const float dg = __ldg(P.diag + i);
-        const float4 ap = make_float4(fmaf(dg, pi.x, -a.x), fmaf(dg, pi.y, -a.y), fmaf(dg, pi.z, -a.z), fmaf(dg, pi.w, -a.w));
+        float4 ap = make_float4(fmaf(dg, pi.x, -a.x), fmaf(dg, pi.y, -a.y), fmaf(dg, pi.z, -a.z), fmaf(dg, pi.w, -a.w));
+        if constexpr (MASK) {  // row i clamped in this quad's trial: r, p and x stay 0 there (a quad never spans two trials)
+          const int t = (M.col0 + 4 * lane) / M.cols;
+          if (__ldg(M.slot + (size_t)i * M.trials + t) >= 0) ap = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
         st4(P.ap + o, ap);
         dot[0].x = fmaf(pi.x, ap.x, dot[0].x);
         dot[0].y = fmaf(pi.y, ap.y, dot[0].y);
@@ -326,6 +340,7 @@ int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const floa
   // Layer-side conversions (GLL.py:66 float64 output, GLL.py:104 the incoming gradient): the on-chip kernels read / write the
   // caller's arrays themselves; the chunked and the streaming path run the two small kernels around the solve.
   const bool has_src = io != nullptr && io->rhs_src != nullptr, has_copy = io != nullptr && io->x_copy != nullptr;
+  const bool masked = io != nullptr && io->mask_slot != nullptr;
   if (lp > CG_MAX_LP) {
     if (has_src) {
       const int rc = pack_grad(io->rhs_src, io->rhs_kind == 2, m, l, lp, const_cast<float*>(rhs), st, nullptr, 0, io->rhs_scale, io->rhs_scale_f64);
@@ -343,8 +358,15 @@ int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const floa
       const int c0 = c * CG_MAX_LP, cnt = min(CG_MAX_LP, l - c0), lpc = padded_classes(cnt);
       int rc = pack_columns(rhs, m, lp, c0, cnt, rhs_c, lpc, st);
       if (rc) return rc;
+      CgIo mio = {};  // a masked solve: the mask is indexed by the chunk's global columns
+      if (masked) {
+        mio.mask_slot = io->mask_slot;
+        mio.mask_trials = io->mask_trials;
+        mio.mask_cols = io->mask_cols;
+        mio.mask_col0 = io->mask_col0 + c0;
+      }
       rc = cg_run(uu_ptr, uu_col, uu_val, diag, rhs_c, m, cnt, tol, max_iter, x_c, it_c + c, rs_c + c, status_out, sub, sub_bytes, st,
-                  ext_counter);
+                  ext_counter, masked ? &mio : nullptr);
       if (rc) return rc;
       rc = unpack_columns(x_c, m, lpc, c0, cnt, x, lp, st);
       if (rc) return rc;
@@ -381,7 +403,7 @@ int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const floa
   P.x_copy_f64 = io ? io->x_copy_f64 : 0;
   P.rhs_scale = io ? io->rhs_scale : nullptr;
   P.rhs_scale_f64 = io ? io->rhs_scale_f64 : 0;
-  {  // systems that fit on chip (every config except the sharded 1M-node graph) take the shared-memory-resident kernel
+  if (!masked) {  // systems that fit on chip (every config except the sharded 1M-node graph) take the shared-memory-resident kernel
     const char* force = getenv("GLL_B200_CG_PATH");  // "streaming" / "resident" / "small" / "cluster": testing knobs
     const bool only_small = force != nullptr && strcmp(force, "small") == 0;
     const bool force_cluster = force != nullptr && strcmp(force, "cluster") == 0;
@@ -417,11 +439,14 @@ int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const floa
   rpb = ceil_div(rpb, S) * S;  // keep phase-2/3 spans aligned to whole lane groups
   P.rows_per_block = rpb;
   const size_t smem = cg_smem_bytes(lp);
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)cg_persistent_kernel, (int)cg_smem_bytes(CG_MAX_LP)));
+  const void* kern = masked ? (const void*)cg_persistent_kernel<true> : (const void*)cg_persistent_kernel<false>;
+  GLL_CUDA_CHECK(set_max_dynamic_smem_once(kern, (int)cg_smem_bytes(CG_MAX_LP)));
   GLL_CUDA_CHECK(cudaMemsetAsync(P.barrier, 0, 256, st));
-  void* args[] = {&P};
+  CgMask M = {nullptr, 0, 0, 0};
+  if (masked) M = {io->mask_slot, io->mask_trials, io->mask_cols, io->mask_col0};
+  void* args[] = {&P, &M};
   GLL_PROF(KID_CG, st);
-  GLL_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)cg_persistent_kernel, dim3(grid), dim3(CG_THREADS), args, smem, st));
+  GLL_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(CG_THREADS), args, smem, st));
   return has_copy ? unpack_pred(x, m, l, lp, io->x_copy, io->x_copy_f64, st) : GLL_OK;
 }
 

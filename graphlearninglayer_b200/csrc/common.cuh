@@ -97,6 +97,7 @@ enum KernelId {
   KID_EDGE_GRAD, KID_ROW_GATHER, KID_CONVERT, KID_CG_ROWS, KID_LAPLACE_REFINE, KID_LAPLACE_FINISH,
   KID_KNN_SEGMENTS,   // segmented search: upload of seg_ptr and the unit table, per-row column windows
   KID_BATCH_REORDER,  // batched layer: kNN lists to the labeled-first order of the block-diagonal graph
+  KID_LAPLACE_TRIALS_SETUP,  // laplace_learning_trials: the slot table of the labeled rows, index checks
   KID_COUNT
 };
 // RAII: counts the launch; when profiling is on, brackets it with two events on the launch stream.
@@ -178,6 +179,10 @@ struct CgIo {
   const void* rhs_scale;  // optional device scalar multiplied into rhs_src (fp64 if rhs_scale_f64)
   int rhs_scale_f64;
   float uu_degree_hint;   // expected off-diagonal entries per row of the system (0: unknown) -- picks the minibatch kernel
+  // optional row mask of T trials x mask_cols columns (mask_col0: this solve's first column among them): A p is zeroed at (row i,
+  // trial t) where mask_slot[i T + t] >= 0.  A masked solve always runs the streaming kernel.
+  const int* mask_slot;
+  int mask_trials, mask_cols, mask_col0;
 };
 int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const float* diag, const float* rhs, int m,
            int l, float tol, int max_iter, float* x, int* iters_out, float* resid_out, int* status_out, void* ws,

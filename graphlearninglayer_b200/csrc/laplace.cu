@@ -16,6 +16,8 @@
 // writes the correction solve's right-hand-side scale: 1 while some column is above tol, else 0 -- a zero right-hand side
 // stops every CG kernel at iteration 0 and the correction is exactly zero, so the round count is fixed and no host decision
 // is needed.  laplace_finish adds the last correction, writes pred, the argmax labels and the hit count.
+#include <algorithm>
+
 #include "cg_common.cuh"
 #include "common.cuh"
 
@@ -347,6 +349,388 @@ int eval_run(const float* X, const float* Y, int B, int n, int d, int k, int l, 
   return GLL_OK;
 }
 
+// ---------------------------------------------------------------------------------------------- T trials on one graph
+// gll_laplace_eval_trials: trial t clamps the k_lab rows train_idx[t] to the label rows Y[t] and solves the other rows.  The graph
+// is the same in every trial, so the stages run once with k_lab = 0: the system is the FULL graph A = D + tau I - W over all n
+// rows, and trial t masks its clamped rows out of its own columns (cg_persistent_kernel<true>: A p is zeroed there, so r, p and
+// x stay 0 on those rows).  Every [n][C] array has C = T lpad columns, lpad = padded_classes(l): trial t owns the columns
+// [t lpad, t lpad + l), so a class quad never spans two trials.  slot[i T + t] = s when train_idx[t, s] == i, else -1.
+
+// slot / bad from train_idx: slot is -1 on entry (memset), bad zero.  An index outside [0, n) or a repeat (the atomicCAS from -1
+// fails) makes the trial invalid; no index is used before it has been checked.
+__global__ void laplace_trials_setup_kernel(const void* __restrict__ idx, int is_i64, int n, int T, int k_lab, int* __restrict__ slot,
+                                            int* __restrict__ bad, int* __restrict__ info) {
+  const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= (long long)T * k_lab) return;
+  const int t = (int)(q / k_lab), s = (int)(q - (long long)t * k_lab);
+  const long long i = is_i64 ? __ldg(reinterpret_cast<const long long*>(idx) + q) : (long long)__ldg(reinterpret_cast<const int*>(idx) + q);
+  bool ok = i >= 0 && i < n;
+  if (ok) ok = atomicCAS(slot + (size_t)i * T + t, -1, s) == -1;
+  if (!ok) {
+    bad[t] = 1;
+    atomicOr(info + GLL_INFO_STATUS, GLL_STATUS_BAD_INDEX);
+  }
+}
+
+struct TrialsRefineParams {
+  const int* row_ptr;  // full graph, n rows
+  const int* col;
+  const float* w;
+  const float* Y;        // T x k_lab x l
+  const int* slot;       // [n][T]
+  const int* bad;        // [T]
+  const double* x_prev;  // [n][C], or NULL
+  const float* e;        // [n][C] fp32 correction (round 0: the initial solution), or NULL: x = 0
+  double* x_out;         // [n][C], or NULL
+  double* r_out;         // [n][C]: right-hand side of the next solve (padding columns stay 0)
+  double* partial;       // [gx][T l]
+  double* colnorm;       // [T l]
+  double* resid;         // [T] or NULL
+  double* scale;         // 1 scalar
+  unsigned* ticket;      // 1
+  int* info;
+  int n, T, k_lab, l, lpad, gx, cw, round;  // round < 0: r = b only (x = 0), no stop-rule bookkeeping
+  double tau, tol;
+};
+
+// laplace_refine_kernel per (row, trial column): block = RL row lanes x CW of the T l class columns, blockIdx.y picks the chunk of
+// CW columns.  A row clamped in trial t, and every row of an invalid trial, has r = 0; a neighbour j clamped in trial t reads
+// u_j = Y[t, slot], the others the iterate.  Column partials are added in CTA order by the last CTA (one integer ticket); it
+// writes each valid trial's largest column norm (resid: NaN for an invalid trial), and the correction scale is 1 while any
+// column of any valid trial is above tol.  No floating-point atomics.
+__global__ void __launch_bounds__(LR_THREADS) laplace_refine_trials_kernel(TrialsRefineParams P) {
+  __shared__ double red[LR_THREADS];
+  __shared__ bool last;
+  const int cw = P.cw, rl_count = LR_THREADS / cw, TL = P.T * P.l;
+  const int tid = threadIdx.x, rl = tid / cw, cc = tid - rl * cw;
+  const int c = blockIdx.y * cw + cc;
+  const bool active = rl < rl_count && c < TL;
+  double acc = 0.0;
+  if (active) {
+    const int T = P.T, l = P.l, t = c / l, cl = c - t * l;
+    const size_t C = (size_t)T * P.lpad, sc = (size_t)t * P.lpad + cl;
+    const float* Yt = P.Y + (size_t)t * P.k_lab * l + cl;
+    const bool valid = __ldg(P.bad + t) == 0;
+    for (int i = blockIdx.x * rl_count + rl; i < P.n; i += P.gx * rl_count) {
+      const size_t o = (size_t)i * C + sc;
+      const double xi = (P.x_prev ? __ldg(P.x_prev + o) : 0.0) + (P.e ? (double)__ldg(P.e + o) : 0.0);
+      if (P.x_out) P.x_out[o] = xi;
+      if (!valid || __ldg(P.slot + (size_t)i * T + t) >= 0) {
+        P.r_out[o] = 0.0;
+        continue;
+      }
+      const int e1 = __ldg(P.row_ptr + i + 1);
+      double s = 0.0, deg = 0.0;
+      for (int e = __ldg(P.row_ptr + i); e < e1; ++e) {
+        const int j = __ldg(P.col + e);
+        const double wv = (double)__ldg(P.w + e);
+        const int sj = __ldg(P.slot + (size_t)j * T + t);
+        const size_t oj = (size_t)j * C + sc;
+        const double uj = (sj >= 0) ? (double)__ldg(Yt + (size_t)sj * l)
+                                    : (P.x_prev ? __ldg(P.x_prev + oj) : 0.0) + (P.e ? (double)__ldg(P.e + oj) : 0.0);
+        s = fma(wv, uj - xi, s);
+        deg += wv;
+      }
+      const double r = s - P.tau * xi;
+      P.r_out[o] = r;
+      acc = fma(r, r / (deg + P.tau + 1e-10), acc);
+    }
+  }
+  if (P.round < 0) return;  // grid-uniform
+  red[tid] = acc;
+  __syncthreads();
+  if (tid < cw && c < TL) {
+    double t = 0.0;
+    for (int q = 0; q < rl_count; ++q) t += red[q * cw + tid];
+    P.partial[(size_t)blockIdx.x * TL + c] = t;
+  }
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last = atomicAdd(P.ticket, 1u) == P.gx * gridDim.y - 1u;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  const int lane = tid & 31, warp = tid >> 5;
+  for (int c2 = warp; c2 < TL; c2 += LR_THREADS / 32) {
+    double t = 0.0;
+    for (int q = lane; q < P.gx; q += 32) t += __ldcg(P.partial + (size_t)q * TL + c2);
+    t = warp_sum(t);
+    if (lane == 0) P.colnorm[c2] = sqrt(t);
+  }
+  __syncthreads();
+  // per trial the largest column norm; the maximum over valid trials is exact, so its order does not matter
+  double mx = 0.0;
+  bool bad = false;
+  for (int t = tid; t < P.T; t += LR_THREADS) {
+    double tm = 0.0;
+    bool tb = false;
+    for (int c2 = t * P.l; c2 < (t + 1) * P.l; ++c2) {
+      const double v = P.colnorm[c2];
+      if (!(v == v) || isinf(v)) tb = true;
+      tm = fmax(tm, v);
+    }
+    const bool valid = __ldg(P.bad + t) == 0;
+    if (P.resid != nullptr) P.resid[t] = (tb || !valid) ? __longlong_as_double(0x7ff8000000000000LL) : tm;
+    if (valid) {
+      bad = bad || tb;
+      mx = fmax(mx, tm);
+    }
+  }
+  bad = __syncthreads_or(bad) != 0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(FULL, mx, o));
+  if (lane == 0) red[warp] = mx;
+  __syncthreads();
+  if (tid == 0) {
+    for (int w = 1; w < LR_THREADS / 32; ++w) mx = fmax(mx, red[w]);
+    const bool more = bad || !(mx <= P.tol);
+    *P.scale = more ? 1.0 : 0.0;
+    if (more) P.info[GLL_INFO_LAPLACE_ROUNDS] = P.round + 1;
+    if (bad) atomicOr(P.info + GLL_INFO_STATUS, GLL_STATUS_NONFINITE);
+    const float fr = bad ? __int_as_float(0x7fc00000) : (float)mx;
+    P.info[GLL_INFO_LAPLACE_RESID] = __float_as_int(fr);
+    if (P.round == 0) P.info[GLL_INFO_LAPLACE_RESID0] = __float_as_int(fr);
+    *P.ticket = 0u;  // rewound for the next round
+  }
+}
+
+// Thread per (row i, trial t = blockIdx.y): pred[t, i] = x + e, or the label row where i is clamped in t, or NaN for an invalid
+// trial; labels = first maximal column (-1 for an invalid trial); hits of the unclamped rows counted with one integer atomic per
+// CTA into correct[t] (-1 for an invalid trial).  CTA (0, 0) also writes the correction-CG iteration counts and the status.
+__global__ void __launch_bounds__(LR_THREADS)
+laplace_finish_trials_kernel(const double* __restrict__ x, const float* __restrict__ e, const float* __restrict__ Y,
+                             const int* __restrict__ slot, const int* __restrict__ badv, int n, int T, int k_lab, int l, int lpad,
+                             double* __restrict__ pred, long long* __restrict__ labels, const long long* __restrict__ targets,
+                             unsigned long long* __restrict__ correct, const double* __restrict__ scale,
+                             const int* __restrict__ round_iters, int rounds, int* __restrict__ info) {
+  __shared__ int part[LR_THREADS / 32];
+  const int t = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool valid = __ldg(badv + t) == 0;
+  int hit = 0;
+  if (i < n) {
+    double* p = pred + ((size_t)t * n + i) * l;
+    long long arg = -1;
+    if (!valid) {
+      for (int c = 0; c < l; ++c) p[c] = __longlong_as_double(0x7ff8000000000000LL);
+    } else {
+      const int si = __ldg(slot + (size_t)i * T + t);
+      const size_t o = (size_t)i * T * lpad + (size_t)t * lpad;
+      const float* y = Y + ((size_t)t * k_lab + (si >= 0 ? si : 0)) * l;
+      double best = 0.0;
+      for (int c = 0; c < l; ++c) {
+        const double v = (si >= 0) ? (double)__ldg(y + c) : x[o + c] + (double)__ldg(e + o + c);
+        p[c] = v;
+        if (c == 0 || v > best) {
+          best = v;
+          arg = c;
+        }
+      }
+      if (si < 0 && targets != nullptr) {
+        const long long tg = __ldg(targets + i);
+        hit = (tg >= 0 && tg == arg) ? 1 : 0;
+      }
+    }
+    labels[(size_t)t * n + i] = arg;
+  }
+  if (correct != nullptr) {
+    hit = warp_sum(hit);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = hit;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      int s = 0;
+      for (int w = 0; w < LR_THREADS / 32; ++w) s += part[w];
+      if (!valid) {
+        if (blockIdx.x == 0) correct[t] = ~0ull;  // -1; no other CTA of an invalid trial adds anything
+      } else if (s) {
+        atomicAdd(correct + t, (unsigned long long)s);
+      }
+    }
+  }
+  if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
+    int tot = 0;
+    unsigned packed[2] = {0u, 0u};
+    for (int r = 0; r < rounds; ++r) {
+      const int it = round_iters[r];
+      tot += it;
+      if (r < 4) packed[r >> 1] |= (unsigned)min(it, 65535) << (16 * (r & 1));
+    }
+    info[GLL_INFO_LAPLACE_CG_ITERS] = tot;
+    info[GLL_INFO_LAPLACE_ROUND_ITERS] = (int)packed[0];
+    info[GLL_INFO_LAPLACE_ROUND_ITERS + 1] = (int)packed[1];
+    if (*scale != 0.0) atomicOr(info + GLL_INFO_STATUS, GLL_STATUS_CG_NOT_CONVERGED);  // tol unmet after the last round
+  }
+}
+
+// launch shape of laplace_refine_trials_kernel: CW columns per CTA, column chunks, and row CTAs (about 4 CTAs per SM in all, so
+// the last CTA adds few partials per column)
+struct TrialsGrid {
+  int cw, gy, gx;
+};
+TrialsGrid trials_grid(int n, int T, int l) {
+  const int tl = T * l, cw = min(tl, 32), gy = ceil_div(tl, cw);
+  return {cw, gy, max(1, min(ceil_div(n, LR_THREADS / cw), ceil_div(4 * device_info().sms, gy)))};
+}
+
+// the trials' own buffers, behind the graph state and in front of the stage workspace
+struct TrialsBufs {
+  int* slot;        // [n][T]
+  int* bad;         // [T]
+  float* rhs;       // [n][C]: the solves' fp32 right-hand side
+  float* x0;        // [n][C]: the initial solve
+  float* corr;      // [n][C]: the correction solves
+  double* xa;       // [n][C]: the fp64 iterate, ping-pong with xb
+  double* xb;
+  double* r;        // [n][C]
+  double* partial;  // [refine grid x][T l]
+  double* colnorm;  // [T l]
+  double* scale;
+  unsigned* ticket;
+  int* round_iters;  // [GLL_LAPLACE_ROUNDS]
+};
+
+// base == NULL: size query only
+size_t trials_bufs(char* base, int n, int T, int l, TrialsBufs* E) {
+  Carver cv(base, ~(size_t)0);
+  const size_t nc = (size_t)n * T * padded_classes(l), tl = (size_t)T * l;
+  TrialsBufs b;
+  b.slot = cv.take<int>((size_t)n * T);
+  b.bad = cv.take<int>(T);
+  b.rhs = cv.take<float>(nc);
+  b.x0 = cv.take<float>(nc);
+  b.corr = cv.take<float>(nc);
+  b.xa = cv.take<double>(nc);
+  b.xb = cv.take<double>(nc);
+  b.r = cv.take<double>(nc);
+  b.partial = cv.take<double>((size_t)trials_grid(n, T, l).gx * tl);
+  b.colnorm = cv.take<double>(tl);
+  b.scale = cv.take<double>(1);
+  b.ticket = cv.take<unsigned>(1);
+  b.round_iters = cv.take<int>(GLL_LAPLACE_ROUNDS);
+  if (E) *E = b;
+  return align_up(cv.off, 256);
+}
+
+// the sizes gll_laplace_eval_trials accepts
+bool trials_sizes_ok(int n, int d, int k, int l, int T, int k_lab) {
+  if (n < 2 || T < 1 || l < 1 || d < 1 || k_lab < 1 || k_lab >= n) return false;
+  if ((long long)n * T * padded_classes(l) > 0x7fffffffLL) return false;
+  return k >= 2 && k <= 64 && k <= n && (k <= 33 || n >= 256);
+}
+
+// the graph state of the k_lab = 0 stages (a one-column dummy label block, as knn_sym_dist)
+int trials_layout(int n, int k, gll_layout* L) { return gll_state_layout(n, k, 1, 0, L); }
+
+// workspace: [graph state | the trials' buffers | stage workspace (kNN, graph stages, CG over C columns)]
+size_t trials_ws_bytes(int n, int d, int k, int l, int T) {
+  gll_layout L;
+  if (trials_layout(n, k, &L)) return 0;
+  const size_t stage = std::max(gll_workspace_bytes(n, d, k, 1, 0), cg_ws_bytes(n, T * padded_classes(l)));
+  return L.total + trials_bufs(nullptr, n, T, l, nullptr) + stage;
+}
+
+int trials_run(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T, int k_lab, int l,
+               int eps_auto, float eps_fixed, float tau, double tol, int cg_max_iter, double* pred, long long* labels,
+               const long long* targets, long long* correct_out, double* resid_out, int* info, void* workspace, size_t workspace_bytes,
+               cudaStream_t st) {
+  const size_t need = trials_ws_bytes(n, d, k, l, T);
+  if (workspace_bytes < need) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, need);
+    return GLL_ERR_WORKSPACE;
+  }
+  const int lpad = padded_classes(l), C = T * lpad;
+  gll_layout L;
+  if (trials_layout(n, k, &L)) return GLL_ERR_ARG;
+  char* S = (char*)workspace;
+  GraphBufs G = graph_bufs(L, S);
+  G.info = info;
+  TrialsBufs E;
+  const size_t eb = trials_bufs(S + L.total, n, T, l, &E);
+  void* ws = S + L.total + eb;
+  const size_t ws_bytes = workspace_bytes - L.total - eb;
+
+  GLL_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int) * GLL_INFO_WORDS, st));
+  GLL_CUDA_CHECK(cudaMemsetAsync(E.ticket, 0, sizeof(unsigned), st));
+  GLL_CUDA_CHECK(cudaMemsetAsync(E.slot, 0xff, sizeof(int) * (size_t)n * T, st));  // -1: not labeled
+  GLL_CUDA_CHECK(cudaMemsetAsync(E.bad, 0, sizeof(int) * (size_t)T, st));
+  GLL_CUDA_CHECK(cudaMemsetAsync(E.r, 0, sizeof(double) * (size_t)n * C, st));  // padding columns of the right-hand side
+  if (correct_out) GLL_CUDA_CHECK(cudaMemsetAsync(correct_out, 0, sizeof(long long) * (size_t)T, st));
+  {
+    GLL_PROF(KID_LAPLACE_TRIALS_SETUP, st);
+    laplace_trials_setup_kernel<<<ceil_div((long long)T * k_lab, 256), 256, 0, st>>>(train_idx, idx_is_i64, n, T, k_lab, E.slot, E.bad,
+                                                                                    info);
+    GLL_LAUNCH_CHECK();
+  }
+  int rc = knn_run(X, n, d, k, 0, n, G.knn_idx, G.knn_dist, info, ws, ws_bytes, st);
+  if (rc) return rc;
+  rc = graph_stages_run(G, nullptr, n, k, 1, 0, eps_auto, eps_fixed, tau, 0, 6, ws, ws_bytes, st);
+  if (rc) return rc;
+
+  const TrialsGrid tg = trials_grid(n, T, l);
+  TrialsRefineParams P;
+  P.row_ptr = G.row_ptr;
+  P.col = G.col;
+  P.w = G.w;
+  P.Y = Y;
+  P.slot = E.slot;
+  P.bad = E.bad;
+  P.r_out = E.r;
+  P.partial = E.partial;
+  P.colnorm = E.colnorm;
+  P.resid = resid_out;
+  P.scale = E.scale;
+  P.ticket = E.ticket;
+  P.info = info;
+  P.n = n;
+  P.T = T;
+  P.k_lab = k_lab;
+  P.l = l;
+  P.lpad = lpad;
+  P.gx = tg.gx;
+  P.cw = tg.cw;
+  P.tau = (double)tau;
+  P.tol = tol;
+  const dim3 grid(tg.gx, tg.gy);
+  // r = b at x = 0, exactly in fp64: the first solve's right-hand side
+  P.x_prev = nullptr;
+  P.e = nullptr;
+  P.x_out = nullptr;
+  P.round = -1;
+  {
+    GLL_PROF(KID_LAPLACE_REFINE, st);
+    laplace_refine_trials_kernel<<<grid, LR_THREADS, 0, st>>>(P);
+    GLL_LAUNCH_CHECK();
+  }
+  unsigned* barrier = (unsigned*)(info + GLL_INFO_CG_BARRIER);
+  CgIo io = {E.r, 2, nullptr, 0, nullptr, 0, 0.f, E.slot, T, lpad, 0};
+  rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, E.rhs, n, C, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, E.x0,
+              info + GLL_INFO_CG_ITERS_FWD, (float*)(info + GLL_INFO_CG_RESID_FWD), nullptr, ws, ws_bytes, st, barrier, &io);
+  if (rc) return rc;
+  io.rhs_scale = E.scale;
+  io.rhs_scale_f64 = 1;
+  for (int r = 0; r < GLL_LAPLACE_ROUNDS; ++r) {
+    P.x_out = (r % 2 == 0) ? E.xa : E.xb;
+    P.x_prev = (r == 0) ? nullptr : (r % 2 == 0 ? E.xb : E.xa);
+    P.e = (r == 0) ? E.x0 : E.corr;
+    P.round = r;
+    {
+      GLL_PROF(KID_LAPLACE_REFINE, st);
+      laplace_refine_trials_kernel<<<grid, LR_THREADS, 0, st>>>(P);
+      GLL_LAUNCH_CHECK();
+    }
+    rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, E.rhs, n, C, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, E.corr, E.round_iters + r,
+                nullptr, nullptr, ws, ws_bytes, st, barrier, &io);
+    if (rc) return rc;
+  }
+  {
+    GLL_PROF(KID_LAPLACE_FINISH, st);
+    laplace_finish_trials_kernel<<<dim3(ceil_div(n, LR_THREADS), T), LR_THREADS, 0, st>>>(
+        P.x_out, E.corr, Y, E.slot, E.bad, n, T, k_lab, l, lpad, pred, labels, targets, (unsigned long long*)correct_out, E.scale,
+        E.round_iters, GLL_LAPLACE_ROUNDS, info);
+    GLL_LAUNCH_CHECK();
+  }
+  return GLL_OK;
+}
+
 }  // namespace
 }  // namespace gll
 
@@ -387,6 +771,24 @@ int gll_laplace_eval_batched(const float* X, const float* Y, int B, int n, int d
   GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
   return eval_run(X, Y, B, n, d, k, l, k_lab, eps_auto, eps_fixed, tau, tol, cg_max_iter, pred, labels, targets, correct_out, resid_out,
                   info, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+size_t gll_laplace_eval_trials_workspace_bytes(int n, int d, int k, int l, int T, int k_lab) {
+  if (!trials_sizes_ok(n, d, k, l, T, k_lab)) return 0;
+  return trials_ws_bytes(n, d, k, l, T);
+}
+
+int gll_laplace_eval_trials(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T, int k_lab,
+                            int l, int eps_auto, float eps_fixed, float tau, double tol, int cg_max_iter, double* pred,
+                            long long* labels, const long long* targets, long long* correct_out, double* resid_out, int* info,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  GLL_REQUIRE(X && train_idx && Y && pred && labels && info && workspace, "null pointer");
+  GLL_REQUIRE(n >= 2 && T >= 1 && (long long)n * T * padded_classes(l) <= 0x7fffffffLL, "need n >= 2, T >= 1 and n T lpad < 2^31");
+  GLL_REQUIRE(k >= 2 && k <= 64 && k <= n && (k <= 33 || n >= 256), "k must be in [2, 64] (n >= 256 when k > 33) and <= n");
+  GLL_REQUIRE(d >= 1 && l >= 1 && k_lab >= 1 && k_lab < n, "bad sizes");
+  GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
+  return trials_run(X, n, d, k, train_idx, idx_is_i64, Y, T, k_lab, l, eps_auto, eps_fixed, tau, tol, cg_max_iter, pred, labels, targets,
+                    correct_out, resid_out, info, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -18,6 +18,15 @@ B independent graphs of the same shape in one call (features (B, n, d), label_ma
 (B, m, l), labels (B, m), correct (B,).  Every graph meets the stop rule on its own; the solver's step lengths are shared by
 the graphs, so pred matches per-graph laplace_learning calls to solver accuracy (bit for bit at B = 1).  See
 gll_laplace_eval_batched in include/gll_b200.h.
+
+    res = laplace_learning_trials(features, train_idx, label_matrix, k=50, epsilon='auto', tau=0.0, tol=1e-10, targets=None)
+
+T labeled sets on ONE set of features (n, d) in any row order: train_idx (T, k_lab) lists the labeled rows of each trial,
+label_matrix (T, k_lab, l) their labels, targets (n,); pred (T, n, l), labels (T, n), correct (T,) over the rows not labeled in
+that trial.  The graph is built once; all T l class columns are solved against it with each trial's labeled rows masked out of
+its own columns, every column with its own step lengths.  A trial with an index outside [0, n) or a repeated index is invalid:
+pred NaN, labels -1, correct -1 and a warning; the other trials are unaffected.  See gll_laplace_eval_trials in
+include/gll_b200.h.
 """
 from __future__ import annotations
 
@@ -30,7 +39,7 @@ from . import _lib
 from .GLL import _bytes, _cg_maxit, _check_status, _require_cuda, _stream_ptr, as_features, decode_info, parse_epsilon
 from ._lib import lib
 
-__all__ = ["laplace_learning", "laplace_learning_batched", "LaplaceResult", "last_eval_info"]
+__all__ = ["laplace_learning", "laplace_learning_batched", "laplace_learning_trials", "LaplaceResult", "last_eval_info"]
 
 
 class LaplaceResult(NamedTuple):
@@ -41,10 +50,11 @@ class LaplaceResult(NamedTuple):
 
 _last_info: Optional[torch.Tensor] = None
 _last_resid: Optional[torch.Tensor] = None  # per-graph residuals of the last call when it was batched
+_last_resid_trials: Optional[torch.Tensor] = None  # per-trial residuals of the last call when it was a trials call
 
 
 def _check_args(n, d, k_lab, l, k, epsilon, tol, total_rows, rows_name):
-    """The size, epsilon and tol checks both entry points share; returns (eps_auto, eps_fixed)."""
+    """The size, epsilon and tol checks the entry points share; returns (eps_auto, eps_fixed)."""
     if not (0 < k_lab < n):
         raise ValueError(f"need 0 < k_lab < n (k_lab={k_lab}, n={n}); labeled rows come first (GLL.py:11)")
     if l < 1 or d < 1:
@@ -91,8 +101,8 @@ def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int 
                                   correct.data_ptr() if correct is not None else None, info.data_ptr(), ws.data_ptr(), ws_bytes,
                                   _stream_ptr(dev))
     _lib.check(rc, "gll_laplace_eval")
-    global _last_info, _last_resid
-    _last_info, _last_resid = info, None
+    global _last_info, _last_resid, _last_resid_trials
+    _last_info, _last_resid, _last_resid_trials = info, None, None
     _check_status(info, "Laplace-learning")
     return LaplaceResult(pred, labels, correct)
 
@@ -138,16 +148,74 @@ def laplace_learning_batched(features: torch.Tensor, label_matrix: torch.Tensor,
                                           correct.data_ptr() if correct is not None else None, resid.data_ptr(), info.data_ptr(),
                                           ws.data_ptr(), ws_bytes, _stream_ptr(dev))
     _lib.check(rc, "gll_laplace_eval_batched")
-    global _last_info, _last_resid
-    _last_info, _last_resid = info, resid
+    global _last_info, _last_resid, _last_resid_trials
+    _last_info, _last_resid, _last_resid_trials = info, resid, None
+    _check_status(info, "Laplace-learning")
+    return LaplaceResult(pred, labels, correct)
+
+
+def laplace_learning_trials(features: torch.Tensor, train_idx: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto",
+                            tau: float = 0.0, tol: float = 1e-10, targets: Optional[torch.Tensor] = None) -> LaplaceResult:
+    """T labeled sets on one graph.  features (n, d) CUDA tensor in any row order; train_idx (T, k_lab) int64 or int32, the labeled
+    rows of trial t (read on the device: no host copy); label_matrix (T, k_lab, l) one-hot float32 or int64, row s of trial t
+    labels row train_idx[t, s]; targets (n,) int64 or None, a negative target is not counted.  Returns pred (T, n, l) float64,
+    labels (T, n) int64 and correct (T,) int64 (None without targets), counting the rows not labeled in that trial.  A labeled
+    row gets its label row and that row's argmax.  Trial t equals laplace_learning on features[perm_t], perm_t = [train_idx[t],
+    the other rows in natural order], on its unlabeled rows; the graph is built once in natural order, so on exact distance ties
+    the kNN tie-break follows natural order rather than perm_t."""
+    if features.dim() != 2:
+        raise ValueError("features must be (n, d)")
+    if train_idx.dim() != 2:
+        raise ValueError("train_idx must be (T, k_lab)")
+    if train_idx.dtype not in (torch.int64, torch.int32):
+        raise ValueError(f"train_idx must be int64 or int32, got {train_idx.dtype}")
+    if label_matrix.dim() != 3:
+        raise ValueError("label_matrix must be (T, k_lab, l)")
+    n, d = features.shape
+    T, k_lab = train_idx.shape
+    if T < 1 or tuple(label_matrix.shape[:2]) != (T, k_lab):
+        raise ValueError(f"label_matrix must be (T, k_lab, l) = ({T}, {k_lab}, l) with T >= 1, got {tuple(label_matrix.shape)}")
+    l = label_matrix.shape[2]
+    k = int(k)
+    eps_auto, eps_fixed = _check_args(n, d, k_lab, l, k, epsilon, tol, n, "n")
+    lpad = (l + 3) // 4 * 4
+    if n * T * lpad >= 2 ** 31:
+        raise ValueError(f"n T lpad must be < 2^31 (n={n}, T={T}, lpad={lpad})")
+    if targets is not None and tuple(targets.shape) != (n,):
+        raise ValueError(f"targets must be ({n},), got {tuple(targets.shape)}")
+    _require_cuda(features, "features")
+    dev = features.device
+    Xc = as_features(features)
+    idx = train_idx.detach().to(device=dev).contiguous()
+    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
+    tg = None
+    if targets is not None:
+        tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
+    with torch.cuda.device(dev):
+        ws_bytes = lib.gll_laplace_eval_trials_workspace_bytes(n, d, k, l, T, k_lab)
+        ws = _bytes(ws_bytes, dev)
+        pred = torch.empty((T, n, l), dtype=torch.float64, device=dev)
+        labels = torch.empty((T, n), dtype=torch.int64, device=dev)
+        correct = torch.empty(T, dtype=torch.int64, device=dev) if tg is not None else None
+        resid = torch.empty(T, dtype=torch.float64, device=dev)
+        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
+        rc = lib.gll_laplace_eval_trials(Xc.data_ptr(), n, d, k, idx.data_ptr(), int(idx.dtype == torch.int64), Y.data_ptr(), T, k_lab,
+                                         l, eps_auto, eps_fixed, float(tau), float(tol), _cg_maxit(), pred.data_ptr(),
+                                         labels.data_ptr(), tg.data_ptr() if tg is not None else None,
+                                         correct.data_ptr() if correct is not None else None, resid.data_ptr(), info.data_ptr(),
+                                         ws.data_ptr(), ws_bytes, _stream_ptr(dev))
+    _lib.check(rc, "gll_laplace_eval_trials")
+    global _last_info, _last_resid, _last_resid_trials
+    _last_info, _last_resid, _last_resid_trials = info, None, resid
     _check_status(info, "Laplace-learning")
     return LaplaceResult(pred, labels, correct)
 
 
 def last_eval_info() -> dict:
-    """Device status block of the most recent laplace_learning or laplace_learning_batched call (synchronises).  Keys follow
-    GLL_INFO_* in include/gll_b200.h; after a batched call the residuals are the maximum over graphs, the iteration counts those
-    of the whole batch, and resid_per_graph lists each graph's largest column norm of the last round."""
+    """Device status block of the most recent laplace_learning, laplace_learning_batched or laplace_learning_trials call
+    (synchronises).  Keys follow GLL_INFO_* in include/gll_b200.h; after a batched call the residuals are the maximum over graphs,
+    the iteration counts those of the whole batch, and resid_per_graph lists each graph's largest column norm of the last round.
+    After a trials call the same holds over the valid trials, and resid_per_trial lists each trial's (NaN for an invalid one)."""
     if _last_info is None:
         return {}
     v = _last_info.cpu().numpy()
@@ -157,4 +225,5 @@ def last_eval_info() -> dict:
     return dict(decode_info(v), cg_iters_first=int(v[_lib.INFO_CG_ITERS_FWD]), rounds=int(v[_lib.INFO_LAPLACE_ROUNDS]),
                 cg_iters_correction=int(v[_lib.INFO_LAPLACE_CG_ITERS]), round_iters=round_iters, resid_first=float(f[_lib.INFO_LAPLACE_RESID0]),
                 resid=float(f[_lib.INFO_LAPLACE_RESID]),
-                **({} if _last_resid is None else dict(resid_per_graph=[float(x) for x in _last_resid.cpu().numpy()])))
+                **({} if _last_resid is None else dict(resid_per_graph=[float(x) for x in _last_resid.cpu().numpy()])),
+                **({} if _last_resid_trials is None else dict(resid_per_trial=[float(x) for x in _last_resid_trials.cpu().numpy()])))

@@ -32,6 +32,7 @@ extern "C" {
 #define GLL_STATUS_EPS_TINY 2         /* GLL.py:240-241 warns "Epsilon in KNN is very close to zero." */
 #define GLL_STATUS_NONFINITE 4
 #define GLL_STATUS_KNN_FALLBACK 8     /* some rows needed the exact brute-force kNN fallback (informational) */
+#define GLL_STATUS_BAD_INDEX 16       /* gll_laplace_eval_trials: a trial's labeled-row index is outside [0, n) or repeated */
 
 /* slots of the int32 info[16] block that lives in the state buffer */
 #define GLL_INFO_STATUS 0
@@ -366,6 +367,32 @@ int gll_laplace_eval_batched(const float* X, const float* Y, int B, int n, int d
                              float eps_fixed, float tau, double tol, int cg_max_iter, double* pred, long long* labels,
                              const long long* targets, long long* correct_out, double* resid_out, int* info,
                              void* workspace, size_t workspace_bytes, void* stream);
+
+/* T trials of gll_laplace_eval on ONE set of features: trial t labels the k_lab rows train_idx[t] (T x k_lab, int64 when
+ * idx_is_i64, else int32; device) with Y[t] (T x k_lab x l fp32) and solves the other n - k_lab rows.  X (n x d) is in any row
+ * order.  The graph (kNN, CSR, eps, W, degrees) is built once on X in natural order, as gll_laplace_eval's stages with no labeled
+ * rows; trial t's result is gll_laplace_eval on X[perm_t], perm_t = [train_idx[t], the other rows in natural order], mapped back
+ * to natural order.  Without exact distance ties the graph is the permuted graph of every trial; on exact ties the index
+ * tie-break of the kNN search follows natural order, not perm_t.
+ *   Solve: all T l class columns against one full-graph system A = D + tau I - W; trial t's labeled rows are masked out of its
+ *   columns (A p is zeroed there), each column keeps its own CG step lengths, and the fp64 refinement stops when every class column
+ *   of every valid trial has ||M (b - A x)||_2 <= tol over that trial's unlabeled rows (M, D as gll_laplace_eval).
+ *   Invalid trials: a train_idx row with an index outside [0, n) or a repeated index never causes an out-of-bounds access; the
+ *   trial gets a zero right-hand side (it neither stops nor slows the others), pred NaN, labels -1, correct -1, resid NaN, and
+ *   GLL_STATUS_BAD_INDEX is set.  The other trials are unaffected.
+ *   Sizes: n >= 2, T >= 1, n T lpad < 2^31 (lpad = gll_padded_classes(l)), 2 <= k <= 64, k <= n, n >= 256 when k > 33,
+ *   1 <= k_lab < n, l >= 1, d >= 1, tol > 0, cg_max_iter >= 1.
+ *   Outputs: pred T x n x l fp64 and labels T x n int64 (a row labeled in trial t gets its label row and that row's argmax);
+ *   targets (n int64, may be NULL; negative = not scored); correct_out (T int64, may be NULL) counts per trial the rows that are
+ *   not labeled in it and whose label equals their target; resid_out (T fp64, may be NULL) = per trial the largest column norm of
+ *   the last round.  info: as gll_laplace_eval, residual slots holding the maximum over valid trials.  Bad arguments return
+ *   GLL_ERR_ARG before any CUDA call; the workspace query returns 0 for them.  Nothing syncs with the host and nothing is copied,
+ *   so the call can be captured in a CUDA graph. */
+size_t gll_laplace_eval_trials_workspace_bytes(int n, int d, int k, int l, int T, int k_lab);
+int gll_laplace_eval_trials(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T,
+                            int k_lab, int l, int eps_auto, float eps_fixed, float tau, double tol, int cg_max_iter, double* pred,
+                            long long* labels, const long long* targets, long long* correct_out, double* resid_out, int* info,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
