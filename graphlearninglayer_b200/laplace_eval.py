@@ -49,8 +49,7 @@ class LaplaceResult(NamedTuple):
 
 
 _last_info: Optional[torch.Tensor] = None
-_last_resid: Optional[torch.Tensor] = None  # per-graph residuals of the last call when it was batched
-_last_resid_trials: Optional[torch.Tensor] = None  # per-trial residuals of the last call when it was a trials call
+_last_resid: Optional[tuple] = None  # (key, per-group residuals) of the last call when it was batched or a trials call
 
 
 def _check_args(n, d, k_lab, l, k, epsilon, tol, total_rows, rows_name):
@@ -67,6 +66,33 @@ def _check_args(n, d, k_lab, l, k, epsilon, tol, total_rows, rows_name):
     return eps
 
 
+def _run(name, features, label_matrix, targets, lead, ws_sizes, pred_shape, groups, eps, tau, tol, resid_key=None):
+    """Converts the inputs, allocates the outputs and the workspace, runs gll_<name> on the current stream and records its info
+    for last_eval_info().  lead(X, Y) gives the arguments in front of eps_auto, with X and Y the converted features and labels;
+    groups is the shape of correct and of the residuals reported under resid_key."""
+    _require_cuda(features, "features")
+    dev = features.device
+    Xc = as_features(features)
+    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
+    tg = None if targets is None else targets.detach().to(device=dev, dtype=torch.int64).contiguous()
+    with torch.cuda.device(dev):
+        ws_bytes = getattr(lib, f"gll_{name}_workspace_bytes")(*ws_sizes)
+        ws = _bytes(ws_bytes, dev)
+        pred = torch.empty(pred_shape, dtype=torch.float64, device=dev)
+        labels = torch.empty(pred_shape[:-1], dtype=torch.int64, device=dev)
+        correct = None if tg is None else torch.empty(groups, dtype=torch.int64, device=dev)
+        resid = None if resid_key is None else torch.empty(groups, dtype=torch.float64, device=dev)
+        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
+        outs = [None if t is None else t.data_ptr() for t in (pred, labels, tg, correct)] + ([] if resid is None else [resid.data_ptr()])
+        rc = getattr(lib, f"gll_{name}")(*lead(Xc.data_ptr(), Y.data_ptr()), *eps, float(tau), float(tol), _cg_maxit(), *outs,
+                                         info.data_ptr(), ws.data_ptr(), ws_bytes, _stream_ptr(dev))
+    _lib.check(rc, f"gll_{name}")
+    global _last_info, _last_resid
+    _last_info, _last_resid = info, None if resid is None else (resid_key, resid)
+    _check_status(info, "Laplace-learning")
+    return LaplaceResult(pred, labels, correct)
+
+
 def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto", tau: float = 0.0,
                      tol: float = 1e-10, targets: Optional[torch.Tensor] = None) -> LaplaceResult:
     """features (n, d) CUDA tensor with the k_lab labeled rows FIRST (GLL.py:11); label_matrix (k_lab, l) one-hot float32 or
@@ -78,33 +104,12 @@ def laplace_learning(features: torch.Tensor, label_matrix: torch.Tensor, k: int 
     n, d = features.shape
     k_lab, l = label_matrix.shape
     k = int(k)
-    eps_auto, eps_fixed = _check_args(n, d, k_lab, l, k, epsilon, tol, n, "n")
+    eps = _check_args(n, d, k_lab, l, k, epsilon, tol, n, "n")
     m = n - k_lab
     if targets is not None and tuple(targets.shape) != (m,):
         raise ValueError(f"targets must be ({m},), got {tuple(targets.shape)}")
-    _require_cuda(features, "features")
-    dev = features.device
-    Xc = as_features(features)
-    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
-    tg = None
-    if targets is not None:
-        tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
-    with torch.cuda.device(dev):
-        ws_bytes = lib.gll_laplace_eval_workspace_bytes(n, d, k, l, k_lab)
-        ws = _bytes(ws_bytes, dev)
-        pred = torch.empty((m, l), dtype=torch.float64, device=dev)
-        labels = torch.empty(m, dtype=torch.int64, device=dev)
-        correct = torch.empty((), dtype=torch.int64, device=dev) if tg is not None else None
-        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
-        rc = lib.gll_laplace_eval(Xc.data_ptr(), Y.data_ptr(), n, d, k, l, k_lab, eps_auto, eps_fixed, float(tau), float(tol),
-                                  _cg_maxit(), pred.data_ptr(), labels.data_ptr(), tg.data_ptr() if tg is not None else None,
-                                  correct.data_ptr() if correct is not None else None, info.data_ptr(), ws.data_ptr(), ws_bytes,
-                                  _stream_ptr(dev))
-    _lib.check(rc, "gll_laplace_eval")
-    global _last_info, _last_resid, _last_resid_trials
-    _last_info, _last_resid, _last_resid_trials = info, None, None
-    _check_status(info, "Laplace-learning")
-    return LaplaceResult(pred, labels, correct)
+    return _run("laplace_eval", features, label_matrix, targets, lambda X, Y: (X, Y, n, d, k, l, k_lab), (n, d, k, l, k_lab), (m, l),
+                (), eps, tau, tol)
 
 
 def laplace_learning_batched(features: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto", tau: float = 0.0,
@@ -123,35 +128,12 @@ def laplace_learning_batched(features: torch.Tensor, label_matrix: torch.Tensor,
         raise ValueError(f"B n must be < 2^31 (B={B}, n={n})")
     _, k_lab, l = label_matrix.shape
     k = int(k)
-    eps_auto, eps_fixed = _check_args(n, d, k_lab, l, k, epsilon, tol, B * n, "B n")
+    eps = _check_args(n, d, k_lab, l, k, epsilon, tol, B * n, "B n")
     m = n - k_lab
     if targets is not None and tuple(targets.shape) != (B, m):
         raise ValueError(f"targets must be ({B}, {m}), got {tuple(targets.shape)}")
-    _require_cuda(features, "features")
-    dev = features.device
-    Xc = as_features(features)
-    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
-    tg = None
-    if targets is not None:
-        tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
-    with torch.cuda.device(dev):
-        ws_bytes = lib.gll_laplace_eval_batched_workspace_bytes(B, n, d, k, l, k_lab)
-        ws = _bytes(ws_bytes, dev)
-        pred = torch.empty((B, m, l), dtype=torch.float64, device=dev)
-        labels = torch.empty((B, m), dtype=torch.int64, device=dev)
-        correct = torch.empty(B, dtype=torch.int64, device=dev) if tg is not None else None
-        resid = torch.empty(B, dtype=torch.float64, device=dev)
-        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
-        rc = lib.gll_laplace_eval_batched(Xc.data_ptr(), Y.data_ptr(), B, n, d, k, l, k_lab, eps_auto, eps_fixed, float(tau),
-                                          float(tol), _cg_maxit(), pred.data_ptr(), labels.data_ptr(),
-                                          tg.data_ptr() if tg is not None else None,
-                                          correct.data_ptr() if correct is not None else None, resid.data_ptr(), info.data_ptr(),
-                                          ws.data_ptr(), ws_bytes, _stream_ptr(dev))
-    _lib.check(rc, "gll_laplace_eval_batched")
-    global _last_info, _last_resid, _last_resid_trials
-    _last_info, _last_resid, _last_resid_trials = info, resid, None
-    _check_status(info, "Laplace-learning")
-    return LaplaceResult(pred, labels, correct)
+    return _run("laplace_eval_batched", features, label_matrix, targets, lambda X, Y: (X, Y, B, n, d, k, l, k_lab),
+                (B, n, d, k, l, k_lab), (B, m, l), (B,), eps, tau, tol, "resid_per_graph")
 
 
 def laplace_learning_trials(features: torch.Tensor, train_idx: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto",
@@ -177,38 +159,19 @@ def laplace_learning_trials(features: torch.Tensor, train_idx: torch.Tensor, lab
         raise ValueError(f"label_matrix must be (T, k_lab, l) = ({T}, {k_lab}, l) with T >= 1, got {tuple(label_matrix.shape)}")
     l = label_matrix.shape[2]
     k = int(k)
-    eps_auto, eps_fixed = _check_args(n, d, k_lab, l, k, epsilon, tol, n, "n")
-    lpad = (l + 3) // 4 * 4
+    eps = _check_args(n, d, k_lab, l, k, epsilon, tol, n, "n")
+    lpad = lib.gll_padded_classes(l)
     if n * T * lpad >= 2 ** 31:
         raise ValueError(f"n T lpad must be < 2^31 (n={n}, T={T}, lpad={lpad})")
+    if T * l > 65535 * 32:  # the refinement grid's column chunks (gridDim.y)
+        raise ValueError(f"T l must be <= 2097120 (T={T}, l={l})")
     if targets is not None and tuple(targets.shape) != (n,):
         raise ValueError(f"targets must be ({n},), got {tuple(targets.shape)}")
-    _require_cuda(features, "features")
-    dev = features.device
-    Xc = as_features(features)
-    idx = train_idx.detach().to(device=dev).contiguous()
-    Y = label_matrix.detach().to(device=dev, dtype=torch.float32).contiguous()
-    tg = None
-    if targets is not None:
-        tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
-    with torch.cuda.device(dev):
-        ws_bytes = lib.gll_laplace_eval_trials_workspace_bytes(n, d, k, l, T, k_lab)
-        ws = _bytes(ws_bytes, dev)
-        pred = torch.empty((T, n, l), dtype=torch.float64, device=dev)
-        labels = torch.empty((T, n), dtype=torch.int64, device=dev)
-        correct = torch.empty(T, dtype=torch.int64, device=dev) if tg is not None else None
-        resid = torch.empty(T, dtype=torch.float64, device=dev)
-        info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
-        rc = lib.gll_laplace_eval_trials(Xc.data_ptr(), n, d, k, idx.data_ptr(), int(idx.dtype == torch.int64), Y.data_ptr(), T, k_lab,
-                                         l, eps_auto, eps_fixed, float(tau), float(tol), _cg_maxit(), pred.data_ptr(),
-                                         labels.data_ptr(), tg.data_ptr() if tg is not None else None,
-                                         correct.data_ptr() if correct is not None else None, resid.data_ptr(), info.data_ptr(),
-                                         ws.data_ptr(), ws_bytes, _stream_ptr(dev))
-    _lib.check(rc, "gll_laplace_eval_trials")
-    global _last_info, _last_resid, _last_resid_trials
-    _last_info, _last_resid, _last_resid_trials = info, None, resid
-    _check_status(info, "Laplace-learning")
-    return LaplaceResult(pred, labels, correct)
+    _require_cuda(features, "features")  # before train_idx is copied anywhere
+    idx = train_idx.detach().to(device=features.device).contiguous()
+    return _run("laplace_eval_trials", features, label_matrix, targets,
+                lambda X, Y: (X, n, d, k, idx.data_ptr(), int(idx.dtype == torch.int64), Y, T, k_lab, l), (n, d, k, l, T, k_lab),
+                (T, n, l), (T,), eps, tau, tol, "resid_per_trial")
 
 
 def last_eval_info() -> dict:
@@ -225,5 +188,4 @@ def last_eval_info() -> dict:
     return dict(decode_info(v), cg_iters_first=int(v[_lib.INFO_CG_ITERS_FWD]), rounds=int(v[_lib.INFO_LAPLACE_ROUNDS]),
                 cg_iters_correction=int(v[_lib.INFO_LAPLACE_CG_ITERS]), round_iters=round_iters, resid_first=float(f[_lib.INFO_LAPLACE_RESID0]),
                 resid=float(f[_lib.INFO_LAPLACE_RESID]),
-                **({} if _last_resid is None else dict(resid_per_graph=[float(x) for x in _last_resid.cpu().numpy()])),
-                **({} if _last_resid_trials is None else dict(resid_per_trial=[float(x) for x in _last_resid_trials.cpu().numpy()])))
+                **({} if _last_resid is None else {_last_resid[0]: [float(x) for x in _last_resid[1].cpu().numpy()]}))

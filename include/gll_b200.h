@@ -380,8 +380,8 @@ int gll_laplace_eval_batched(const float* X, const float* Y, int B, int n, int d
  *   Invalid trials: a train_idx row with an index outside [0, n) or a repeated index never causes an out-of-bounds access; the
  *   trial gets a zero right-hand side (it neither stops nor slows the others), pred NaN, labels -1, correct -1, resid NaN, and
  *   GLL_STATUS_BAD_INDEX is set.  The other trials are unaffected.
- *   Sizes: n >= 2, T >= 1, n T lpad < 2^31 (lpad = gll_padded_classes(l)), 2 <= k <= 64, k <= n, n >= 256 when k > 33,
- *   1 <= k_lab < n, l >= 1, d >= 1, tol > 0, cg_max_iter >= 1.
+ *   Sizes: n >= 2, T >= 1, n T lpad < 2^31 (lpad = gll_padded_classes(l)), T l <= 2097120, 2 <= k <= 64, k <= n, n >= 256
+ *   when k > 33, 1 <= k_lab < n, l >= 1, d >= 1, tol > 0, cg_max_iter >= 1.
  *   Outputs: pred T x n x l fp64 and labels T x n int64 (a row labeled in trial t gets its label row and that row's argmax);
  *   targets (n int64, may be NULL; negative = not scored); correct_out (T int64, may be NULL) counts per trial the rows that are
  *   not labeled in it and whose label equals their target; resid_out (T fp64, may be NULL) = per trial the largest column norm of

@@ -75,15 +75,17 @@ def test_c_argument_checks(libmod):
            dict(T=0), dict(n=1 << 20, T=1 << 10, l=3),                              # T >= 1, n T lpad < 2^31
            dict(k=1), dict(k=65), dict(n=40, k=41, k_lab=10), dict(n=255, k=34),   # 2 <= k <= 64, k <= n, n >= 256 when k > 33
            dict(k_lab=0), dict(k_lab=300), dict(l=0), dict(d=0),                    # 1 <= k_lab < n, l >= 1, d >= 1
-           dict(tol=0.0), dict(tol=-1.0), dict(maxit=0))                            # tol > 0, cg_max_iter >= 1
+           dict(tol=0.0), dict(tol=-1.0), dict(maxit=0),                            # tol > 0, cg_max_iter >= 1
+           dict(T=1 << 19, l=4), dict(n=40, k=20, k_lab=10, T=1 << 16, l=33))      # T l <= 65535 * 32 (refinement grid)
     for kw in bad:
         assert call(**kw) == ERR_ARG, kw
     wsb = lib.gll_laplace_eval_trials_workspace_bytes  # (n, d, k, l, T, k_lab)
     for args in ((300, 8, 50, 3, 0, 30), (1 << 20, 8, 25, 3, 1 << 10, 30), (300, 8, 1, 3, 4, 30), (300, 8, 65, 3, 4, 30),
                  (40, 8, 41, 3, 4, 10), (255, 8, 34, 3, 4, 10), (300, 8, 50, 3, 4, 0), (300, 8, 50, 3, 4, 300),
-                 (300, 8, 50, 0, 4, 30), (300, 0, 50, 3, 4, 30)):
+                 (300, 8, 50, 0, 4, 30), (300, 0, 50, 3, 4, 30), (300, 8, 50, 4, 1 << 19, 30), (40, 8, 20, 33, 1 << 16, 10)):
         assert wsb(*args) == 0, args
     assert wsb(300, 8, 50, 3, 4, 30) > 0 and wsb(2000, 64, 50, 37, 4, 74) > 0
+    assert wsb(40, 8, 20, 32, 65535, 10) > 0 and wsb(40, 8, 20, 1, 65535 * 32, 10) > 0  # T l = 65535 * 32 is accepted
 
 
 @pytest.mark.parametrize("kwargs, exc, match", [
@@ -98,7 +100,9 @@ def test_c_argument_checks(libmod):
     (dict(I=torch.zeros(2, 300, dtype=torch.long), Y=torch.zeros(2, 300, 3)), ValueError, "k_lab"),
     (dict(Y=torch.zeros(2, 30, 0)), ValueError, "class column"), (dict(epsilon="knn"), ValueError, "epsilon"),
     (dict(tol=0.0), ValueError, "tol"), (dict(targets=torch.zeros(270, dtype=torch.long)), ValueError, "targets"),
-    (dict(targets=torch.zeros(2, 300, dtype=torch.long)), ValueError, "targets")])
+    (dict(targets=torch.zeros(2, 300, dtype=torch.long)), ValueError, "targets"),
+    (dict(I=torch.zeros(1, 30, dtype=torch.long).expand(1 << 19, 30), Y=torch.zeros(1, 30, 4).expand(1 << 19, 30, 4)), ValueError,
+     "T l must be")])
 def test_python_validation_before_any_device_call(libmod, kwargs, exc, match):
     import graphlearninglayer_b200 as pkg
 
@@ -457,6 +461,29 @@ def test_deterministic_and_graph_capturable(gpu):
     g.replay()
     torch.cuda.synchronize()
     assert torch.equal(c.pred, ref.pred) and torch.equal(c.labels, ref.labels) and torch.equal(c.correct, ref.correct)
+
+
+@pytest.mark.gpu
+def test_more_trials_than_a_grid_dimension(gpu):
+    """T = 65 536 trials, one more than a grid's y extent: the last trial against a T = 1 call on its labeled set"""
+    n, l, k_lab, T = 200, 3, 12, 1 << 16
+    X, y = _data(16, n, 16, l)
+    rng = np.random.default_rng(17)
+    idx = np.argsort(rng.random((T, n)), axis=1)[:, :k_lab].astype(np.int64)
+    Ys = np.eye(l, dtype=np.float32)[y[idx]]
+    res = _run(gpu, X, idx, Ys, y, k=20)
+    torch.cuda.synchronize()
+    assert res.pred.shape == (T, n, l) and res.correct.shape == (T,)
+    info = _info()
+    assert info["status"] & ~8 == 0 and len(info["resid_per_trial"]) == T
+    assert np.all(np.asarray(info["resid_per_trial"]) <= 1e-10)  # NaN fails
+    one = _run(gpu, X, idx[-1:], Ys[-1:], y, k=20)
+    torch.cuda.synchronize()
+    a, b = res.pred[-1].cpu().numpy(), one.pred[0].cpu().numpy()
+    assert O.max_rel(a, b) < 1e-6
+    assert _labels_match(res.labels[-1].cpu().numpy(), b, one.labels[0].cpu().numpy())
+    flips = int((res.labels[-1] != one.labels[0]).sum())
+    assert abs(int(res.correct[-1]) - int(one.correct[0])) <= flips
 
 
 @pytest.mark.gpu
