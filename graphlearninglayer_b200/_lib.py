@@ -79,6 +79,7 @@ def _load():
                                   vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp])
     sig("gll_cg_solve", i32, [vp, vp, vp, vp, vp, i32, i32, f32, i32, vp, vp, vp, vp, vp, sz, vp])
     sig("gll_cg_solve_hint", i32, [vp, vp, vp, vp, vp, i32, i32, f32, i32, vp, vp, vp, vp, vp, sz, vp, f32])
+    sig("gll_cg_kernel", i32, [i32, i32, f32])
     sig("gll_backward_edges", i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp])
     sig("gll_debug_gram_tile", i32, [vp, i32, i32, i32, i32, vp, vp, vp, sz, vp])
     sig("gll_base_cache_bytes", sz, [i32])
@@ -135,7 +136,7 @@ EXPORTS = ["gll_last_error", "gll_version", "gll_device_sm_count", "gll_kernel_c
            "gll_launch_count", "gll_profile_enable", "gll_profile_collect", "gll_debug_cg_trace", "gll_debug_knn_trace", "gll_padded_classes", "gll_max_edges",
            "gll_state_layout", "gll_workspace_bytes", "gll_knn_workspace_bytes", "gll_graph_workspace_bytes",
            "gll_weights_workspace_bytes", "gll_cg_workspace_bytes", "gll_knn", "gll_graph_build", "gll_edge_weights",
-           "gll_cg_solve", "gll_cg_solve_hint", "gll_backward_edges", "gll_forward", "gll_backward", "gll_backward_scaled", "gll_knn_rows_workspace_bytes", "gll_knn_rows",
+           "gll_cg_solve", "gll_cg_solve_hint", "gll_cg_kernel", "gll_backward_edges", "gll_forward", "gll_backward", "gll_backward_scaled", "gll_knn_rows_workspace_bytes", "gll_knn_rows",
            "gll_backward_edges_rows", "gll_pack_columns", "gll_unpack_columns", "gll_unpack_pred", "gll_pack_grad",
            "gll_cg_rows_workspace_bytes", "gll_cg_rows_init", "gll_cg_rows_spmv", "gll_cg_rows_update", "gll_ce_loss", "gll_ce_loss_workspace_bytes",
            "gll_cg_rows_peer_mail_bytes", "gll_cg_rows_peer_flag_bytes", "gll_cg_rows_init_p2p", "gll_cg_rows_spmv_p2p",

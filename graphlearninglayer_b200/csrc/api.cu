@@ -481,16 +481,34 @@ int gll_edge_weights(const int* knn_idx, const float* knn_dist, const int* row_p
 int gll_cg_solve(const int* uu_ptr, const int* uu_col, const float* uu_val, const float* diag, const float* rhs, int m, int l,
                  float tol, int max_iter, float* x, int* iters_out, float* resid_out, int* status_out, void* workspace,
                  size_t workspace_bytes, void* stream) {
-  return cg_run(uu_ptr, uu_col, uu_val, diag, rhs, m, l, tol, max_iter, x, iters_out, resid_out, status_out, workspace,
-                workspace_bytes, (cudaStream_t)stream);
+  return gll_cg_solve_hint(uu_ptr, uu_col, uu_val, diag, rhs, m, l, tol, max_iter, x, iters_out, resid_out, status_out, workspace,
+                           workspace_bytes, stream, 0.f);
 }
 
 int gll_cg_solve_hint(const int* uu_ptr, const int* uu_col, const float* uu_val, const float* diag, const float* rhs, int m, int l,
                       float tol, int max_iter, float* x, int* iters_out, float* resid_out, int* status_out, void* workspace,
                       size_t workspace_bytes, void* stream, float uu_degree_hint) {
-  const CgIo io = {nullptr, 0, nullptr, 0, nullptr, 0, uu_degree_hint};
-  return cg_run(uu_ptr, uu_col, uu_val, diag, rhs, m, l, tol, max_iter, x, iters_out, resid_out, status_out, workspace,
-                workspace_bytes, (cudaStream_t)stream, nullptr, &io);
+  CgSolve S{};
+  S.ptr = uu_ptr;
+  S.col = uu_col;
+  S.val = uu_val;
+  S.diag = diag;
+  S.m = m;
+  S.rhs = rhs;
+  S.x = x;
+  S.l = l;
+  S.tol = tol;
+  S.max_iter = max_iter;
+  S.iters_out = iters_out;
+  S.resid_out = resid_out;
+  S.status_out = status_out;
+  S.uu_degree_hint = uu_degree_hint;
+  return cg_run(S, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int gll_cg_kernel(int m, int l, float uu_degree_hint) {
+  GLL_REQUIRE(m >= 1 && l >= 1 && l <= 128, "need m >= 1 and 1 <= l <= 128");
+  return cg_pick(m, padded_classes(l), uu_degree_hint, false);
 }
 
 int gll_backward_edges(const float* X, int n, int d, int l, int k_lab, int eps_auto, const int* row_ptr, const int* col,
@@ -662,10 +680,15 @@ static int forward_solve(const GraphBufs& B, const float* Y, int n, int k, int l
   const int m = n - k_lab, lp = padded_classes(l);
   int rc = graph_stages_run(B, Y, n, k, l, k_lab, eps_auto, eps_fixed, tau, 0, 6, workspace, workspace_bytes, st);
   if (rc) return rc;
-  const CgIo io = {nullptr, 0, pred_out, pred_is_f64, nullptr, 0, uu_degree_hint(n, k, m)};  // Pred (GLL.py:66) is written by the solver itself
-  return cg_run(B.uu_ptr, B.uu_col, B.uu_val, B.diag, B.rhs, m, l, cg_tol, cg_max_iter, B.ut + (size_t)k_lab * lp,
-                B.info + GLL_INFO_CG_ITERS_FWD, (float*)(B.info + GLL_INFO_CG_RESID_FWD), B.info + GLL_INFO_STATUS, workspace,
-                workspace_bytes, st, (unsigned*)(B.info + GLL_INFO_CG_BARRIER), &io);
+  CgSolve S = cg_system(B, m, l, cg_tol, cg_max_iter);
+  S.x = B.ut + (size_t)k_lab * lp;
+  S.iters_out = B.info + GLL_INFO_CG_ITERS_FWD;
+  S.resid_out = (float*)(B.info + GLL_INFO_CG_RESID_FWD);
+  S.status_out = B.info + GLL_INFO_STATUS;
+  S.x_copy = pred_out;  // Pred (GLL.py:66) is written by the solver itself
+  S.x_copy_f64 = pred_is_f64;
+  S.uu_degree_hint = uu_degree_hint(n, k, m);
+  return cg_run(S, workspace, workspace_bytes, st);
 }
 
 int gll_forward(const float* X, const float* Y, int n, int d, int k, int l, int k_lab, int eps_auto, float eps_fixed,
@@ -795,10 +818,17 @@ int gll_backward_scaled(const float* X, const void* grad_out, int grad_is_f64, c
   const int m = n - k_lab, lp = padded_classes(l);
   // GLL.py:104: the solver reads the incoming gradient itself; the labeled rows of the padded adjoint solution (zeros) are
   // never read -- edge_grad substitutes them
-  const CgIo io = {grad_out, grad_is_f64 ? 2 : 1, nullptr, 0, scale, scale_is_f64, uu_degree_hint(n, k, m)};
-  rc = cg_run(B.uu_ptr, B.uu_col, B.uu_val, B.diag, B.rhs, m, l, cg_tol, cg_max_iter, B.wt + (size_t)k_lab * lp,
-              B.info + GLL_INFO_CG_ITERS_BWD, (float*)(B.info + GLL_INFO_CG_RESID_BWD), B.info + GLL_INFO_STATUS, workspace,
-              workspace_bytes, st, (unsigned*)(B.info + GLL_INFO_CG_BARRIER), &io);
+  CgSolve S = cg_system(B, m, l, cg_tol, cg_max_iter);
+  S.x = B.wt + (size_t)k_lab * lp;
+  S.iters_out = B.info + GLL_INFO_CG_ITERS_BWD;
+  S.resid_out = (float*)(B.info + GLL_INFO_CG_RESID_BWD);
+  S.status_out = B.info + GLL_INFO_STATUS;
+  S.rhs_src = grad_out;
+  S.rhs_kind = grad_is_f64 ? 2 : 1;
+  S.rhs_scale = scale;
+  S.rhs_scale_f64 = scale_is_f64;
+  S.uu_degree_hint = uu_degree_hint(n, k, m);
+  rc = cg_run(S, workspace, workspace_bytes, st);
   if (rc) return rc;
   return backward_edges_run(X, n, d, l, k_lab, eps_auto, B, dX, 0, n, 3, st);
 }

@@ -23,12 +23,6 @@ namespace gll {
 namespace {
 
 
-__device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
 __device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned& epoch) {
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -36,36 +30,11 @@ __device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned& epoch)
     __threadfence();
     atomicAdd(counter, 1u);
     const unsigned target = epoch * gridDim.x;
-    while (ld_acquire(counter) < target) {
+    while (ld_acquire_u32(counter) < target) {
     }
     __threadfence();
   }
   __syncthreads();
-}
-
-__device__ __forceinline__ float4 ldcg4(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
-__device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
-
-// sum over the neighbour-slot index s of lane = s*Q + q; result valid on lanes < Q
-__device__ __forceinline__ float4 reduce_over_s(float4 a, int s, int S, int Q) {
-  int top = 1;
-  while (top < S) top <<= 1;
-  int span = S;
-  for (int st = top >> 1; st >= 1; st >>= 1) {
-    float4 o;
-    o.x = __shfl_down_sync(FULL, a.x, st * Q);
-    o.y = __shfl_down_sync(FULL, a.y, st * Q);
-    o.z = __shfl_down_sync(FULL, a.z, st * Q);
-    o.w = __shfl_down_sync(FULL, a.w, st * Q);
-    if (s < st && s + st < span) {
-      a.x += o.x;
-      a.y += o.y;
-      a.z += o.z;
-      a.w += o.w;
-    }
-    span = min(span, st);
-  }
-  return a;
 }
 
 // Deterministic grid-wide sum of NV float4 accumulators per lane (lane owns class quad q), with a grid barrier.
@@ -107,17 +76,11 @@ __device__ __forceinline__ void grid_reduce(float4 (&acc)[NV], const CgParams& P
   __syncthreads();
 }
 
-// Masked operator of laplace_learning_trials: column c of this solve is column col0 + c of `trials` trials of `cols` columns each,
-// and A p is zeroed at (row i, trial t) when slot[i trials + t] >= 0.  A separate parameter, so that CgParams (shared with the
-// on-chip kernels) keeps its layout.
-struct CgMask {
-  const int* slot;
-  int trials, cols, col0;
-};
-
-// MASK = false is the unmasked solve and never reads M
+// MASK: the masked operator of laplace_learning_trials.  Column c of this solve is column mask_col0 + c of mask_trials trials
+// of mask_cols columns each, and A p is zeroed at (row i, trial t) when mask_slot[i mask_trials + t] >= 0.  MASK = false never
+// reads the mask.
 template <bool MASK>
-__global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P, CgMask M) {
+__global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P) {
   extern __shared__ __align__(16) double sm[];
   const int lp = P.lp, Q = lp >> 2, S = 32 / Q;
   double* wpart = sm;                            // [2][CG_WARPS][lp]
@@ -215,8 +178,8 @@ __global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P
         const float dg = __ldg(P.diag + i);
         float4 ap = make_float4(fmaf(dg, pi.x, -a.x), fmaf(dg, pi.y, -a.y), fmaf(dg, pi.z, -a.z), fmaf(dg, pi.w, -a.w));
         if constexpr (MASK) {  // row i clamped in this quad's trial: r, p and x stay 0 there (a quad never spans two trials)
-          const int t = (M.col0 + 4 * lane) / M.cols;
-          if (__ldg(M.slot + (size_t)i * M.trials + t) >= 0) ap = make_float4(0.f, 0.f, 0.f, 0.f);
+          const int t = (P.mask_col0 + 4 * lane) / P.mask_cols;
+          if (__ldg(P.mask_slot + (size_t)i * P.mask_trials + t) >= 0) ap = make_float4(0.f, 0.f, 0.f, 0.f);
         }
         st4(P.ap + o, ap);
         dot[0].x = fmaf(pi.x, ap.x, dot[0].x);
@@ -280,26 +243,33 @@ __global__ void __launch_bounds__(CG_THREADS, 1) cg_persistent_kernel(CgParams P
     grid_barrier(P.barrier, epoch);
   }
 
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    const float resid = (float)sqrt(maxrr);
-    if (P.iters_out) *P.iters_out = it;
-    if (P.resid_out) *P.resid_out = resid;
-    if (P.status_out) {
-      int st = 0;
-      if (nonfinite) st |= GLL_STATUS_NONFINITE;
-      if (!nonfinite && !(sqrt(maxrr) <= tol)) st |= GLL_STATUS_CG_NOT_CONVERGED;
-      if (st) atomicOr(P.status_out, st);
-    }
-  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) cg_write_stats(P, it, (float)sqrt(maxrr), nonfinite, sqrt(maxrr), tol);
 }
 
 size_t cg_smem_bytes(int lp) {
   return sizeof(double) * ((size_t)2 * CG_WARPS * lp + 2 * lp + 2 * lp) + sizeof(float) * 2 * lp;
 }
 
-int cg_grid(int m) {
-  int g = ceil_div(m, CG_WARPS);
-  return max(1, min(g, device_info().sms));
+// Streaming kernel: the layer's conversions run as separate kernels around the solve.
+int cg_streaming_launch(CgParams P, cudaStream_t st) {
+  const int m = P.m, l = P.l, lp = P.lp;
+  if (P.rhs_src != nullptr) {
+    const int rc = pack_grad(P.rhs_src, P.rhs_kind == 2, m, l, lp, const_cast<float*>(P.rhs), st, nullptr, 0, P.rhs_scale, P.rhs_scale_f64);
+    if (rc) return rc;
+    P.rhs_src = nullptr;
+  }
+  void* x_copy = P.x_copy;
+  P.x_copy = nullptr;
+  const int grid = max(1, min(ceil_div(m, CG_WARPS), device_info().sms));
+  const int S = 32 / (lp / 4);
+  P.rows_per_block = ceil_div(ceil_div(m, grid), S) * S;  // keep phase-2/3 spans aligned to whole lane groups
+  const void* kern = P.mask_slot ? (const void*)cg_persistent_kernel<true> : (const void*)cg_persistent_kernel<false>;
+  GLL_CUDA_CHECK(set_max_dynamic_smem_once(kern, (int)cg_smem_bytes(CG_MAX_LP)));
+  GLL_CUDA_CHECK(cudaMemsetAsync(P.barrier, 0, 256, st));
+  void* args[] = {&P};
+  GLL_PROF(KID_CG, st);
+  GLL_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(CG_THREADS), args, cg_smem_bytes(lp), st));
+  return x_copy ? unpack_pred(P.x, m, l, lp, x_copy, P.x_copy_f64, st) : GLL_OK;
 }
 
 }  // namespace
@@ -327,23 +297,37 @@ size_t cg_ws_bytes(int m, int l) {
          cg_resident_ws_bytes(m, lp);
 }
 
-int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const float* diag, const float* rhs, int m, int l,
-           float tol, int max_iter, float* x, int* iters_out, float* resid_out, int* status_out, void* ws, size_t ws_bytes,
-           cudaStream_t st, unsigned* ext_counter, const CgIo* io) {
-  GLL_REQUIRE(uu_ptr && uu_col && uu_val && diag && rhs && x && ws, "null pointer");
-  const int lp = padded_classes(l);
+// Systems that fit on chip (every config except the sharded 1M-node graph) take an on-chip kernel.  The cluster kernel gathers
+// neighbour rows through distributed shared memory, which moves few transactions per clock: it wins on SPARSE systems (C2: 1.4
+// off-diagonal entries per row, C3: 3.2 -- 35 us per solve against 41 for the one-CTA kernel) and loses on dense ones (C1: 14.5
+// per row -- 154 us against 94 for the multi-CTA kernel).  The host cannot see nnz; the layer passes what it expects,
+// (k - 1) m / n, and callers that pass nothing get the other kernels.  GLL_B200_CG_PATH ("streaming" / "resident" / "small" /
+// "cluster") is a testing knob: "small" and "cluster" put that kernel first, any other value skips both minibatch kernels.
+int cg_pick(int m, int lp, float uu_degree_hint, bool masked) {
+  if (masked) return GLL_CG_KERNEL_STREAMING;
+  const char* force = getenv("GLL_B200_CG_PATH");
+  const bool unset = force == nullptr || force[0] == 0;
+  const bool small = !unset && strcmp(force, "small") == 0, cluster = !unset && strcmp(force, "cluster") == 0;
+  if (!unset && strcmp(force, "streaming") == 0) return GLL_CG_KERNEL_STREAMING;
+  if (unset || small || cluster) {
+    const bool sparse = uu_degree_hint > 0.f && uu_degree_hint <= 5.f;
+    if ((cluster || (unset && sparse)) && cg_cluster_fits(m, lp)) return GLL_CG_KERNEL_CLUSTER;
+    if (cg_small_fits(m, lp)) return GLL_CG_KERNEL_SMALL;
+  }
+  return cg_resident_fits(m, lp) ? GLL_CG_KERNEL_RESIDENT : GLL_CG_KERNEL_STREAMING;
+}
+
+int cg_run(const CgSolve& S, void* ws, size_t ws_bytes, cudaStream_t st) {
+  GLL_REQUIRE(S.ptr && S.col && S.val && S.diag && S.rhs && S.x && ws, "null pointer");
+  const int m = S.m, l = S.l, lp = padded_classes(l);
   if (ws_bytes < cg_ws_bytes(m, l)) {
     set_error("CG workspace too small: %zu < %zu", ws_bytes, cg_ws_bytes(m, l));
     return GLL_ERR_WORKSPACE;
   }
   Carver cv(ws, ws_bytes);
-  // Layer-side conversions (GLL.py:66 float64 output, GLL.py:104 the incoming gradient): the on-chip kernels read / write the
-  // caller's arrays themselves; the chunked and the streaming path run the two small kernels around the solve.
-  const bool has_src = io != nullptr && io->rhs_src != nullptr, has_copy = io != nullptr && io->x_copy != nullptr;
-  const bool masked = io != nullptr && io->mask_slot != nullptr;
   if (lp > CG_MAX_LP) {
-    if (has_src) {
-      const int rc = pack_grad(io->rhs_src, io->rhs_kind == 2, m, l, lp, const_cast<float*>(rhs), st, nullptr, 0, io->rhs_scale, io->rhs_scale_f64);
+    if (S.rhs_src != nullptr) {
+      const int rc = pack_grad(S.rhs_src, S.rhs_kind == 2, m, l, lp, const_cast<float*>(S.rhs), st, nullptr, 0, S.rhs_scale, S.rhs_scale_f64);
       if (rc) return rc;
     }
     const int chunks = ceil_div(l, CG_MAX_LP);
@@ -353,101 +337,46 @@ int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const floa
     float* rs_c = cv.take<float>(chunks);
     const size_t sub_bytes = cg_ws_bytes(m, CG_MAX_LP);
     void* sub = cv.take<char>(sub_bytes);
-    GLL_CUDA_CHECK(cudaMemsetAsync(x, 0, sizeof(float) * (size_t)m * lp, st));  // padded class columns read as zero
+    GLL_CUDA_CHECK(cudaMemsetAsync(S.x, 0, sizeof(float) * (size_t)m * lp, st));  // padded class columns read as zero
     for (int c = 0; c < chunks; ++c) {
       const int c0 = c * CG_MAX_LP, cnt = min(CG_MAX_LP, l - c0), lpc = padded_classes(cnt);
-      int rc = pack_columns(rhs, m, lp, c0, cnt, rhs_c, lpc, st);
+      int rc = pack_columns(S.rhs, m, lp, c0, cnt, rhs_c, lpc, st);
       if (rc) return rc;
-      CgIo mio = {};  // a masked solve: the mask is indexed by the chunk's global columns
-      if (masked) {
-        mio.mask_slot = io->mask_slot;
-        mio.mask_trials = io->mask_trials;
-        mio.mask_cols = io->mask_cols;
-        mio.mask_col0 = io->mask_col0 + c0;
-      }
-      rc = cg_run(uu_ptr, uu_col, uu_val, diag, rhs_c, m, cnt, tol, max_iter, x_c, it_c + c, rs_c + c, status_out, sub, sub_bytes, st,
-                  ext_counter, masked ? &mio : nullptr);
+      // a chunk: packed columns, no conversions, no sparsity hint; the mask is indexed by the chunk's global columns
+      CgSolve C = S;
+      C.rhs = rhs_c;
+      C.x = x_c;
+      C.l = cnt;
+      C.iters_out = it_c + c;
+      C.resid_out = rs_c + c;
+      C.rhs_src = nullptr;
+      C.rhs_scale = nullptr;
+      C.x_copy = nullptr;
+      C.uu_degree_hint = 0.f;
+      C.mask_col0 = S.mask_col0 + c0;
+      rc = cg_run(C, sub, sub_bytes, st);
       if (rc) return rc;
-      rc = unpack_columns(x_c, m, lpc, c0, cnt, x, lp, st);
+      rc = unpack_columns(x_c, m, lpc, c0, cnt, S.x, lp, st);
       if (rc) return rc;
     }
-    cg_combine_stats_kernel<<<1, 1, 0, st>>>(it_c, rs_c, chunks, iters_out, resid_out);
+    cg_combine_stats_kernel<<<1, 1, 0, st>>>(it_c, rs_c, chunks, S.iters_out, S.resid_out);
     GLL_LAUNCH_CHECK();
-    return has_copy ? unpack_pred(x, m, l, lp, io->x_copy, io->x_copy_f64, st) : GLL_OK;
+    return S.x_copy ? unpack_pred(S.x, m, l, lp, S.x_copy, S.x_copy_f64, st) : GLL_OK;
   }
-  CgParams P;
-  P.ptr = uu_ptr;
-  P.col = uu_col;
-  P.val = uu_val;
-  P.diag = diag;
-  P.rhs = rhs;
-  P.x = x;
+  CgParams P{S};
+  P.lp = lp;
   P.r = cv.take<float>((size_t)m * lp);
   P.p = cv.take<float>((size_t)m * lp);
   P.ap = cv.take<float>((size_t)m * lp);
   P.partial = cv.take<double>((size_t)2 * (2 * CG_MAX_LP) * device_info().sms);
   P.barrier = cv.take<unsigned>(64);
-  P.m = m;
-  P.l = l;
-  P.lp = lp;
-  P.max_iter = max_iter;
-  P.tol = tol;
-  P.iters_out = iters_out;
-  P.resid_out = resid_out;
-  P.status_out = status_out;
-  P.rows_per_block = 0;
-  P.ext_counter = ext_counter;
-  P.rhs_src = io ? io->rhs_src : nullptr;
-  P.rhs_kind = io ? io->rhs_kind : 0;
-  P.x_copy = io ? io->x_copy : nullptr;
-  P.x_copy_f64 = io ? io->x_copy_f64 : 0;
-  P.rhs_scale = io ? io->rhs_scale : nullptr;
-  P.rhs_scale_f64 = io ? io->rhs_scale_f64 : 0;
-  if (!masked) {  // systems that fit on chip (every config except the sharded 1M-node graph) take the shared-memory-resident kernel
-    const char* force = getenv("GLL_B200_CG_PATH");  // "streaming" / "resident" / "small" / "cluster": testing knobs
-    const bool only_small = force != nullptr && strcmp(force, "small") == 0;
-    const bool force_cluster = force != nullptr && strcmp(force, "cluster") == 0;
-    // The cluster kernel gathers neighbour rows through distributed shared memory, which moves few transactions per clock: it
-    // wins on SPARSE systems (C2: 1.4 off-diagonal entries per row, C3: 3.2 -- 35 us per solve against 41 for the one-CTA kernel)
-    // and loses on dense ones (C1: 14.5 per row -- 154 us against 94 for the multi-CTA kernel).  The host cannot see nnz; the
-    // layer passes what it expects, (k - 1) m / n, and callers that pass nothing get the other kernels.
-    const bool sparse = io != nullptr && io->uu_degree_hint > 0.f && io->uu_degree_hint <= 5.f;
-    if (force == nullptr || force[0] == 0 || only_small || force_cluster) {  // minibatch-sized systems: the latency-organised kernels
-      int rc = (force_cluster || (sparse && !only_small)) ? cg_cluster_try(P, st) : 0;  // one cluster of eight CTAs (64 <= m <= 2048)
-      if (rc < 0) return rc;
-      if (rc == 1) return GLL_OK;
-      rc = cg_small_try(P, st);  // one CTA, a thread per row (m <= 512)
-      if (rc < 0) return rc;
-      if (rc == 1) return GLL_OK;
-    }
-    if (!(force && strcmp(force, "streaming") == 0)) {
-      void* scratch = cv.take<char>(cg_resident_ws_bytes(m, lp));
-      const int rc = cg_resident_try(P, scratch, st);
-      if (rc < 0) return rc;
-      if (rc == 1) return GLL_OK;
-    }
+  void* scratch = cv.take<char>(cg_resident_ws_bytes(m, lp));
+  switch (cg_pick(m, lp, S.uu_degree_hint, S.mask_slot != nullptr)) {
+    case GLL_CG_KERNEL_CLUSTER: return cg_cluster_launch(P, st);    // one cluster of eight CTAs (64 <= m <= 2048)
+    case GLL_CG_KERNEL_SMALL: return cg_small_launch(P, st);        // one CTA (m <= 512)
+    case GLL_CG_KERNEL_RESIDENT: return cg_resident_launch(P, scratch, st);
+    default: return cg_streaming_launch(P, st);
   }
-  if (has_src) {  // streaming kernel: conversions as separate kernels
-    const int rc = pack_grad(io->rhs_src, io->rhs_kind == 2, m, l, lp, const_cast<float*>(rhs), st, nullptr, 0, io->rhs_scale, io->rhs_scale_f64);
-    if (rc) return rc;
-    P.rhs_src = nullptr;
-  }
-  P.x_copy = nullptr;
-  const int grid = cg_grid(m);
-  const int S = 32 / (lp / 4);
-  int rpb = ceil_div(m, grid);
-  rpb = ceil_div(rpb, S) * S;  // keep phase-2/3 spans aligned to whole lane groups
-  P.rows_per_block = rpb;
-  const size_t smem = cg_smem_bytes(lp);
-  const void* kern = masked ? (const void*)cg_persistent_kernel<true> : (const void*)cg_persistent_kernel<false>;
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once(kern, (int)cg_smem_bytes(CG_MAX_LP)));
-  GLL_CUDA_CHECK(cudaMemsetAsync(P.barrier, 0, 256, st));
-  CgMask M = {nullptr, 0, 0, 0};
-  if (masked) M = {io->mask_slot, io->mask_trials, io->mask_cols, io->mask_col0};
-  void* args[] = {&P, &M};
-  GLL_PROF(KID_CG, st);
-  GLL_CUDA_CHECK(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(CG_THREADS), args, smem, st));
-  return has_copy ? unpack_pred(x, m, l, lp, io->x_copy, io->x_copy_f64, st) : GLL_OK;
 }
 
 }  // namespace gll

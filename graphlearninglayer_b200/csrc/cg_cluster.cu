@@ -8,16 +8,13 @@
 //      fp32 and finishes with one float4 butterfly; the partial sums (fp64) go into a slot per (CTA, part)
 //   C  thread c adds the slots of class column c in a fixed order and derives alpha / beta; stop test
 //   D  vector updates, new u
-// Two shapes of the same kernel:
-//   * ONE CTA of 1024 threads for up to 512 rows (the former one-CTA kernel, cg_small.cu, took 3.1 us per iteration with a
-//     thread per row: a warp walked the longest of its 32 rows serially and nine warps added 512 rows each);
-//   * ONE CLUSTER of eight CTAs for up to 2048 rows: a CTA owns an eighth of the rows, neighbour rows are gathered from the
-//     owner's shared memory (ld.shared::cluster, addresses precomputed with mapa), the partial sums are written into a slot of
-//     EVERY CTA's shared memory (st.shared::cluster) and two barrier.cluster per iteration replace the two grid barriers of
-//     the multi-CTA kernel (cg_resident.cu: 1.2 us each through L2).
-// No global-memory traffic inside the loop.
+// ONE CLUSTER of eight CTAs of 320 threads runs systems of 64 to 2048 rows: a CTA owns an eighth of the rows, neighbour rows are
+// gathered from the owner's shared memory (ld.shared::cluster, addresses precomputed with mapa), the partial sums are written
+// into a slot of EVERY CTA's shared memory (st.shared::cluster) and two barrier.cluster per iteration replace the two grid
+// barriers of the multi-CTA kernel (cg_resident.cu: 1.2 us each through L2).  No global-memory traffic inside the loop.
+// It takes a system when cg_pick routes it here (a sparsity hint of at most 5 entries per row, or GLL_B200_CG_PATH=cluster)
+// and its items (class quads x rows per CTA) fit four per thread; the others go to cg_small.cu or cg_resident.cu.
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "cg_common.cuh"
@@ -25,6 +22,12 @@
 namespace gll {
 namespace {
 
+constexpr int CC_CTAS = 8;
+// (256 / 320 / 384 threads per CTA measured the same at C2, 2.95-3.2 us per iteration; the same item layout on ONE CTA: 3.8 us
+//  with 512 threads, 5.0 us with 1024 (spills at 64 registers) -- an iteration is ~450 mostly dependent instructions per warp,
+//  and what the cluster buys is a shorter chain per warp, not bandwidth)
+constexpr int CC_THREADS = 320;
+constexpr int CC_WARPS = CC_THREADS / 32;
 constexpr int CC_MAX_NIT = 4;
 constexpr size_t CC_SMEM_BUDGET = 208 * 1024;  // (512 rows x 12 class columns on one CTA: 145 KB of vectors and products)
 
@@ -33,14 +36,9 @@ __device__ __forceinline__ uint32_t cc_rank() {
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
   return r;
 }
-template <int CTAS>
-__device__ __forceinline__ void cc_sync() {  // everybody in the CTA (cluster) is here, and their shared-memory writes are visible
-  if (CTAS == 1) {
-    __syncthreads();
-  } else {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-  }
+__device__ __forceinline__ void cc_sync() {  // everybody in the cluster is here, and their shared-memory writes are visible
+  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 __device__ __forceinline__ uint32_t cc_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 // cluster-window address of the same shared-memory offset in CTA `rank` (a CTA's own shared::cta addresses are valid there too)
@@ -57,10 +55,6 @@ __device__ __forceinline__ float4 cc_ld4(uint32_t addr) {
 __device__ __forceinline__ void cc_st_f64(uint32_t addr, double v) {
   asm volatile("st.shared::cluster.f64 [%0], %1;" ::"r"(addr), "d"(v) : "memory");
 }
-__device__ __forceinline__ float4 cc_zero4() { return make_float4(0.f, 0.f, 0.f, 0.f); }
-__device__ __forceinline__ void cc_fma4(float4& a, float w, const float4& u) {
-  a.x = fmaf(w, u.x, a.x); a.y = fmaf(w, u.y, a.y); a.z = fmaf(w, u.z, a.z); a.w = fmaf(w, u.w, a.w);
-}
 
 struct CcShape {
   int R;         // rows per CTA (a multiple of 32)
@@ -69,18 +63,17 @@ struct CcShape {
   int edge_cap;  // edges of a CTA's slice that fit in shared memory
 };
 
-template <int NIT, int CTAS, int THREADS>
-__global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcShape S, unsigned long long* trace) {
+template <int NIT>
+__global__ void __launch_bounds__(CC_THREADS, 1) cg_cluster_kernel(CgParams P, CcShape S, unsigned long long* trace) {
   // debug timeline (gll_debug_cg_trace, tools/cg_small_trace.py): trace[pass * 8 + phase] = SM clock of CTA 0, thread 0
 #define CC_STAMP(phase) do { if (trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0 && iter < 15) trace[iter * 8 + (phase)] = (unsigned long long)clock64(); } while (0)
-  constexpr int WARPS = THREADS / 32;
   extern __shared__ __align__(16) unsigned char sm_raw[];
   const int lp = P.lp, Q = lp >> 2, m = P.m, E3 = 3 * lp, R = S.R;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0) trace[15 * 8 + 7] = (unsigned long long)clock64();  // kernel entry
-  const int rank = (CTAS == 1) ? 0 : (int)cc_rank();
+  const int rank = (int)cc_rank();
   const int row0 = rank * R, rows = max(0, min(R, m - row0));  // my rows (R = rows per CTA, the same in every CTA)
-  const int nslots = CTAS * S.nparts;
+  const int nslots = CC_CTAS * S.nparts;
   // ---- shared memory (identical layout in every CTA: remote addresses are local offsets mapped with mapa) ----
   float* us = reinterpret_cast<float*>(sm_raw);                              // [R][lp]   u = r / diag of my rows
   float4* prod = reinterpret_cast<float4*>(us + (size_t)R * lp);             // [3][Q][R] r*u, w*u, r*r per item
@@ -97,16 +90,15 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
 
   const uint32_t us_s = cc_smem_u32(us), part_s = cc_smem_u32(part);
   auto u_row_addr = [&](int j) {
-    if (CTAS == 1) return us_s + (uint32_t)(j * lp) * 4u;
     const int owner = j / R;
     return cc_mapa(us_s + (uint32_t)((j - owner * R) * lp) * 4u, (uint32_t)owner);
   };
   const int e_begin = (rows > 0) ? __ldg(P.ptr + row0) : 0;
   const int nnz = (rows > 0) ? __ldg(P.ptr + row0 + rows) - e_begin : 0;
   const bool cached = nnz <= S.edge_cap;  // (always at minibatch sizes; otherwise the edges are read from global memory)
-  for (int i = tid; i <= rows; i += THREADS) lptr[i] = __ldg(P.ptr + row0 + i) - e_begin;
+  for (int i = tid; i <= rows; i += CC_THREADS) lptr[i] = __ldg(P.ptr + row0 + i) - e_begin;
   if (cached)
-    for (int e = tid; e < nnz; e += THREADS) {
+    for (int e = tid; e < nnz; e += CC_THREADS) {
       eaddr[e] = u_row_addr(__ldg(P.col + e_begin + e));
       eval[e] = __ldg(P.val + e_begin + e);
     }
@@ -118,17 +110,17 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
   float4 r[NIT], p[NIT], s[NIT];
 #pragma unroll
   for (int k = 0; k < NIT; ++k) {
-    const int it = tid + k * THREADS;
+    const int it = tid + k * CC_THREADS;
     quad[k] = it / R;
     lrow[k] = it - quad[k] * R;
     on[k] = quad[k] < Q && lrow[k] < rows;
     dg[k] = on[k] ? __ldg(P.diag + row0 + lrow[k]) : 1.f;
     dinv[k] = on[k] ? 1.f / dg[k] : 0.f;
-    r[k] = on[k] ? cg_load_rhs4(P, row0 + lrow[k], quad[k]) : cc_zero4();
-    p[k] = s[k] = cc_zero4();
+    r[k] = on[k] ? cg_load_rhs4(P, row0 + lrow[k], quad[k]) : zero4();
+    p[k] = s[k] = zero4();
     if (quad[k] < Q) {
-      xs[(size_t)quad[k] * R + lrow[k]] = cc_zero4();
-      *reinterpret_cast<float4*>(us + (size_t)lrow[k] * lp + 4 * quad[k]) = make_float4(r[k].x * dinv[k], r[k].y * dinv[k], r[k].z * dinv[k], r[k].w * dinv[k]);
+      xs[(size_t)quad[k] * R + lrow[k]] = zero4();
+      *reinterpret_cast<float4*>(us + (size_t)lrow[k] * lp + 4 * quad[k]) = scale4(r[k], dinv[k]);
     }
   }
   // per-column CG scalars: thread c owns class column c (every CTA computes identical values)
@@ -137,7 +129,7 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
   double tol2 = 0.0;
   int iter = 0;
   bool bad_any = false;
-  cc_sync<CTAS>();  // every CTA's u and edge addresses are in place
+  cc_sync();  // every CTA's u and edge addresses are in place
 
   while (true) {
     CC_STAMP(0);
@@ -145,7 +137,7 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
 #pragma unroll
     for (int k = 0; k < NIT; ++k) {
       if (quad[k] < Q) {
-        float4 a = cc_zero4();
+        float4 a = zero4();
         if (on[k]) {
           const int e1 = lptr[lrow[k] + 1];
           const uint32_t qoff = 16u * (uint32_t)quad[k];
@@ -156,26 +148,26 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
             for (; e + 4 <= e1; e += 4) {
               const uint32_t a0 = eaddr[e], a1 = eaddr[e + 1], a2 = eaddr[e + 2], a3 = eaddr[e + 3];
               const float4 u0 = cc_ld4(a0 + qoff), u1 = cc_ld4(a1 + qoff), u2 = cc_ld4(a2 + qoff), u3 = cc_ld4(a3 + qoff);
-              cc_fma4(a, eval[e], u0);
-              cc_fma4(a, eval[e + 1], u1);
-              cc_fma4(a, eval[e + 2], u2);
-              cc_fma4(a, eval[e + 3], u3);
+              fma4(a, eval[e], u0);
+              fma4(a, eval[e + 1], u1);
+              fma4(a, eval[e + 2], u2);
+              fma4(a, eval[e + 3], u3);
             }
             if (e + 2 <= e1) {
               const uint32_t a0 = eaddr[e], a1 = eaddr[e + 1];
               const float4 u0 = cc_ld4(a0 + qoff), u1 = cc_ld4(a1 + qoff);
-              cc_fma4(a, eval[e], u0);
-              cc_fma4(a, eval[e + 1], u1);
+              fma4(a, eval[e], u0);
+              fma4(a, eval[e + 1], u1);
               e += 2;
             }
-            if (e < e1) cc_fma4(a, eval[e], cc_ld4(eaddr[e] + qoff));
+            if (e < e1) fma4(a, eval[e], cc_ld4(eaddr[e] + qoff));
           } else {
-            for (; e < e1; ++e) cc_fma4(a, __ldg(P.val + e_begin + e), cc_ld4(u_row_addr(__ldg(P.col + e_begin + e)) + qoff));
+            for (; e < e1; ++e) fma4(a, __ldg(P.val + e_begin + e), cc_ld4(u_row_addr(__ldg(P.col + e_begin + e)) + qoff));
           }
         }
-        const float4 u4 = make_float4(r[k].x * dinv[k], r[k].y * dinv[k], r[k].z * dinv[k], r[k].w * dinv[k]);
+        const float4 u4 = scale4(r[k], dinv[k]);
         const float4 w4 = on[k] ? make_float4(fmaf(dg[k], u4.x, -a.x), fmaf(dg[k], u4.y, -a.y), fmaf(dg[k], u4.z, -a.z), fmaf(dg[k], u4.w, -a.w))
-                                : cc_zero4();
+                                : zero4();
         const size_t o = (size_t)quad[k] * R + lrow[k];
         ws[o] = w4;
         prod[o] = make_float4(r[k].x * u4.x, r[k].y * u4.y, r[k].z * u4.z, r[k].w * u4.w);
@@ -188,11 +180,11 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
     __syncthreads();
     // ================= B: partial sums, one warp per (product, class quad, row part), into a slot of EVERY CTA =================
 #pragma unroll 1
-    for (int sj = warp; sj < 3 * Q * S.nparts; sj += WARPS) {
+    for (int sj = warp; sj < 3 * Q * S.nparts; sj += CC_WARPS) {
       const int job = sj / S.nparts, pt = sj - job * S.nparts;
       const float4* src = prod + (size_t)job * R;
       const int i1 = min(R, (pt + 1) * S.part_rows);
-      float4 f = cc_zero4();  // fp32 inside a part (<= a few hundred rows, as in the former one-CTA kernel), fp64 across parts and CTAs
+      float4 f = zero4();  // fp32 inside a part (<= a few hundred rows, as in the former one-CTA kernel), fp64 across parts and CTAs
       for (int i = pt * S.part_rows + lane; i < i1; i += 32) {  // rows beyond `rows` hold zeros (items that are not `on`)
         const float4 v = src[i];
         f.x += v.x; f.y += v.y; f.z += v.z; f.w += v.w;
@@ -204,11 +196,11 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
         f.z += __shfl_xor_sync(FULL, f.z, o);
         f.w += __shfl_xor_sync(FULL, f.w, o);
       }
-      // lane c < CTAS sends the four sums to CTA c (job = v * Q + quad  ->  element v * lp + 4 * quad + j)
-      if (lane < CTAS) {
+      // lane c < CC_CTAS sends the four sums to CTA c (job = v * Q + quad  ->  element v * lp + 4 * quad + j)
+      if (lane < CC_CTAS) {
         const int v = job / Q, qd = job - v * Q;
         const uint32_t off = part_s + (uint32_t)((rank * S.nparts + pt) * E3 + v * lp + 4 * qd) * 8u;
-        const uint32_t dst = (CTAS == 1) ? off : cc_mapa(off, (uint32_t)lane);
+        const uint32_t dst = cc_mapa(off, (uint32_t)lane);
         cc_st_f64(dst, (double)f.x);
         cc_st_f64(dst + 8u, (double)f.y);
         cc_st_f64(dst + 16u, (double)f.z);
@@ -216,7 +208,7 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
       }
     }
     CC_STAMP(5);
-    cc_sync<CTAS>();  // (1) all partial sums have landed
+    cc_sync();  // (1) all partial sums have landed
     CC_STAMP(1);
     if (tid < E3) {
       double t = 0.0;
@@ -238,18 +230,7 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
       float al = 0.f, be = 0.f;
       if (!frozen && rr > tol2) {
         live = 1;
-        const float bb = (iter == 0) ? 0.f : (float)g_new * inv_g_old;
-        const double den = d_new - (double)bb * g_new * (double)inv_a_old;
-        if (den > 0.0 && g_new > 0.0) {
-          // approximate reciprocals (MUFU.RCP, deterministic): alpha and beta only have to be the SAME numbers in every CTA
-          const float rg = __fdividef(1.f, (float)g_new);
-          al = __fdividef((float)g_new, (float)den);
-          be = bb;
-          inv_a_old = (float)den * rg;
-          inv_g_old = rg;
-        } else {
-          frozen = true;  // breakdown at the fp32 floor: stop moving this column
-        }
+        cg_column_step(g_new, d_new, iter == 0, inv_g_old, inv_a_old, frozen, al, be);
       }
       alpha[tid] = al;
       beta[tid] = be;
@@ -269,22 +250,14 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
         const float4 be = *reinterpret_cast<const float4*>(beta + 4 * quad[k]);
         const float di = dinv[k];
         const size_t o = (size_t)quad[k] * R + lrow[k];
-        const float4 w4 = ws[o];
         float4 x4 = xs[o];
-        p[k].x = fmaf(be.x, p[k].x, r[k].x * di); p[k].y = fmaf(be.y, p[k].y, r[k].y * di);
-        p[k].z = fmaf(be.z, p[k].z, r[k].z * di); p[k].w = fmaf(be.w, p[k].w, r[k].w * di);
-        s[k].x = fmaf(be.x, s[k].x, w4.x); s[k].y = fmaf(be.y, s[k].y, w4.y);
-        s[k].z = fmaf(be.z, s[k].z, w4.z); s[k].w = fmaf(be.w, s[k].w, w4.w);
-        x4.x = fmaf(al.x, p[k].x, x4.x); x4.y = fmaf(al.y, p[k].y, x4.y);
-        x4.z = fmaf(al.z, p[k].z, x4.z); x4.w = fmaf(al.w, p[k].w, x4.w);
-        r[k].x = fmaf(-al.x, s[k].x, r[k].x); r[k].y = fmaf(-al.y, s[k].y, r[k].y);
-        r[k].z = fmaf(-al.z, s[k].z, r[k].z); r[k].w = fmaf(-al.w, s[k].w, r[k].w);
+        cg_cg_update(al, be, scale4(r[k], di), ws[o], x4, r[k], p[k], s[k]);
         xs[o] = x4;
-        *reinterpret_cast<float4*>(us + (size_t)lrow[k] * lp + 4 * quad[k]) = make_float4(r[k].x * di, r[k].y * di, r[k].z * di, r[k].w * di);
+        *reinterpret_cast<float4*>(us + (size_t)lrow[k] * lp + 4 * quad[k]) = scale4(r[k], di);
       }
     }
     CC_STAMP(6);
-    cc_sync<CTAS>();  // (2) the new u is visible to everybody; the slots of `part` may be rewritten
+    cc_sync();  // (2) the new u is visible to everybody; the slots of `part` may be rewritten
   }
 #undef CC_STAMP
 
@@ -298,16 +271,9 @@ __global__ void __launch_bounds__(THREADS, 1) cg_cluster_kernel(CgParams P, CcSh
   if (rank == 0 && tid == 0) {
     double mx = 0.0;
     for (int c = 0; c < lp; ++c) mx = fmax(mx, red[2 * lp + c]);
-    if (P.iters_out) *P.iters_out = iter;
-    if (P.resid_out) *P.resid_out = (float)sqrt(mx);
-    if (P.status_out) {
-      int st = 0;
-      if (bad_any) st |= GLL_STATUS_NONFINITE;
-      if (!bad_any && !(mx <= tol2)) st |= GLL_STATUS_CG_NOT_CONVERGED;
-      if (st) atomicOr(P.status_out, st);
-    }
+    cg_write_stats(P, iter, (float)sqrt(mx), bad_any, mx, tol2);
   }
-  if (CTAS > 1) cc_sync<CTAS>();  // nobody exits while a peer may still read its u rows or write into its slots
+  cc_sync();  // nobody exits while a peer may still read its u rows or write into its slots
 }
 
 size_t cc_fixed_smem(int R, int lp, int nslots) {
@@ -317,55 +283,59 @@ size_t cc_fixed_smem(int R, int lp, int nslots) {
   return align_up(b, 16);
 }
 
-template <int CTAS, int THREADS>
-int cc_launch(const CgParams& P, cudaStream_t st) {
-  const int lp = P.lp, Q = lp >> 2;
+struct CcPlan {
+  int nit;  // items per thread; 0: the system does not fit
   CcShape S;
-  S.R = ceil_div(ceil_div(P.m, CTAS), 32) * 32;  // whole warps of rows per class quad
-  const long long items = (long long)Q * S.R;
-  const int nit = (int)((items + THREADS - 1) / THREADS);
-  if (nit > CC_MAX_NIT) return 0;
-  S.nparts = max(1, min((THREADS / 32) / (3 * Q), S.R / 32));  // use the warps that the (product, quad) jobs leave idle
+  size_t smem;
+};
+
+CcPlan cluster_plan(int m, int lp) {
+  CcPlan p = {};
+  if (m < 64 || m > 2048) return p;  // below 64 rows there is nothing to share
+  const int Q = lp >> 2;
+  CcShape& S = p.S;
+  S.R = ceil_div(ceil_div(m, CC_CTAS), 32) * 32;  // whole warps of rows per class quad
+  const int nit = (int)(((long long)Q * S.R + CC_THREADS - 1) / CC_THREADS);
+  if (nit > CC_MAX_NIT) return p;
+  S.nparts = max(1, min(CC_WARPS / (3 * Q), S.R / 32));  // use the warps that the (product, quad) jobs leave idle
   S.part_rows = ceil_div(ceil_div(S.R, S.nparts), 32) * 32;
-  const size_t fixed = cc_fixed_smem(S.R, lp, CTAS * S.nparts);
-  if (fixed + 16384 > CC_SMEM_BUDGET) return 0;
+  const size_t fixed = cc_fixed_smem(S.R, lp, CC_CTAS * S.nparts);
+  if (fixed + 16384 > CC_SMEM_BUDGET) return p;
   S.edge_cap = (int)((CC_SMEM_BUDGET - fixed) / 8);
-  const size_t smem = fixed + (size_t)S.edge_cap * 8;
-  const void* kern = nit == 1   ? (const void*)cg_cluster_kernel<1, CTAS, THREADS>
-                     : nit == 2 ? (const void*)cg_cluster_kernel<2, CTAS, THREADS>
-                     : nit == 3 ? (const void*)cg_cluster_kernel<3, CTAS, THREADS>
-                                : (const void*)cg_cluster_kernel<4, CTAS, THREADS>;
+  p.smem = fixed + (size_t)S.edge_cap * 8;
+  p.nit = nit;
+  return p;
+}
+
+}  // namespace
+
+bool cg_cluster_fits(int m, int lp) { return cluster_plan(m, lp).nit > 0; }
+
+int cg_cluster_launch(const CgParams& P, cudaStream_t st) {
+  static const void* const kernels[CC_MAX_NIT] = {(const void*)cg_cluster_kernel<1>, (const void*)cg_cluster_kernel<2>,
+                                                  (const void*)cg_cluster_kernel<3>, (const void*)cg_cluster_kernel<4>};
+  CcPlan pl = cluster_plan(P.m, P.lp);
+  const void* kern = kernels[pl.nit - 1];
   GLL_CUDA_CHECK(set_max_dynamic_smem_once(kern, (int)CC_SMEM_BUDGET));
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(CTAS);
-  cfg.blockDim = dim3(THREADS);
-  cfg.dynamicSmemBytes = smem;
+  cfg.gridDim = dim3(CC_CTAS);
+  cfg.blockDim = dim3(CC_THREADS);
+  cfg.dynamicSmemBytes = pl.smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CTAS;
+  attr[0].val.clusterDim.x = CC_CTAS;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   CgParams Pc = P;
   unsigned long long* trace = (unsigned long long*)cg_get_trace();
-  void* args[] = {&Pc, &S, &trace};
+  void* args[] = {&Pc, &pl.S, &trace};
   GLL_PROF(KID_CG, st);
   GLL_CUDA_CHECK(cudaLaunchKernelExC(&cfg, kern, args));
-  return 1;
-}
-
-}  // namespace
-
-// 1: the solve was taken; 0: the system is not of this kind (caller falls through to the other kernels); < 0: error
-int cg_cluster_try(const CgParams& P, cudaStream_t st) {
-  if (P.m < 64 || P.m > 2048) return 0;  // below 64 rows there is nothing to share
-  // (256 / 320 / 384 threads per CTA measured the same at C2, 2.95-3.2 us per iteration; the same item layout on ONE CTA: 3.8 us
-  //  with 512 threads, 5.0 us with 1024 (spills at 64 registers) -- an iteration is ~450 mostly dependent instructions per warp,
-  //  and what the cluster buys is a shorter chain per warp, not bandwidth)
-  return cc_launch<8, 320>(P, st);
+  return GLL_OK;
 }
 
 }  // namespace gll

@@ -19,8 +19,8 @@
 //     reads all G x 3l partials with coalesced loads and adds them in the same fixed order, so all CTAs take identical
 //     branches and the result is bit-reproducible (no floating-point atomics).
 //   * the SpMV is bound by the L1TEX wavefront rate (one 128-byte line per gathered row of u: ~2 us for the 2.5 k gathers
-//     of a CTA), so it issues exactly one gather per edge and nothing else: rows are cut into SEGMENTS of 8 edges
-//     (built once per solve in shared memory), a thread owns one (segment, class quad) and has its 8 loads in flight at
+//     of a CTA), so it issues exactly one gather per edge and nothing else: rows are cut into SEGMENTS of 10 edges
+//     (built once per solve in shared memory), a thread owns one (segment, class quad) and has its 10 loads in flight at
 //     once -- no idle lanes for short rows, no tail for hub rows (degree 91 against a mean of 26) -- and u rows of 48
 //     bytes are stored with a 64-byte stride so that no gather straddles a line.  Segment sums are added per row in a
 //     second, shared-memory-only pass.
@@ -38,7 +38,7 @@ constexpr int CR_WARPS = CR_THREADS / 32;
 // Edges per segment = independent gathers in flight per thread.  10 makes the C4-size system (97 rows x ~26 edges x 3
 // class quads per CTA) exactly one round of <= 1024 (segment, quad) tasks; with 8 it is 1092 tasks = a second, nearly
 // empty round that costs a full L2 round trip.
-constexpr int CR_SEG_DEFAULT = 10;
+constexpr int CR_SEG = 10;
 constexpr size_t CR_SMEM_BUDGET = 200 * 1024;
 constexpr int CR_MAX_GRID = 160;  // the sum over CTAs keeps CR_MAX_GRID / 32 loads per lane in flight
 
@@ -53,12 +53,6 @@ struct CrParams {
   unsigned long long* trace;  // debug: [grid][16 passes][16 phases] clock64 stamps (NULL = off)
 };
 
-__device__ __forceinline__ float4 ldcg4(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
 __device__ __forceinline__ void red_release_add_u32(unsigned* p, unsigned v) {
   asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
@@ -74,14 +68,6 @@ __device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned target)
   }
   __syncthreads();
 }
-
-__device__ __forceinline__ void fma4(float4& acc, float w, const float4& v) {
-  acc.x = fmaf(w, v.x, acc.x);
-  acc.y = fmaf(w, v.y, acc.y);
-  acc.z = fmaf(w, v.z, acc.z);
-  acc.w = fmaf(w, v.w, acc.w);
-}
-__device__ __forceinline__ float4 scale4(const float4& a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
 
 // debug timeline (TRACE instantiation only).  BAR.SYNC is deferred-blocking (a clock read right behind it can run before the barrier releases), so
 // the stamp first touches shared memory, which waits for the barrier.
@@ -130,17 +116,10 @@ __device__ __forceinline__ void write_stats(const CgParams& P, const double* red
   double mx_all = 0.0;
 #pragma unroll 1
   for (int c = 0; c < lp; ++c) mx_all = fmax(mx_all, red[2 * lp + c]);
-  if (P.iters_out) *P.iters_out = iter;
-  if (P.resid_out) *P.resid_out = sqrtf((float)mx_all);
-  if (P.status_out) {
-    int st = 0;
-    if (bad) st |= GLL_STATUS_NONFINITE;
-    if (!bad && !(mx_all <= tol2)) st |= GLL_STATUS_CG_NOT_CONVERGED;
-    if (st) atomicOr(P.status_out, st);
-  }
+  cg_write_stats(P, iter, sqrtf((float)mx_all), bad, mx_all, tol2);
 }
 
-template <bool SINGLE, int CR_SEG, bool TRACE>
+template <bool SINGLE, bool TRACE>
 __global__ void __launch_bounds__(CR_THREADS, 1) cg_resident_kernel(CrParams R) {
   extern __shared__ __align__(16) unsigned char sm_raw[];
   const CgParams& P = R.cg;
@@ -371,25 +350,12 @@ __global__ void __launch_bounds__(CR_THREADS, 1) cg_resident_kernel(CrParams R) 
     if (tid < lp) {
       const int c = tid;
       const double tol2 = ctrl->tol2;
-      // quotients in fp32 (alpha and beta are fp32 anyway); the cancellation-prone difference in fp64
       const double g_new = red[c], d_new = red[lp + c], rr = red[2 * lp + c];
       bad = (!(rr == rr) || rr > 1.0e300) ? 1 : 0;
       float al = 0.f, be = 0.f;
       if (!frozen[c] && rr > tol2) {  // columns that broke down are frozen for good
         live = 1;
-        const float bb = (iter == 0) ? 0.f : (float)g_new * inv_g_old[c];
-        const double den = d_new - (double)bb * g_new * (double)inv_a_old[c];
-        if (den > 0.0 && g_new > 0.0) {
-          // approximate reciprocals (MUFU.RCP, deterministic): alpha and beta only have to be the SAME numbers in every
-          // CTA and in the x and r updates, their last bits do not matter to CG
-          const float rg = __fdividef(1.f, (float)g_new);
-          al = __fdividef((float)g_new, (float)den);
-          be = bb;
-          inv_a_old[c] = (float)den * rg;
-          inv_g_old[c] = rg;
-        } else {
-          frozen[c] = 1;  // breakdown (rounding at the fp32 floor): stop moving this column
-        }
+        cg_column_step(g_new, d_new, iter == 0, inv_g_old[c], inv_a_old[c], frozen[c], al, be);
       }
       alpha[c] = al;
       beta[c] = be;
@@ -420,10 +386,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) cg_resident_kernel(CrParams R) 
       float4 x4 = *reinterpret_cast<const float4*>(xs + o), r4 = *reinterpret_cast<const float4*>(rs + o);
       float4 p4 = *reinterpret_cast<const float4*>(ps + o), s4 = *reinterpret_cast<const float4*>(ss + o);
       const float4 w4 = *reinterpret_cast<const float4*>(ws + o);
-      p4.x = fmaf(be.x, p4.x, r4.x * di); p4.y = fmaf(be.y, p4.y, r4.y * di); p4.z = fmaf(be.z, p4.z, r4.z * di); p4.w = fmaf(be.w, p4.w, r4.w * di);
-      s4.x = fmaf(be.x, s4.x, w4.x); s4.y = fmaf(be.y, s4.y, w4.y); s4.z = fmaf(be.z, s4.z, w4.z); s4.w = fmaf(be.w, s4.w, w4.w);
-      x4.x = fmaf(al.x, p4.x, x4.x); x4.y = fmaf(al.y, p4.y, x4.y); x4.z = fmaf(al.z, p4.z, x4.z); x4.w = fmaf(al.w, p4.w, x4.w);
-      r4.x = fmaf(-al.x, s4.x, r4.x); r4.y = fmaf(-al.y, s4.y, r4.y); r4.z = fmaf(-al.z, s4.z, r4.z); r4.w = fmaf(-al.w, s4.w, r4.w);
+      cg_cg_update(al, be, scale4(r4, di), w4, x4, r4, p4, s4);
       *reinterpret_cast<float4*>(xs + o) = x4;
       *reinterpret_cast<float4*>(rs + o) = r4;
       *reinterpret_cast<float4*>(ps + o) = p4;
@@ -460,21 +423,17 @@ struct CrPlan {
   size_t smem;
 };
 
-CrPlan plan(int m, int lp, int seg) {
+CrPlan plan(int m, int lp) {
   CrPlan p;
   p.ok = 0;
   const int sms = device_info().sms;
-  const size_t per_seg = align_up(sizeof(int) * seg + sizeof(float) * seg + sizeof(float) * lp, 16);
+  const size_t per_seg = align_up(sizeof(int) * CR_SEG + sizeof(float) * CR_SEG + sizeof(float) * lp, 16);
   int grid;
   // whole system in one SM (no grid-wide exchange at all) when the vectors and ~5 segments per row fit
   if (fixed_smem(m, lp, true) + per_seg * 5 * (size_t)m <= CR_SMEM_BUDGET * 3 / 4)
     grid = 1;
   else
     grid = max(2, min(min(sms, CR_MAX_GRID), ceil_div(m, 96)));
-  if (const char* e = getenv("GLL_B200_CG_GRID")) {  // debug: sweep the number of CTAs
-    const int g = atoi(e);
-    if (g >= 2 && g <= min(sms, CR_MAX_GRID) && grid > 1) grid = g;
-  }
   int rows_cap = ceil_div(m, grid);
   if (grid > 1 && fixed_smem(rows_cap, lp, false) + 4 * 1024 > CR_SMEM_BUDGET) {
     grid = min(sms, CR_MAX_GRID);
@@ -501,15 +460,10 @@ size_t cg_resident_ws_bytes(int m, int lp) {
   return align_up(sizeof(float) * (size_t)m * ustride_of(lp), 256) + align_up(sizeof(double) * 3 * (size_t)lp * sms, 256) + 256 + 256;
 }
 
-static int cg_seg() {
-  const char* e = getenv("GLL_B200_CG_SEG");  // debug: 8 or 10
-  return (e && atoi(e) == 8) ? 8 : CR_SEG_DEFAULT;
-}
+bool cg_resident_fits(int m, int lp) { return plan(m, lp).ok != 0; }
 
-int cg_resident_try(const CgParams& P, void* scratch, cudaStream_t st) {
-  const int seg = cg_seg();
-  const CrPlan pl = plan(P.m, P.lp, seg);
-  if (!pl.ok) return 0;
+int cg_resident_launch(const CgParams& P, void* scratch, cudaStream_t st) {
+  const CrPlan pl = plan(P.m, P.lp);
   CrParams R;
   R.cg = P;
   Carver cv(scratch, cg_resident_ws_bytes(P.m, P.lp));
@@ -522,9 +476,9 @@ int cg_resident_try(const CgParams& P, void* scratch, cudaStream_t st) {
   R.rows_cap = pl.rows_cap;
   R.seg_cap = pl.seg_cap;
   R.trace = g_cg_trace;
-  const void* k_single = seg == 8 ? (const void*)cg_resident_kernel<true, 8, false> : (const void*)cg_resident_kernel<true, 10, false>;
-  const void* k_multi = seg == 8 ? (const void*)cg_resident_kernel<false, 8, false> : (const void*)cg_resident_kernel<false, 10, false>;
-  if (R.trace != nullptr) k_multi = (const void*)cg_resident_kernel<false, 10, true>;  // debug timeline (gll_debug_cg_trace)
+  const void* k_single = (const void*)cg_resident_kernel<true, false>;
+  const void* k_multi = (const void*)cg_resident_kernel<false, false>;
+  if (R.trace != nullptr) k_multi = (const void*)cg_resident_kernel<false, true>;  // debug timeline (gll_debug_cg_trace)
   GLL_CUDA_CHECK(set_max_dynamic_smem_once(k_single, (int)CR_SMEM_BUDGET));
   GLL_CUDA_CHECK(set_max_dynamic_smem_once(k_multi, (int)CR_SMEM_BUDGET));
   void* args[] = {&R};
@@ -538,7 +492,7 @@ int cg_resident_try(const CgParams& P, void* scratch, cudaStream_t st) {
     // cooperative launch: all CTAs are co-resident, which the grid barrier relies on
     GLL_CUDA_CHECK(cudaLaunchCooperativeKernel(k_multi, dim3(pl.grid), dim3(CR_THREADS), args, pl.smem, st));
   }
-  return 1;
+  return GLL_OK;
 }
 
 }  // namespace gll

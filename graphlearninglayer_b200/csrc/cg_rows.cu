@@ -65,7 +65,6 @@ RowsState carve(void* ws, size_t ws_bytes, int rows_local, int lp) {
 }
 
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
-__device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 
 // ---- peer-memory mode ----
 constexpr int MAX_PEERS = 8;
@@ -147,28 +146,6 @@ rows_init_kernel(const float* __restrict__ diag, const float* __restrict__ rhs, 
   if (PR.world > 0) publish_epoch(PR, 0, epoch, S.ticket2);
 }
 
-// sum over the neighbour-slot index s of lane = s*Q + q; valid on lanes < Q
-__device__ __forceinline__ float4 reduce_slots(float4 a, int s, int S, int Q) {
-  int top = 1;
-  while (top < S) top <<= 1;
-  int span = S;
-  for (int st = top >> 1; st >= 1; st >>= 1) {
-    float4 o;
-    o.x = __shfl_down_sync(FULL, a.x, st * Q);
-    o.y = __shfl_down_sync(FULL, a.y, st * Q);
-    o.z = __shfl_down_sync(FULL, a.z, st * Q);
-    o.w = __shfl_down_sync(FULL, a.w, st * Q);
-    if (s < st && s + st < span) {
-      a.x += o.x;
-      a.y += o.y;
-      a.z += o.z;
-      a.w += o.w;
-    }
-    span = min(span, st);
-  }
-  return a;
-}
-
 // w = A u on the rank's rows; lane = (neighbour slot s, class quad q), 128-bit gathers of u_j, four gathers in flight
 __global__ void __launch_bounds__(RW_THREADS)
 rows_spmv_kernel(const int* __restrict__ ptr, const int* __restrict__ col, const float* __restrict__ val, const float* __restrict__ diag,
@@ -210,7 +187,7 @@ rows_spmv_kernel(const int* __restrict__ ptr, const int* __restrict__ col, const
         }
       }
     }
-    a = reduce_slots(a, s, NS, Q);
+    a = reduce_over_s(a, s, NS, Q);
     if (lane < Q) {
       const size_t lo = (size_t)(i - row_lo) * lp + 4 * lane;
       const float4 ui = ld4(u_full + (size_t)i * lp + 4 * lane);
@@ -361,10 +338,7 @@ rows_update_kernel(const float* __restrict__ diag, int lp, int row_lo, int row_h
     const float4 al = ld4(alpha + 4 * q), be = ld4(beta + 4 * q);
     const float4 u = ld4(u_full + go), w = ld4(S.w + lo);
     float4 p = ld4(S.p + lo), sv = ld4(S.s + lo), xv = ld4(x + go), r = ld4(S.r + lo);
-    p.x = fmaf(be.x, p.x, u.x); p.y = fmaf(be.y, p.y, u.y); p.z = fmaf(be.z, p.z, u.z); p.w = fmaf(be.w, p.w, u.w);
-    sv.x = fmaf(be.x, sv.x, w.x); sv.y = fmaf(be.y, sv.y, w.y); sv.z = fmaf(be.z, sv.z, w.z); sv.w = fmaf(be.w, sv.w, w.w);
-    xv.x = fmaf(al.x, p.x, xv.x); xv.y = fmaf(al.y, p.y, xv.y); xv.z = fmaf(al.z, p.z, xv.z); xv.w = fmaf(al.w, p.w, xv.w);
-    r.x = fmaf(-al.x, sv.x, r.x); r.y = fmaf(-al.y, sv.y, r.y); r.z = fmaf(-al.z, sv.z, r.z); r.w = fmaf(-al.w, sv.w, r.w);
+    cg_cg_update(al, be, u, w, xv, r, p, sv);
     const float dinv = 1.f / __ldg(diag + i);
     st4(S.p + lo, p);
     st4(S.s + lo, sv);

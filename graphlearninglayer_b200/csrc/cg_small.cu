@@ -21,14 +21,6 @@ constexpr int CS_WARPS = CS_THREADS / 32;
 constexpr int CS_MAX_NIT = 4;
 constexpr size_t CS_SMEM_BUDGET = 160 * 1024;
 
-__device__ __forceinline__ float4 f4zero() { return make_float4(0.f, 0.f, 0.f, 0.f); }
-__device__ __forceinline__ float4 f4scale(const float4& a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
-__device__ __forceinline__ void f4fma(float4& acc, float w, const float4& v) {
-  acc.x = fmaf(w, v.x, acc.x);
-  acc.y = fmaf(w, v.y, acc.y);
-  acc.z = fmaf(w, v.z, acc.z);
-  acc.w = fmaf(w, v.w, acc.w);
-}
 __device__ __forceinline__ float4 f4mul(const float4& a, const float4& b) { return make_float4(a.x * b.x, a.y * b.y, a.z * b.z, a.w * b.w); }
 __device__ __forceinline__ float4 f4butterfly(float4 a) {
 #pragma unroll
@@ -88,10 +80,10 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
     on[k] = quad[k] < Q && row[k] < m;
     dg[k] = on[k] ? __ldg(P.diag + row[k]) : 1.f;
     dinv[k] = on[k] ? 1.f / dg[k] : 0.f;
-    r[k] = on[k] ? cg_load_rhs4(P, row[k], quad[k]) : f4zero();
-    x[k] = p[k] = s[k] = w[k] = f4zero();
+    r[k] = on[k] ? cg_load_rhs4(P, row[k], quad[k]) : zero4();
+    x[k] = p[k] = s[k] = w[k] = zero4();
     uoff[k] = (quad[k] < Q) ? 4 * quad[k] : 0;
-    if (quad[k] < Q) *reinterpret_cast<float4*>(us + (size_t)row[k] * lp + 4 * quad[k]) = f4scale(r[k], dinv[k]);
+    if (quad[k] < Q) *reinterpret_cast<float4*>(us + (size_t)row[k] * lp + 4 * quad[k]) = scale4(r[k], dinv[k]);
   }
   // per-column CG scalars live in warp 0: lane owns columns lane, lane + 32, ...
   constexpr int CPL = CG_MAX_LP / 32;
@@ -120,7 +112,7 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
     {
       float4 a[NIT];
 #pragma unroll
-      for (int k = 0; k < NIT; ++k) a[k] = f4zero();
+      for (int k = 0; k < NIT; ++k) a[k] = zero4();
       // no branches inside the edge loop (items beyond the last quad gather quad 0 and are discarded below), and one
       // copy per address space of the CSR: otherwise every gather re-derives the shared-memory window (S2UR in the loop)
       auto walk = [&](const int* __restrict__ cj, const float* __restrict__ cv) {
@@ -132,7 +124,7 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
           const float we = cv[e];
           const uint32_t uj = us_s + (uint32_t)(cj[e] * lp) * 4u;
 #pragma unroll
-          for (int k = 0; k < NIT; ++k) f4fma(a[k], we, lds128(uj + 4u * (uint32_t)uoff[k]));
+          for (int k = 0; k < NIT; ++k) fma4(a[k], we, lds128(uj + 4u * (uint32_t)uoff[k]));
         }
       };
       if (row[0] < m) {
@@ -145,10 +137,10 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
 #pragma unroll
       for (int k = 0; k < NIT; ++k) {
         if (quad[k] < Q) {
-          const float4 u4 = f4scale(r[k], dinv[k]);
+          const float4 u4 = scale4(r[k], dinv[k]);
           w[k] = make_float4(fmaf(dg[k], u4.x, -a[k].x), fmaf(dg[k], u4.y, -a[k].y), fmaf(dg[k], u4.z, -a[k].z),
                              fmaf(dg[k], u4.w, -a[k].w));
-          if (!on[k]) w[k] = f4zero();
+          if (!on[k]) w[k] = zero4();
           const size_t o = (size_t)quad[k] * rows_pad + row[k];
           prod[o] = f4mul(r[k], u4);
           prod[(size_t)Q * rows_pad + o] = f4mul(w[k], u4);
@@ -164,11 +156,11 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
 #pragma unroll 1
     for (int job = warp; job < 3 * Q; job += CS_WARPS) {
       const float4* src = prod + (size_t)job * rows_pad;
-      float4 t0 = f4zero(), t1 = f4zero();
+      float4 t0 = zero4(), t1 = zero4();
 #pragma unroll 4
       for (int i = lane; i < rows_pad; i += 64) {
         const float4 v0 = src[i];
-        const float4 v1 = (i + 32 < rows_pad) ? src[i + 32] : f4zero();
+        const float4 v1 = (i + 32 < rows_pad) ? src[i + 32] : zero4();
         t0.x += v0.x; t0.y += v0.y; t0.z += v0.z; t0.w += v0.w;
         t1.x += v1.x; t1.y += v1.y; t1.z += v1.z; t1.w += v1.w;
       }
@@ -209,22 +201,8 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
           if (c < lp) {
             const float g_new = red[c], d_new = red[lp + c];
             float al = 0.f, be = 0.f;
-            if (!frozen[j] && rrc[j] > tol2) {
-              const float bb = (iter == 0) ? 0.f : g_new * inv_g_old[j];
-              // the cancellation-prone difference in fp64, the quotients in fp32 (alpha and beta are fp32 anyway)
-              const double den = (double)d_new - (double)bb * (double)g_new * (double)inv_a_old[j];
-              if (den > 0.0 && g_new > 0.f) {
-                // approximate reciprocals (MUFU.RCP, deterministic), as in cg_resident.cu: the last bits of alpha / beta do
-                // not matter to CG, three IEEE divisions in this one-warp section cost ~0.2 us per pass
-                const float rg = __fdividef(1.f, g_new);
-                al = __fdividef(g_new, (float)den);
-                be = bb;
-                inv_a_old[j] = (float)den * rg;
-                inv_g_old[j] = rg;
-              } else {
-                frozen[j] = true;  // breakdown at the fp32 floor: stop moving this column
-              }
-            }
+            // (approximate reciprocals: three IEEE divisions in this one-warp section cost ~0.2 us per pass)
+            if (!frozen[j] && rrc[j] > tol2) cg_column_step(g_new, d_new, iter == 0, inv_g_old[j], inv_a_old[j], frozen[j], al, be);
             alpha[c] = al;
             beta[c] = be;
           }
@@ -242,15 +220,8 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
         const float4 al = *reinterpret_cast<const float4*>(alpha + 4 * quad[k]);
         const float4 be = *reinterpret_cast<const float4*>(beta + 4 * quad[k]);
         const float di = dinv[k];
-        p[k].x = fmaf(be.x, p[k].x, r[k].x * di); p[k].y = fmaf(be.y, p[k].y, r[k].y * di);
-        p[k].z = fmaf(be.z, p[k].z, r[k].z * di); p[k].w = fmaf(be.w, p[k].w, r[k].w * di);
-        s[k].x = fmaf(be.x, s[k].x, w[k].x); s[k].y = fmaf(be.y, s[k].y, w[k].y);
-        s[k].z = fmaf(be.z, s[k].z, w[k].z); s[k].w = fmaf(be.w, s[k].w, w[k].w);
-        x[k].x = fmaf(al.x, p[k].x, x[k].x); x[k].y = fmaf(al.y, p[k].y, x[k].y);
-        x[k].z = fmaf(al.z, p[k].z, x[k].z); x[k].w = fmaf(al.w, p[k].w, x[k].w);
-        r[k].x = fmaf(-al.x, s[k].x, r[k].x); r[k].y = fmaf(-al.y, s[k].y, r[k].y);
-        r[k].z = fmaf(-al.z, s[k].z, r[k].z); r[k].w = fmaf(-al.w, s[k].w, r[k].w);
-        *reinterpret_cast<float4*>(us + (size_t)row[k] * lp + 4 * quad[k]) = f4scale(r[k], di);
+        cg_cg_update(al, be, scale4(r[k], di), w[k], x[k], r[k], p[k], s[k]);
+        *reinterpret_cast<float4*>(us + (size_t)row[k] * lp + 4 * quad[k]) = scale4(r[k], di);
       }
     }
     __syncthreads();
@@ -263,54 +234,48 @@ __global__ void __launch_bounds__(CS_THREADS, 1) cg_small_kernel(CgParams P, int
       *reinterpret_cast<float4*>(P.x + (size_t)row[k] * lp + 4 * quad[k]) = x[k];
       cg_store_copy4(P, row[k], quad[k], x[k]);
     }
-  if (tid == 0) {  // warp 0 holds the stop state
-    if (P.iters_out) *P.iters_out = iter;
-    if (P.resid_out) *P.resid_out = sqrtf(mx_all);
-    if (P.status_out) {
-      int st = 0;
-      if (bad) st |= GLL_STATUS_NONFINITE;
-      if (!bad && !(mx_all <= tol2)) st |= GLL_STATUS_CG_NOT_CONVERGED;
-      if (st) atomicOr(P.status_out, st);
-    }
-  }
+  if (tid == 0) cg_write_stats(P, iter, sqrtf(mx_all), bad, mx_all, tol2);  // warp 0 holds the stop state
 }
 
-size_t small_fixed_smem(int m, int lp, int rows_pad, int nit) {
+struct CsPlan {
+  int nit;  // items per thread; 0: the system does not fit
+  int rows_pad, csr_cap;
+  size_t smem;
+};
+
+CsPlan small_plan(int m, int lp) {
+  CsPlan p = {};
+  if (m > CS_THREADS) return p;
+  p.rows_pad = 32;  // a power of two, so that it divides the CTA size: every thread's items then share their row
+  while (p.rows_pad < m) p.rows_pad <<= 1;
   const int Q = lp >> 2;
-  (void)nit;
-  return sizeof(float) * (size_t)rows_pad * lp + 16 * (size_t)3 * Q * rows_pad + sizeof(float) * 5 * (size_t)lp + 16 +
-         sizeof(int) * ((size_t)m + 1) + 64;
+  const int nit = (int)(((long long)Q * p.rows_pad + CS_THREADS - 1) / CS_THREADS);
+  if (nit > CS_MAX_NIT) return p;
+  const size_t fixed = sizeof(float) * (size_t)p.rows_pad * lp + 16 * (size_t)3 * Q * p.rows_pad + sizeof(float) * 5 * (size_t)lp + 16 +
+                       sizeof(int) * ((size_t)m + 1) + 64;
+  if (fixed + 4096 > CS_SMEM_BUDGET) return p;
+  p.csr_cap = (int)((CS_SMEM_BUDGET - fixed) / 8);
+  p.smem = fixed + (size_t)p.csr_cap * 8;
+  p.nit = nit;
+  return p;
 }
 
 }  // namespace
 
-// 1: the solve was taken; 0: the system is not "small" (caller falls through to the other kernels); < 0: error
-int cg_small_try(const CgParams& P, cudaStream_t st) {
-  const int lp = P.lp, Q = lp >> 2;
-  if (P.m > CS_THREADS) return 0;
-  int rows_pad = 32;  // a power of two, so that it divides the CTA size: every thread's items then share their row
-  while (rows_pad < P.m) rows_pad <<= 1;
-  const long long items = (long long)Q * rows_pad;
-  const int nit = (int)((items + CS_THREADS - 1) / CS_THREADS);
-  if (nit > CS_MAX_NIT) return 0;
-  const size_t fixed = small_fixed_smem(P.m, lp, rows_pad, nit);
-  if (fixed + 4096 > CS_SMEM_BUDGET) return 0;
-  const int csr_cap = (int)((CS_SMEM_BUDGET - fixed) / 8);
-  const size_t smem = fixed + (size_t)csr_cap * 8;
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)cg_small_kernel<1>, (int)CS_SMEM_BUDGET));
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)cg_small_kernel<2>, (int)CS_SMEM_BUDGET));
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)cg_small_kernel<3>, (int)CS_SMEM_BUDGET));
-  GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)cg_small_kernel<4>, (int)CS_SMEM_BUDGET));
+bool cg_small_fits(int m, int lp) { return small_plan(m, lp).nit > 0; }
+
+int cg_small_launch(const CgParams& P, cudaStream_t st) {
+  static const void* const kernels[CS_MAX_NIT] = {(const void*)cg_small_kernel<1>, (const void*)cg_small_kernel<2>,
+                                                  (const void*)cg_small_kernel<3>, (const void*)cg_small_kernel<4>};
+  CsPlan pl = small_plan(P.m, P.lp);
+  const void* kern = kernels[pl.nit - 1];
+  GLL_CUDA_CHECK(set_max_dynamic_smem_once(kern, (int)CS_SMEM_BUDGET));
+  CgParams Pc = P;
   unsigned long long* trace = (unsigned long long*)cg_get_trace();
+  void* args[] = {&Pc, &pl.rows_pad, &pl.csr_cap, &trace};
   GLL_PROF(KID_CG, st);
-  switch (nit) {
-    case 1: cg_small_kernel<1><<<1, CS_THREADS, smem, st>>>(P, rows_pad, csr_cap, trace); break;
-    case 2: cg_small_kernel<2><<<1, CS_THREADS, smem, st>>>(P, rows_pad, csr_cap, trace); break;
-    case 3: cg_small_kernel<3><<<1, CS_THREADS, smem, st>>>(P, rows_pad, csr_cap, trace); break;
-    default: cg_small_kernel<4><<<1, CS_THREADS, smem, st>>>(P, rows_pad, csr_cap, trace); break;
-  }
-  GLL_LAUNCH_CHECK();
-  return 1;
+  GLL_CUDA_CHECK(cudaLaunchKernel(kern, dim3(1), dim3(CS_THREADS), args, pl.smem, st));
+  return GLL_OK;
 }
 
 }  // namespace gll

@@ -169,25 +169,53 @@ int batched_knn_run(const float* X, int B, int n, int d, int k, int k_lab, const
 size_t weights_ws_bytes(int n, int k);
 size_t graph_weights_ws_bytes(int n, int k);
 
-// optional fused conversions of the layer: rhs_src = the caller's [m][l] right-hand side (rhs_kind 1 fp32 / 2 fp64; `rhs` is then
-// scratch), x_copy = an extra [m][l] copy of the solution (fp64 if x_copy_f64)
-struct CgIo {
-  const void* rhs_src;
-  int rhs_kind;
-  void* x_copy;
-  int x_copy_f64;
-  const void* rhs_scale;  // optional device scalar multiplied into rhs_src (fp64 if rhs_scale_f64)
-  int rhs_scale_f64;
-  float uu_degree_hint;   // expected off-diagonal entries per row of the system (0: unknown) -- picks the minibatch kernel
+// One CG solve (cg.cu).  Callers value-initialise it ({}) and set what they use by name.
+struct CgSolve {
+  // the system A = diag - offdiag(val) on m rows (compact CSR), rhs and x [m][lp] with lp = padded_classes(l)
+  const int* ptr;
+  const int* col;
+  const float* val;
+  const float* diag;
+  const float* rhs;
+  float* x;
+  unsigned* ext_counter;  // optional [2], zero on entry: the on-chip kernel's grid barrier and exit ticket.  The kernel leaves
+                          // both zero again, so one memset per forward (the info block) serves the forward AND the adjoint solve
+  int* iters_out;         // device pointers, each may be NULL
+  float* resid_out;
+  int* status_out;
+  // Fused conversions of the layer (the on-chip kernels do them in place; cg_run runs separate kernels for the others):
+  const void* rhs_src;    // if set: the right-hand side is this [m][l] array (rhs_kind 1: fp32, 2: fp64); `rhs` is then scratch
+  void* x_copy;           // if set: the solution is also written as an [m][l] array (fp64 if x_copy_f64, else fp32)
+  const void* rhs_scale;  // optional device scalar (fp64 if rhs_scale_f64, else fp32) multiplied into rhs_src: the upstream gradient
+                          // of a loss head whose d loss / d pred is rhs_src (losses.py: LaplaceLearningCELoss)
+  int m, l, max_iter;
+  float tol;  // > 0: absolute; < 0: |tol| times the largest column 2-norm of rhs
+  int rhs_kind, x_copy_f64, rhs_scale_f64;
+  float uu_degree_hint;  // expected off-diagonal entries per row of the system (0: unknown) -- picks the minibatch kernel
   // optional row mask of T trials x mask_cols columns (mask_col0: this solve's first column among them): A p is zeroed at (row i,
   // trial t) where mask_slot[i T + t] >= 0.  A masked solve always runs the streaming kernel.
   const int* mask_slot;
   int mask_trials, mask_cols, mask_col0;
 };
-int cg_run(const int* uu_ptr, const int* uu_col, const float* uu_val, const float* diag, const float* rhs, int m,
-           int l, float tol, int max_iter, float* x, int* iters_out, float* resid_out, int* status_out, void* ws,
-           size_t ws_bytes, cudaStream_t st, unsigned* ext_counter = nullptr, const CgIo* io = nullptr);
+int cg_run(const CgSolve& S, void* ws, size_t ws_bytes, cudaStream_t st);
+// the unlabeled system of B with right-hand side B.rhs and the barrier words of B.info (which are zeroed with the info block)
+inline CgSolve cg_system(const GraphBufs& B, int m, int l, float tol, int max_iter) {
+  CgSolve S{};
+  S.ptr = B.uu_ptr;
+  S.col = B.uu_col;
+  S.val = B.uu_val;
+  S.diag = B.diag;
+  S.m = m;
+  S.rhs = B.rhs;
+  S.l = l;
+  S.tol = tol;
+  S.max_iter = max_iter;
+  S.ext_counter = (unsigned*)(B.info + GLL_INFO_CG_BARRIER);
+  return S;
+}
 size_t cg_ws_bytes(int m, int l);
+// the kernel cg_run takes for a system of m rows and lp <= CG_MAX_LP padded class columns: GLL_CG_KERNEL_*
+int cg_pick(int m, int lp, float uu_degree_hint, bool masked);
 
 // row-partitioned CG (cg_rows.cu): stage launchers.  peers == NULL: the host runs the NCCL collectives between them;
 // otherwise the exchanges are fused into the kernels over peer memory (epoch = flag value of this stage, see cg_rows.cu)

@@ -489,17 +489,26 @@ int eval_run(const float* X, const float* Y, int B, int n, int d, int k, int l, 
   if (rc) return rc;
   float* x0 = G.ut + (size_t)K * u.P.lp;
   float* corr = G.wt;  // the adjoint's region, free in an evaluation
-  unsigned* barrier = (unsigned*)(info + GLL_INFO_CG_BARRIER);  // zeroed with info, rewound by the kernels
   // No sparsity hint (0): the evaluation system is never routed to the cluster kernel.  No status pointer either: an inner solve
   // that stops at the fp32 floor is not a failure -- the fp64 rounds decide convergence.  B graphs are one block-diagonal system:
   // every CG solves them together, with step lengths shared by the graphs (per class column).
-  rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, x0,
-              info + GLL_INFO_CG_ITERS_FWD, (float*)(info + GLL_INFO_CG_RESID_FWD), nullptr, u.ws, u.ws_bytes, st, barrier, nullptr);
+  CgSolve S = cg_system(G, m, l, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter);
+  S.x = x0;
+  S.iters_out = info + GLL_INFO_CG_ITERS_FWD;
+  S.resid_out = (float*)(info + GLL_INFO_CG_RESID_FWD);
+  rc = cg_run(S, u.ws, u.ws_bytes, st);
   if (rc) return rc;
-  const CgIo io = {u.E.r, 2, nullptr, 0, u.E.scale, 1, 0.f};
+  CgSolve R = S;  // the correction of a refinement round
+  R.x = corr;
+  R.tol = -(float)GLL_LAPLACE_CG_RTOL;
+  R.resid_out = nullptr;
+  R.rhs_src = u.E.r;
+  R.rhs_kind = 2;
+  R.rhs_scale = u.E.scale;
+  R.rhs_scale_f64 = 1;
   return refine_rounds<UnionRows>(u.P, x0, corr, pred, u.E.xa, [&](int* iters) {
-    return cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, G.rhs, m, l, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, corr, iters, nullptr,
-                  nullptr, u.ws, u.ws_bytes, st, barrier, &io);
+    R.iters_out = iters;
+    return cg_run(R, u.ws, u.ws_bytes, st);
   }, st);
 }
 
@@ -538,16 +547,27 @@ int trials_run(const float* X, int n, int d, int k, const void* train_idx, int i
   P0.round = -1;
   rc = launch_refine<TrialRows>(P0, st);
   if (rc) return rc;
-  unsigned* barrier = (unsigned*)(info + GLL_INFO_CG_BARRIER);
-  CgIo io = {E.r, 2, nullptr, 0, nullptr, 0, 0.f, E.slot, T, u.P.lp, 0};
-  rc = cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, E.rhs, n, C, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter, E.x0,
-              info + GLL_INFO_CG_ITERS_FWD, (float*)(info + GLL_INFO_CG_RESID_FWD), nullptr, u.ws, u.ws_bytes, st, barrier, &io);
+  CgSolve S = cg_system(G, n, C, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter);
+  S.rhs = E.rhs;
+  S.x = E.x0;
+  S.iters_out = info + GLL_INFO_CG_ITERS_FWD;
+  S.resid_out = (float*)(info + GLL_INFO_CG_RESID_FWD);
+  S.rhs_src = E.r;
+  S.rhs_kind = 2;
+  S.mask_slot = E.slot;
+  S.mask_trials = T;
+  S.mask_cols = u.P.lp;
+  rc = cg_run(S, u.ws, u.ws_bytes, st);
   if (rc) return rc;
-  io.rhs_scale = E.scale;
-  io.rhs_scale_f64 = 1;
+  CgSolve R = S;  // the correction of a refinement round
+  R.x = E.corr;
+  R.tol = -(float)GLL_LAPLACE_CG_RTOL;
+  R.resid_out = nullptr;
+  R.rhs_scale = E.scale;
+  R.rhs_scale_f64 = 1;
   return refine_rounds<TrialRows>(u.P, E.x0, E.corr, E.xb, E.xa, [&](int* iters) {
-    return cg_run(G.uu_ptr, G.uu_col, G.uu_val, G.diag, E.rhs, n, C, -(float)GLL_LAPLACE_CG_RTOL, cg_max_iter, E.corr, iters, nullptr,
-                  nullptr, u.ws, u.ws_bytes, st, barrier, &io);
+    R.iters_out = iters;
+    return cg_run(R, u.ws, u.ws_bytes, st);
   }, st);
 }
 

@@ -179,6 +179,14 @@ int gll_cg_solve_hint(const int* uu_ptr, const int* uu_col, const float* uu_val,
                       const float* rhs, int m, int l, float tol, int max_iter, float* x, int* iters_out,
                       float* resid_out, int* status_out, void* workspace, size_t workspace_bytes, void* stream,
                       float uu_degree_hint);
+/* Host-only query (no GPU needed): the kernel gll_cg_solve_hint runs for m rows, 1 <= l <= 128 class columns and the hint,
+ * under the current GLL_B200_CG_PATH; GLL_ERR_ARG outside that range.  More than 128 columns are solved in chunks of 128, each
+ * picked on its own without the hint. */
+#define GLL_CG_KERNEL_STREAMING 0 /* vectors in global memory, any size */
+#define GLL_CG_KERNEL_RESIDENT 1  /* multi-CTA, vectors and matrix slices in shared memory */
+#define GLL_CG_KERNEL_SMALL 2     /* one CTA, up to 512 rows */
+#define GLL_CG_KERNEL_CLUSTER 3   /* one cluster of eight CTAs, 64 to 2048 rows, sparse systems */
+int gll_cg_kernel(int m, int l, float uu_degree_hint);
 
 /* K5+K6. Backward edge pass (GLL.py:104-159): G_ij = -<wt_i-wt_j, ut_i-ut_j>, gv = G*V, b_i = sum_j G_ij modV_ij
  * (auto only), dX_i = sum_j t_ij (x_i - x_j) with t_ij = gv_ij - [j==kappa(i)] b_i - [kappa(j)==i] b_j. */

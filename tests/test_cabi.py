@@ -109,3 +109,38 @@ def test_peer_table_matches_the_header(libmod):
     assert lib.gll_cg_rows_peer_mail_bytes() == 2 * 8 * 3 * 128 * 8  # [2 parities][8 ranks][3 dots x 128 columns] doubles
     assert lib.gll_ce_loss_workspace_bytes(512) == 0 and lib.gll_ce_loss_workspace_bytes(100000) > 0
     assert lib.gll_cg_rows_workspace_bytes(1000, 10) > 4 * 1000 * 12 * 4
+
+
+STREAMING, RESIDENT, SMALL, CLUSTER = 0, 1, 2, 3  # GLL_CG_KERNEL_*
+
+
+@pytest.mark.parametrize("path,cases", [
+    # (m, l, hint) -> kernel.  Unset or empty: cluster for 0 < hint <= 5 where it fits, else small where it fits, else resident
+    # where it fits, else streaming.
+    ("", [((63, 10, 1.4), SMALL), ((64, 10, 1.4), CLUSTER), ((2048, 10, 1.4), CLUSTER), ((2049, 10, 1.4), RESIDENT),
+          ((300, 10, 0.0), SMALL), ((300, 10, 5.0), CLUSTER), ((300, 10, 5.01), SMALL),
+          ((2048, 20, 1.4), CLUSTER), ((2048, 21, 1.4), RESIDENT),
+          ((512, 10, 0.0), SMALL), ((513, 10, 0.0), RESIDENT), ((512, 16, 0.0), SMALL), ((512, 17, 0.0), RESIDENT),
+          ((700, 40, 0.0), RESIDENT), ((3000, 10, 0.0), RESIDENT), ((1_000_000, 10, 0.0), STREAMING)]),
+    ("small", [((300, 10, 1.4), SMALL), ((512, 16, 1.4), SMALL), ((700, 10, 1.4), RESIDENT), ((1_000_000, 10, 0.0), STREAMING)]),
+    ("cluster", [((300, 10, 0.0), CLUSTER), ((63, 10, 0.0), SMALL), ((700, 40, 0.0), CLUSTER), ((700, 100, 0.0), RESIDENT),
+                 ((2049, 10, 0.0), RESIDENT), ((1_000_000, 10, 0.0), STREAMING)]),
+    ("resident", [((300, 10, 1.4), RESIDENT), ((64, 1, 0.0), RESIDENT), ((1_000_000, 10, 0.0), STREAMING)]),
+    ("streaming", [((300, 10, 1.4), STREAMING), ((3000, 10, 0.0), STREAMING)]),
+    ("other", [((300, 10, 1.4), RESIDENT), ((1_000_000, 10, 0.0), STREAMING)]),
+])
+def test_cg_kernel_table(libmod, monkeypatch, path, cases):
+    """gll_cg_kernel: which CG kernel a solve of m rows and l classes takes, under GLL_B200_CG_PATH, at the edges of each kernel.
+    lp = 4 ceil(l / 4) padded columns, Q = lp / 4 class quads.  The expected values follow from the size rules of the kernels:
+      cluster  64 <= m <= 2048; R = 32 ceil(ceil(m / 8) / 32) rows per CTA; Q R items over 320 threads, at most 4 per thread;
+               shared memory within 208 KB.  (2048, 20): R = 256, Q = 5, 1280 items = 4 per thread; (2048, 21): Q = 6, 5 per
+               thread.  (700, 40): R = 96, Q = 10, 3 per thread and 118 KB: it fits; (700, 100): Q = 25, 8 per thread.
+      small    m <= 512; rows padded to a power of two P >= 32; Q P items over 512 threads, at most 4 per thread; shared memory
+               within 160 KB.  (512, 16): Q = 4, 4 per thread and 134 KB; (512, 17): Q = 5, 5 per thread.
+      resident fits unless a CTA's rows (m over up to 148 SMs) overflow 200 KB of shared memory: 10^6 rows do.
+    "small" / "cluster" put that kernel first and ignore the hint; any other non-empty value skips both minibatch kernels."""
+    monkeypatch.setenv("GLL_B200_CG_PATH", path)
+    lib = libmod.lib
+    got = [lib.gll_cg_kernel(m, l, h) for (m, l, h), _ in cases]
+    assert got == [k for _, k in cases]
+    assert lib.gll_cg_kernel(100, 0, 0.0) == -1 and lib.gll_cg_kernel(100, 129, 0.0) == -1 and lib.gll_cg_kernel(0, 10, 0.0) == -1

@@ -399,13 +399,15 @@ def test_cg_vs_direct_solve(gll, monkeypatch, l, path):
     assert true_res < 5e-5  # fp32 storage of A and x bounds the true residual
 
 
-@pytest.mark.parametrize("m,l", [(64, 1), (65, 13), (511, 10), (2048, 3), (2048, 16), (700, 40)])
+@pytest.mark.parametrize("m,l", [(64, 1), (65, 13), (511, 10), (2048, 3), (2048, 16), (700, 40), (700, 100)])
 def test_cg_cluster_kernel_edge_sizes(gll, monkeypatch, m, l):
-    """The eight-CTA cluster kernel at the edges of its range (64 and 2048 rows, a last CTA with one row or none, one class, up to
-    four items per thread; 40 classes at 700 rows exceed its item budget and must fall through to another kernel).  Forced: the
-    stage entry point passes no sparsity hint and would pick the other kernels."""
+    """The eight-CTA cluster kernel (GLL_CG_KERNEL_CLUSTER = 3) at the edges of its range (64 and 2048 rows, a last CTA with one
+    row or none, one class, up to four items per thread; 40 classes at 700 rows are 3 items per thread).  100 classes at 700 rows
+    are 8 items per thread, beyond its budget: that system falls through to the multi-CTA kernel (GLL_CG_KERNEL_RESIDENT = 1).
+    Forced: the stage entry point passes no sparsity hint and would pick the other kernels."""
     _, _lib = gll
     monkeypatch.setenv("GLL_B200_CG_PATH", "cluster")
+    assert _lib.lib.gll_cg_kernel(m, l, 0.0) == (1 if (m, l) == (700, 100) else 3)
     X, Y, *_ = O.synth_inputs(31 + m + l, 120, m, 20, l, 1.5)
     f = O.forward(X, Y, 0.03, 1.0, solver="lu")
     x, iters, resid, status = run_cg(_lib, f.Luu, f.B, tol=1e-7)
