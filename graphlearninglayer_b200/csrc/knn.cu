@@ -10,7 +10,8 @@
 //                 (bit-symmetric in i,j), order by (distance, index), emit k entries with self in slot 0, and
 //                 PROVE completeness: every non-candidate has approximate distance >= L_i, so its true distance
 //                 is >= L_i - err; rows where that does not exceed the k-th exact distance are queued for
-//   fallback    : brute-force fp64 search for the queued rows only.
+//   fallback    : brute-force fp64 search for the queued rows only, one pass per 32 neighbours.
+// k in (33, 64] takes two candidate rounds of KC; the same re-rank kernel ranks both rounds' lists together (ROUNDS = 2).
 //
 // This file holds the fp32 SIMT Gram path (tiny graphs; any d, any alignment), the operand-split kernels, re-rank and
 // fallback, and the host code of every search.  The tcgen05/TMA Gram path (n >= 256, any d: rows are zero-padded to a multiple
@@ -380,6 +381,7 @@ knn_gemm_topk_kernel(const float* __restrict__ X, const float* __restrict__ sq, 
 namespace {
 
 constexpr int RERANK_WARPS = 4;
+constexpr int FB_WARPS = 8;
 
 template <bool VEC4>
 __device__ __forceinline__ double exact_d2(const float* __restrict__ xi_s, const float* __restrict__ xj, int d,
@@ -443,7 +445,121 @@ __device__ __forceinline__ double knn_err_bound(float err_coef, float sqi, const
   return (double)err_coef * ((double)sqi + sqm) + 2.0 * rterm * 1.000001;
 }
 
-template <bool VEC4>
+// The order of every output list: (exact distance, index).
+__device__ __forceinline__ bool pair_less(double ad, int aj, double bd, int bj) { return ad < bd || (ad == bd && aj < bj); }
+
+// Rank of the lane's pair (d2, j): how many of the warp's valid pairs (wd, wj), R per lane and j >= 0, order before it.
+template <int R>
+__device__ __forceinline__ int pair_rank(const double (&wd)[R], const int (&wj)[R], double d2, int j) {
+  int rank = 0;
+#pragma unroll
+  for (int s = 0; s < R; ++s) {
+    for (int c = 0; c < KC; ++c) {
+      const double od = __shfl_sync(FULL, wd[s], c);
+      const int oj = __shfl_sync(FULL, wj[s], c);
+      if (oj >= 0 && (od < d2 || (od == d2 && oj < j))) ++rank;  // pair_less spelled out: the compiler then selects, not branches
+    }
+  }
+  return rank;
+}
+
+// One lane's part of output row i: its pair (d2, j), when valid, in slot 1 + rank if that is one of the row's k - 1 neighbour
+// slots; with `self` also row i itself, at distance 0, in slot 0.
+__device__ __forceinline__ void emit_row(int* __restrict__ knn_idx, float* __restrict__ knn_dist, int i, int k, int rank,
+                                         bool valid, double d2, int j, bool self) {
+  if (valid && rank < k - 1) {
+    knn_idx[(size_t)i * k + 1 + rank] = j;
+    knn_dist[(size_t)i * k + 1 + rank] = (float)sqrt(d2);
+  }
+  if (self) {
+    knn_idx[(size_t)i * k] = i;
+    knn_dist[(size_t)i * k] = 0.f;
+  }
+}
+
+// Completeness proof of re-ranked row i: every column outside its candidate lists has approximate distance >= lower, so exact
+// distance >= lower - errb.  The lists hold the k - 1 nearest when that exceeds d_k, the exact distance ranked k - 2, or when
+// no column was left out (lower = +inf).  A row that fails, or is forced (GLL_B200_KNN_FORCE_FALLBACK, tests), goes to flag_rows.
+template <int R>
+__device__ __forceinline__ void prove_or_flag(const double (&d2)[R], const int (&j)[R], const int (&rank)[R], int k, float lower,
+                                              double errb, bool force, int i, int* __restrict__ flag_count,
+                                              int* __restrict__ flag_rows, int lane) {
+  bool ok = false;
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const unsigned who = __ballot_sync(FULL, j[r] >= 0 && rank[r] == k - 2);
+    if (who) {
+      const double dk = __shfl_sync(FULL, d2[r], __ffs(who) - 1);
+      ok = ((double)lower - errb > dk) || (lower == INFINITY);
+    }
+  }
+  if (force) ok = false;
+  if (!ok && lane == 0) {
+    int p = atomicAdd(flag_count, 1);
+    flag_rows[p] = i;
+  }
+}
+
+__device__ __forceinline__ void list_insert_d(double& md, int& mj, double xd, int xj, int lane) {
+  bool lt = (md < xd) || (md == xd && mj < xj);
+  int pos = __popc(__ballot_sync(FULL, lt));
+  double pd = __shfl_up_sync(FULL, md, 1);
+  int pj = __shfl_up_sync(FULL, mj, 1);
+  if (lane > pos) {
+    md = pd;
+    mj = pj;
+  } else if (lane == pos) {
+    md = xd;
+    mj = xj;
+  }
+}
+
+// Merge the ascending 32-list (od, oj) into the ascending 32-list (md, mj), one (distance, index) pair per lane, padding
+// (INFINITY, 0x7fffffff) at the end: min(A[i], B[31 - i]) holds the 32 smallest of the union as a bitonic sequence, five
+// compare-exchange steps put it in order.  Replaces up to 32 serial insertions per list.
+__device__ __forceinline__ void dlist_merge_sorted(double& md, int& mj, double od, int oj, int lane) {
+  const double rd = __shfl_sync(FULL, od, 31 - lane);
+  const int rj = __shfl_sync(FULL, oj, 31 - lane);
+  if (pair_less(rd, rj, md, mj)) {
+    md = rd;
+    mj = rj;
+  }
+#pragma unroll
+  for (int j = 16; j >= 1; j >>= 1) {
+    const double pd = __shfl_xor_sync(FULL, md, j);
+    const int pj = __shfl_xor_sync(FULL, mj, j);
+    const bool keep_min = (lane & j) == 0;
+    const bool p_less = pair_less(pd, pj, md, mj);
+    if (p_less == keep_min) {
+      md = pd;
+      mj = pj;
+    }
+  }
+}
+
+// k in (33, 64] (the evaluation path, utils.laplace asks for k = 50; the layer itself uses k = 25) takes two candidate rounds
+// of 32, the second excluding the first by key.  One warp per row: union of the row's candidate sets of one round -> one
+// sorted 32-list; optionally its last key
+__global__ void __launch_bounds__(RERANK_WARPS * 32)
+knn_merge_kernel(int row_end, CandLayout lay, const u64* __restrict__ cand, u64* __restrict__ merged, u64* __restrict__ excl) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int i = lay.row_begin + blockIdx.x * RERANK_WARPS + warp;
+  if (i >= row_end) return;
+  const int splits = cand_lists(lay, i);
+  u64 mine = KEY_INF;
+  for (int s = 0; s < splits; ++s) {
+    list_merge_set(mine, cand[((size_t)i * lay.stride + s) * KC + lane], lane);
+  }
+  merged[(size_t)(i - lay.row_begin) * KC + lane] = mine;
+  if (excl != nullptr && lane == KC - 1) excl[i] = mine;  // KEY_INF if fewer than 32 columns exist: round 2 finds nothing
+}
+
+// Exact re-rank of rows [lay.row_begin, row_end), one warp per row, and the rows' completeness proof.
+// ROUNDS = 1 (k <= 33): the row's candidate sets in `cand` under `lay`, merged here into one sorted list; candidates that
+//   cannot be among the k - 1 nearest are skipped.
+// ROUNDS = 2 (33 < k <= 64): `cand` holds the two rounds' merged lists (knn_merge_kernel), [2][rows][KC]; first-round members
+//   that come back in round 2 are dropped, and all 64 candidates are ranked together.
+template <bool VEC4, int ROUNDS>
 __global__ void __launch_bounds__(RERANK_WARPS * 32)
 knn_rerank_kernel(const float* __restrict__ X, const float* __restrict__ sq, const unsigned* __restrict__ sqmax_bits,
                   int n, int d, int k, int row_end, CandLayout lay, const u64* __restrict__ cand, float err_coef,
@@ -470,174 +586,83 @@ knn_rerank_kernel(const float* __restrict__ X, const float* __restrict__ sq, con
     for (int t = lane; t < d; t += 32) xi[t] = X[(size_t)i * d + t];
   }
 
-  u64 mine = KEY_INF;
-  const int splits = cand_lists(lay, i);
-  if (splits == 1 && lay.tc == 0) {
-    mine = cand[(size_t)i * lay.stride * KC + lane];  // SIMT lists are sorted
-  } else {
-    for (int s = 0; s < splits; ++s) {  // tensor-core lists are unsorted sets: merge by insertion
-      list_merge_set(mine, cand[((size_t)i * lay.stride + s) * KC + lane], lane);
+  u64 keys[ROUNDS];  // the row's candidates, one per lane and round
+  if constexpr (ROUNDS == 1) {
+    keys[0] = KEY_INF;
+    const int splits = cand_lists(lay, i);
+    if (splits == 1 && lay.tc == 0) {
+      keys[0] = cand[(size_t)i * lay.stride * KC + lane];  // SIMT lists are sorted
+    } else {
+      for (int s = 0; s < splits; ++s) {  // tensor-core lists are unsorted sets: merge by insertion
+        list_merge_set(keys[0], cand[((size_t)i * lay.stride + s) * KC + lane], lane);
+      }
     }
+  } else {
+    const size_t r = (size_t)(i - lay.row_begin) * KC + lane;
+    keys[0] = cand[r];
+    keys[1] = cand[(size_t)(row_end - lay.row_begin) * KC + r];
   }
-  u64 last = __shfl_sync(FULL, mine, KC - 1);
+  u64 last = __shfl_sync(FULL, keys[ROUNDS - 1], KC - 1);
   const float lower = (last == KEY_INF) ? INFINITY : key_dist(last);  // every non-candidate has d~^2 >= lower
   __syncwarp();
-
-  // Candidates whose approximate distance exceeds the (k-1)-th approximate distance by more than twice the error bound
-  // cannot be among the k-1 nearest (k-1 others are provably closer): their exact distance is not needed.
-  const double errb = knn_err_bound(err_coef, sq[i], sqmax_bits);
-  const u64 kth = __shfl_sync(FULL, mine, k - 2);
-  const float cutoff = (kth == KEY_INF) ? INFINITY : (float)((double)key_dist(kth) + 2.0 * errb + 1e-30) * (1.f + 1e-6f);
-  double myd2 = INFINITY;
-  int myj = -1;
-  for (int c = 0; c < KC; ++c) {
-    u64 kc = __shfl_sync(FULL, mine, c);
-    if (kc == KEY_INF) break;
-    if (c > k - 2 && key_dist(kc) > cutoff) break;  // sorted: everything behind is farther still
-    int j = key_idx(kc);
-    double v = use_reg ? exact_d2_reg(xr, X + (size_t)j * d, d >> 2, lane) : exact_d2<VEC4>(xi, X + (size_t)j * d, d, lane);
-    if (lane == c) {
-      myd2 = v;
-      myj = j;
+  if constexpr (ROUNDS == 2) {
+    // the second round re-admits first-round members whose stored value ties with the first round's 32nd (knn_tc.cu): drop them
+    bool dup = false;
+    for (int c = 0; c < KC; ++c) {
+      const u64 oa = __shfl_sync(FULL, keys[0], c);
+      dup |= (oa != KEY_INF && keys[1] != KEY_INF && key_idx(oa) == key_idx(keys[1]));
     }
+    if (dup) keys[1] = KEY_INF;
   }
-  int rank = 0;
-  for (int c = 0; c < KC; ++c) {
-    double od = __shfl_sync(FULL, myd2, c);
-    int oj = __shfl_sync(FULL, myj, c);
-    if (oj >= 0 && (od < myd2 || (od == myd2 && oj < myj))) ++rank;
-  }
-  if (myj >= 0 && rank < k - 1) {
-    knn_idx[(size_t)i * k + 1 + rank] = myj;
-    knn_dist[(size_t)i * k + 1 + rank] = (float)sqrt(myd2);
-  }
-  if (lane == 0) {
-    knn_idx[(size_t)i * k] = i;
-    knn_dist[(size_t)i * k] = 0.f;
-  }
-  // completeness proof
-  unsigned who = __ballot_sync(FULL, myj >= 0 && rank == k - 2);
-  bool ok = false;
-  if (who) {
-    double dk = __shfl_sync(FULL, myd2, __ffs(who) - 1);
-    ok = ((double)lower - errb > dk) || (lower == INFINITY);
-  }
-  if (i - lay.row_begin < force_rows) ok = false;  // GLL_B200_KNN_FORCE_FALLBACK (tests): treat the first rows as unproven
-  if (!ok && lane == 0) {
-    int p = atomicAdd(flag_count, 1);
-    flag_rows[p] = i;
-  }
-}
 
-constexpr int FB_WARPS = 8;
-
-__device__ __forceinline__ void list_insert_d(double& md, int& mj, double xd, int xj, int lane) {
-  bool lt = (md < xd) || (md == xd && mj < xj);
-  int pos = __popc(__ballot_sync(FULL, lt));
-  double pd = __shfl_up_sync(FULL, md, 1);
-  int pj = __shfl_up_sync(FULL, mj, 1);
-  if (lane > pos) {
-    md = pd;
-    mj = pj;
-  } else if (lane == pos) {
-    md = xd;
-    mj = xj;
+  const double errb = knn_err_bound(err_coef, sq[i], sqmax_bits);
+  float cutoff = INFINITY;
+  if constexpr (ROUNDS == 1) {
+    // Candidates whose approximate distance exceeds the (k-1)-th approximate distance by more than twice the error bound
+    // cannot be among the k-1 nearest (k-1 others are provably closer): their exact distance is not needed.
+    const u64 kth = __shfl_sync(FULL, keys[0], k - 2);
+    cutoff = (kth == KEY_INF) ? INFINITY : (float)((double)key_dist(kth) + 2.0 * errb + 1e-30) * (1.f + 1e-6f);
   }
-}
-
-// Merge the ascending 32-list (od, oj) into the ascending 32-list (md, mj), one (distance, index) pair per lane, padding
-// (INFINITY, 0x7fffffff) at the end: min(A[i], B[31 - i]) holds the 32 smallest of the union as a bitonic sequence, five
-// compare-exchange steps put it in order.  Replaces up to 32 serial insertions per list.
-__device__ __forceinline__ bool pair_less(double ad, int aj, double bd, int bj) { return ad < bd || (ad == bd && aj < bj); }
-__device__ __forceinline__ void dlist_merge_sorted(double& md, int& mj, double od, int oj, int lane) {
-  const double rd = __shfl_sync(FULL, od, 31 - lane);
-  const int rj = __shfl_sync(FULL, oj, 31 - lane);
-  if (pair_less(rd, rj, md, mj)) {
-    md = rd;
-    mj = rj;
+  double myd2[ROUNDS];
+  int myj[ROUNDS];
+#pragma unroll
+  for (int r = 0; r < ROUNDS; ++r) {
+    myd2[r] = INFINITY;
+    myj[r] = -1;
   }
 #pragma unroll
-  for (int j = 16; j >= 1; j >>= 1) {
-    const double pd = __shfl_xor_sync(FULL, md, j);
-    const int pj = __shfl_xor_sync(FULL, mj, j);
-    const bool keep_min = (lane & j) == 0;
-    const bool p_less = pair_less(pd, pj, md, mj);
-    if (p_less == keep_min) {
-      md = pd;
-      mj = pj;
+  for (int r = 0; r < ROUNDS; ++r) {
+    for (int c = 0; c < KC; ++c) {
+      u64 kc = __shfl_sync(FULL, keys[r], c);
+      if (kc == KEY_INF) {
+        if (ROUNDS == 1) break;  // a sorted list ends here; round 2's list has holes where returning members were dropped
+        continue;
+      }
+      if (ROUNDS == 1 && c > k - 2 && key_dist(kc) > cutoff) break;  // sorted: everything behind is farther still
+      int j = key_idx(kc);
+      double v = use_reg ? exact_d2_reg(xr, X + (size_t)j * d, d >> 2, lane) : exact_d2<VEC4>(xi, X + (size_t)j * d, d, lane);
+      if (lane == c) {
+        myd2[r] = v;
+        myj[r] = j;
+      }
     }
   }
+  int rank[ROUNDS];
+#pragma unroll
+  for (int r = 0; r < ROUNDS; ++r) rank[r] = pair_rank(myd2, myj, myd2[r], myj[r]);
+#pragma unroll
+  for (int r = 0; r < ROUNDS; ++r)
+    emit_row(knn_idx, knn_dist, i, k, rank[r], myj[r] >= 0, myd2[r], myj[r], lane == 0 && r == ROUNDS - 1);
+  prove_or_flag(myd2, myj, rank, k, lower, errb, i - lay.row_begin < force_rows, i, flag_count, flag_rows, lane);
 }
 
-template <bool VEC4>
-__global__ void __launch_bounds__(FB_WARPS * 32)
-knn_fallback_kernel(const float* __restrict__ X, int n, int d, int k, const int* __restrict__ flag_count,
-                    const int* __restrict__ flag_rows, int* __restrict__ knn_idx, float* __restrict__ knn_dist,
-                    int* __restrict__ info, const int2* __restrict__ win) {
-  extern __shared__ __align__(16) float xs[];
-  __shared__ double sd[FB_WARPS][32];
-  __shared__ int sj[FB_WARPS][32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int nflag = *flag_count;
-  if (blockIdx.x == 0 && threadIdx.x == 0 && info != nullptr) {
-    info[GLL_INFO_KNN_FALLBACK_ROWS] = nflag;
-    if (nflag > 0) atomicOr(&info[GLL_INFO_STATUS], GLL_STATUS_KNN_FALLBACK);
-  }
-  for (int f = blockIdx.x; f < nflag; f += gridDim.x) {
-    const int i = flag_rows[f];
-    const int2 w = (win != nullptr) ? win[i] : make_int2(0, n);  // a segmented search scans the row's own segment
-    for (int t = threadIdx.x; t < d; t += blockDim.x) xs[t] = X[(size_t)i * d + t];
-    __syncthreads();
-    // k - 1 <= 32 neighbours fit one 32-wide list; larger k takes a second scan that only admits pairs beyond the 32nd
-    // (distance, index) of the first scan
-    double ex_d = -1.0;
-    int ex_j = -1;
-    for (int pass = 0; pass * 32 < k - 1; ++pass) {
-      double md = INFINITY;
-      int mj = 0x7fffffff;
-      for (int j = w.x + warp; j < w.y; j += FB_WARPS) {
-        if (j == i) continue;
-        double v = exact_d2<VEC4>(xs, X + (size_t)j * d, d, lane);
-        if (v > ex_d || (v == ex_d && j > ex_j)) list_insert_d(md, mj, v, j, lane);
-      }
-      sd[warp][lane] = md;
-      sj[warp][lane] = mj;
-      __syncthreads();
-      if (warp == 0) {
-        for (int w = 1; w < FB_WARPS; ++w)
-          for (int t = 0; t < 32; ++t) {
-            int xj = sj[w][t];
-            if (xj == 0x7fffffff) break;
-            list_insert_d(md, mj, sd[w][t], xj, lane);
-          }
-        const int slot = pass * 32 + lane;
-        if (slot < k - 1 && mj != 0x7fffffff) {
-          knn_idx[(size_t)i * k + 1 + slot] = mj;
-          knn_dist[(size_t)i * k + 1 + slot] = (float)sqrt(md);
-        }
-        if (lane == 0 && pass == 0) {
-          knn_idx[(size_t)i * k] = i;
-          knn_dist[(size_t)i * k] = 0.f;
-        }
-        if (lane == 31) {  // threshold for the next scan
-          sd[0][0] = md;
-          sj[0][0] = mj;
-        }
-      }
-      __syncthreads();
-      ex_d = sd[0][0];
-      ex_j = sj[0][0];
-      __syncthreads();
-    }
-    __syncthreads();
-  }
-}
-
-// ---- brute-force fallback for k - 1 <= 32, fast for FEW rows: the flagged rows' column ranges are dealt to all CTAs ----
+// ---- brute-force fallback, fast for FEW rows: the flagged rows' column ranges are dealt to all CTAs ----
 // (a flagged row used to be one CTA's job: 171 ms for two rows of a 1M-node graph.)  Task t = (flagged row f, column chunk c)
-// with C = max(1, G / nflag) chunks per row; every task leaves the 32 smallest (exact fp64 distance, index) pairs of its
-// chunk; with C == 1 that is the row's answer, otherwise the last CTA to finish merges the C lists of every row.
-template <bool VEC4>
+// with C = max(1, G / nflag) chunks per row; every task leaves the 32 smallest admitted (exact fp64 distance, index) pairs of
+// its chunk; with C == 1 that is the row's answer, otherwise the last CTA to finish merges the C lists of every row.  Each pass
+// finds 32 neighbours: pass 0 writes slot 0 and slots 1 .. min(32, k - 1); pass 1 (k > 33) admits only the pairs ordered after
+// the row's 32nd neighbour and writes slots 33 .. k - 1.  PASS is a template argument so that pass 0 carries no trace of pass 1.
+template <bool VEC4, int PASS>
 __global__ void __launch_bounds__(FB_WARPS * 32)
 knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const int* __restrict__ flag_count,
                          const int* __restrict__ flag_rows, int* __restrict__ knn_idx, float* __restrict__ knn_dist,
@@ -648,6 +673,8 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
   __shared__ int sj[FB_WARPS][32];
   __shared__ int last_cta;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int base = 32 * PASS;  // the pass's first neighbour slot is 1 + base
+  const bool self = lane == 0 && PASS == 0;
   const int nflag = *flag_count;
   if (blockIdx.x == 0 && threadIdx.x == 0 && info != nullptr) {
     info[GLL_INFO_KNN_FALLBACK_ROWS] = nflag;
@@ -664,6 +691,17 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
     __syncthreads();  // the previous task's readers of xs / sd / sj are done
     for (int q = threadIdx.x; q < d; q += blockDim.x) xs[q] = X[(size_t)i * d + q];
     __syncthreads();
+    // pass 1 admits pairs after (ex_d, ex_j): the 32nd neighbour as pass 0 wrote it, its distance recomputed by the same
+    // exact_d2 (bit for bit the double pass 0 ranked it by).  Pass 0 leaves slot 32 unwritten when fewer than 32 columns have
+    // a distance (NaN features): a stale index outside the window is not dereferenced and admits nothing.
+    double ex_d = -INFINITY;
+    int ex_j = -1;
+    if constexpr (PASS == 1) {
+      ex_j = knn_idx[(size_t)i * k + 32];
+      const bool written = ex_j >= w.x && ex_j < w.y;
+      ex_d = written ? exact_d2<VEC4>(xs, X + (size_t)ex_j * d, d, lane) : INFINITY;
+      ex_j = written ? ex_j : 0x7fffffff;
+    }
     double md = INFINITY, thr_d = INFINITY;
     int mj = 0x7fffffff, thr_j = 0x7fffffff;
     // four columns per trip: their row loads and butterflies are independent (one column at a time is a chain of L2 round trips)
@@ -678,7 +716,8 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
       for (int u = 0; u < 4; ++u) {
         const int j = jb + u;
         if (j >= j1 || j == i) continue;
-        if (v[u] < thr_d || (v[u] == thr_d && j < thr_j)) {  // warp-uniform: only pairs that enter the list pay for the insertion
+        // warp-uniform: only pairs that enter the list pay for the insertion (and for pass 1's lower bound)
+        if (pair_less(v[u], j, thr_d, thr_j) && (PASS == 0 || pair_less(ex_d, ex_j, v[u], j))) {
           list_insert_d(md, mj, v[u], j, lane);
           thr_d = __shfl_sync(FULL, md, 31);
           thr_j = __shfl_sync(FULL, mj, 31);
@@ -691,14 +730,7 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
     if (warp == 0) {
       for (int w = 1; w < FB_WARPS; ++w) dlist_merge_sorted(md, mj, sd[w][lane], sj[w][lane], lane);
       if (C == 1) {
-        if (lane < k - 1 && mj != 0x7fffffff) {
-          knn_idx[(size_t)i * k + 1 + lane] = mj;
-          knn_dist[(size_t)i * k + 1 + lane] = (float)sqrt(md);
-        }
-        if (lane == 0) {
-          knn_idx[(size_t)i * k] = i;
-          knn_dist[(size_t)i * k] = 0.f;
-        }
+        emit_row(knn_idx, knn_dist, i, k, base + lane, mj != 0x7fffffff, md, mj, self);
       } else {
         part_d[(size_t)t * 32 + lane] = md;
         part_j[(size_t)t * 32 + lane] = mj;
@@ -733,14 +765,7 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
 #pragma unroll
         for (int u = 0; u < 4; ++u) dlist_merge_sorted(md, mj, ld[u], lj[u], lane);
       }
-      if (lane < k - 1 && mj != 0x7fffffff) {
-        knn_idx[(size_t)i * k + 1 + lane] = mj;
-        knn_dist[(size_t)i * k + 1 + lane] = (float)sqrt(md);
-      }
-      if (lane == 0) {
-        knn_idx[(size_t)i * k] = i;
-        knn_dist[(size_t)i * k] = 0.f;
-      }
+      emit_row(knn_idx, knn_dist, i, k, base + lane, mj != 0x7fffffff, md, mj, self);
     }
     return;
   }
@@ -766,113 +791,8 @@ knn_fallback_scan_kernel(const float* __restrict__ X, int n, int d, int k, const
     __syncthreads();
     if (warp == 0) {
       for (int w = 1; w < FB_WARPS; ++w) dlist_merge_sorted(md, mj, sd[w][lane], sj[w][lane], lane);
-      if (lane < k - 1 && mj != 0x7fffffff) {
-        knn_idx[(size_t)i * k + 1 + lane] = mj;
-        knn_dist[(size_t)i * k + 1 + lane] = (float)sqrt(md);
-      }
-      if (lane == 0) {
-        knn_idx[(size_t)i * k] = i;
-        knn_dist[(size_t)i * k] = 0.f;
-      }
+      emit_row(knn_idx, knn_dist, i, k, base + lane, mj != 0x7fffffff, md, mj, self);
     }
-  }
-}
-
-
-// ---------------------------------------------------------------------------------------------------------
-// k in (33, 64]: two candidate rounds of 32 (the second excludes the first by key), merged and re-ranked together.
-// Used by the evaluation path (utils.laplace asks for k = 50, utils.py:651); the layer itself uses k = 25.
-// ---------------------------------------------------------------------------------------------------------
-// one warp per row: union of the row's candidate sets of one round -> one sorted 32-list; optionally its last key
-__global__ void __launch_bounds__(RERANK_WARPS * 32)
-knn_merge_kernel(int row_end, CandLayout lay, const u64* __restrict__ cand, u64* __restrict__ merged, u64* __restrict__ excl) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int i = lay.row_begin + blockIdx.x * RERANK_WARPS + warp;
-  if (i >= row_end) return;
-  const int splits = cand_lists(lay, i);
-  u64 mine = KEY_INF;
-  for (int s = 0; s < splits; ++s) {
-    list_merge_set(mine, cand[((size_t)i * lay.stride + s) * KC + lane], lane);
-  }
-  merged[(size_t)(i - lay.row_begin) * KC + lane] = mine;
-  if (excl != nullptr && lane == KC - 1) excl[i] = mine;  // KEY_INF if fewer than 32 columns exist: round 2 finds nothing
-}
-
-template <bool VEC4>
-__global__ void __launch_bounds__(RERANK_WARPS * 32)
-knn_rerank64_kernel(const float* __restrict__ X, const float* __restrict__ sq, const unsigned* __restrict__ sqmax_bits, int n, int d,
-                    int k, int row_begin, int row_end, const u64* __restrict__ m1, const u64* __restrict__ m2, float err_coef,
-                    int* __restrict__ knn_idx, float* __restrict__ knn_dist, int* __restrict__ flag_count,
-                    int* __restrict__ flag_rows, int force_rows) {
-  extern __shared__ __align__(16) float xs[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int i = row_begin + blockIdx.x * RERANK_WARPS + warp;
-  if (i >= row_end) return;
-  float* xi = xs + (size_t)warp * d;
-  for (int t = lane; t < d; t += 32) xi[t] = X[(size_t)i * d + t];
-  __syncwarp();
-  const u64 ca = m1[(size_t)(i - row_begin) * KC + lane];
-  u64 cb = m2[(size_t)(i - row_begin) * KC + lane];
-  const u64 last = __shfl_sync(FULL, cb, KC - 1);
-  const float lower = (last == KEY_INF) ? INFINITY : key_dist(last);  // every non-candidate has d~^2 >= lower
-  // the second round re-admits first-round members whose stored value ties with the first round's 32nd (knn_tc.cu): drop them
-  {
-    bool dup = false;
-    for (int c = 0; c < KC; ++c) {
-      const u64 oa = __shfl_sync(FULL, ca, c);
-      dup |= (oa != KEY_INF && cb != KEY_INF && key_idx(oa) == key_idx(cb));
-    }
-    if (dup) cb = KEY_INF;
-  }
-  double da = INFINITY, db = INFINITY;
-  int ja = -1, jb = -1;
-  for (int c = 0; c < 2 * KC; ++c) {
-    const u64 kc = __shfl_sync(FULL, (c < KC) ? ca : cb, c & (KC - 1));
-    if (kc == KEY_INF) continue;
-    const int j = key_idx(kc);
-    const double v = exact_d2<VEC4>(xi, X + (size_t)j * d, d, lane);
-    if (lane == (c & (KC - 1))) {
-      if (c < KC) {
-        da = v;
-        ja = j;
-      } else {
-        db = v;
-        jb = j;
-      }
-    }
-  }
-  int ra = 0, rb = 0;
-  for (int c = 0; c < 2 * KC; ++c) {
-    const double od = __shfl_sync(FULL, (c < KC) ? da : db, c & (KC - 1));
-    const int oj = __shfl_sync(FULL, (c < KC) ? ja : jb, c & (KC - 1));
-    if (oj < 0) continue;
-    ra += (od < da || (od == da && oj < ja)) ? 1 : 0;
-    rb += (od < db || (od == db && oj < jb)) ? 1 : 0;
-  }
-  if (ja >= 0 && ra < k - 1) {
-    knn_idx[(size_t)i * k + 1 + ra] = ja;
-    knn_dist[(size_t)i * k + 1 + ra] = (float)sqrt(da);
-  }
-  if (jb >= 0 && rb < k - 1) {
-    knn_idx[(size_t)i * k + 1 + rb] = jb;
-    knn_dist[(size_t)i * k + 1 + rb] = (float)sqrt(db);
-  }
-  if (lane == 0) {
-    knn_idx[(size_t)i * k] = i;
-    knn_dist[(size_t)i * k] = 0.f;
-  }
-  // completeness proof against the (k-1)-th exact distance
-  const unsigned wa = __ballot_sync(FULL, ja >= 0 && ra == k - 2), wb = __ballot_sync(FULL, jb >= 0 && rb == k - 2);
-  bool ok = false;
-  if (wa | wb) {
-    const double dk = wa ? __shfl_sync(FULL, da, __ffs(wa) - 1) : __shfl_sync(FULL, db, __ffs(wb) - 1);
-    const double errb = knn_err_bound(err_coef, sq[i], sqmax_bits);
-    ok = ((double)lower - errb > dk) || (lower == INFINITY);
-  }
-  if (i - row_begin < force_rows) ok = false;  // GLL_B200_KNN_FORCE_FALLBACK (tests): treat the first rows as unproven
-  if (!ok && lane == 0) {
-    int p = atomicAdd(flag_count, 1);
-    flag_rows[p] = i;
   }
 }
 
@@ -957,7 +877,7 @@ KnnPlan knn_plan(int n, int d, int row_begin, int row_end, int col_begin = 0, co
 // What a kNN entry takes from its workspace; the members it does not use stay NULL.
 struct KnnBufs {
   float* sq;
-  unsigned* small;     // small[0]: bits of max |x|^2, small[1]: flag_count, small[8]: fallback ticket (zeroed per search)
+  unsigned* small;     // small[0]: bits of max |x|^2, small[1]: flag_count, small[8 + pass]: fallback tickets (zeroed per search)
   int* flag_count;
   u64* cand;           // the plan's rows x lay.stride lists, indexed by GLOBAL row: where row 0 would live
   int* flag_rows;
@@ -1051,49 +971,42 @@ int launch_norms(const float* X, int n, int d, const TcPlan& plan, const KnnBufs
 }
 
 // Exact re-rank of rows [lay.row_begin, row_end), their completeness proof, and the brute-force search of the rows it could not
-// prove.  k <= 33: the candidate lists `cand` under `lay`; k > 33: b.merged, the two rounds' merged lists.
+// prove, one fallback pass per 32 neighbours.  k <= 33: the candidate lists `cand` under `lay`; k > 33: b.merged, the two rounds'
+// merged lists.
 int knn_finish(const float* X, int n, int d, int k, int row_end, const CandLayout& lay, const u64* cand, float err_coef,
                const KnnBufs& b, int* knn_idx, float* knn_dist, int* info, cudaStream_t st) {
   const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
   const bool two_rounds = k > KC + 1;
-  const int row_begin = lay.row_begin, blocks = ceil_div(row_end - row_begin, RERANK_WARPS);
+  const int blocks = ceil_div(row_end - lay.row_begin, RERANK_WARPS);
   const size_t smem = sizeof(float) * (size_t)RERANK_WARPS * d, fsmem = sizeof(float) * (size_t)d;
   const char* force = getenv("GLL_B200_KNN_FORCE_FALLBACK");
   const int force_rows = force ? atoi(force) : 0;
   const bool no_fallback = getenv("GLL_B200_KNN_DEBUG") != nullptr;  // timing experiments: every row would be "unproven"
-  if (two_rounds) {
-    auto kern = vec4 ? knn_rerank64_kernel<true> : knn_rerank64_kernel<false>;
+  {
+    auto kern = two_rounds ? (vec4 ? knn_rerank_kernel<true, 2> : knn_rerank_kernel<false, 2>)
+                           : (vec4 ? knn_rerank_kernel<true, 1> : knn_rerank_kernel<false, 1>);
     GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)smem));
     GLL_PROF(KID_RERANK, st);
-    kern<<<blocks, RERANK_WARPS * 32, smem, st>>>(X, b.sq, b.small, n, d, k, row_begin, row_end, b.merged,
-                                                 b.merged + (size_t)(row_end - row_begin) * KC, err_coef, knn_idx, knn_dist,
-                                                 b.flag_count, b.flag_rows, force_rows);
-  } else {
-    auto kern = vec4 ? knn_rerank_kernel<true> : knn_rerank_kernel<false>;
-    GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)smem));
-    GLL_PROF(KID_RERANK, st);
-    kern<<<blocks, RERANK_WARPS * 32, smem, st>>>(X, b.sq, b.small, n, d, k, row_end, lay, cand, err_coef, knn_idx, knn_dist,
-                                                 b.flag_count, b.flag_rows, force_rows);
+    kern<<<blocks, RERANK_WARPS * 32, smem, st>>>(X, b.sq, b.small, n, d, k, row_end, lay, two_rounds ? b.merged : cand, err_coef,
+                                                 knn_idx, knn_dist, b.flag_count, b.flag_rows, force_rows);
   }
   GLL_LAUNCH_CHECK();
   if (no_fallback) return GLL_OK;
-  if (two_rounds) {
-    auto kern = vec4 ? knn_fallback_kernel<true> : knn_fallback_kernel<false>;
+  // the rows' column ranges dealt to all CTAs; each pass has its own ticket word
+  const int fblocks = knn_fallback_grid();
+  double* part_d = reinterpret_cast<double*>(b.fb_scratch);
+  int* part_j = reinterpret_cast<int*>(part_d + (size_t)fblocks * 32);
+  for (int pass = 0; pass * 32 < k - 1; ++pass) {
+    auto kern = vec4 ? (pass ? knn_fallback_scan_kernel<true, 1> : knn_fallback_scan_kernel<true, 0>)
+                     : (pass ? knn_fallback_scan_kernel<false, 1> : knn_fallback_scan_kernel<false, 0>);
     GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)fsmem));
-    GLL_PROF(KID_KNN_FALLBACK, st);
-    kern<<<device_info().sms, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, b.flag_count, b.flag_rows, knn_idx, knn_dist, info, b.win);
-  } else {
-    // the rows' column ranges dealt to all CTAs
-    const int fblocks = knn_fallback_grid();
-    double* part_d = reinterpret_cast<double*>(b.fb_scratch);
-    int* part_j = reinterpret_cast<int*>(part_d + (size_t)fblocks * 32);
-    auto kern = vec4 ? knn_fallback_scan_kernel<true> : knn_fallback_scan_kernel<false>;
-    GLL_CUDA_CHECK(set_max_dynamic_smem_once((const void*)kern, (int)fsmem));
-    GLL_PROF(KID_KNN_FALLBACK, st);
-    kern<<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, b.flag_count, b.flag_rows, knn_idx, knn_dist, info, part_d, part_j,
-                                                b.small + 8, b.win);
+    {
+      GLL_PROF(KID_KNN_FALLBACK, st);
+      kern<<<fblocks, FB_WARPS * 32, fsmem, st>>>(X, n, d, k, b.flag_count, b.flag_rows, knn_idx, knn_dist, pass ? nullptr : info,
+                                                  part_d, part_j, b.small + 8 + pass, b.win);
+    }
+    GLL_LAUNCH_CHECK();
   }
-  GLL_LAUNCH_CHECK();
   return GLL_OK;
 }
 

@@ -780,7 +780,7 @@ knn_gram_topk_tc_kernel(const __grid_constant__ CUtensorMap mapAH, const __grid_
             // stored value is >= the first round's 32nd value, except that 32nd entry itself.  (Not "key > 32nd key": a column
             // that TIES with the 32nd value and has a smaller index may have been evicted from its set in the first round --
             // the entry a set drops among tied maxima is picked by slot, not by index -- and would be lost to both rounds.
-            // First-round members that tie come back as duplicates; knn_rerank64 drops them by index.)
+            // First-round members that tie come back as duplicates; the re-rank drops them by index.)
             bool fresh = true;
             if (P.excl != nullptr) {
               const u64 key = make_key(unshift(__uint_as_float(kbits), sqi_row), j0 + c);

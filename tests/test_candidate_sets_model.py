@@ -111,7 +111,7 @@ def run_two_rounds(v, rule2):
     sub = run_row(v[idx], 4, 32, 4, "next_bucket")[:KC]
     r2 = [(s, idx[j]) for s, j in sub]
     first_members = {j for _, j in r1}
-    r2_new = [x for x in r2 if x[1] not in first_members]          # knn_rerank64 drops the first round's members by index
+    r2_new = [x for x in r2 if x[1] not in first_members]          # the k > 33 re-rank drops the first round's members by index
     return r1, r2, r2_new
 
 

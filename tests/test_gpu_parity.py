@@ -206,15 +206,20 @@ def test_knn_one_pass_full_size_matches_two_pass(gll, monkeypatch):
     assert int(info0[_lib.INFO_KNN_FALLBACK_ROWS].item()) <= 4 and int(info1[_lib.INFO_KNN_FALLBACK_ROWS].item()) == 0
 
 
+@pytest.mark.parametrize("k", [25, 50, 64])
 @pytest.mark.parametrize("forced", [1, 3, 700, 5000])
-def test_knn_fallback_rows_dealt_over_all_ctas(gll, monkeypatch, forced):
+def test_knn_fallback_rows_dealt_over_all_ctas(gll, monkeypatch, forced, k):
     """Rows whose completeness proof fails are redone by exact brute force; few rows are split into column chunks over all
-    CTAs and merged (1, 3: chunked; 700, 5000: one or more rows per CTA).  Forced here for the first rows: same lists."""
+    CTAs and merged (1, 3: chunked; 700, 5000: one or more rows per CTA), one pass per 32 neighbours (k = 50, 64: the second
+    pass starts after the 32nd).  Forced here for the first rows: same lists."""
     _, _lib = gll
     X, *_ = O.synth_inputs(12, 3000, 1777, 200, 10, 3.5)
-    i0, d0, info0 = run_knn(_lib, X)
+    i0, d0, info0 = run_knn(_lib, X, k)
     monkeypatch.setenv("GLL_B200_KNN_FORCE_FALLBACK", str(forced))
-    i1, d1, info1 = run_knn(_lib, X)
+    fb = _lib.kernel_names().index("knn_fallback")
+    before = _lib.launch_count(fb)
+    i1, d1, info1 = run_knn(_lib, X, k)
+    assert _lib.launch_count(fb) == before + (2 if k > 33 else 1)
     assert int(info1[_lib.INFO_KNN_FALLBACK_ROWS].item()) >= min(forced, X.shape[0])
     assert torch.equal(i0, i1) and torch.equal(d0, d1)
 
@@ -959,13 +964,15 @@ def test_knn_large_k_with_duplicates(gll):
     assert np.array_equal(idx.cpu().numpy()[50:120, :50], ref_ind[50:120])  # ties resolved by index in both
 
 
-@pytest.mark.parametrize("k", [25, 50])
-def test_knn_lattice_points_massive_ties(gll, monkeypatch, k):
+@pytest.mark.parametrize("k,forced", [(25, 0), (50, 0), (50, 3000)], ids=["25", "50", "50-fallback"])
+def test_knn_lattice_points_massive_ties(gll, monkeypatch, k, forced):
     """Features on a small integer lattice: squared distances take a handful of values, so nearly every candidate decision is a
     value tie (within one row's set, between the sets of a row, between the two rounds of a k > 33 search).  The lists must be
-    the oracle's -- ties by index -- whatever the packed, truncated keys of the tensor-core epilogue do with equal values."""
+    the oracle's -- ties by index -- whatever the packed, truncated keys of the tensor-core epilogue do with equal values.
+    50-fallback: every row through the brute-force fallback, whose second pass starts after a 32nd neighbour that ties."""
     _, _lib = gll
     monkeypatch.setenv("GLL_B200_KNN_PATH", "tc")
+    monkeypatch.setenv("GLL_B200_KNN_FORCE_FALLBACK", str(forced))
     rng = np.random.default_rng(11)
     X = rng.integers(0, 3, size=(3000, 10)).astype(np.float32)
     ref_ind, ref_dist = O.exact_knn(X, k, slack=600)
