@@ -97,12 +97,10 @@ ProfScope::~ProfScope() {
 
 namespace {
 
-// rhs = grad_output padded to lp class columns (fp32); optionally also wt[0 : zero_count] = 0 (the labeled rows of the
-// padded adjoint solution, GLL.py:104) so that the backward needs no separate memset
+// rhs = grad_output padded to lp class columns (fp32)
 __global__ void pack_grad_kernel(const void* __restrict__ g, int is_f64, int m, int l, int lp, float* __restrict__ rhs,
-                                 float* __restrict__ zero_ptr, long long zero_count, const void* __restrict__ scale, int scale_f64) {
+                                 const void* __restrict__ scale, int scale_f64) {
   long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  for (long long z = t; z < zero_count; z += (long long)gridDim.x * blockDim.x) zero_ptr[z] = 0.f;
   if (t >= (long long)m * lp) return;
   int r = (int)(t / lp), c = (int)(t % lp);
   const double sc = (scale == nullptr) ? 1.0 : (scale_f64 ? *(const double*)scale : (double)*(const float*)scale);
@@ -267,10 +265,9 @@ int unpack_columns(const float* src, int rows, int lp_src, int c0, int cnt, floa
   return GLL_OK;
 }
 
-int pack_grad(const void* g, int is_f64, int m, int l, int lp, float* rhs, cudaStream_t st, float* zero_ptr, long long zero_count,
-              const void* scale, int scale_f64) {
+int pack_grad(const void* g, int is_f64, int m, int l, int lp, float* rhs, cudaStream_t st, const void* scale, int scale_f64) {
   GLL_PROF(KID_PACK, st);
-  pack_grad_kernel<<<ceil_div((long long)m * lp, 256), 256, 0, st>>>(g, is_f64, m, l, lp, rhs, zero_ptr, zero_count, scale, scale_f64);
+  pack_grad_kernel<<<ceil_div((long long)m * lp, 256), 256, 0, st>>>(g, is_f64, m, l, lp, rhs, scale, scale_f64);
   GLL_LAUNCH_CHECK();
   return GLL_OK;
 }

@@ -55,134 +55,70 @@ edge_grad_kernel(int row_begin, int row_end, int lp, int k_lab, int eps_auto, co
   }
 }
 
-constexpr int ROW_CHUNK = 128;
-
-template <int W>
-__device__ __forceinline__ void load_chunk(const float* __restrict__ base, int c, float (&v)[W]) {
-  if constexpr (W == 4) {
-    const float4 t = __ldg(reinterpret_cast<const float4*>(base) + c);
-    v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-  } else {
-    v[0] = __ldg(base + c);
-  }
+// One W-float chunk of a feature row (W = 4: a float4, W = 1: a float), its update acc += t (x_i - x_j) in fp64 accumulators,
+// and its store.  float4 chunks take the difference in fp32 (exact enough: one rounding), single floats in fp64; each form
+// keeps the results its path has always given.
+__device__ __forceinline__ void accumulate_chunk(double (&acc)[4], double t, float4 xi, float4 xj) {
+  acc[0] = fma(t, (double)(xi.x - xj.x), acc[0]);
+  acc[1] = fma(t, (double)(xi.y - xj.y), acc[1]);
+  acc[2] = fma(t, (double)(xi.z - xj.z), acc[2]);
+  acc[3] = fma(t, (double)(xi.w - xj.w), acc[3]);
 }
+__device__ __forceinline__ void accumulate_chunk(double (&acc)[1], double t, float xi, float xj) {
+  acc[0] += t * ((double)xi - (double)xj);
+}
+__device__ __forceinline__ float4 round_chunk(const double (&acc)[4]) {
+  return make_float4((float)acc[0], (float)acc[1], (float)acc[2], (float)acc[3]);
+}
+__device__ __forceinline__ float round_chunk(const double (&acc)[1]) { return (float)acc[0]; }
 
-// block per row; a thread owns up to 4 feature chunks (W floats each) per pass and keeps them in registers
-template <int W>
-__global__ void __launch_bounds__(256)
-row_gather_kernel(const float* __restrict__ X, int row_begin, int d, int eps_auto, const int* __restrict__ row_ptr,
+template <int W> struct Chunk { using T = float; };
+template <> struct Chunk<4> { using T = float4; };
+
+// Warp per row: a lane owns NV W-float chunks of the feature row (chunk = lane + 32 u), so one neighbour row is NV coalesced
+// loads of 32 W floats.  W = 4 needs d % 4 == 0 and 16-byte aligned X and dX; W = 1 takes any d and alignment.  Edge
+// metadata (column, t_ij) is prepared 32 edges at a time, one edge per lane; edges with t_ij == 0 (both ends labeled: most
+// edges of a minibatch graph) are dropped with a ballot; the row of the NEXT surviving edge is already in flight while the
+// current one is accumulated (fp64 accumulators).  Four rows per CTA: many rows in flight per SM, where a CTA per row spent
+// its life waiting on five dependent loads.
+template <int W, int NV>
+__global__ void __launch_bounds__(128)
+row_gather_kernel(const float* __restrict__ X, int row_begin, int row_end, int d, int eps_auto, const int* __restrict__ row_ptr,
                   const int* __restrict__ col, const int* __restrict__ kappa, const float* __restrict__ gv,
                   const float* __restrict__ bvec, float* __restrict__ dX) {
-  __shared__ int sj[ROW_CHUNK];
-  __shared__ float stc[ROW_CHUNK];
-  const int i = row_begin + blockIdx.x;
-  const int e0 = row_ptr[i], e1 = row_ptr[i + 1];
-  const int ki = eps_auto ? kappa[i] : -1;
-  const float bi = eps_auto ? bvec[i] : 0.f;
-  const int cols = d / W;
-  const float* xrow = X + (size_t)i * d;
-  for (int cbase = 0; cbase < cols; cbase += 4 * blockDim.x) {
-    double acc[4][W];
-    float xi[4][W];
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const int c = cbase + u * blockDim.x + threadIdx.x;
-#pragma unroll
-      for (int t = 0; t < W; ++t) acc[u][t] = 0.0, xi[u][t] = 0.f;
-      if (c < cols) load_chunk<W>(xrow, c, xi[u]);
-    }
-    for (int eb = e0; eb < e1; eb += ROW_CHUNK) {
-      const int cnt = min(ROW_CHUNK, e1 - eb);
-      __syncthreads();
-      for (int t = threadIdx.x; t < cnt; t += blockDim.x) {
-        const int j = col[eb + t];
-        float tc = gv[eb + t];
-        if (eps_auto) {
-          if (j == ki) tc -= bi;
-          if (kappa[j] == i) tc -= bvec[j];
-        }
-        sj[t] = j;
-        stc[t] = tc;
-      }
-      __syncthreads();
-      for (int t = 0; t < cnt; ++t) {
-        const float tc = stc[t];
-        if (tc == 0.f) continue;
-        const float* xj = X + (size_t)sj[t] * d;
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int c = cbase + u * blockDim.x + threadIdx.x;
-          if (c < cols) {
-            float v[W];
-            load_chunk<W>(xj, c, v);
-#pragma unroll
-            for (int q = 0; q < W; ++q) acc[u][q] += (double)tc * ((double)xi[u][q] - (double)v[q]);
-          }
-        }
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const int c = cbase + u * blockDim.x + threadIdx.x;
-      if (c < cols) {
-        if constexpr (W == 4) {
-          reinterpret_cast<float4*>(dX + (size_t)i * d)[c] =
-              make_float4((float)acc[u][0], (float)acc[u][1], (float)acc[u][2], (float)acc[u][3]);
-        } else {
-          dX[(size_t)i * d + c] = (float)acc[u][0];
-        }
-      }
-    }
-  }
-}
-
-// Warp per row (vectorised path, d % 4 == 0): a lane owns NV float4 chunks of the feature row (chunk = lane + 32 u), so one
-// neighbour row is NV coalesced 512-byte loads.  Edge metadata (column, t_ij) is prepared 32 edges at a time, one edge per
-// lane; edges with t_ij == 0 (both ends labeled: most edges of a minibatch graph) are dropped with a ballot; the row of
-// the NEXT surviving edge is already in flight while the current one is accumulated (fp64 accumulators).
-// Four rows per CTA: many more rows in flight per SM than the block-per-row kernel, whose CTAs spent their life waiting on
-// five dependent loads.
-template <int NV>
-__global__ void __launch_bounds__(128)
-row_gather_warp_kernel(const float* __restrict__ X, int row_begin, int row_end, int d, int eps_auto, const int* __restrict__ row_ptr,
-                       const int* __restrict__ col, const int* __restrict__ kappa, const float* __restrict__ gv,
-                       const float* __restrict__ bvec, float* __restrict__ dX) {
+  using V = typename Chunk<W>::T;
   const int lane = threadIdx.x & 31;
   // rows are taken from the END: an unlabeled row (they come last, GLL.py:11) gathers ~30 neighbour rows one after the other,
   // a labeled row one or two -- started last, the long chains were the kernel's tail (35 us at C2 for 60 MB of gathers)
   const int i = row_end - 1 - (blockIdx.x * 4 + (threadIdx.x >> 5));
   if (i < row_begin) return;
-  const int cols = d >> 2;
+  const int cols = W == 4 ? d >> 2 : d;
   const int e0 = __ldg(row_ptr + i), e1 = __ldg(row_ptr + i + 1);
   const int ki = eps_auto ? __ldg(kappa + i) : -1;
   const float bi = eps_auto ? __ldg(bvec + i) : 0.f;
-  const float4* xrow = reinterpret_cast<const float4*>(X + (size_t)i * d);
+  const V* xrow = reinterpret_cast<const V*>(X + (size_t)i * d);
   for (int cbase = 0; cbase < cols; cbase += 32 * NV) {
-    float4 xi[NV];
-    double acc[NV][4];
+    V xi[NV];
+    double acc[NV][W];
 #pragma unroll
     for (int u = 0; u < NV; ++u) {
       const int c = cbase + lane + 32 * u;
-      xi[u] = (c < cols) ? __ldg(xrow + c) : make_float4(0.f, 0.f, 0.f, 0.f);
-      acc[u][0] = acc[u][1] = acc[u][2] = acc[u][3] = 0.0;
+      xi[u] = (c < cols) ? __ldg(xrow + c) : V{};
+#pragma unroll
+      for (int q = 0; q < W; ++q) acc[u][q] = 0.0;
     }
-    auto fetch = [&](int j, float4 (&v)[NV]) {
-      const float4* xj = reinterpret_cast<const float4*>(X + (size_t)j * d);
+    auto fetch = [&](int j, V (&v)[NV]) {
+      const V* xj = reinterpret_cast<const V*>(X + (size_t)j * d);
 #pragma unroll
       for (int u = 0; u < NV; ++u) {
         const int c = cbase + lane + 32 * u;
-        v[u] = (c < cols) ? __ldg(xj + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[u] = (c < cols) ? __ldg(xj + c) : V{};
       }
     };
-    auto accumulate = [&](float tc, const float4 (&v)[NV]) {
+    auto accumulate = [&](float tc, const V (&v)[NV]) {
       const double t = (double)tc;
 #pragma unroll
-      for (int u = 0; u < NV; ++u) {  // the difference is exact enough in fp32 (one rounding); products and sums in fp64
-        acc[u][0] = fma(t, (double)(xi[u].x - v[u].x), acc[u][0]);
-        acc[u][1] = fma(t, (double)(xi[u].y - v[u].y), acc[u][1]);
-        acc[u][2] = fma(t, (double)(xi[u].z - v[u].z), acc[u][2]);
-        acc[u][3] = fma(t, (double)(xi[u].w - v[u].w), acc[u][3]);
-      }
+      for (int u = 0; u < NV; ++u) accumulate_chunk(acc[u], t, xi[u], v[u]);
     };
     for (int eb = e0; eb < e1; eb += 32) {
       const int e = eb + lane;
@@ -198,7 +134,7 @@ row_gather_warp_kernel(const float* __restrict__ X, int row_begin, int row_end, 
       }
       unsigned live = __ballot_sync(FULL, tc != 0.f);
       if (live == 0) continue;
-      float4 va[NV], vb[NV];
+      V va[NV], vb[NV];
       int t = __ffs(live) - 1;
       live &= live - 1;
       fetch(__shfl_sync(FULL, j, t), va);
@@ -223,11 +159,11 @@ row_gather_warp_kernel(const float* __restrict__ X, int row_begin, int row_end, 
         accumulate(tcb, vb);
       }
     }
-    float4* out = reinterpret_cast<float4*>(dX + (size_t)i * d);
+    V* out = reinterpret_cast<V*>(dX + (size_t)i * d);
 #pragma unroll
     for (int u = 0; u < NV; ++u) {
       const int c = cbase + lane + 32 * u;
-      if (c < cols) out[c] = make_float4((float)acc[u][0], (float)acc[u][1], (float)acc[u][2], (float)acc[u][3]);
+      if (c < cols) out[c] = round_chunk(acc[u]);
     }
   }
 }
@@ -251,18 +187,16 @@ int backward_edges_run(const float* X, int n, int d, int l, int k_lab, int eps_a
   if (phases & 2) {  // K6: needs b of ALL rows (neighbours j with kappa(j) = i)
     const bool vec4 = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && ((reinterpret_cast<uintptr_t>(dX) & 15) == 0);
     const int cols = vec4 ? d / 4 : d;
-    int threads = min(256, max(32, ceil_div(cols, 32) * 32));
+    // NV: as few column passes as the registers allow, with few idle lanes (W = 1, NV = 16: 132 registers, no spills).
+    // Measured at C2 on a B200 at 1000 W (tools/row_gather_bench.py): d = 130 takes 20.6 us at NV = 8, 28.7 at 16; d = 2051
+    // takes 174 us at NV = 16, 218 at 8.
+    auto* kernel = vec4 ? (cols <= 32 ? row_gather_kernel<4, 1> : cols <= 64 ? row_gather_kernel<4, 2> : row_gather_kernel<4, 4>)
+                        : (cols <= 32    ? row_gather_kernel<1, 1>
+                           : cols <= 128 ? row_gather_kernel<1, 4>
+                           : cols <= 256 ? row_gather_kernel<1, 8>
+                                         : row_gather_kernel<1, 16>);
     GLL_PROF(KID_ROW_GATHER, st);
-    if (vec4) {
-      const int grid = ceil_div(rows, 4);
-      if (cols <= 32)
-        row_gather_warp_kernel<1><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
-      else if (cols <= 64)
-        row_gather_warp_kernel<2><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
-      else
-        row_gather_warp_kernel<4><<<grid, 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
-    } else
-      row_gather_kernel<1><<<rows, threads, 0, st>>>(X, row_begin, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
+    kernel<<<ceil_div(rows, 4), 128, 0, st>>>(X, row_begin, row_end, d, eps_auto, B.row_ptr, B.col, B.kappa, B.gv, B.bvec, dX);
   }
   GLL_LAUNCH_CHECK();
   return GLL_OK;

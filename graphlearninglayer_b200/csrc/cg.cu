@@ -254,7 +254,7 @@ size_t cg_smem_bytes(int lp) {
 int cg_streaming_launch(CgParams P, cudaStream_t st) {
   const int m = P.m, l = P.l, lp = P.lp;
   if (P.rhs_src != nullptr) {
-    const int rc = pack_grad(P.rhs_src, P.rhs_kind == 2, m, l, lp, const_cast<float*>(P.rhs), st, nullptr, 0, P.rhs_scale, P.rhs_scale_f64);
+    const int rc = pack_grad(P.rhs_src, P.rhs_kind == 2, m, l, lp, const_cast<float*>(P.rhs), st, P.rhs_scale, P.rhs_scale_f64);
     if (rc) return rc;
     P.rhs_src = nullptr;
   }
@@ -327,7 +327,7 @@ int cg_run(const CgSolve& S, void* ws, size_t ws_bytes, cudaStream_t st) {
   Carver cv(ws, ws_bytes);
   if (lp > CG_MAX_LP) {
     if (S.rhs_src != nullptr) {
-      const int rc = pack_grad(S.rhs_src, S.rhs_kind == 2, m, l, lp, const_cast<float*>(S.rhs), st, nullptr, 0, S.rhs_scale, S.rhs_scale_f64);
+      const int rc = pack_grad(S.rhs_src, S.rhs_kind == 2, m, l, lp, const_cast<float*>(S.rhs), st, S.rhs_scale, S.rhs_scale_f64);
       if (rc) return rc;
     }
     const int chunks = ceil_div(l, CG_MAX_LP);

@@ -241,8 +241,8 @@ int unpack_columns(const float* src, int rows, int lp_src, int c0, int cnt, floa
 
 
 // small utility kernels (api.cu)
-int pack_grad(const void* g, int is_f64, int m, int l, int lp, float* rhs, cudaStream_t st, float* zero_ptr = nullptr,
-              long long zero_count = 0, const void* scale = nullptr, int scale_f64 = 0);
+int pack_grad(const void* g, int is_f64, int m, int l, int lp, float* rhs, cudaStream_t st, const void* scale = nullptr,
+              int scale_f64 = 0);
 int unpack_pred(const float* ut_u, int m, int l, int lp, void* pred, int is_f64, cudaStream_t st);
 
 inline int padded_classes(int l) { return (l + 3) / 4 * 4; }

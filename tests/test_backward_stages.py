@@ -1,6 +1,6 @@
-"""Stage tests of the backward edge pass -- K5 `edge_grad_kernel` and every K6 `row_gather_*` variant (csrc/backward.cu) --
-and of the row normalisation pair (`gll_normalize_rows` / `_backward`, csrc/api.cu), each against a plain fp64
-restatement of the same operation on the same fp32 inputs.
+"""Stage tests of the backward edge pass -- K5 `edge_grad_kernel` and every K6 `row_gather_kernel` instantiation
+(csrc/backward.cu) -- and of the row normalisation pair (`gll_normalize_rows` / `_backward`, csrc/api.cu), each against a
+plain fp64 restatement of the same operation on the same fp32 inputs.
 
 The per-edge reference (GLL.py:104-159, as in test_gpu_parity._stagewise_fp64_check), over a CSR (row_ptr, col, dist, w):
     wt[:k_lab] := 0
@@ -171,15 +171,24 @@ class Stage:
         return self.kappa is not None
 
 
-def run_edges(gll, S, phases=3, rows=None, out=None):
+def run_edges(gll, S, phases=3, rows=None, out=None, shift=0):
     """gll_backward_edges (rows None) or gll_backward_edges_rows on S's inputs.  out: host (gv, bvec, dX) the device buffers
-    start from (default NaN).  Returns host copies of (gv, bvec, dX)."""
+    start from (default NaN).  shift: X and dX start that many floats past a 16-byte boundary.  Returns host copies of
+    (gv, bvec, dX)."""
     torch, _, _lib, dev_t = gll
     f32, i32 = torch.float32, torch.int32
+
+    def dev_shifted(a, k):
+        buf = torch.empty(a.size + k, dtype=f32, device="cuda")
+        assert buf.data_ptr() % 16 == 0
+        buf[k:] = dev_t(a, f32).ravel()
+        return buf[k:].view(a.shape)
+
     if out is None:
         out = (np.full(S.E, np.nan, np.float32), np.full(S.n, np.nan, np.float32), np.full((S.n, S.d), np.nan, np.float32))
-    gv, bvec, dX = (dev_t(a, f32) for a in out)
-    X, rp, col = dev_t(S.X, f32), dev_t(S.row_ptr, i32), dev_t(S.col, i32)
+    gv, bvec = (dev_t(a, f32) for a in out[:2])
+    X, dX = dev_shifted(S.X, shift), dev_shifted(out[2], shift)
+    rp, col = dev_t(S.row_ptr, i32), dev_t(S.col, i32)
     dist, w, eps, ut, wt = (dev_t(a, f32) for a in (S.dist, S.w, S.eps, S.ut, S.wt))
     kappa = dev_t(S.kappa, i32) if S.auto else None
     args = (X.data_ptr(), S.n, S.d, S.l, S.k_lab, int(S.auto), rp.data_ptr(), col.data_ptr(), dist.data_ptr(), w.data_ptr(),
@@ -248,17 +257,30 @@ def test_edge_grad_vs_reference(gll, k_lab, m, l, eps):
 # ----------------------------------------------------------------------------------------------------------------
 # 2. K6 on every variant
 # ----------------------------------------------------------------------------------------------------------------
-# d % 4 != 0 -> row_gather_kernel<1> (d <= 32: 32 threads; 2051: 256 threads and three column passes); otherwise
-# row_gather_warp_kernel<NV>: 128 -> NV 1, 132 / 256 -> NV 2, 260 / 512 -> NV 4 one pass, 516 -> two passes, 2048 -> four
+# row_gather_kernel<W, NV>, column passes of 32 NV chunks of W floats.  d % 4 != 0 -> W = 1: 1 / 3 / 19 -> NV 1, 99 -> NV 4,
+# 130 -> NV 8, 515 -> NV 16 two passes, 2051 -> five.  Otherwise W = 4: 128 -> NV 1, 132 / 256 -> NV 2, 260 / 512 -> NV 4
+# one pass, 516 -> two passes, 2048 -> four.
 @pytest.mark.gpu
 @pytest.mark.parametrize("eps", ["auto", 1.0])
-@pytest.mark.parametrize("d", [1, 3, 19, 128, 132, 256, 260, 512, 516, 2048, 2051])
+@pytest.mark.parametrize("d", [1, 3, 19, 99, 128, 130, 132, 256, 260, 512, 515, 516, 2048, 2051])
 def test_row_gather_every_variant(gll, d, eps):
     X = gaussian_points(100 + d, 320, d)
     S = Stage.from_graph(X, 64, 5, eps, seed=d)
     gv, bvec, dX = run_edges(gll, S)
     check_k5(S, gv, bvec, f"K5 d={d} eps={eps}")
     check_k6(S, gv, bvec, dX, f"K6 d={d} eps={eps}")
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("eps", ["auto", 1.0])
+def test_row_gather_misaligned_rows(gll, eps):
+    """d % 4 == 0 with X and dX one float past a 16-byte boundary: float chunks (W = 1), not float4 loads."""
+    d = 512
+    X = gaussian_points(100 + d, 320, d)
+    S = Stage.from_graph(X, 64, 5, eps, seed=d)
+    gv, bvec, dX = run_edges(gll, S, shift=1)
+    check_k5(S, gv, bvec, f"K5 d={d} misaligned eps={eps}")
+    check_k6(S, gv, bvec, dX, f"K6 d={d} misaligned eps={eps}")
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -269,8 +291,8 @@ def test_row_gather_every_variant(gll, d, eps):
 @pytest.mark.parametrize("hub", ["labeled", "unlabeled"])
 @pytest.mark.parametrize("d", [2048, 2051])
 def test_row_gather_planted_hub(gll, d, hub, eps):
-    """Unit-sphere points and the origin, every row's nearest neighbour: the origin's row has n - 1 edges (five 128-edge
-    chunks of the scalar kernel, twenty 32-edge ballots of the warp kernel)."""
+    """Unit-sphere points and the origin, every row's nearest neighbour: the origin's row has n - 1 edges (twenty 32-edge
+    ballots of row_gather_kernel, each column pass)."""
     n, k_lab = 641, 100
     X = gaussian_points(7 + d, n, d)
     X /= np.linalg.norm(X, axis=1, keepdims=True)

@@ -43,7 +43,7 @@ def launches(path, out):
 
 NAME_MAP = {"knn_gram_topk_tc_kernel": "knn_gram_topk_tcgen05", "knn_rerank_kernel": "knn_rerank", "cg_resident_kernel": "cg_persistent",
             "cg_persistent_kernel": "cg_persistent", "cg_small_kernel": "cg_persistent", "row_gather_kernel": "row_gather",
-            "row_gather_warp_kernel": "row_gather", "edge_grad_kernel": "edge_grad", "graph_weights_kernel": "graph_build"}
+            "edge_grad_kernel": "edge_grad", "graph_weights_kernel": "graph_build"}
 TRAFFIC = {}
 
 
