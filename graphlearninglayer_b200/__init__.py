@@ -4,6 +4,7 @@
     from graphlearninglayer_b200 import laplace_learning        # utils.laplace on GPU features, no host round trip
     from graphlearninglayer_b200 import laplace_learning_batched  # the same over B independent graphs (B, n, d)
     from graphlearninglayer_b200 import laplace_learning_trials  # T labeled sets on one graph (n, d)
+    from graphlearninglayer_b200 import poisson_learning         # Poisson learning of T labeled sets on one graph (n, d)
     from graphlearninglayer_b200 import LaplaceLearningSparseHardBatched  # B independent graphs (B, n, d) in one call
 
 The names resolve lazily so that ``python -m graphlearninglayer_b200.build`` can run before the shared library
@@ -12,10 +13,10 @@ CPU or PyTorch fallback.
 """
 __all__ = ["LaplaceLearningSparseHard", "LaplaceLearningSparseHardNormalized", "LaplaceLearningSparseHardBatched", "knn_sym_dist", "stable_conjgrad", "last_info", "GLL",
            "GraphedStep", "BaseSetEvaluator", "laplace_learning", "LaplaceResult",
-           "laplace_learning_batched", "laplace_learning_trials"]
+           "laplace_learning_batched", "laplace_learning_trials", "poisson_learning"]
 _ELSEWHERE = {"GraphedStep": ".graphed", "BaseSetEvaluator": ".evalcache", "laplace_learning": ".laplace_eval",
               "LaplaceResult": ".laplace_eval", "laplace_learning_batched": ".laplace_eval",
-              "laplace_learning_trials": ".laplace_eval"}
+              "laplace_learning_trials": ".laplace_eval", "poisson_learning": ".laplace_eval"}
 
 
 def __getattr__(name):

@@ -126,6 +126,9 @@ def _load():
     sig("gll_laplace_eval_trials_workspace_bytes", sz, [i32, i32, i32, i32, i32, i32])
     sig("gll_laplace_eval_trials", i32, [vp, i32, i32, i32, vp, i32, vp, i32, i32, i32, i32, f32, f32, C.c_double, i32, vp, vp, vp,
                                          vp, vp, vp, vp, sz, vp])
+    sig("gll_poisson_eval_workspace_bytes", sz, [i32, i32, i32, i32, i32, i32])
+    sig("gll_poisson_eval", i32, [vp, i32, i32, i32, vp, i32, vp, i32, i32, i32, i32, f32, C.c_double, i32, vp, vp, vp, vp, vp, vp,
+                                  vp, sz, vp])
     return lib
 
 
@@ -145,7 +148,8 @@ EXPORTS = ["gll_last_error", "gll_version", "gll_device_sm_count", "gll_kernel_c
            "gll_base_cache_build", "gll_knn_cached_workspace_bytes", "gll_knn_cached", "gll_laplace_eval_workspace_bytes",
            "gll_laplace_eval", "gll_knn_segments_workspace_bytes", "gll_knn_segments", "gll_knn_segments_units",
            "gll_batched_workspace_bytes", "gll_forward_batched", "gll_laplace_eval_batched_workspace_bytes", "gll_laplace_eval_batched",
-           "gll_laplace_eval_trials_workspace_bytes", "gll_laplace_eval_trials"]
+           "gll_laplace_eval_trials_workspace_bytes", "gll_laplace_eval_trials", "gll_poisson_eval_workspace_bytes",
+           "gll_poisson_eval"]
 
 
 def check(rc: int, what: str) -> None:

@@ -72,7 +72,7 @@ std::atomic<long long> g_launches[KID_COUNT];
 const char* const g_kernel_names[KID_COUNT] = {
     "sqnorm", "knn_gram_topk_simt", "knn_gram_topk_tcgen05", "knn_rerank", "knn_fallback", "graph_build", "edge_weights",
     "cg_persistent", "pack_unpack", "edge_grad", "row_gather", "convert", "cg_rows", "laplace_refine", "laplace_finish",
-    "knn_segment_setup", "batch_reorder", "laplace_trials_setup"};
+    "knn_segment_setup", "batch_reorder", "laplace_trials_setup", "poisson_mean", "poisson_center"};
 }  // namespace
 
 ProfScope::ProfScope(int id_, cudaStream_t st_) : id(id_), st(st_), slot(nullptr) {

@@ -98,6 +98,8 @@ enum KernelId {
   KID_KNN_SEGMENTS,   // segmented search: upload of seg_ptr and the unit table, per-row column windows
   KID_BATCH_REORDER,  // batched layer: kNN lists to the labeled-first order of the block-diagonal graph
   KID_LAPLACE_TRIALS_SETUP,  // laplace_learning_trials: the slot table of the labeled rows, index checks
+  KID_POISSON_MEAN,          // poisson_learning: each trial's mean label row, the centre of its source term
+  KID_POISSON_CENTER,        // poisson_learning: degree-weighted column means of the solution, subtracted by laplace_finish
   KID_COUNT
 };
 // RAII: counts the launch; when profiling is on, brackets it with two events on the launch stream.

@@ -7,10 +7,13 @@
 //                                laplace_finish
 //   gll_laplace_eval_trials:     the same on one graph built with k_lab = 0, T labeled sets masked into one full-graph system;
 //                                the first right-hand side is laplace_refine's x = 0 pass
+//   gll_poisson_eval:            the trials' graph, slot table and rounds with nothing clamped: L u = b on all n rows, b the
+//                                centred source of the labeled rows; poisson_center before laplace_finish
 //
-// Both solves are R row groups x T column groups of l class columns: B graphs are R = B, T = 1 (UnionRows), the trials R = 1 and
-// T trials (TrialRows).  laplace_refine and laplace_finish are written once over those two policies, which say only where a row
-// and its columns live, whether a row is clamped in a column group, and what a neighbour's value is.
+// The solves are R row groups x T column groups of l class columns: B graphs are R = B, T = 1 (UnionRows), the trials R = 1 and
+// T trials (TrialRows), Poisson learning the same with no clamped row (PoissonRows).  laplace_refine and laplace_finish are
+// written once over those policies, which say only where a row and its columns live, whether a row is clamped in a column group,
+// what a neighbour's value is, and whether the system has a source term (and then a centred solution).
 //
 // laplace_refine (round r) reads x_{r-1} (fp64) and the previous fp32 correction e_{r-1}, and writes x_r = x_{r-1} + e_{r-1}
 // to the OTHER fp64 buffer (neighbour rows are read while rows are written, so the rounds ping-pong between two buffers).  In
@@ -61,6 +64,8 @@ struct LaplaceParams {
   unsigned long long* correct;  // [R T] or NULL
   int R, rows, T, l, lp, k_lab, gx, cw, fb, gs, round;
   double tau, tol;
+  const double* ybar;  // Poisson: [T l] each trial's mean label row
+  double* cmean;       // Poisson: [T l] the degree-weighted mean of each column, subtracted by laplace_finish
 };
 
 __device__ __forceinline__ bool group_valid(const LaplaceParams& P, int t) { return P.bad == nullptr || __ldg(P.bad + t) == 0; }
@@ -69,6 +74,7 @@ __device__ __forceinline__ bool group_valid(const LaplaceParams& P, int t) { ret
 // puts its k_lab = B k_lab labeled rows first, so row i is CSR row k_lab + i and a neighbour j < k_lab is label row j.  x and r
 // are [m][l], e [m][lp] and never NULL; no row is clamped.  The policy is built for one column c of the l.
 struct UnionRows {
+  static constexpr bool poisson = false;
   const LaplaceParams& P;
   const int t = 0, c;
   __device__ UnionRows(const LaplaceParams& P, int c) : P(P), c(c) {}
@@ -85,6 +91,7 @@ struct UnionRows {
 // t lpad + cl of the C = T lpad columns of x, e and r.  Row i is clamped in trial t when slot[i T + t] >= 0, and a clamped
 // neighbour reads its label row Y[t, slot].  x_prev and e may be NULL (x = 0).
 struct TrialRows {
+  static constexpr bool poisson = false;
   const LaplaceParams& P;
   const int t, cl;
   const size_t C, sc;
@@ -101,6 +108,19 @@ struct TrialRows {
   __device__ double u(int j) const {
     const int s = slot(j);
     return s >= 0 ? (double)__ldg(yrow(s)) : x(j);
+  }
+};
+
+// Poisson learning: the trials' layout and slot table, but no row is clamped (a neighbour's value is always the iterate) and the
+// system L u = b has a source term, b_i = Y[t, s] - ybar[t] on the row labeled by slot s of trial t, else 0, formed on the fly.
+// slot() still says which rows are labeled: laplace_finish does not count them.
+struct PoissonRows : TrialRows {
+  static constexpr bool poisson = true;
+  __device__ PoissonRows(const LaplaceParams& P, int c) : TrialRows(P, c) {}
+  __device__ double u(int j) const { return x(j); }
+  __device__ double source(int i) const {
+    const int s = slot(i);
+    return s >= 0 ? (double)__ldg(yrow(s)) - __ldg(P.ybar + (size_t)t * P.l + cl) : 0.0;
   }
 };
 
@@ -125,7 +145,7 @@ __global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(LaplaceParam
       const size_t o = rows.xo(i);
       const double xi = rows.x(i);
       if (P.x_out) P.x_out[o] = xi;
-      if (!valid || rows.slot(i) >= 0) {
+      if (!valid || (!Rows::poisson && rows.slot(i) >= 0)) {
         P.r_out[o] = 0.0;
         continue;
       }
@@ -137,7 +157,8 @@ __global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(LaplaceParam
         s = fma(wv, rows.u(j) - xi, s);
         deg += wv;
       }
-      const double r = s - P.tau * xi;
+      double r = s - P.tau * xi;
+      if constexpr (Rows::poisson) r += rows.source(i);
       P.r_out[o] = r;
       acc = fma(r, r / (deg + P.tau + 1e-10), acc);
     }
@@ -216,7 +237,7 @@ __global__ void __launch_bounds__(LR_THREADS) laplace_refine_kernel(LaplaceParam
 }
 
 // Thread per (row, group): group q = (row group g, column group t) = (q / T, q % T) owns the fb CTAs [q fb, (q + 1) fb).  pred =
-// x + e, or the label row where the row is clamped, or NaN for an invalid group; labels = first maximal column (-1 for an invalid
+// x + e (Poisson: minus the column's cmean), or the label row where the row is clamped, or NaN for an invalid group; labels = first maximal column (-1 for an invalid
 // group); hits of the unclamped rows counted with one integer atomic per CTA into correct[q] (-1 for an invalid group).  CTA 0
 // also writes the correction-CG iteration counts and the convergence status.
 template <class Rows>
@@ -238,7 +259,8 @@ __global__ void __launch_bounds__(LR_THREADS) laplace_finish_kernel(LaplaceParam
       const size_t xo = rows.xo(i), eo = rows.eo(i);
       double best = 0.0;
       for (int c = 0; c < P.l; ++c) {
-        const double v = (s >= 0) ? (double)__ldg(rows.yrow(s) + c) : P.x_out[xo + c] + (double)__ldg(P.e + eo + c);
+        double v = (!Rows::poisson && s >= 0) ? (double)__ldg(rows.yrow(s) + c) : P.x_out[xo + c] + (double)__ldg(P.e + eo + c);
+        if constexpr (Rows::poisson) v -= __ldg(P.cmean + (size_t)t * P.l + c);
         p[c] = v;
         if (c == 0 || v > best) {
           best = v;
@@ -297,6 +319,69 @@ __global__ void laplace_trials_setup_kernel(const void* __restrict__ idx, int is
   }
 }
 
+// Poisson learning: ybar[t l + c] = the mean of Y[t, :, c], summed in fp64 in slot order
+__global__ void poisson_mean_kernel(const float* __restrict__ Y, int T, int k_lab, int l, double* __restrict__ ybar) {
+  const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= (long long)T * l) return;
+  const long long t = q / l, c = q - t * l;
+  double s = 0.0;
+  for (int j = 0; j < k_lab; ++j) s += (double)__ldg(Y + (t * k_lab + j) * l + c);
+  ybar[q] = s / (double)k_lab;
+}
+
+// Poisson learning, after the last correction: cmean[c] = sum_i D_i u_ic / sum_i D_i over all n rows, u = x_out + e, D the fp64
+// row sums of W (as laplace_refine).  L u = b fixes u only up to a constant per column, and that constant moves the argmax, so
+// laplace_finish subtracts cmean: the result has zero degree-weighted mean, the limit of Jacobi-CG from x = 0 that fp32 rounding
+// drifts away from.  Launch shape, per-CTA partials and the last CTA's sums in CTA order as laplace_refine (no floating-point
+// atomics); partial holds the [gx][T l] sums of D u, then those of D.
+__global__ void __launch_bounds__(LR_THREADS) poisson_center_kernel(LaplaceParams P) {
+  __shared__ double red[2][LR_THREADS];
+  __shared__ bool last;
+  const int cw = P.cw, rl_count = LR_THREADS / cw, TL = P.T * P.l;
+  const int tid = threadIdx.x, rl = tid / cw, cc = tid - rl * cw;
+  const int c = blockIdx.y * cw + cc;
+  double du = 0.0, dd = 0.0;
+  if (rl < rl_count && c < TL) {
+    const PoissonRows rows(P, c);
+    for (int i = blockIdx.x * rl_count + rl; i < P.rows; i += P.gx * rl_count) {
+      const int e1 = __ldg(P.row_ptr + i + 1);
+      double deg = 0.0;
+      for (int e = __ldg(P.row_ptr + i); e < e1; ++e) deg += (double)__ldg(P.w + e);
+      du = fma(deg, P.x_out[rows.xo(i)] + (double)__ldg(P.e + rows.eo(i)), du);
+      dd += deg;
+    }
+  }
+  red[0][tid] = du;
+  red[1][tid] = dd;
+  __syncthreads();
+  if (tid < cw && c < TL) {
+    double a = 0.0, b = 0.0;
+    for (int q = 0; q < rl_count; ++q) {
+      a += red[0][q * cw + tid];
+      b += red[1][q * cw + tid];
+    }
+    P.partial[(size_t)blockIdx.x * TL + c] = a;
+    P.partial[((size_t)P.gx + blockIdx.x) * TL + c] = b;
+  }
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last = atomicAdd(P.ticket, 1u) == P.gx * gridDim.y - 1u;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  const int lane = tid & 31, warp = tid >> 5;
+  for (int c2 = warp; c2 < TL; c2 += LR_THREADS / 32) {
+    double a = 0.0, b = 0.0;
+    for (int q = lane; q < P.gx; q += 32) {
+      a += __ldcg(P.partial + (size_t)q * TL + c2);
+      b += __ldcg(P.partial + ((size_t)P.gx + q) * TL + c2);
+    }
+    a = warp_sum(a);
+    b = warp_sum(b);
+    if (lane == 0) P.cmean[c2] = a / b;
+  }
+}
+
 // Launch shape of laplace_refine over `cols` columns and row groups of `rows` rows: cw columns per CTA, gy column chunks, gx CTAs
 // per row group, at most 4 per SM (spread: about 4 per SM over all chunks, so the last CTA of the trials adds few partials per
 // column).  The shape fixes the order of the column sums, and with it the bits of resid.
@@ -308,9 +393,12 @@ RefineGrid refine_grid(int rows, int cols, bool spread) {
   return {cw, gy, max(1, min(ceil_div(rows, LR_THREADS / cw), spread ? ceil_div(ctas, gy) : ctas))};
 }
 
+// The three evaluations: B graphs, the Laplace trials and Poisson learning (the trials' layout plus its source and centring).
+enum EvalKind { EVAL_GRAPHS, EVAL_TRIALS, EVAL_POISSON };
+
 // The evaluation's own buffers, behind the graph state and in front of the stage workspace.  The trials add the slot table, bad,
 // an fp32 right-hand side, first solution and correction of C = T lpad columns (B graphs use the graph state's) and a second fp64
-// iterate (B graphs ping-pong with the caller's pred).
+// iterate (B graphs ping-pong with the caller's pred).  Poisson learning adds ybar, cmean and a second half of partial.
 struct EvalBufs {
   int* slot;  // [n][T]
   int* bad;   // [T]
@@ -326,11 +414,14 @@ struct EvalBufs {
   double* scale;
   unsigned* ticket;  // [R + 1]
   int* round_iters;  // [GLL_LAPLACE_ROUNDS]
+  double* ybar;      // [T l]
+  double* cmean;     // [T l]
 };
 
 // base == NULL: size query only
-size_t eval_bufs(char* base, int R, int rows, int T, int l, bool trials, EvalBufs* E) {
+size_t eval_bufs(char* base, int R, int rows, int T, int l, EvalKind kind, EvalBufs* E) {
   Carver cv(base, ~(size_t)0);
+  const bool trials = kind != EVAL_GRAPHS;
   const size_t N = (size_t)R * rows, tl = (size_t)T * l, nx = trials ? N * T * padded_classes(l) : N * l;
   EvalBufs b = {};
   if (trials) {
@@ -343,12 +434,16 @@ size_t eval_bufs(char* base, int R, int rows, int T, int l, bool trials, EvalBuf
   }
   b.xa = cv.take<double>(nx);
   b.r = cv.take<double>(nx);
-  b.partial = cv.take<double>((size_t)R * refine_grid(rows, T * l, trials).gx * tl);
+  b.partial = cv.take<double>((kind == EVAL_POISSON ? 2 : 1) * (size_t)R * refine_grid(rows, T * l, trials).gx * tl);
   b.colnorm = cv.take<double>(R * tl);
   b.gmax = trials ? b.colnorm : cv.take<double>(R);
   b.scale = cv.take<double>(1);
   b.ticket = cv.take<unsigned>((size_t)R + 1);
   b.round_iters = cv.take<int>(GLL_LAPLACE_ROUNDS);
+  if (kind == EVAL_POISSON) {
+    b.ybar = cv.take<double>(tl);
+    b.cmean = cv.take<double>(tl);
+  }
   if (E) *E = b;
   return align_up(cv.off, 256);
 }
@@ -360,18 +455,19 @@ size_t eval_ws_bytes(int B, int n, int d, int k, int l, int k_lab) {
   if (gll_state_layout(B * n, k, l, B * k_lab, &L)) return 0;
   const size_t stage = (B == 1) ? gll_workspace_bytes(n, d, k, l, k_lab) : batched_ws_bytes(B, n, d, k, l, k_lab);
   if (stage == 0) return 0;
-  return L.total + eval_bufs(nullptr, B, n - k_lab, 1, l, false, nullptr) + stage;
+  return L.total + eval_bufs(nullptr, B, n - k_lab, 1, l, EVAL_GRAPHS, nullptr) + stage;
 }
 
 // the graph state of the trials' k_lab = 0 stages (a one-column dummy label block, as knn_sym_dist)
 int trials_layout(int n, int k, gll_layout* L) { return gll_state_layout(n, k, 1, 0, L); }
 
-// workspace of T trials: [graph state | the evaluation's buffers | stage workspace (kNN, graph stages, CG over C columns)]
-size_t trials_ws_bytes(int n, int d, int k, int l, int T) {
+// workspace of T trials (kind: EVAL_TRIALS or EVAL_POISSON): [graph state | the evaluation's buffers | stage workspace (kNN,
+// graph stages, CG over C columns)]
+size_t trials_ws_bytes(int n, int d, int k, int l, int T, EvalKind kind) {
   gll_layout L;
   if (trials_layout(n, k, &L)) return 0;
   const size_t stage = std::max(gll_workspace_bytes(n, d, k, 1, 0), cg_ws_bytes(n, T * padded_classes(l)));
-  return L.total + eval_bufs(nullptr, 1, n, T, l, true, nullptr) + stage;
+  return L.total + eval_bufs(nullptr, 1, n, T, l, kind, nullptr) + stage;
 }
 
 // a run's carved workspace; P holds what both kernels read, the rounds fill in the iterates
@@ -385,7 +481,7 @@ struct Run {
 
 // Checks and carves the workspace [graph state | the evaluation's buffers | stage workspace] of a run that needs `need` bytes,
 // zeroes info, the tickets and the hit counts, and fills the kernels' parameters.
-int begin_run(const gll_layout& L, size_t need, bool trials, int R, int rows, int T, int l, int k_lab, const float* Y, float tau,
+int begin_run(const gll_layout& L, size_t need, EvalKind kind, int R, int rows, int T, int l, int k_lab, const float* Y, float tau,
               double tol, double* pred, long long* labels, const long long* targets, long long* correct_out, double* resid_out,
               int* info, void* workspace, size_t workspace_bytes, cudaStream_t st, Run* run) {
   if (workspace_bytes < need) {
@@ -396,7 +492,8 @@ int begin_run(const gll_layout& L, size_t need, bool trials, int R, int rows, in
   Run& u = *run;
   u.G = graph_bufs(L, S);
   u.G.info = info;  // the caller's info block in place of the state's
-  const size_t eb = eval_bufs(S + L.total, R, rows, T, l, trials, &u.E);
+  const bool trials = kind != EVAL_GRAPHS;
+  const size_t eb = eval_bufs(S + L.total, R, rows, T, l, kind, &u.E);
   u.ws = S + L.total + eb;
   u.ws_bytes = workspace_bytes - L.total - eb;
   GLL_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int) * GLL_INFO_WORDS, st));
@@ -436,6 +533,8 @@ int begin_run(const gll_layout& L, size_t need, bool trials, int R, int rows, in
   P.fb = ceil_div(rows, LR_THREADS);
   P.tau = (double)tau;
   P.tol = tol;
+  P.ybar = u.E.ybar;
+  P.cmean = u.E.cmean;
   return GLL_OK;
 }
 
@@ -464,6 +563,11 @@ int refine_rounds(LaplaceParams P, const float* x0, const float* corr, double* f
     rc = correction(P.round_iters + r);
     if (rc) return rc;
   }
+  if constexpr (Rows::poisson) {
+    GLL_PROF(KID_POISSON_CENTER, st);
+    poisson_center_kernel<<<dim3(P.gx, ceil_div(P.T * P.l, P.cw)), LR_THREADS, 0, st>>>(P);
+    GLL_LAUNCH_CHECK();
+  }
   GLL_PROF(KID_LAPLACE_FINISH, st);
   laplace_finish_kernel<Rows><<<P.R * P.T * P.fb, LR_THREADS, 0, st>>>(P);
   GLL_LAUNCH_CHECK();
@@ -478,7 +582,7 @@ int eval_run(const float* X, const float* Y, int B, int n, int d, int k, int l, 
   gll_layout L;
   if (gll_state_layout(N, k, l, K, &L)) return GLL_ERR_ARG;
   Run u;
-  int rc = begin_run(L, eval_ws_bytes(B, n, d, k, l, k_lab), false, B, n - k_lab, 1, l, K, Y, tau, tol, pred, labels, targets,
+  int rc = begin_run(L, eval_ws_bytes(B, n, d, k, l, k_lab), EVAL_GRAPHS, B, n - k_lab, 1, l, K, Y, tau, tol, pred, labels, targets,
                      correct_out, resid_out, info, workspace, workspace_bytes, st, &u);
   if (rc) return rc;
   const GraphBufs& G = u.G;
@@ -517,6 +621,10 @@ int eval_run(const float* X, const float* Y, int B, int n, int d, int k, int l, 
 // rows, and trial t masks its clamped rows out of its own columns (cg_persistent_kernel<true>: A p is zeroed there, so r, p and
 // x stay 0 on those rows).  Every [n][C] array has C = T lpad columns, lpad = padded_classes(l): trial t owns the columns
 // [t lpad, t lpad + l), so a class quad never spans two trials.  slot[i T + t] = s when train_idx[t, s] == i, else -1.
+// gll_poisson_eval (Rows = PoissonRows) is the same with tau = 0 and no mask: every trial solves L u = b on all n rows, b its
+// centred source (poisson_mean, then laplace_refine's x = 0 pass), so cg_run picks its kernel by size; poisson_center runs before
+// laplace_finish.
+template <class Rows>
 int trials_run(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T, int k_lab, int l,
                int eps_auto, float eps_fixed, float tau, double tol, int cg_max_iter, double* pred, long long* labels,
                const long long* targets, long long* correct_out, double* resid_out, int* info, void* workspace, size_t workspace_bytes,
@@ -524,7 +632,8 @@ int trials_run(const float* X, int n, int d, int k, const void* train_idx, int i
   gll_layout L;
   if (trials_layout(n, k, &L)) return GLL_ERR_ARG;
   Run u;
-  int rc = begin_run(L, trials_ws_bytes(n, d, k, l, T), true, 1, n, T, l, k_lab, Y, tau, tol, pred, labels, targets, correct_out,
+  constexpr EvalKind kind = Rows::poisson ? EVAL_POISSON : EVAL_TRIALS;
+  int rc = begin_run(L, trials_ws_bytes(n, d, k, l, T, kind), kind, 1, n, T, l, k_lab, Y, tau, tol, pred, labels, targets, correct_out,
                      resid_out, info, workspace, workspace_bytes, st, &u);
   if (rc) return rc;
   const GraphBufs& G = u.G;
@@ -539,13 +648,18 @@ int trials_run(const float* X, int n, int d, int k, const void* train_idx, int i
                                                                                     info);
     GLL_LAUNCH_CHECK();
   }
+  if constexpr (Rows::poisson) {
+    GLL_PROF(KID_POISSON_MEAN, st);
+    poisson_mean_kernel<<<ceil_div((long long)T * l, 256), 256, 0, st>>>(Y, T, k_lab, l, E.ybar);
+    GLL_LAUNCH_CHECK();
+  }
   rc = knn_run(X, n, d, k, 0, n, G.knn_idx, G.knn_dist, info, u.ws, u.ws_bytes, st);
   if (rc) return rc;
   rc = graph_stages_run(G, nullptr, n, k, 1, 0, eps_auto, eps_fixed, tau, 0, 6, u.ws, u.ws_bytes, st);
   if (rc) return rc;
   LaplaceParams P0 = u.P;  // r = b at x = 0, exactly in fp64: the first solve's right-hand side
   P0.round = -1;
-  rc = launch_refine<TrialRows>(P0, st);
+  rc = launch_refine<Rows>(P0, st);
   if (rc) return rc;
   CgSolve S = cg_system(G, n, C, -(float)GLL_LAPLACE_CG_RTOL0, cg_max_iter);
   S.rhs = E.rhs;
@@ -554,9 +668,11 @@ int trials_run(const float* X, int n, int d, int k, const void* train_idx, int i
   S.resid_out = (float*)(info + GLL_INFO_CG_RESID_FWD);
   S.rhs_src = E.r;
   S.rhs_kind = 2;
-  S.mask_slot = E.slot;
-  S.mask_trials = T;
-  S.mask_cols = u.P.lp;
+  if constexpr (!Rows::poisson) {
+    S.mask_slot = E.slot;
+    S.mask_trials = T;
+    S.mask_cols = u.P.lp;
+  }
   rc = cg_run(S, u.ws, u.ws_bytes, st);
   if (rc) return rc;
   CgSolve R = S;  // the correction of a refinement round
@@ -565,7 +681,7 @@ int trials_run(const float* X, int n, int d, int k, const void* train_idx, int i
   R.resid_out = nullptr;
   R.rhs_scale = E.scale;
   R.rhs_scale_f64 = 1;
-  return refine_rounds<TrialRows>(u.P, E.x0, E.corr, E.xb, E.xa, [&](int* iters) {
+  return refine_rounds<Rows>(u.P, E.x0, E.corr, E.xb, E.xa, [&](int* iters) {
     R.iters_out = iters;
     return cg_run(R, u.ws, u.ws_bytes, st);
   }, st);
@@ -638,7 +754,7 @@ int gll_laplace_eval_batched(const float* X, const float* Y, int B, int n, int d
 }
 
 size_t gll_laplace_eval_trials_workspace_bytes(int n, int d, int k, int l, int T, int k_lab) {
-  return trials_sizes_error(n, d, k, l, T, k_lab) ? 0 : trials_ws_bytes(n, d, k, l, T);
+  return trials_sizes_error(n, d, k, l, T, k_lab) ? 0 : trials_ws_bytes(n, d, k, l, T, EVAL_TRIALS);
 }
 
 int gll_laplace_eval_trials(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T, int k_lab,
@@ -648,8 +764,23 @@ int gll_laplace_eval_trials(const float* X, int n, int d, int k, const void* tra
   GLL_REQUIRE(X && train_idx && Y && pred && labels && info && workspace, "null pointer");
   if (const char* why = trials_sizes_error(n, d, k, l, T, k_lab)) return refuse(why);
   GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
-  return trials_run(X, n, d, k, train_idx, idx_is_i64, Y, T, k_lab, l, eps_auto, eps_fixed, tau, tol, cg_max_iter, pred, labels, targets,
-                    correct_out, resid_out, info, workspace, workspace_bytes, (cudaStream_t)stream);
+  return trials_run<TrialRows>(X, n, d, k, train_idx, idx_is_i64, Y, T, k_lab, l, eps_auto, eps_fixed, tau, tol, cg_max_iter, pred, labels,
+                               targets, correct_out, resid_out, info, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+size_t gll_poisson_eval_workspace_bytes(int n, int d, int k, int l, int T, int k_lab) {
+  return trials_sizes_error(n, d, k, l, T, k_lab) ? 0 : trials_ws_bytes(n, d, k, l, T, EVAL_POISSON);
+}
+
+int gll_poisson_eval(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T, int k_lab, int l,
+                     int eps_auto, float eps_fixed, double tol, int cg_max_iter, double* pred, long long* labels,
+                     const long long* targets, long long* correct_out, double* resid_out, int* info, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  GLL_REQUIRE(X && train_idx && Y && pred && labels && info && workspace, "null pointer");
+  if (const char* why = trials_sizes_error(n, d, k, l, T, k_lab)) return refuse(why);
+  GLL_REQUIRE(tol > 0.0 && cg_max_iter >= 1, "tol must be > 0 and cg_max_iter >= 1");
+  return trials_run<PoissonRows>(X, n, d, k, train_idx, idx_is_i64, Y, T, k_lab, l, eps_auto, eps_fixed, 0.f, tol, cg_max_iter, pred,
+                                 labels, targets, correct_out, resid_out, info, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

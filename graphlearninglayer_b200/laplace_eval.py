@@ -27,6 +27,12 @@ that trial.  The graph is built once; all T l class columns are solved against i
 its own columns, every column with its own step lengths.  A trial with an index outside [0, n) or a repeated index is invalid:
 pred NaN, labels -1, correct -1 and a warning; the other trials are unaffected.  See gll_laplace_eval_trials in
 include/gll_b200.h.
+
+    res = poisson_learning(features, train_idx, label_matrix, k=50, epsilon='auto', tol=1e-10, targets=None)
+
+Poisson learning (Calder et al., ICML 2020; graphlearning's ssl.poisson without class priors) of the same T labeled sets on the
+same graph: L u = b on all n rows, b = each labeled row's label minus the trial's mean label row, u with zero degree-weighted mean
+per column; pred (T, n, l) is u on every row, labeled rows included.  See gll_poisson_eval in include/gll_b200.h.
 """
 from __future__ import annotations
 
@@ -39,7 +45,8 @@ from . import _lib
 from .GLL import _bytes, _cg_maxit, _check_status, _require_cuda, _stream_ptr, as_features, decode_info, parse_epsilon
 from ._lib import lib
 
-__all__ = ["laplace_learning", "laplace_learning_batched", "laplace_learning_trials", "LaplaceResult", "last_eval_info"]
+__all__ = ["laplace_learning", "laplace_learning_batched", "laplace_learning_trials", "poisson_learning", "LaplaceResult",
+           "last_eval_info"]
 
 
 class LaplaceResult(NamedTuple):
@@ -49,7 +56,7 @@ class LaplaceResult(NamedTuple):
 
 
 _last_info: Optional[torch.Tensor] = None
-_last_resid: Optional[tuple] = None  # (key, per-group residuals) of the last call when it was batched or a trials call
+_last_resid: Optional[tuple] = None  # (key, per-group residuals) of the last call when it was batched, trials or Poisson
 
 
 def _check_args(n, d, k_lab, l, k, epsilon, tol, total_rows, rows_name):
@@ -69,7 +76,7 @@ def _check_args(n, d, k_lab, l, k, epsilon, tol, total_rows, rows_name):
 def _run(name, features, label_matrix, targets, lead, ws_sizes, pred_shape, groups, eps, tau, tol, resid_key=None):
     """Converts the inputs, allocates the outputs and the workspace, runs gll_<name> on the current stream and records its info
     for last_eval_info().  lead(X, Y) gives the arguments in front of eps_auto, with X and Y the converted features and labels;
-    groups is the shape of correct and of the residuals reported under resid_key."""
+    groups is the shape of correct and of the residuals reported under resid_key.  tau None: the entry point takes no tau."""
     _require_cuda(features, "features")
     dev = features.device
     Xc = as_features(features)
@@ -84,7 +91,8 @@ def _run(name, features, label_matrix, targets, lead, ws_sizes, pred_shape, grou
         resid = None if resid_key is None else torch.empty(groups, dtype=torch.float64, device=dev)
         info = torch.empty(_lib.INFO_WORDS, dtype=torch.int32, device=dev)
         outs = [None if t is None else t.data_ptr() for t in (pred, labels, tg, correct)] + ([] if resid is None else [resid.data_ptr()])
-        rc = getattr(lib, f"gll_{name}")(*lead(Xc.data_ptr(), Y.data_ptr()), *eps, float(tau), float(tol), _cg_maxit(), *outs,
+        taus = () if tau is None else (float(tau),)
+        rc = getattr(lib, f"gll_{name}")(*lead(Xc.data_ptr(), Y.data_ptr()), *eps, *taus, float(tol), _cg_maxit(), *outs,
                                          info.data_ptr(), ws.data_ptr(), ws_bytes, _stream_ptr(dev))
     _lib.check(rc, f"gll_{name}")
     global _last_info, _last_resid
@@ -145,6 +153,26 @@ def laplace_learning_trials(features: torch.Tensor, train_idx: torch.Tensor, lab
     row gets its label row and that row's argmax.  Trial t equals laplace_learning on features[perm_t], perm_t = [train_idx[t],
     the other rows in natural order], on its unlabeled rows; the graph is built once in natural order, so on exact distance ties
     the kNN tie-break follows natural order rather than perm_t."""
+    return _run_trials("laplace_eval_trials", features, train_idx, label_matrix, k, epsilon, tau, tol, targets)
+
+
+def poisson_learning(features: torch.Tensor, train_idx: torch.Tensor, label_matrix: torch.Tensor, k: int = 50, epsilon="auto",
+                     tol: float = 1e-10, targets: Optional[torch.Tensor] = None) -> LaplaceResult:
+    """Poisson learning of T labeled sets on one graph, with laplace_learning_trials' arguments and no tau.  Trial t solves
+    L u = b on all n rows (L = D - W of laplace_learning_trials' graph, nothing clamped), b = Y[t, s] - mean_s Y[t, s] on the row
+    train_idx[t, s] and 0 elsewhere, to the stop rule ||M (b - L u)||_2 <= tol per class column, and returns the u with
+    sum_i D_i u[i, c] = 0 per column.  Returns pred (T, n, l) float64 = u on every row (labeled rows included, not their label
+    row), labels (T, n) int64 = first maximal column and correct (T,) int64 (None without targets) over the rows not labeled in
+    that trial.  Class priors are not applied: rescale pred and take the argmax to use them.  A trial with an invalid index is
+    invalid as in laplace_learning_trials; a trial whose labels are all equal has a zero source and gives u = 0, labels 0.  On a
+    graph with several connected components the system is solvable only when each component's source sums to zero; otherwise
+    'max iter reached' is warned and the result is unspecified."""
+    return _run_trials("poisson_eval", features, train_idx, label_matrix, k, epsilon, None, tol, targets)
+
+
+def _run_trials(name, features, train_idx, label_matrix, k, epsilon, tau, tol, targets):
+    """The checks and the call of the entry points over T labeled sets on one graph (gll_<name>: laplace_eval_trials, or
+    poisson_eval with tau None)."""
     if features.dim() != 2:
         raise ValueError("features must be (n, d)")
     if train_idx.dim() != 2:
@@ -169,16 +197,17 @@ def laplace_learning_trials(features: torch.Tensor, train_idx: torch.Tensor, lab
         raise ValueError(f"targets must be ({n},), got {tuple(targets.shape)}")
     _require_cuda(features, "features")  # before train_idx is copied anywhere
     idx = train_idx.detach().to(device=features.device).contiguous()
-    return _run("laplace_eval_trials", features, label_matrix, targets,
+    return _run(name, features, label_matrix, targets,
                 lambda X, Y: (X, n, d, k, idx.data_ptr(), int(idx.dtype == torch.int64), Y, T, k_lab, l), (n, d, k, l, T, k_lab),
                 (T, n, l), (T,), eps, tau, tol, "resid_per_trial")
 
 
 def last_eval_info() -> dict:
-    """Device status block of the most recent laplace_learning, laplace_learning_batched or laplace_learning_trials call
-    (synchronises).  Keys follow GLL_INFO_* in include/gll_b200.h; after a batched call the residuals are the maximum over graphs,
+    """Device status block of the most recent laplace_learning, laplace_learning_batched, laplace_learning_trials or
+    poisson_learning call (synchronises).  Keys follow GLL_INFO_* in include/gll_b200.h; after a batched call the residuals are the maximum over graphs,
     the iteration counts those of the whole batch, and resid_per_graph lists each graph's largest column norm of the last round.
-    After a trials call the same holds over the valid trials, and resid_per_trial lists each trial's (NaN for an invalid one)."""
+    After a trials or Poisson call the same holds over the valid trials, and resid_per_trial lists each trial's (NaN for an
+    invalid one)."""
     if _last_info is None:
         return {}
     v = _last_info.cpu().numpy()

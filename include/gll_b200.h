@@ -402,6 +402,32 @@ int gll_laplace_eval_trials(const float* X, int n, int d, int k, const void* tra
                             long long* labels, const long long* targets, long long* correct_out, double* resid_out, int* info,
                             void* workspace, size_t workspace_bytes, void* stream);
 
+/* Poisson learning (Calder, Cook, Thorpe, Slepcev, ICML 2020; graphlearning's ssl.poisson without class priors) for T labeled
+ * sets on ONE set of features, with the arguments of gll_laplace_eval_trials and no tau.
+ *   Graph: gll_laplace_eval_trials' graph, built once on X in natural order; D = row sums of the stored fp32 W in fp64, L = D - W.
+ *   Source: ybar_t = (1/k_lab) sum_s Y[t, s]; b_t[i] = Y[t, s] - ybar_t on the row i = train_idx[t, s], else 0 (Y need not be
+ *   one-hot).  Solve L u_t = b_t on ALL n rows: nothing is clamped, labeled rows are unknowns like the others.
+ *   Normalisation: sum_i D_i u_t[i, c] = 0 for every class column c.  L u = b fixes u only up to a constant per column and that
+ *   constant moves the argmax, so it is part of the result; it is enforced after the last round (exact arithmetic Jacobi-CG from 0
+ *   lands there; fp32 rounding drifts along the null space).
+ *   Stop rule: as gll_laplace_eval_trials with tau = 0 and no clamped row: every class column of every valid trial has
+ *   ||M (b - L x)||_2 <= tol over all n rows, M = diag(D + 1e-10)^(-1/2).  The schedule is GLL_LAPLACE_*'s.
+ *   Outputs: pred T x n x l fp64 = u_t on every row (labeled rows included: they do NOT get their label row back); labels T x n
+ *   int64 = first maximal column; targets, correct_out (rows not labeled in trial t with label == target >= 0) and resid_out as
+ *   gll_laplace_eval_trials.
+ *   Invalid trials: exactly gll_laplace_eval_trials' rules (GLL_STATUS_BAD_INDEX; pred NaN, labels -1, correct -1, resid NaN; the
+ *   other trials unaffected).  A trial whose source is zero (e.g. all its labeled rows carry the same label) gives u = 0 and labels
+ *   0; it meets the stop rule at the first round.  A graph with several connected components is solvable only when each
+ *   component's source sums to zero; otherwise the call neither faults nor hangs, GLL_STATUS_CG_NOT_CONVERGED (or _NONFINITE) is
+ *   set and the outputs are unspecified.
+ *   Sizes: gll_laplace_eval_trials' rules.  Bad arguments return GLL_ERR_ARG before any CUDA call; the workspace query returns 0
+ *   for them.  Nothing syncs with the host and nothing is copied, so the call can be captured in a CUDA graph. */
+size_t gll_poisson_eval_workspace_bytes(int n, int d, int k, int l, int T, int k_lab);
+int gll_poisson_eval(const float* X, int n, int d, int k, const void* train_idx, int idx_is_i64, const float* Y, int T, int k_lab,
+                     int l, int eps_auto, float eps_fixed, double tol, int cg_max_iter, double* pred, long long* labels,
+                     const long long* targets, long long* correct_out, double* resid_out, int* info, void* workspace,
+                     size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
